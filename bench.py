@@ -17,6 +17,8 @@ A step = one evaluation of {NLML, dNLML/dtheta} of the loadest-gp model on one s
   --impl reference : the reference's CPU path restated by the oracle (dense covariance build, torch.linalg.cholesky,
             autograd backward -- what discontinuum/engines/gpytorch.py:353,384 executes), float64, every host thread,
             MEASURED at n = 16 384 itself (one timed evaluation) with n = 4096 / 8192 alongside.
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned (DIR/nlml.npy, DIR/grad.npy,
+            float64).  The inputs depend only on the arguments, so two builds can be compared output for output.
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -115,6 +117,15 @@ def fp64_peak_live(local: int):
             "how": f"torch.matmul float64 {n}^3 (cuBLAS DGEMM): best of 8 / mean of {reps} back to back, CUDA events"}
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """One float64 DIR/<name>.npy per array."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def cpu_eval(n: int, mode: str = "autograd"):
     """One oracle NLML+grad evaluation at size n on the host: dense covariance build + torch.linalg.cholesky + backward.
     mode "autograd": autograd straight through the Cholesky factorisation (what the reference's objective.backward()
@@ -202,7 +213,12 @@ def main():
     ap.add_argument("--c5-n", type=int, default=32768)
     ap.add_argument("--c5-m", type=int, default=100000)
     ap.add_argument("--c5-draws", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the NLML and gradient of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path only")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -264,6 +280,8 @@ def main():
     clocks = sampler.stop()
     if any(infos) or not np.isfinite(val):
         raise RuntimeError(f"factorisation failed inside the timed region: info={infos} nlml={val}")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"nlml": np.array([val]), "grad": grad})
 
     # ---- phase split of one evaluation (CUDA events on the launching stream inside libdgp)
     eng.set_timing(True)

@@ -1,5 +1,5 @@
 """Run by tests/test_reference_integration.py in a fresh process, only where the reference's sources are readable
-(/root/reference/src: the build container).  INTEGRATION.md section 1, executed: the reference's OWN data mixin (its DataManager
+(DISCONTINUUM_REFERENCE = its src/ directory).  INTEGRATION.md section 1, executed: the reference's OWN data mixin (its DataManager
 and pipelines) and its OWN plot mixin, composed with `MarginalB200` exactly as a maintainer would,
 
     class LoadestGPMarginalB200(LoadestDataMixin, LoadestPlotMixin, MarginalB200): ...
@@ -17,7 +17,7 @@ from unittest.mock import MagicMock
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get("DISCONTINUUM_REFERENCE", "/root/reference/src")
+REF = os.environ["DISCONTINUUM_REFERENCE"]
 sys.path[:0] = [os.path.join(ROOT, "oracle", "gpytorch_standin"), HERE, ROOT]
 
 

@@ -4,6 +4,8 @@ the oracle's objective, and the array-level data pipelines reproduce the referen
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -33,10 +35,15 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_engine_fails_loudly_without_gpu():
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(capi.DgpError, match="no CUDA device"):
-        capi.Engine(max_n=128)
+    """Run in a fresh process with every device hidden, so that this also holds on a machine that has a GPU."""
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "import pytest\n"
+            "from discontinuum_b200 import capi\n"
+            "with pytest.raises(capi.DgpError, match='no CUDA device'):\n"
+            "    capi.Engine(max_n=128)\n") % ROOT
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                       text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
 
 
 def test_loadest_spec_structure():
