@@ -63,8 +63,6 @@ _SIGNATURES = [
     ("dgp_nlml_grad_launch", C.c_int, [_P, _P, C.c_double]),
     ("dgp_nlml_grad_wait", C.c_int, [_P, _P, _P]),
     ("dgp_nlml_grad_ready", C.c_int, [_P]),
-    ("dgp_partition_device", C.c_int, [C.c_int, C.c_int, _P]),
-    ("dgp_create_partitioned", C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int]),
     ("dgp_factorize", C.c_int, [_P, _P, C.c_double, _P]),
     ("dgp_predict", C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P]),
     ("dgp_mean_functional_grad", C.c_int, [_P, _P, C.c_int, _P, _P, _P]),
@@ -154,18 +152,6 @@ def _ptr(a) -> Tuple[int, int]:
 
 def _f64(a) -> np.ndarray:
     return np.ascontiguousarray(np.asarray(a, dtype=np.float64))
-
-
-def partition_device(device: int, parts: int) -> Tuple[int, int]:
-    """Split the SMs of `device` into `parts` disjoint partitions (CUDA green contexts).  Returns (partitions, SMs per
-    partition); idempotent per process and device (the first split stays)."""
-    lib = load_library()
-    sms = C.c_int(0)
-    rc = lib.dgp_partition_device(int(device), int(parts), C.byref(sms))
-    if rc < 1:
-        msg = lib.dgp_last_error(None)
-        raise DgpError(f"dgp_partition_device failed ({rc}): {msg.decode() if msg else ''}")
-    return rc, sms.value
 
 
 class BatchEngine:
@@ -271,15 +257,10 @@ class BatchEngine:
 class Engine:
     """One libdgp handle: the resident training set of one site and its factorisation workspace."""
 
-    def __init__(self, max_n: int, max_m: int = 2048, device: int = 0, stream: int = 0, partition: Optional[int] = None):
-        """partition: index of an SM partition made by `partition_device` (the engine's kernels then only run on
-        that slice of the GPU: concurrent sites do not queue behind each other's long tiles)."""
+    def __init__(self, max_n: int, max_m: int = 2048, device: int = 0, stream: int = 0):
         self.lib = load_library()
         self._h = _P()
-        if partition is not None:
-            rc = self.lib.dgp_create_partitioned(C.byref(self._h), int(device), int(max_n), int(max_m), int(partition))
-        else:
-            rc = self.lib.dgp_create(C.byref(self._h), int(device), int(max_n), int(max_m), _P(stream) if stream else None)
+        rc = self.lib.dgp_create(C.byref(self._h), int(device), int(max_n), int(max_m), _P(stream) if stream else None)
         if rc != 0:
             msg = self.lib.dgp_last_error(None)
             self._h = _P()

@@ -14,7 +14,7 @@
 //   deterministic reductions -> {nlml, info, grad} -> pinned host buffer.
 // Three padded n x n panels: bufA (work matrix, then T = L^-1 and scratch, then Ky^-1), bufL (L, lower), bufU (U = L^-T,
 // upper).  Covariance tiles come from one of two generators with the same per-entry arithmetic (dgp_cov.cuh): up to
-// DGP_PREGEN_MIN_NB block columns, for the prediction / sampling matrices and with DGP_PREGEN=0 a tile is generated in shared
+// DGP_PREGEN_MIN_NB block columns and for the prediction / sampling matrices a tile is generated in shared
 // memory in the epilogue of its first trailing update (out = K - sum) and K itself is never stored; for larger training
 // matrices a standalone generator writes the lower tiles of K into the work matrix strip by strip on the low-priority stream
 // while the first panel is factored (measured faster: the generator's FP64 arithmetic shares the datapath with DMMA and is
@@ -58,19 +58,13 @@ PFN_encodeTiled get_encode() {
 
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
-// ---- green contexts (driver API, resolved at run time like the tensor-map encoder: libdgp does not link libcuda)
-template <typename F>
-F driver_fn(const char* name) {
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint(name, &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) return nullptr;
-  return (F)p;
-}
-struct SmPartitions {
-  int parts = 0, sms = 0;
-  std::vector<CUgreenCtx> ctx;
-};
-SmPartitions g_partitions[64];
+// the factorisation schedule of both engines (DESIGN.md 4.5): panels of PANEL_BLOCKS block columns; trailing updates in
+// column strips of STRIP_BLOCKS block columns, strip j on stream j mod 2
+constexpr int PANEL_BLOCKS = 4;
+constexpr int STRIP_BLOCKS = 8;
+static_assert(STRIP_BLOCKS % PANEL_BLOCKS == 0, "a strip holds whole panels");
+// the merges of the inverse are launched as the factorisation passes them up to this many block columns (single-site engine)
+constexpr int EAGER_INV_MAX_NB = 96;
 
 }  // namespace
 
@@ -84,27 +78,13 @@ struct dgp_handle_s {
   cudaEvent_t ev_lo[2] = {nullptr, nullptr};
   bool own_stream = false;
   std::vector<cudaEvent_t> evs;      // look-ahead dependencies (no timing)
-  bool lookahead = true;
-  int panel_blocks = 4;              // block columns per panel of the two-level Cholesky
-  bool pdl = true;                   // programmatic dependent launch along the panel chain (DGP_PDL=0: off)
-  bool chain_half = true;            // 64-row half tiles for the panel chain's small launches (DGP_CHAIN_HALF=0: off)
   cudaStream_t stream_t2 = nullptr;  // second trailing-update stream (same priority as `stream`): column strips alternate
-  int eager_inv = 1;                 // merges of the inverse launched as the factorisation passes them (DGP_EAGER_INV=0: after it)
-  int eager_lag = 0;                 // ... released this many block columns late (DGP_EAGER_LAG)
-  int eager_max_h = 0;               // above 96 block columns: highest merge level that goes early (DGP_EAGER_MAXH; 0 = none: measured no gain at n = 16384 for 4 / 8 / 16 / 32)
-  int strip_blocks = 8;              // width of a column strip in block columns (DGP_STRIP_BLOCKS, 0: one stream, no strips)
-  bool inpanel_left = false;         // in-panel updates left-looking (one rank-(128 j) update per column; DGP_INPANEL_LEFT=1)
-  bool pregen = true;                // standalone covariance generator ahead of the factorisation (DGP_PREGEN=0: first-touch generation)
-  struct GraphSlot { cudaGraphExec_t exec = nullptr; double jitter = 0.0; bool seen = false; long long launches = 0; };
-  GraphSlot graphs[3];               // per evaluation level (nlml / nlml+grad / factorize)
-  bool use_graphs = false;  // opt-in (DGP_GRAPHS=1): replay loses the stream priorities of the look-ahead, measured slower
   int max_n = 0, max_pad = 0, max_m = 0;
   int n = 0, npad = 0, nb = 0, sms = 148;
   bool have_train = false, factorized = false, have_T = false, debug_kinv = false, timing = false;
   bool lu_zeroed = false;  // bufL / bufU cleared for the current leading dimension (see k_potf2_v2, zero_lu)
   int zeroed_npad = 0;     // ... which is this one
   dgp_spec spec;       // internal copy: the caller's spec + derived sin/cos feature columns of periodic factors
-  dgp_spec user_spec;  // as passed to dgp_set_train
   // device buffers
   double *bufA = nullptr, *bufL = nullptr, *bufU = nullptr, *DI = nullptr;
   double *X = nullptr, *y = nullptr, *noise = nullptr, *Xw = nullptr, *r = nullptr, *z = nullptr, *alpha = nullptr;
@@ -202,12 +182,6 @@ static cudaError_t launch_ex(void (*kern)(KArgs...), int grid, int block, size_t
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
-// L2-aware tile order of the LAUUM / inverse launches (DGP_RASTER=0: the round-1 row-by-row order)
-static int raster_on() {
-  static const int v = getenv("DGP_RASTER") ? atoi(getenv("DGP_RASTER")) != 0 : 1;
-  return v;
-}
-
 static const BatchTab g_no_batch = {};   // count == 0: single-site launch
 static const P2Batch g_no_p2batch = {};
 
@@ -218,33 +192,12 @@ static int launch_gemm(HT h, const CUtensorMap& a, const CUtensorMap& b, const G
   if (st == nullptr) st = h->stream;
   if (bt == nullptr) bt = &g_no_batch;
   static bool attr_set[64] = {false};  // per device: function attributes belong to the device's context
-  static int smem_bytes = SM_TOTAL;
   const int dev = (h->device >= 0 && h->device < 64) ? h->device : 0;
   if (!attr_set[dev]) {
-    const char* pad = getenv("DGP_SMEM_PAD");  // experiment knob: extra bytes force 1 CTA / SM
-    if (pad) smem_bytes = SM_TOTAL + atoi(pad);
-    CK(h, cudaFuncSetAttribute(k_gemm<INIT, EPI, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    CK(h, cudaFuncSetAttribute(k_gemm<INIT, EPI, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_TOTAL));
     attr_set[dev] = true;
   }
-  if (INIT == INIT_COV) {   // first-touch tiles: alternate "generate first" / "generate last" by wave-sized groups of CTAs
-    static const int gen_first = getenv("DGP_GEN_FIRST") ? atoi(getenv("DGP_GEN_FIRST")) : 0;   // measured: no gain (DESIGN 4.6)
-    if (gen_first > 0 && g.ntiles > h->sms) {
-      GemmArgs g2 = g;
-      g2.gen_first_mod = h->sms * gen_first;
-      CK(h, launch_ex(k_gemm<INIT, EPI, MT>, g.ntiles, GEMM_THREADS, (size_t)smem_bytes, st, pdl, a, b, h->spec, g2, *bt));
-      h->launches++;
-      return 0;
-    }
-  }
-  static const int stagger = getenv("DGP_STAGGER_NS") ? atoi(getenv("DGP_STAGGER_NS")) : 0;
-  if (stagger > 0 && MT == 8 && g.ntiles > 2 * h->sms) {
-    GemmArgs g2 = g;
-    g2.stagger_ns = stagger; g2.stagger_lo = h->sms;
-    CK(h, launch_ex(k_gemm<INIT, EPI, MT>, g.ntiles, GEMM_THREADS, (size_t)smem_bytes, st, pdl, a, b, h->spec, g2, *bt));
-    h->launches++;
-    return 0;
-  }
-  CK(h, launch_ex(k_gemm<INIT, EPI, MT>, g.ntiles * (MT == 8 ? 1 : 2), GEMM_THREADS, (size_t)smem_bytes, st, pdl, a, b, h->spec, g, *bt));
+  CK(h, launch_ex(k_gemm<INIT, EPI, MT>, g.ntiles * (MT == 8 ? 1 : 2), GEMM_THREADS, (size_t)SM_TOTAL, st, pdl, a, b, h->spec, g, *bt));
   h->launches++;
   return 0;
 }
@@ -289,53 +242,20 @@ int dgp_create(dgp_handle* out, int device, int max_n, int max_m, void* stream) 
     cudaDeviceGetStreamPriorityRange(&lo, &hi);
     if (stream) { h->stream = (cudaStream_t)stream; }
     else {
-      const char* p3 = getenv("DGP_PRIO3");
-      if (p3 == nullptr || atoi(p3) != 0) {
-        cudaStreamCreateWithPriority(&h->stream, cudaStreamNonBlocking, (lo + hi) / 2);
-        cudaStreamCreateWithPriority(&h->stream_lo, cudaStreamNonBlocking, lo);
-        cudaEventCreateWithFlags(&h->ev_lo[0], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&h->ev_lo[1], cudaEventDisableTiming);
-      } else {
-        cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
-      }
+      cudaStreamCreateWithPriority(&h->stream, cudaStreamNonBlocking, (lo + hi) / 2);
       h->own_stream = true;
     }
+    // the phases after the factorisation get a lowest-priority stream of the handle's own, also behind a caller's stream
+    cudaStreamCreateWithPriority(&h->stream_lo, cudaStreamNonBlocking, lo);
+    cudaEventCreateWithFlags(&h->ev_lo[0], cudaEventDisableTiming);
+    cudaEventCreateWithFlags(&h->ev_lo[1], cudaEventDisableTiming);
     cudaStreamCreateWithPriority(&h->stream_hi, cudaStreamNonBlocking, hi);
     {  // second trailing-update stream at the priority of `stream` (whoever created that)
       int pr = (lo + hi) / 2;
       if (cudaStreamGetPriority(h->stream, &pr) != cudaSuccess) { cudaGetLastError(); pr = (lo + hi) / 2; }
       cudaStreamCreateWithPriority(&h->stream_t2, cudaStreamNonBlocking, pr);
     }
-    if (h->stream_lo == nullptr && (getenv("DGP_PRIO3") == nullptr || atoi(getenv("DGP_PRIO3")) != 0)) {
-      // caller's stream: the phases after the factorisation still get a lowest-priority stream of the handle's own
-      cudaStreamCreateWithPriority(&h->stream_lo, cudaStreamNonBlocking, lo);
-      cudaEventCreateWithFlags(&h->ev_lo[0], cudaEventDisableTiming);
-      cudaEventCreateWithFlags(&h->ev_lo[1], cudaEventDisableTiming);
-    }
-    const char* ei = getenv("DGP_EAGER_INV");
-    if (ei) h->eager_inv = atoi(ei);
-    const char* em = getenv("DGP_EAGER_MAXH");
-    if (em && atoi(em) >= 0) h->eager_max_h = atoi(em);
-    const char* el = getenv("DGP_EAGER_LAG");
-    if (el && atoi(el) >= 0) h->eager_lag = atoi(el) / 8 * 8;
-    const char* sb = getenv("DGP_STRIP_BLOCKS");
-    if (sb && atoi(sb) >= 0 && atoi(sb) <= 4096) h->strip_blocks = atoi(sb);
-    const char* la = getenv("DGP_LOOKAHEAD");
-    if (la) h->lookahead = atoi(la) != 0;
-    const char* ug = getenv("DGP_GRAPHS");
-    if (ug) h->use_graphs = atoi(ug) != 0;
     h->trace_path = getenv("DGP_TRACE");
-    const char* pd = getenv("DGP_PDL");
-    if (pd) h->pdl = atoi(pd) != 0;
-    if (h->use_graphs) h->pdl = false;
-    const char* ch = getenv("DGP_CHAIN_HALF");
-    if (ch) h->chain_half = atoi(ch) != 0;
-    const char* pb = getenv("DGP_PANEL_BLOCKS");
-    if (pb && atoi(pb) >= 1 && atoi(pb) <= 64) h->panel_blocks = atoi(pb);
-    const char* pg = getenv("DGP_PREGEN");
-    if (pg) h->pregen = atoi(pg) != 0;
-    const char* il = getenv("DGP_INPANEL_LEFT");
-    if (il) h->inpanel_left = atoi(il) != 0;
   }
   const size_t np = h->max_pad, mc = h->max_m, nbm = np / 128;
   auto A = [&](double** p, size_t count) { return cudaMalloc((void**)p, count * sizeof(double)); };
@@ -360,86 +280,8 @@ int dgp_create(dgp_handle* out, int device, int max_n, int max_m, void* stream) 
     dgp_destroy(h);
     return -2;
   }
-  cudaFuncSetAttribute(k_potf2, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM);
   cudaFuncSetAttribute(k_potf2_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM);
   *out = h;
-  return 0;
-}
-
-int dgp_partition_device(int device, int parts, int* sms_out) {
-  if (device < 0 || device >= 64 || parts < 1) DGP_FAIL((dgp_handle) nullptr, -1, "dgp_partition_device: bad arguments");
-  SmPartitions& P = g_partitions[device];
-  if (P.parts > 0) { if (sms_out) *sms_out = P.sms; return P.parts; }  // one split per device and process
-  if (cudaSetDevice(device) != cudaSuccess || cudaFree(0) != cudaSuccess)
-    DGP_FAIL((dgp_handle) nullptr, -2, "dgp_partition_device: no CUDA device %d", device);
-  typedef CUresult (*PFN_devres)(CUdevice, CUdevResource*, CUdevResourceType);
-  typedef CUresult (*PFN_split)(CUdevResource*, unsigned int*, const CUdevResource*, CUdevResource*, unsigned int, unsigned int);
-  typedef CUresult (*PFN_desc)(CUdevResourceDesc*, CUdevResource*, unsigned int);
-  typedef CUresult (*PFN_gcreate)(CUgreenCtx*, CUdevResourceDesc, CUdevice, unsigned int);
-  typedef CUresult (*PFN_devget)(CUdevice*, int);
-  PFN_devres f_res = driver_fn<PFN_devres>("cuDeviceGetDevResource");
-  PFN_split f_split = driver_fn<PFN_split>("cuDevSmResourceSplitByCount");
-  PFN_desc f_desc = driver_fn<PFN_desc>("cuDevResourceGenerateDesc");
-  PFN_gcreate f_create = driver_fn<PFN_gcreate>("cuGreenCtxCreate");
-  PFN_devget f_dev = driver_fn<PFN_devget>("cuDeviceGet");
-  if (!f_res || !f_split || !f_desc || !f_create || !f_dev)
-    DGP_FAIL((dgp_handle) nullptr, -3, "dgp_partition_device: green-context entry points not available in this driver");
-  CUdevice dev;
-  CUresult r = f_dev(&dev, device);
-  CUdevResource all;
-  if (r == CUDA_SUCCESS) r = f_res(dev, &all, CU_DEV_RESOURCE_TYPE_SM);
-  if (r != CUDA_SUCCESS) DGP_FAIL((dgp_handle) nullptr, -3, "cuDeviceGetDevResource failed (%d)", (int)r);
-  const int total = (int)all.sm.smCount;
-  int per = total / parts / 8 * 8;  // partitions are multiples of 8 SMs on sm_90+
-  if (per < 8) DGP_FAIL((dgp_handle) nullptr, -1, "dgp_partition_device: %d partitions of >= 8 SMs do not fit %d SMs", parts, total);
-  std::vector<CUdevResource> groups((size_t)parts);
-  unsigned int nb = (unsigned int)parts;
-  CUdevResource rest;
-  r = f_split(groups.data(), &nb, &all, &rest, 0, (unsigned int)per);
-  if (r != CUDA_SUCCESS || nb < 1) DGP_FAIL((dgp_handle) nullptr, -3, "cuDevSmResourceSplitByCount failed (%d)", (int)r);
-  P.ctx.clear();
-  for (unsigned int i = 0; i < nb; i++) {
-    CUdevResourceDesc desc;
-    CUgreenCtx g;
-    r = f_desc(&desc, &groups[i], 1);
-    if (r == CUDA_SUCCESS) r = f_create(&g, desc, dev, CU_GREEN_CTX_DEFAULT_STREAM);
-    if (r != CUDA_SUCCESS) DGP_FAIL((dgp_handle) nullptr, -3, "cuGreenCtxCreate failed for partition %u (%d)", i, (int)r);
-    P.ctx.push_back(g);
-  }
-  P.parts = (int)P.ctx.size();
-  P.sms = (int)groups[0].sm.smCount;
-  if (sms_out) *sms_out = P.sms;
-  return P.parts;
-}
-
-int dgp_create_partitioned(dgp_handle* out, int device, int max_n, int max_m, int part) {
-  if (device < 0 || device >= 64) DGP_FAIL((dgp_handle) nullptr, -1, "dgp_create_partitioned: bad device");
-  SmPartitions& P = g_partitions[device];
-  if (part < 0 || part >= P.parts) DGP_FAIL((dgp_handle) nullptr, -1, "dgp_create_partitioned: partition %d of %d (call dgp_partition_device first)", part, P.parts);
-  typedef CUresult (*PFN_gstream)(CUstream*, CUgreenCtx, unsigned int, int);
-  PFN_gstream f_stream = driver_fn<PFN_gstream>("cuGreenCtxStreamCreate");
-  if (!f_stream) DGP_FAIL((dgp_handle) nullptr, -3, "cuGreenCtxStreamCreate not available");
-  if (cudaSetDevice(device) != cudaSuccess) DGP_FAIL((dgp_handle) nullptr, -2, "no CUDA device %d", device);
-  int lo = 0, hi = 0;
-  cudaDeviceGetStreamPriorityRange(&lo, &hi);
-  CUstream st = nullptr, st_hi = nullptr;
-  CUresult r = f_stream(&st, P.ctx[(size_t)part], CU_STREAM_NON_BLOCKING, lo);
-  if (r == CUDA_SUCCESS) r = f_stream(&st_hi, P.ctx[(size_t)part], CU_STREAM_NON_BLOCKING, hi);
-  if (r != CUDA_SUCCESS) DGP_FAIL((dgp_handle) nullptr, -3, "cuGreenCtxStreamCreate failed (%d)", (int)r);
-  int rc = dgp_create(out, device, max_n, max_m, (void*)st);
-  if (rc != 0) { cudaStreamDestroy((cudaStream_t)st); cudaStreamDestroy((cudaStream_t)st_hi); return rc; }
-  dgp_handle h = *out;
-  cudaStreamDestroy(h->stream_hi);          // the look-ahead stream must live in the partition as well
-  h->stream_hi = (cudaStream_t)st_hi;
-  cudaStreamDestroy(h->stream_t2);          // one trailing-update stream inside a partition (no column strips)
-  h->stream_t2 = nullptr;
-  if (h->stream_lo) {                       // ... and no helper stream outside it for the inverse / LAUUM phases
-    cudaStreamDestroy(h->stream_lo);
-    h->stream_lo = nullptr;
-    for (int i = 0; i < 2; i++) if (h->ev_lo[i]) { cudaEventDestroy(h->ev_lo[i]); h->ev_lo[i] = nullptr; }
-  }
-  h->own_stream = true;                     // both streams are the handle's to destroy
-  h->sms = P.sms;
   return 0;
 }
 
@@ -452,7 +294,6 @@ int dgp_destroy(dgp_handle h) {
   if (h->stream_t2) { cudaStreamSynchronize(h->stream_t2); cudaStreamDestroy(h->stream_t2); }
   for (int i = 0; i < 2; i++) if (h->ev_lo[i]) cudaEventDestroy(h->ev_lo[i]);
   for (cudaEvent_t e : h->evs) cudaEventDestroy(e);
-  for (auto& gs : h->graphs) if (gs.exec) cudaGraphExecDestroy(gs.exec);
   double* bufs[] = {h->bufA, h->bufL, h->bufU, h->DI, h->X, h->y, h->noise, h->Xw, h->r, h->z, h->alpha, h->theta,
                     h->scal, h->gpart, h->zpart, h->cvec, h->vvec, h->gam, h->tmpz, h->mfg_out, h->wpart, h->Kx, h->Xs, h->Xws, h->means, h->dot, h->vpart, h->mu, h->var};
   for (double* p : bufs) if (p) cudaFree(p);
@@ -509,12 +350,11 @@ static int check_spec(HT h, const dgp_spec* sp) {
 
 // Append sinpi / cospi feature columns for periodic factors while the feature table has room (see dgp_cov.cuh).
 static void augment_spec(dgp_spec* sp) {
-  static const bool off = getenv("DGP_NO_SINCOS_COLS") != nullptr;
   for (int t = 0; t < sp->nterms; t++)
     for (int f = 0; f < sp->term[t].nfactors; f++) {
       dgp_factor& fa = sp->term[t].factor[f];
       fa.pad_ = 0;
-      if (off || fa.kind != DGP_PERIODIC) continue;
+      if (fa.kind != DGP_PERIODIC) continue;
       // reuse the pair of an earlier factor on the same column and period
       for (int c = 0; c + 1 < sp->ncols && fa.pad_ == 0; c++)
         if (sp->col[c].kind == DGP_COL_SINP && sp->col[c].src == fa.col[0] && sp->col[c].theta == fa.period) fa.pad_ = c + 1;
@@ -536,13 +376,6 @@ int dgp_set_train(dgp_handle h, const dgp_spec* spec, const double* X, const dou
   int rc = check_spec(h, spec);
   if (rc) return rc;
   CK(h, cudaSetDevice(h->device));
-  if (!h->have_train || n != h->n || memcmp(&h->user_spec, spec, sizeof(dgp_spec)) != 0) {
-    for (auto& gs : h->graphs) {  // captured launch sequences bake in n and the spec
-      if (gs.exec) cudaGraphExecDestroy(gs.exec);
-      gs = dgp_handle_s::GraphSlot();
-    }
-  }
-  h->user_spec = *spec;
   h->spec = *spec;
   augment_spec(&h->spec);
   h->n = n;
@@ -586,7 +419,7 @@ static GemmArgs base_args(dgp_handle h, int mode, int step) {
   memset(&g, 0, sizeof(g));
   g.mode = mode; g.step = step; g.nb = h->nb; g.n = h->n;
   g.ldc = h->npad; g.sign = 1.0;
-  g.Xw = h->Xw; g.noise = h->noise; g.theta = h->theta; g.alpha = h->alpha; g.part = h->gpart;
+  g.Xw = h->Xw; g.noise = h->noise; g.theta = h->theta; g.part = h->gpart;
   return g;
 }
 
@@ -617,19 +450,19 @@ static int ensure_events(dgp_handle h, size_t count) {
   return 0;
 }
 
-// Two-level right-looking Cholesky with look-ahead.  Block columns are grouped in panels of `pw` blocks.
+// Two-level right-looking Cholesky with look-ahead.  Block columns are grouped in panels of PANEL_BLOCKS blocks.
 // Stream P (high priority) runs the latency-bound work of one panel, block column by block column:
 //   potf2(s) -> TRSM(s) (all rows below) [-> forward substitution(s)] -> rank-128 update of the panel's own
 //   remaining columns.
-// Stream T runs the throughput-bound rank-(128 pw) update of everything right of the panel, split in two
-// launches: the next panel's columns first (all panel p+1 reads), then the rest, which overlaps panel p+1 on P.
+// Streams T and T2 run the throughput-bound rank-(128 pw) update of everything right of the panel in column strips: the
+// next panel's columns first (all panel p+1 reads), then the rest, which overlaps panel p+1 on P.
 // The wide update reads/writes each trailing tile once per panel instead of once per block column.
-// one rank-(128 kb) update launch: block columns [o, o + w) (M_TRAIL_COL) or the lower triangle from block o (M_TRAIL)
-static int launch_trail(dgp_handle h, const CholBufs& b, int mode, int k0, int kb, int o, int w, int ntiles, bool first_touch,
+// one rank-(128 kb) update launch of block columns [o, o + w)
+static int launch_trail(dgp_handle h, const CholBufs& b, int k0, int kb, int o, int w, int ntiles, bool first_touch,
                         double jitter, cudaStream_t st, bool half_tiles = false, bool pdl = false) {
-  GemmArgs g = base_args(h, mode, k0);
+  GemmArgs g = base_args(h, M_TRAIL_COL, k0);
   g.nb = b.nb; g.ldc = b.ld;
-  g.aux0 = (mode == M_TRAIL_COL) ? (o | (w << 16)) : o;
+  g.aux0 = o | (w << 16);
   g.aux1 = kb;
   g.aux2 = first_touch ? 0 : 1;
   g.C = b.A; g.ntiles = ntiles; g.sign = -1.0; g.jitter = jitter;
@@ -647,7 +480,7 @@ static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool ge
   const int nb = b.nb;
   const long long ld = b.ld;
   int rc;
-  const bool pdl = h->pdl && !h->trace_path;  // the trace's events would sit between the kernels
+  const bool pdl = !h->trace_path;  // the trace's events would sit between the kernels
   // timing experiments only (results are garbage), compiled in with -DDGP_EXPERIMENTS and never in the shipped library:
   // DGP_SKIP bit 0: no diagonal-block kernel, 1: no panel solve, 2: no in-panel update
 #ifdef DGP_EXPERIMENTS
@@ -659,17 +492,12 @@ static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool ge
     const size_t off = (size_t)s * 128 * ld + (size_t)s * 128;
     const bool inplace = (b.L == b.A);
     trace_mark(h, P, "potf2<", s);
-    static const bool potf2_v1 = getenv("DGP_POTF2_V1") != nullptr && atoi(getenv("DGP_POTF2_V1")) != 0;
     // T_ss is read by the panel solve from the diagonal block of the work matrix: the contiguous copy in DI is only
     // written for the in-place factorisation and for the forward-substitution kernel of the NLML-only path
-    const bool t_in_a = !potf2_v1 && !inplace && !fwd;
+    const bool t_in_a = !inplace && !fwd;
     // the zero sub-blocks of bufL / bufU were cleared by dgp_set_train and only this kernel ever writes them
     const bool lu_clean = !inplace && h->lu_zeroed && b.L == h->bufL && (b.U == nullptr || b.U == h->bufU);
-    if (skip & 1) {}
-    else if (potf2_v1)
-      k_potf2<<<1, PF_THREADS, PF_SMEM, P>>>(b.A + off, b.L + off, b.U ? b.U + off : nullptr, ld,
-                                             b.DI + (size_t)s * 128 * 128, b.scal, s * 128, inplace ? nullptr : b.A + off);
-    else  // dependent launch behind the in-panel update of the previous block column (same stream, nothing in between)
+    if (!(skip & 1))  // dependent launch behind the in-panel update of the previous block column (same stream, nothing in between)
       CK(h, launch_ex(k_potf2_v2, 1, P2_THREADS, (size_t)P2_SMEM, P, pdl && s > pb && !inplace && !fwd, (const double*)(b.A + off), b.L + off,
                       b.U ? b.U + off : (double*)nullptr, ld, t_in_a ? (double*)nullptr : b.DI + (size_t)s * 128 * 128, b.scal, s * 128,
                       inplace ? (double*)nullptr : b.A + off, lu_clean ? 0 : 1, g_no_p2batch));
@@ -684,9 +512,9 @@ static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool ge
       if (inplace) { g.C = b.P; g.ldc = 128; g.aux0 = 1; }  // both half-tiles read the whole block: stage, then copy
       g.aux1 = t_in_a ? 1 : 0;
       const CUtensorMap& tB = t_in_a ? *b.tA : *b.tDI;
-      // half tiles while the launch is smaller than the GPU (chain_half: 2 m 64x64-row CTAs fit the 2 x SMs slots)
-      if (h->chain_half && 4 * m <= 2 * h->sms) { if ((rc = launch_gemm<INIT_ZERO, EPI_STORE, 4>(h, *b.tA, tB, g, P, pdl && !potf2_v1))) return rc; }
-      else if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, *b.tA, tB, g, P, pdl && !potf2_v1))) return rc;
+      // half tiles while the launch is smaller than the GPU (2 m 64x64-row CTAs fit the 2 x SMs slots)
+      if (4 * m <= 2 * h->sms) { if ((rc = launch_gemm<INIT_ZERO, EPI_STORE, 4>(h, *b.tA, tB, g, P, pdl))) return rc; }
+      else if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, *b.tA, tB, g, P, pdl))) return rc;
       if (inplace) {
         k_copy_panel<<<m, 256, 0, P>>>(b.P, b.A, ld, s);
         h->launches++;
@@ -699,17 +527,12 @@ static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool ge
       h->launches++;
       CK(h, cudaGetLastError());
     }
-    if (s + 1 < pe && !(skip & 4)) {  // in-panel update of the panel's own remaining columns, rows >= s + 1
+    if (s + 1 < pe && !(skip & 4)) {  // in-panel update: rank-128 update of the panel's own block columns (s, pe), rows >= s + 1
       const bool waited = (s == pb && mid_wait != nullptr);
       if (waited) CK(h, cudaStreamWaitEvent(P, mid_wait, 0));
-      if (h->inpanel_left) {  // left-looking: column s + 1 takes the panel's columns [pb, s] in one rank-(128 (s+1-pb)) update
-        if ((rc = launch_trail(h, b, M_TRAIL_COL, pb, s + 1 - pb, s + 1, 1, m * 2, generate && pb == 0, jitter, P,
-                               h->chain_half && 4 * m <= 2 * h->sms, pdl && !inplace && !fwd && !waited))) return rc;
-      } else {                // right-looking: rank-128 update of block columns (s, pe)
-        const int w = pe - s - 1;
-        if ((rc = launch_trail(h, b, M_TRAIL_COL, s, 1, s + 1, w, m * 2 * w, generate && s == 0, jitter, P,
-                               h->chain_half && 4 * m * w <= 2 * h->sms, pdl && !inplace && !fwd && !waited))) return rc;
-      }
+      const int w = pe - s - 1;
+      if ((rc = launch_trail(h, b, s, 1, s + 1, w, m * 2 * w, generate && s == 0, jitter, P, 4 * m * w <= 2 * h->sms,
+                             pdl && !inplace && !fwd && !waited))) return rc;
       trace_mark(h, P, "inpanel>", s);
     }
   }
@@ -720,32 +543,27 @@ static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool ge
 // block columns of L, and the diagonal blocks of T and U up to there, are final behind that event)
 struct PanelHook { int (*fn)(dgp_handle, void*, cudaEvent_t, int) = nullptr; void* ctx = nullptr; };
 
+// the standalone generator covers every matrix it is used for with at least two column strips
+static_assert(DGP_PREGEN_MIN_NB >= STRIP_BLOCKS, "pre-generated matrices span more than one strip");
+
 static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jitter, bool fwd, PanelHook hook = PanelHook()) {
   const int nb = b.nb;
   const long long ld = b.ld;
   int rc;
-  cudaStream_t T = h->stream, P = h->lookahead ? h->stream_hi : h->stream;
-  const int pw = h->panel_blocks;
+  cudaStream_t T = h->stream, P = h->stream_hi, T2 = h->stream_t2;
+  constexpr int pw = PANEL_BLOCKS, sw = STRIP_BLOCKS;
   const int npanels = (nb + pw - 1) / pw;
-  // column strips of the trailing updates (see below): width in block columns, a multiple of the panel width
-  const int sw = (h->strip_blocks + pw - 1) / pw * pw;
-  cudaStream_t T2 = (P != T && sw > 0 && h->stream_t2 != nullptr && !h->use_graphs) ? h->stream_t2 : nullptr;
   bool any2 = false;
-  const int nstrips = sw > 0 ? (nb + sw - 1) / sw : 0;
-  // DGP_PREGEN (default on): the covariance matrix is written by a standalone generator, strip by strip on the
+  const int nstrips = (nb + sw - 1) / sw;
+  // above DGP_PREGEN_MIN_NB block columns the covariance matrix is written by a standalone generator, strip by strip on the
   // low-priority stream while the first panel is factored, and the first trailing update reads it like any later one
-  const bool pregen = generate && h->pregen && nb > DGP_PREGEN_MIN_NB;
-  const bool pregen_strips = pregen && T2 != nullptr && h->stream_lo != nullptr && nstrips > 1;
+  const bool pregen = generate && nb > DGP_PREGEN_MIN_NB;
   if ((rc = ensure_events(h, 3 * (size_t)npanels + 3 + (size_t)nstrips))) return rc;
   auto ev_gen = [&](int j) { return h->evs[3 * (size_t)npanels + 2 + j]; };
   auto ev_panel = [&](int p) { return h->evs[3 * p]; };
   auto ev_cols = [&](int p) { return h->evs[3 * p + 1]; };   // all columns of panel p have the updates of panels < p
   auto ev_col0 = [&](int p) { return h->evs[3 * p + 2]; };   // ... its first block column has them
-  if (pregen && !pregen_strips) {   // one trailing stream: everything up front, in stream order
-    k_cov_lower<<<dim3(nb * 4, nb), 256, 0, T>>>(h->spec, h->theta, h->Xw, h->noise, jitter, b.A, ld, h->n, 0);
-    h->launches++;
-    CK(h, cudaGetLastError());
-  } else if (pregen) {
+  if (pregen) {
     k_cov_lower<<<dim3(nb * 4, sw), 256, 0, T>>>(h->spec, h->theta, h->Xw, h->noise, jitter, b.A, ld, h->n, 0);
     h->launches++;
     CK(h, cudaGetLastError());
@@ -765,25 +583,22 @@ static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jit
     h->launches++;
     CK(h, cudaGetLastError());
   }
-  if (P != T) {
-    CK(h, cudaEventRecord(ev_cols(0), T));
-    CK(h, cudaStreamWaitEvent(P, ev_cols(0), 0));
-  }
+  CK(h, cudaEventRecord(ev_cols(0), T));
+  CK(h, cudaStreamWaitEvent(P, ev_cols(0), 0));
   for (int p = 0; p < npanels; p++) {
     const int pb = p * pw, pe = (pb + pw < nb) ? pb + pw : nb;
-    if (P != T && p > 0) CK(h, cudaStreamWaitEvent(P, ev_col0(p), 0));
-    if ((rc = factor_panel(h, b, pb, pe, generate && !pregen, jitter, fwd, P, (P != T && p > 0) ? ev_cols(p) : nullptr))) return rc;
-    if (P != T) {
-      CK(h, cudaEventRecord(ev_panel(p), P));
-      CK(h, cudaStreamWaitEvent(T, ev_panel(p), 0));
-      if (hook.fn && pe < nb && (rc = hook.fn(h, hook.ctx, ev_panel(p), pe))) return rc;
-    }
-    if (pe < nb && T2 != nullptr) {
+    if (p > 0) CK(h, cudaStreamWaitEvent(P, ev_col0(p), 0));
+    if ((rc = factor_panel(h, b, pb, pe, generate && !pregen, jitter, fwd, P, p > 0 ? ev_cols(p) : nullptr))) return rc;
+    CK(h, cudaEventRecord(ev_panel(p), P));
+    CK(h, cudaStreamWaitEvent(T, ev_panel(p), 0));
+    if (hook.fn && pe < nb && (rc = hook.fn(h, hook.ctx, ev_panel(p), pe))) return rc;
+    if (pe < nb) {
       // Column strips on two streams.  The trailing matrix is cut into fixed strips of `sw` block columns; strip j is
       // always updated on stream j mod 2, so the strips of one stream form their own dependency chain (panel after
       // panel) and the two streams never wait for each other: while one launch drains its last partial wave, the other
       // stream's CTAs take the free slots (a single stream loses about half a wave per launch, 3 launches per panel).
       // The next panel's columns are the head of their strip: first column | its other columns | the rest of the strip.
+      // Launches with fewer tiles than the GPU has CTA slots run on 64-row half tiles (a K = 512 tile is 34 us on its own).
       const int ne = (pe + pw < nb) ? pe + pw : nb, w = ne - pe, m = nb - pe;
       const int slots = 2 * h->sms;
       const bool first = generate && p == 0 && !pregen;
@@ -795,44 +610,28 @@ static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jit
           if (!used2) { used2 = true; cudaStreamWaitEvent(T2, ev_panel(p), 0); }
           S = T2;
         }
-        if (pregen_strips && p == 0 && j > 0) cudaStreamWaitEvent(S, ev_gen(j), 0);
+        if (pregen && p == 0 && j > 0) cudaStreamWaitEvent(S, ev_gen(j), 0);
         return S;
       };
       cudaStream_t S0 = strip_stream(j0);
       trace_mark(h, S0, "cols<", p);
-      if ((rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, pe, 1, m * 2, first, jitter, S0, h->chain_half && m * 2 <= slots))) return rc;
+      if ((rc = launch_trail(h, b, pb, pe - pb, pe, 1, m * 2, first, jitter, S0, m * 2 <= slots))) return rc;
       CK(h, cudaEventRecord(ev_col0(p + 1), S0));
-      if (w > 1 && (rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, pe + 1, w - 1, (m - 1) * 2 * (w - 1), first, jitter, S0,
-                                      h->chain_half && (m - 1) * 2 * (w - 1) <= slots))) return rc;
+      if (w > 1 && (rc = launch_trail(h, b, pb, pe - pb, pe + 1, w - 1, (m - 1) * 2 * (w - 1), first, jitter, S0,
+                                      (m - 1) * 2 * (w - 1) <= slots))) return rc;
       trace_mark(h, S0, "cols>", p);
       CK(h, cudaEventRecord(ev_cols(p + 1), S0));
       const int e0 = ((j0 + 1) * sw < nb) ? (j0 + 1) * sw : nb;
       if (ne < e0) {
         const int tiles = (nb - ne) * 2 * (e0 - ne);
-        if ((rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, ne, e0 - ne, tiles, first, jitter, S0, h->chain_half && tiles <= slots))) return rc;
+        if ((rc = launch_trail(h, b, pb, pe - pb, ne, e0 - ne, tiles, first, jitter, S0, tiles <= slots))) return rc;
       }
       for (int j = j0 + 1; j * sw < nb; j++) {
         const int o = j * sw, wj = (o + sw < nb) ? sw : nb - o, tiles = (nb - o) * 2 * wj;
-        if ((rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, o, wj, tiles, first, jitter, strip_stream(j), h->chain_half && tiles <= slots))) return rc;
+        if ((rc = launch_trail(h, b, pb, pe - pb, o, wj, tiles, first, jitter, strip_stream(j), tiles <= slots))) return rc;
       }
       trace_mark(h, T, "rest>", p);
       if (used2) any2 = true;
-    } else if (pe < nb) {  // rank-(128 (pe - pb)) update right of the panel: next panel's columns, then the rest
-      const int ne = (pe + pw < nb) ? pe + pw : nb, w = ne - pe, m = nb - pe;
-      // the first column of the next panel is all its diagonal block and panel solve wait for: update it on its own
-      trace_mark(h, T, "cols<", p);
-      // (half tiles while a launch has fewer tiles than the GPU has CTA slots: a K = 512 tile is 34 us on its own)
-      const int slots = 2 * h->sms;
-      if ((rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, pe, 1, m * 2, generate && p == 0 && !pregen, jitter, T, h->chain_half && m * 2 <= slots))) return rc;
-      if (P != T) CK(h, cudaEventRecord(ev_col0(p + 1), T));
-      if (w > 1 && (rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, pe + 1, w - 1, (m - 1) * 2 * (w - 1), generate && p == 0 && !pregen, jitter, T,
-                                      h->chain_half && (m - 1) * 2 * (w - 1) <= slots))) return rc;
-      trace_mark(h, T, "cols>", p);
-      if (P != T) CK(h, cudaEventRecord(ev_cols(p + 1), T));
-      const int m2 = nb - ne;
-      if (m2 > 0 && (rc = launch_trail(h, b, M_TRAIL, pb, pe - pb, ne, 0, m2 * (m2 + 1), generate && p == 0 && !pregen, jitter, T,
-                                       h->chain_half && m2 * (m2 + 1) <= slots))) return rc;
-      trace_mark(h, T, "rest>", p);
     }
   }
   if (any2) {  // the caller continues on T
@@ -847,7 +646,7 @@ static int run_potrf(dgp_handle h, double jitter, bool fwd, PanelHook hook = Pan
   return potrf_core(h, b, true, jitter, fwd, hook);
 }
 
-// U = L^-T (upper) by recursive doubling: the diagonal 128-blocks come from k_potf2 (U_ss in bufU, T_ss = L_ss^-1 in
+// U = L^-T (upper) by recursive doubling: the diagonal 128-blocks come from k_potf2_v2 (U_ss in bufU, T_ss = L_ss^-1 in
 // the diagonal blocks of bufA); level h merges neighbouring block ranges [o, o+h) | [o+h, o+2h):
 //   M'  = U11 L21'          -> scratch, upper triangle of bufA          (long-K tiles, no read-modify-write)
 //   U12 = -M' T22'          -> bufU
@@ -861,28 +660,23 @@ struct InvProgress {
   int done[16];       // per level (hb = 1 << l): leading pairs already launched
   bool want_T;
   cudaStream_t W;
-  int lag;            // release the merges `lag` block columns late (DGP_EAGER_LAG)
-  int max_h;          // highest level (block count of a merged range) launched before the factorisation is complete
 };
 
 static int trtri_advance(dgp_handle h, InvProgress& ip, int F) {
   const int nb = h->nb;
   int rc, lv = 0;
   for (int hb = 1; hb < nb; hb *= 2, lv++) {
-    if (F < nb && hb > ip.max_h) break;   // while the factorisation runs: only the levels whose tiles are short
     const int npairs = (nb - hb + 2 * hb - 1) / (2 * hb);  // pairs whose second range is non-empty
     const int avail = F >= nb ? npairs : F / (2 * hb);
     const int pr0 = ip.done[lv], cnt = avail - pr0;
     if (cnt <= 0) continue;
     {
       GemmArgs g = base_args(h, M_INV_M, pr0);
-      g.raster = raster_on();
       g.aux0 = hb; g.aux1 = cnt; g.C = h->bufA; g.ntiles = cnt * hb * 2 * hb;
       if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmU, h->tmL, g, ip.W))) return rc;
     }
     {
       GemmArgs g = base_args(h, M_INV_U, pr0);
-      g.raster = raster_on();
       g.aux0 = hb; g.aux1 = cnt; g.C = h->bufU; g.ntiles = cnt * hb * 2 * hb; g.sign = -1.0;
       if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmA, h->tmA, g, ip.W))) return rc;
     }
@@ -898,10 +692,9 @@ static int trtri_advance(dgp_handle h, InvProgress& ip, int F) {
 
 static int eager_hook(dgp_handle h, void* ctx, cudaEvent_t ev_panel, int pe) {
   InvProgress& ip = *(InvProgress*)ctx;
-  const int F = pe - ip.lag;
-  if (F < 2 || (F & 7) != 0) return 0;   // every 8 block columns: 4 / 2 / 1 new pairs at the three lowest levels
+  if ((pe & 7) != 0) return 0;   // every 8 block columns: 4 / 2 / 1 new pairs at the three lowest levels
   CK(h, cudaStreamWaitEvent(ip.W, ev_panel, 0));
-  return trtri_advance(h, ip, F);
+  return trtri_advance(h, ip, pe);
 }
 
 static int run_trtri(dgp_handle h, InvProgress& ip) {
@@ -917,20 +710,12 @@ static int run_trtri(dgp_handle h, InvProgress& ip) {
   return 0;
 }
 
+// LAUUM stores the lower tiles of Ky^-1 (8 n^2 / 2 B, over T, which is dead by now) and a separate high-occupancy pass
+// contracts W = alpha alpha' - Ky^-1 with the regenerated dK/dtheta tiles (measured 3-4 ms faster at n = 16384 than the
+// contraction fused into the LAUUM epilogue, whose dependent FP64 chains wait behind the co-resident CTA's DMMA issue).
 static int run_lauum_grad(dgp_handle h) {
   GemmArgs g = base_args(h, M_LAUUM, 0);
-  g.raster = raster_on();
-  g.C = h->bufA; g.ntiles = lauum_slots(h->nb, g.raster);
-  g.Kinv = h->debug_kinv ? h->bufA : nullptr;
-  // Default: LAUUM stores the lower tiles of Ky^-1 (8 n^2 / 2 B, over T, which is dead by now) and a separate
-  // high-occupancy pass contracts W = alpha alpha' - Ky^-1 with the regenerated dK/dtheta tiles.  DGP_FUSED_GRAD=1
-  // selects the contraction fused into the LAUUM epilogue instead (no Ky^-1 round trip; measured 3-4 ms slower at
-  // n = 16384 because the epilogue's dependent FP64 chains wait behind the co-resident CTA's DMMA issue).
-  static const bool fused = getenv("DGP_FUSED_GRAD") != nullptr && atoi(getenv("DGP_FUSED_GRAD")) != 0;
-  if (fused) {  // per-tile partials are indexed by the CTA: row-by-row order, one CTA per tile
-    g.raster = 0; g.ntiles = h->nb * (h->nb + 1);
-    return launch_gemm<INIT_ZERO, EPI_GRAD>(h, h->tmU, h->tmU, g);
-  }
+  g.C = h->bufA; g.ntiles = lauum_slots(h->nb);
   int rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmU, h->tmU, g);
   if (rc) return rc;
   k_grad_contract<<<h->nb * (h->nb + 1), 128, 0, h->stream>>>(h->spec, h->theta, h->Xw, h->alpha, h->bufA, h->npad, h->n, h->gpart);
@@ -952,43 +737,35 @@ static int evaluate_enqueue(dgp_handle h, double jitter, int level) {
   int rc;
   CK(h, cudaMemcpyAsync(h->theta, h->h_theta, sizeof(double) * h->spec.ntheta, cudaMemcpyHostToDevice, h->stream));
   if ((rc = run_features(h))) return rc;
-  // the O(n^3) phases after the factorisation go to the low-priority stream (when the handle has one)
+  // the O(n^3) phases after the factorisation go to the low-priority stream
   cudaStream_t main_stream = h->stream;
-  const bool lo = level >= 1 && h->stream_lo != nullptr && !h->use_graphs;
   InvProgress ip;
   memset(&ip, 0, sizeof(ip));
-  ip.want_T = (level == 2); ip.W = lo ? h->stream_lo : main_stream; ip.lag = h->eager_lag;
-  // (measured: every level is a gain up to n = 8192 and for batches; at n = 16384 the long low-priority tiles of the high
-  // levels cost the chain of the last panels as much as they fill -- there only the levels up to eager_max_h go early)
-  ip.max_h = (h->eager_inv > 1 || h->nb <= 96) ? (1 << 20) : h->eager_max_h;
+  ip.want_T = (level == 2); ip.W = h->stream_lo;
+  // (measured: releasing the merges as the factorisation passes them is a gain at every level up to n = 8192 and for
+  // batches; at n = 16384 the long low-priority tiles cost the chain of the last panels as much as they fill, and no level
+  // gained there -- above EAGER_INV_MAX_NB block columns the inverse starts after the factorisation)
   PanelHook hook;
-  if (lo && h->lookahead && h->eager_inv >= 1 && ip.max_h >= 1) { hook.fn = eager_hook; hook.ctx = &ip; }
+  if (level >= 1 && h->nb <= EAGER_INV_MAX_NB) { hook.fn = eager_hook; hook.ctx = &ip; }
   if ((rc = run_potrf(h, jitter, level == 0, hook))) return rc;  // level >= 1: z = U'r after the inverse instead
   if (h->timing) CK(h, cudaEventRecord(h->ev[1], h->stream));
   if (level >= 1) {
-    if (lo) {
-      CK(h, cudaEventRecord(h->ev_lo[0], main_stream));
-      CK(h, cudaStreamWaitEvent(h->stream_lo, h->ev_lo[0], 0));
-      h->stream = h->stream_lo;
-    }
+    CK(h, cudaEventRecord(h->ev_lo[0], main_stream));
+    CK(h, cudaStreamWaitEvent(h->stream_lo, h->ev_lo[0], 0));
+    h->stream = h->stream_lo;
     rc = run_trtri(h, ip);
     if (!rc && h->timing) { cudaEventRecord(h->ev[2], h->stream); }
     if (!rc && level == 1) rc = run_lauum_grad(h);
     if (!rc && h->timing) { cudaEventRecord(h->ev[3], h->stream); }
-    if (lo) {
-      cudaEventRecord(h->ev_lo[1], h->stream_lo);
-      h->stream = main_stream;
-      CK(h, cudaStreamWaitEvent(main_stream, h->ev_lo[1], 0));
-    }
+    cudaEventRecord(h->ev_lo[1], h->stream_lo);
+    h->stream = main_stream;
+    CK(h, cudaStreamWaitEvent(main_stream, h->ev_lo[1], 0));
     if (rc) return rc;
   }
   if ((rc = run_finish(h, level == 1))) return rc;
   return 0;
 }
 
-// The launch sequence of an evaluation depends only on (n, level, jitter): the first call of a kind runs eagerly,
-// the second is captured into a CUDA graph (both streams; the look-ahead events become graph edges) and every
-// later call replays it, so that the ~10^3 launches cost one cudaGraphLaunch on the host.
 static int evaluate_launch(dgp_handle h, const double* theta, double jitter, int level) {
   // level 0: nlml ; 1: nlml + grad ; 2: factorize for prediction (L, U, alpha, T)
   if (!h) return -1;
@@ -998,32 +775,9 @@ static int evaluate_launch(dgp_handle h, const double* theta, double jitter, int
   int rc;
   h->factorized = false; h->have_T = false;
   memcpy(h->h_theta, theta, sizeof(double) * h->spec.ntheta);
-  dgp_handle_s::GraphSlot& gs = h->graphs[level];
-  const bool use_graph = h->use_graphs && !h->timing && !h->debug_kinv;
-  if (use_graph && gs.exec != nullptr && gs.jitter == jitter) {
-    CK(h, cudaGraphLaunch(gs.exec, h->stream));
-    h->launches += gs.launches;
-  } else if (use_graph && gs.seen && gs.jitter == jitter) {
-    if (gs.exec != nullptr) { cudaGraphExecDestroy(gs.exec); gs.exec = nullptr; }
-    const long long l0 = h->launches;
-    cudaGraph_t graph = nullptr;
-    CK(h, cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-    rc = evaluate_enqueue(h, jitter, level);
-    cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
-    if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-    if (ce != cudaSuccess) DGP_FAIL(h, -2, "graph capture failed: %s", cudaGetErrorString(ce));
-    ce = cudaGraphInstantiate(&gs.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (ce != cudaSuccess) { gs.exec = nullptr; DGP_FAIL(h, -2, "graph instantiate failed: %s", cudaGetErrorString(ce)); }
-    gs.launches = h->launches - l0;
-    CK(h, cudaGraphLaunch(gs.exec, h->stream));
-  } else {
-    if (gs.exec != nullptr && gs.jitter != jitter) { cudaGraphExecDestroy(gs.exec); gs.exec = nullptr; }
-    gs.seen = true; gs.jitter = jitter;
-    if (h->timing) CK(h, cudaEventRecord(h->ev[0], h->stream));
-    if ((rc = evaluate_enqueue(h, jitter, level))) return rc;
-    if (h->timing) CK(h, cudaEventRecord(h->ev[4], h->stream));
-  }
+  if (h->timing) CK(h, cudaEventRecord(h->ev[0], h->stream));
+  if ((rc = evaluate_enqueue(h, jitter, level))) return rc;
+  if (h->timing) CK(h, cudaEventRecord(h->ev[4], h->stream));
   h->pending = true;
   h->pending_grad = level;
   return 0;
@@ -1411,8 +1165,8 @@ int dgp_dist_dims(dgp_handle h, int m, int S, int world, long long* dims) {
   if (!h->have_train) DGP_FAIL(h, -1, "dgp_dist_dims: no training data");
   const long long mpad = round_up(m, 128), mb = mpad / 128;
   const long long rows_per_rank = ((mb + world - 1) / world) * 128;
-  dims[0] = mpad; dims[1] = h->npad; dims[2] = round_up(S, 128); dims[3] = (long long)h->panel_blocks * 128;
-  dims[4] = (mb + h->panel_blocks - 1) / h->panel_blocks; dims[5] = rows_per_rank;
+  dims[0] = mpad; dims[1] = h->npad; dims[2] = round_up(S, 128); dims[3] = (long long)PANEL_BLOCKS * 128;
+  dims[4] = (mb + PANEL_BLOCKS - 1) / PANEL_BLOCKS; dims[5] = rows_per_rank;
   return 0;
 }
 
@@ -1425,7 +1179,7 @@ int dgp_dist_begin(dgp_handle h, const double* Xs, int m, int S, const double* Z
   CK(h, cudaSetDevice(h->device));
   dgp_dist d = new dgp_dist_s();
   d->h = h; d->m = m; d->mpad = round_up(m, 128); d->mb = d->mpad / 128; d->S = S; d->Spad = round_up(S, 128);
-  d->pw = h->panel_blocks; d->npanels = (d->mb + d->pw - 1) / d->pw; d->rank = rank; d->world = world; d->jitter = jitter;
+  d->pw = PANEL_BLOCKS; d->npanels = (d->mb + d->pw - 1) / d->pw; d->rank = rank; d->world = world; d->jitter = jitter;
   d->VT = VT; d->Od = Od; d->mu = mu;
   const size_t mpad = d->mpad;
   {
@@ -1570,7 +1324,7 @@ int dgp_dist_trail(dgp_dist d, int p, int j_first, int j_last) {
   for (int j = j_first; j <= j_last; j++) {
     if (!d->mine(j)) continue;
     const int jb = j * d->pw, je = (jb + d->pw < d->mb) ? jb + d->pw : d->mb, w = je - jb;
-    if ((rc = launch_trail(h, b, M_TRAIL_COL, pb, pe - pb, jb, w, (d->mb - jb) * 2 * w, false, 0.0, h->stream))) return rc;
+    if ((rc = launch_trail(h, b, pb, pe - pb, jb, w, (d->mb - jb) * 2 * w, false, 0.0, h->stream))) return rc;
   }
   return 0;
 }

@@ -19,16 +19,10 @@ struct dgp_batch_s {
   int device = 0, sms = 148;
   cudaStream_t stream = nullptr, stream_hi = nullptr, stream_lo = nullptr, stream_t2 = nullptr;
   bool own_stream = false;
-  bool eager_inv = true;     // merges of the inverse launched as the factorisation passes them (DGP_EAGER_INV=0: after it)
-  int eager_lag = 0;
-  int strip_blocks = 8;      // column strips of the trailing updates on two streams (DGP_STRIP_BLOCKS; 0: one stream)
   cudaEvent_t ev_lo[2] = {nullptr, nullptr};
   cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   std::vector<cudaEvent_t> evs;
-  int panel_blocks = 4;
-  bool pdl = true, chain_half = true, timing = false;
-  bool pregen = true;        // standalone covariance generator ahead of the factorisation (DGP_PREGEN=0: first-touch generation)
-  bool inpanel_left = false; // in-panel updates left-looking (DGP_INPANEL_LEFT=1; default: right-looking rank-128 updates, like the single-site engine -- the two must agree for bit-identical results)
+  bool timing = false;
   int max_sites = 0, max_pad = 0, max_n = 0;
   int G = 0, NB = 0;
   long long ld = 0;
@@ -83,18 +77,17 @@ GemmArgs b_args(dgp_batch_t b, int mode, double* C, double sign, int ntiles) {
   memset(&g, 0, sizeof(g));
   g.mode = mode; g.nb = b->NB; g.n = 0;
   g.ntiles = ntiles; g.C = C; g.ldc = b->ld; g.sign = sign;
-  g.Xw = b->Xw; g.noise = b->noise; g.theta = b->theta; g.alpha = b->alpha; g.part = b->gpart;
-  g.raster = raster_on();
+  g.Xw = b->Xw; g.noise = b->noise; g.theta = b->theta; g.part = b->gpart;
   return g;
 }
 
-// one rank-(128 kb) update launch over the sites of `tb` (M_TRAIL_COL / M_TRAIL entries); half_limit: largest tile count
-// that still runs on 64-row half tiles (0: never)
-int b_launch_trail(dgp_batch_t b, const TabBuilder& tb, int mode, cudaStream_t st, int half_limit, bool pdl) {
+// one rank-(128 kb) update launch over the sites of `tb` (M_TRAIL_COL entries); half_limit: largest tile count that still
+// runs on 64-row half tiles
+int b_launch_trail(dgp_batch_t b, const TabBuilder& tb, cudaStream_t st, int half_limit, bool pdl) {
   if (tb.total <= 0) return 0;
-  GemmArgs g = b_args(b, mode, b->A, -1.0, tb.total);
+  GemmArgs g = b_args(b, M_TRAIL_COL, b->A, -1.0, tb.total);
   if (tb.any_first) return launch_gemm<INIT_COV, EPI_STORE>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
-  if (b->chain_half && tb.total <= half_limit) return launch_gemm<INIT_LOAD, EPI_STORE, 4>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
+  if (tb.total <= half_limit) return launch_gemm<INIT_LOAD, EPI_STORE, 4>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
   return launch_gemm<INIT_LOAD, EPI_STORE>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
 }
 
@@ -113,13 +106,12 @@ int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg);
 int b_eager(dgp_batch_t b, BInvProgress* ip, cudaEvent_t ev_panel, int pe);
 
 int b_potrf(dgp_batch_t b, BInvProgress* eager) {
-  const int G = b->G, NB = b->NB, pw = b->panel_blocks;
+  const int G = b->G, NB = b->NB;
+  constexpr int pw = PANEL_BLOCKS, sw = STRIP_BLOCKS;
   const long long ld = b->ld;
-  cudaStream_t T = b->stream, P = b->stream_hi;
+  cudaStream_t T = b->stream, P = b->stream_hi, T2 = b->stream_t2;
   const int npanels = (NB + pw - 1) / pw;
   int rc;
-  const int sw = (b->strip_blocks + pw - 1) / pw * pw;
-  cudaStream_t T2 = (sw > 0 && b->stream_t2 != nullptr) ? b->stream_t2 : nullptr;
   bool any2 = false;
   if ((rc = b_ensure_events(b, 3 * (size_t)npanels + 3))) return rc;
   auto ev_panel = [&](int p) { return b->evs[3 * p]; };
@@ -130,13 +122,13 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
   CK(b, cudaGetLastError());
   CK(b, cudaEventRecord(ev_cols(0), T));
   CK(b, cudaStreamWaitEvent(P, ev_cols(0), 0));
-  // standalone generator (potrf_core's DGP_PREGEN schedule): the sites with more than DGP_PREGEN_MIN_NB block columns get their
+  // standalone generator (as in potrf_core): the sites with more than DGP_PREGEN_MIN_NB block columns get their
   // whole lower triangle written on the low-priority stream while the first diagonal blocks are factored, and their first
   // updates read it like any later one.  The same sites by the same rule as the single-site engine: bit-identical results.
   bool pre[DGP_BATCH_MAX];
   bool any_pre = false, wP = false, wT = false, w2 = false;
   for (int i = 0; i < G; i++) {
-    pre[i] = b->pregen && b->nb[i] > DGP_PREGEN_MIN_NB;
+    pre[i] = b->nb[i] > DGP_PREGEN_MIN_NB;
     any_pre |= pre[i];
   }
   cudaEvent_t ev_gen = b->evs[3 * (size_t)npanels + 1];
@@ -165,17 +157,7 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
         const int m = nbi - s - 1;
         trsm.add(i, s, nbi, b->n[i], 0, 1, 0, 2 * m);
         const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
-        if (s + 1 < lpe && b->inpanel_left) {
-          // left-looking inside the panel (option): block column s + 1 takes the panel's columns [lpb, s] in ONE
-          // rank-(128 (s+1-lpb)) update (read and written once per panel instead of once per earlier column).  Since the
-          // tile engine adds a tile's old value in its epilogue (out = old + sign * sum, sums started at zero) the two forms
-          // round differently, and with the C tile prefetched they cost the same (measured): the default is right-looking
-          // in both engines, which keeps batch and single-site results bit-identical.
-          const int lpb = pb - b->off[i];
-          const bool first = (lpb == 0) && !pre[i];   // columns of a site's first panel are generated here
-          inp.add(i, lpb, nbi, b->n[i], (s + 1) | (1 << 16), s + 1 - lpb, first ? 0 : 1, m * 2);
-          inp.any_first |= first && m > 0;
-        } else if (s + 1 < lpe) {
+        if (s + 1 < lpe) {   // right-looking, like the single-site engine: the two must agree for bit-identical results
           const int w = lpe - s - 1;
           const bool first = (s == 0) && !pre[i];
           inp.add(i, s, nbi, b->n[i], (s + 1) | (w << 16), 1, first ? 0 : 1, m * 2 * w);
@@ -184,20 +166,20 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
       }
       if (pk.count == 0) continue;
       // dependent launch behind the in-panel update of the previous block column (same stream, nothing in between)
-      CK(b, launch_ex(k_potf2_v2, pk.count, P2_THREADS, (size_t)P2_SMEM, P, b->pdl && t > pb, (const double*)b->A, b->L, b->U, ld,
+      CK(b, launch_ex(k_potf2_v2, pk.count, P2_THREADS, (size_t)P2_SMEM, P, t > pb, (const double*)b->A, b->L, b->U, ld,
                       (double*)nullptr, b->scal, 0, b->A, 0, pk));
       b->launches++;
       if (trsm.total > 0) {  // panel solve: L[i, s] = A[i, s] T_ss', T_ss read from the diagonal block of the work matrix
         GemmArgs g = b_args(b, M_TRSM, b->L, 1.0, trsm.total);
-        if (b->chain_half && 2 * trsm.total <= slots) { if ((rc = launch_gemm<INIT_ZERO, EPI_STORE, 4>(b, b->tmA, b->tmA, g, P, b->pdl, &trsm.t))) return rc; }
-        else if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmA, b->tmA, g, P, b->pdl, &trsm.t))) return rc;
+        if (2 * trsm.total <= slots) { if ((rc = launch_gemm<INIT_ZERO, EPI_STORE, 4>(b, b->tmA, b->tmA, g, P, true, &trsm.t))) return rc; }
+        else if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmA, b->tmA, g, P, true, &trsm.t))) return rc;
       }
       if (inp.total > 0) {   // rank-128 update of the panel's own remaining columns
         const bool waited = (t == pb && p > 0);
         if (waited) CK(b, cudaStreamWaitEvent(P, ev_cols(p), 0));
         const bool gen_wait = any_pre && !wP;
         if (gen_wait) { wP = true; CK(b, cudaStreamWaitEvent(P, ev_gen, 0)); }
-        if ((rc = b_launch_trail(b, inp, M_TRAIL_COL, P, b->sms, b->pdl && !waited && !gen_wait))) return rc;
+        if ((rc = b_launch_trail(b, inp, P, b->sms, !waited && !gen_wait))) return rc;
       }
     }
     CK(b, cudaEventRecord(ev_panel(p), P));
@@ -207,77 +189,54 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
     // ---- rank-(128 pw) update right of the panel.  Column strips on two streams (potrf_core of dgp_api.cu): fixed strips
     // of `sw` block columns in the end-aligned (global) column numbering, strip j always on stream j mod 2; the next panel's
     // columns are the head of their strip: first column | its other columns | the rest of the strip.
-    if (T2 != nullptr) {
-      const int j0 = pe / sw;
-      bool used2 = false;
-      auto strip_stream = [&](int j) -> cudaStream_t {
-        if ((j & 1) == 0) return T;
-        if (!used2) { used2 = true; cudaStreamWaitEvent(T2, ev_panel(p), 0); }
-        if (any_pre && !w2) { w2 = true; cudaStreamWaitEvent(T2, ev_gen, 0); }
-        return T2;
-      };
-      cudaStream_t S0 = strip_stream(j0);
-      TabBuilder ta(b), tb2(b), tr(b);
-      int jmax = j0;
-      for (int k = 0; k < G; k++) {
-        const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
-        if (lpb < 0 || lpb >= nbi) continue;
-        const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
-        if (lpe >= nbi) continue;
-        const int kb = lpe - lpb, ne = (lpe + pw < nbi) ? lpe + pw : nbi, w = ne - lpe, m = nbi - lpe;
-        const bool first = (lpb == 0) && !pre[i];
-        const int a2 = first ? 0 : 1;
-        ta.add(i, lpb, nbi, b->n[i], lpe | (1 << 16), kb, a2, m * 2);
-        ta.any_first |= first;
-        if (w > 1) { tb2.add(i, lpb, nbi, b->n[i], (lpe + 1) | ((w - 1) << 16), kb, a2, (m - 1) * 2 * (w - 1)); tb2.any_first |= first; }
-        const int e0 = ((j0 + 1) * sw - b->off[i] < nbi) ? (j0 + 1) * sw - b->off[i] : nbi;   // local end of the near strip
-        if (ne < e0) { tr.add(i, lpb, nbi, b->n[i], ne | ((e0 - ne) << 16), kb, a2, (nbi - ne) * 2 * (e0 - ne)); tr.any_first |= first; }
-        const int jl = (b->off[i] + nbi - 1) / sw;   // last global strip this site reaches
-        if (jl > jmax) jmax = jl;
-      }
-      if ((rc = b_launch_trail(b, ta, M_TRAIL_COL, S0, slots, false))) return rc;
-      if (p + 1 < npanels) CK(b, cudaEventRecord(ev_col0(p + 1), S0));
-      if ((rc = b_launch_trail(b, tb2, M_TRAIL_COL, S0, slots, false))) return rc;
-      if (p + 1 < npanels) CK(b, cudaEventRecord(ev_cols(p + 1), S0));
-      if ((rc = b_launch_trail(b, tr, M_TRAIL_COL, S0, slots, false))) return rc;
-      for (int j = j0 + 1; j <= jmax; j++) {
-        TabBuilder ts(b);
-        for (int k = 0; k < G; k++) {
-          const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
-          if (lpb < 0 || lpb >= nbi) continue;
-          const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
-          const int o = j * sw - b->off[i];
-          if (lpe >= nbi || o >= nbi) continue;
-          const int wj = (o + sw < nbi) ? sw : nbi - o;
-          const bool first = (lpb == 0) && !pre[i];
-          ts.add(i, lpb, nbi, b->n[i], o | (wj << 16), lpe - lpb, first ? 0 : 1, (nbi - o) * 2 * wj);
-          ts.any_first |= first;
-        }
-        if (ts.total > 0 && (rc = b_launch_trail(b, ts, M_TRAIL_COL, strip_stream(j), slots, false))) return rc;
-      }
-      if (used2) any2 = true;
-      continue;
-    }
-    // one stream: next panel's first column | its other columns | the rest
-    TabBuilder ta(b), tb2(b), tc(b);
+    const int j0 = pe / sw;
+    bool used2 = false;
+    auto strip_stream = [&](int j) -> cudaStream_t {
+      if ((j & 1) == 0) return T;
+      if (!used2) { used2 = true; cudaStreamWaitEvent(T2, ev_panel(p), 0); }
+      if (any_pre && !w2) { w2 = true; cudaStreamWaitEvent(T2, ev_gen, 0); }
+      return T2;
+    };
+    cudaStream_t S0 = strip_stream(j0);
+    TabBuilder ta(b), tb2(b), tr(b);
+    int jmax = j0;
     for (int k = 0; k < G; k++) {
       const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
       if (lpb < 0 || lpb >= nbi) continue;
       const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
       if (lpe >= nbi) continue;
-      const int kb = lpe - lpb, ne = (lpe + pw < nbi) ? lpe + pw : nbi, w = ne - lpe, m = nbi - lpe, m2 = nbi - ne;
+      const int kb = lpe - lpb, ne = (lpe + pw < nbi) ? lpe + pw : nbi, w = ne - lpe, m = nbi - lpe;
       const bool first = (lpb == 0) && !pre[i];
       const int a2 = first ? 0 : 1;
       ta.add(i, lpb, nbi, b->n[i], lpe | (1 << 16), kb, a2, m * 2);
       ta.any_first |= first;
       if (w > 1) { tb2.add(i, lpb, nbi, b->n[i], (lpe + 1) | ((w - 1) << 16), kb, a2, (m - 1) * 2 * (w - 1)); tb2.any_first |= first; }
-      if (m2 > 0) { tc.add(i, lpb, nbi, b->n[i], ne, kb, a2, m2 * (m2 + 1)); tc.any_first |= first; }
+      const int e0 = ((j0 + 1) * sw - b->off[i] < nbi) ? (j0 + 1) * sw - b->off[i] : nbi;   // local end of the near strip
+      if (ne < e0) { tr.add(i, lpb, nbi, b->n[i], ne | ((e0 - ne) << 16), kb, a2, (nbi - ne) * 2 * (e0 - ne)); tr.any_first |= first; }
+      const int jl = (b->off[i] + nbi - 1) / sw;   // last global strip this site reaches
+      if (jl > jmax) jmax = jl;
     }
-    if ((rc = b_launch_trail(b, ta, M_TRAIL_COL, T, slots, false))) return rc;
-    if (p + 1 < npanels) CK(b, cudaEventRecord(ev_col0(p + 1), T));
-    if ((rc = b_launch_trail(b, tb2, M_TRAIL_COL, T, slots, false))) return rc;
-    if (p + 1 < npanels) CK(b, cudaEventRecord(ev_cols(p + 1), T));
-    if ((rc = b_launch_trail(b, tc, M_TRAIL, T, slots, false))) return rc;
+    if ((rc = b_launch_trail(b, ta, S0, slots, false))) return rc;
+    if (p + 1 < npanels) CK(b, cudaEventRecord(ev_col0(p + 1), S0));
+    if ((rc = b_launch_trail(b, tb2, S0, slots, false))) return rc;
+    if (p + 1 < npanels) CK(b, cudaEventRecord(ev_cols(p + 1), S0));
+    if ((rc = b_launch_trail(b, tr, S0, slots, false))) return rc;
+    for (int j = j0 + 1; j <= jmax; j++) {
+      TabBuilder ts(b);
+      for (int k = 0; k < G; k++) {
+        const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
+        if (lpb < 0 || lpb >= nbi) continue;
+        const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
+        const int o = j * sw - b->off[i];
+        if (lpe >= nbi || o >= nbi) continue;
+        const int wj = (o + sw < nbi) ? sw : nbi - o;
+        const bool first = (lpb == 0) && !pre[i];
+        ts.add(i, lpb, nbi, b->n[i], o | (wj << 16), lpe - lpb, first ? 0 : 1, (nbi - o) * 2 * wj);
+        ts.any_first |= first;
+      }
+      if (ts.total > 0 && (rc = b_launch_trail(b, ts, strip_stream(j), slots, false))) return rc;
+    }
+    if (used2) any2 = true;
   }
   if (any2) {  // the caller continues on T
     CK(b, cudaEventRecord(b->evs[3 * (size_t)npanels], T2));
@@ -292,7 +251,6 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
 struct BInvProgress {
   short done[16][DGP_BATCH_MAX];
   cudaStream_t W;
-  int lag;
 };
 
 int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg) {
@@ -337,10 +295,9 @@ int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg) {
 }
 
 int b_eager(dgp_batch_t b, BInvProgress* ip, cudaEvent_t ev_panel, int pe) {
-  const int F = pe - ip->lag;
-  if (F < 2 || (F & 7) != 0) return 0;
+  if ((pe & 7) != 0) return 0;
   CK(b, cudaStreamWaitEvent(ip->W, ev_panel, 0));
-  return b_trtri_advance(b, *ip, F);
+  return b_trtri_advance(b, *ip, pe);
 }
 
 // the rest of the inverse, then z = U'r, alpha = U z
@@ -362,7 +319,7 @@ int b_lauum_grad(dgp_batch_t b, cudaStream_t W) {
   TabBuilder tb(b);
   for (int k = 0; k < b->G; k++) {
     const int i = b->order[k];
-    tb.add(i, 0, b->nb[i], b->n[i], 0, 0, 0, lauum_slots(b->nb[i], raster_on()));
+    tb.add(i, 0, b->nb[i], b->n[i], 0, 0, 0, lauum_slots(b->nb[i]));
   }
   GemmArgs g = b_args(b, M_LAUUM, b->A, 1.0, tb.total);
   int rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmU, b->tmU, g, W, false, &tb.t);
@@ -385,8 +342,9 @@ int b_enqueue(dgp_batch_t b) {
   CK(b, cudaGetLastError());
   BInvProgress ip;
   memset(&ip, 0, sizeof(ip));
-  ip.W = W; ip.lag = b->eager_lag;
-  if ((rc = b_potrf(b, (b->eager_inv && W != T) ? &ip : nullptr))) return rc;
+  ip.W = W;
+  // the merges of the inverse are released as the factorisation passes them at every size (unlike the single-site engine)
+  if ((rc = b_potrf(b, W != T ? &ip : nullptr))) return rc;
   if (b->timing) CK(b, cudaEventRecord(b->ev[1], T));
   if (W != T) {
     CK(b, cudaEventRecord(b->ev_lo[0], T));
@@ -459,28 +417,12 @@ int dgp_batch_create(dgp_batch* out, int device, int max_sites, int max_n, void*
     b->own_stream = true;
   }
   cudaStreamCreateWithPriority(&b->stream_lo, cudaStreamNonBlocking, lo);
-  const char* ei = getenv("DGP_EAGER_INV");
-  if (ei) b->eager_inv = atoi(ei) != 0;
-  const char* el = getenv("DGP_EAGER_LAG");
-  if (el && atoi(el) >= 0) b->eager_lag = atoi(el) / 8 * 8;
   cudaStreamCreateWithPriority(&b->stream_hi, cudaStreamNonBlocking, hi);
   {
     int pr = (lo + hi) / 2;
     if (cudaStreamGetPriority(b->stream, &pr) != cudaSuccess) { cudaGetLastError(); pr = (lo + hi) / 2; }
     cudaStreamCreateWithPriority(&b->stream_t2, cudaStreamNonBlocking, pr);
   }
-  const char* sbk = getenv("DGP_STRIP_BLOCKS");
-  if (sbk && atoi(sbk) >= 0 && atoi(sbk) <= 4096) b->strip_blocks = atoi(sbk);
-  const char* pd = getenv("DGP_PDL");
-  if (pd) b->pdl = atoi(pd) != 0;
-  const char* ch = getenv("DGP_CHAIN_HALF");
-  if (ch) b->chain_half = atoi(ch) != 0;
-  const char* pbk = getenv("DGP_PANEL_BLOCKS");
-  if (pbk && atoi(pbk) >= 1 && atoi(pbk) <= 64) b->panel_blocks = atoi(pbk);
-  const char* pg = getenv("DGP_PREGEN");
-  if (pg) b->pregen = atoi(pg) != 0;
-  const char* il = getenv("DGP_INPANEL_LEFT");
-  if (il) b->inpanel_left = atoi(il) != 0;
   const size_t np = b->max_pad, S = max_sites, nbm = np / 128;
   cudaError_t r = cudaSuccess;
   auto A = [&](double** p, size_t count) { if (r == cudaSuccess) r = cudaMalloc((void**)p, count * sizeof(double)); };
@@ -531,7 +473,7 @@ int dgp_batch_set_train(dgp_batch b, const dgp_spec* spec, int nsites, const int
   }
   b->ld = npmax;
   b->NB = npmax / 128;
-  const int pw = b->panel_blocks;
+  const int pw = PANEL_BLOCKS;
   memset(&b->sd, 0, sizeof(b->sd));
   b->sd.count = nsites; b->sd.nbmax = b->NB; b->sd.ld = b->ld;
   for (int i = 0; i < nsites; i++) {

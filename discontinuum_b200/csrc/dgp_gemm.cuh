@@ -10,7 +10,7 @@
 // The same kernel runs every O(n^3) phase of the marginal-likelihood evaluation; `mode` selects how a
 // tile index maps to operand panels (decode_job) and the template flags select what the tile starts from
 // (nothing / its old value / a generated covariance tile -- added in the epilogue, the accumulators always start at
-// zero) and the epilogue (store / fused W (.) dK/dtheta contraction / row sum of squares).
+// zero) and the epilogue (store / row sum of squares).
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -25,32 +25,31 @@ constexpr int A_BYTES = BM * BK * 8;   // 16 KB
 constexpr int B_BYTES = BN * BK * 8;   //  8 KB
 constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
 constexpr int GEMM_THREADS = 256;      // 2 warpgroups: 4 consumer warps | 1 producer warp + 3 warps that only give up their registers
-constexpr int WS = BN + 1;             // padded row stride of the W tile in the grad epilogue
+constexpr int WS = BN + 1;             // padded row stride of the W tile in the first-touch epilogue
 #ifndef DGP_COV_V
 #define DGP_COV_V 8
 #endif
 constexpr int COV_V = DGP_COV_V;       // covariance entries a thread evaluates side by side when it generates a tile
 
-enum { M_TRSM = 0, M_TRAIL = 1, M_TRAIL_COL = 2, M_INV_M = 3, M_LAUUM = 4, M_PREDVAR = 5, M_GENERIC = 6, M_INV_U = 7, M_ZL = 8 };
+enum { M_TRSM = 0, M_TRAIL_COL = 2, M_INV_M = 3, M_LAUUM = 4, M_PREDVAR = 5, M_GENERIC = 6, M_INV_U = 7, M_ZL = 8 };
 enum { INIT_ZERO = 0, INIT_LOAD = 1, INIT_COV = 2 };
-enum { EPI_STORE = 0, EPI_GRAD = 1, EPI_SUMSQ = 2 };
+enum { EPI_STORE = 0, EPI_SUMSQ = 2 };
 
 struct GemmArgs {
   int mode, step, nb, n;        // nb = npad / 128, n = valid points
   int ntiles, aux0, aux1, aux2; // mode dependent (M_PREDVAR: aux0 = row blocks of the chunk; M_GENERIC: see decode)
   double* C; long long ldc;     // in/out matrix of the tile
   double sign;                  // EPI_STORE: C = sign * acc  (INIT_LOAD loads sign * C)
-  const double* Xw;             // feature table [npad][DGP_XS]          (INIT_COV, EPI_GRAD)
+  const double* Xw;             // feature table [npad][DGP_XS]          (INIT_COV)
   const double* noise;          // fixed noise [npad]                    (INIT_COV)
-  const double* theta;          // natural parameters on device          (INIT_COV, EPI_GRAD)
-  const double* alpha;          // [npad]                                (EPI_GRAD)
-  double* part;                 // EPI_GRAD: [ntiles][DGP_MAX_THETA]; EPI_SUMSQ: [2 nb][rows]
-  double* Kinv;                 // optional dense Ky^-1 output (EPI_GRAD, debug), ld = ldc
+  const double* theta;          // natural parameters on device          (INIT_COV)
+  const void* reserved0_;       // unused (see reserved3_)
+  double* part;                 // EPI_SUMSQ: [2 nb][rows]
+  const void* reserved1_;       // unused (see reserved3_)
   double jitter;
   int latent;                   // INIT_COV: add only `jitter` on the diagonal (latent posterior covariance)
-  int raster;                   // M_LAUUM / M_INV_M / M_INV_U: tiles enumerated in 8 x 16 super-tiles (see decode_job)
-  int stagger_ns, stagger_lo;   // experiment (DGP_STAGGER_NS): CTAs [lo, 2 lo) of a launch start this many ns late
-  int gen_first_mod;            // INIT_COV: CTAs with (blockIdx / gen_first_mod) odd generate their tile BEFORE the main loop (0: none)
+  int reserved2_;               // unused (see reserved3_)
+  int reserved3_[3];            // unused: k_gemm spills more with a shorter GemmArgs (ptxas -v), so the layout stays fixed
 };
 
 // Batched launches (dgp_batch_*: several independent sites per launch).  A launch covers the tiles of up to
@@ -66,14 +65,14 @@ struct BatchTab {
   BatchEnt e[DGP_BATCH_MAX];
 };
 
-// tile slots of an M_LAUUM launch over nb block rows (raster order: 8-row bands of 8 x 16 cells, see decode_job)
-__host__ __device__ inline int lauum_slots(int nb, int raster) {
+// tile slots of an M_LAUUM launch over nb block rows (8-row bands of 8 x 16 cells, see decode_job)
+__host__ __device__ inline int lauum_slots(int nb) {
   const int B = (nb + 7) / 8;
-  return raster ? 64 * B * (B + 1) : nb * (nb + 1);
+  return 64 * B * (B + 1);
 }
 
 // the fields of GemmArgs that decode_job reads (per site in a batched launch)
-struct JobCtx { int mode, step, nb, aux0, aux1, aux2, raster; };
+struct JobCtx { int mode, step, nb, aux0, aux1, aux2; };
 
 struct Job {
   int rowA, kA, rowB, kB, nk;   // operand panel origins (elements) and number of 16-wide k steps
@@ -103,20 +102,9 @@ __device__ __forceinline__ Job decode_job(const JobCtx& g, int tile, int init_de
       j.nk = h ? 8 : 4;
       j.crow = i * 128; j.ccol = (g.aux0 ? 0 : s * 128) + h * 64;  // aux0 = 1: into a [rows][128] panel buffer
     } break;
-    case M_TRAIL: {  // A[i, c] -= L[i, K] L[c, K]^T, K = block columns [step, step + aux1); lower triangle of the
-                     // trailing matrix with origin block o = aux0: rows i = o + ip, 64-col blocks c = 2 o + cp <= row
-      const int o = g.aux0;
-      const int ip = (isqrt_floor(4 * tile + 1) - 1) >> 1;
-      const int cp = tile - ip * (ip + 1);
-      const int i = o + ip, c = 2 * o + cp;
-      j.rowA = i * 128; j.kA = s * 128;
-      j.rowB = c * 64; j.kB = s * 128;
-      j.nk = 8 * g.aux1;
-      j.crow = i * 128; j.ccol = c * 64;
-      j.init = g.aux2 ? INIT_LOAD : INIT_COV;  // aux2 = 0: first touch of these tiles, generate the covariance
-    } break;
-    case M_TRAIL_COL: {  // the same update on the block columns [o, o + w) only (w = ntiles-independent, in g.latent's
-                         // place: aux0 = o | (w << 16)): rows i >= o, tiles above the diagonal exit
+    case M_TRAIL_COL: {  // A[i, c] -= L[i, K] L[c, K]^T, K = block columns [step, step + aux1), on the block columns
+                         // [o, o + w) (aux0 = o | (w << 16)): rows i >= o, tiles above the diagonal exit.  aux2 = 0: first
+                         // touch of these tiles, generate the covariance
       const int o = g.aux0 & 0xffff, w2 = 2 * (g.aux0 >> 16);
       const int i = o + tile / w2, c = 2 * o + tile % w2;
       j.valid = c <= 2 * i + 1;
@@ -133,16 +121,13 @@ __device__ __forceinline__ Job decode_job(const JobCtx& g, int tile, int init_de
       const int hb = g.aux0, np_ = g.aux1;
       const int pr = tile % np_, w = tile / np_;
       const int o = (s + pr) * 2 * hb;
+      // L2-aware order: the hb x 2hb tiles of a pair in cells of R x 2R tiles (R = min(8, hb)), so that the CTAs resident
+      // together share R row panels and 2R column panels instead of one row panel and ~150 column panels
+      const int R = hb < 8 ? hb : 8, C2 = 2 * R, per = R * C2, cpr = hb / R;
+      const int cell = w / per, within = w % per;
       int jb, ic;
-      if (g.raster) {
-        // L2-aware order: the hb x 2hb tiles of a pair in cells of R x 2R tiles (R = min(8, hb)), so that the CTAs resident
-        // together share R row panels and 2R column panels instead of one row panel and ~150 column panels
-        const int R = hb < 8 ? hb : 8, C2 = 2 * R, per = R * C2, cpr = hb / R;
-        const int cell = w / per, within = w % per;
-        if (g.mode == M_INV_M) { jb = (cell / cpr) * R + within / C2; ic = (cell % cpr) * C2 + within % C2; }
-        else { jb = (cell % cpr) * R + within % R; ic = 2 * hb - 1 - ((cell / cpr) * C2 + within / R); }
-      } else if (g.mode == M_INV_M) { jb = w / (2 * hb); ic = w % (2 * hb); }
-      else { ic = 2 * hb - 1 - w / hb; jb = w % hb; }
+      if (g.mode == M_INV_M) { jb = (cell / cpr) * R + within / C2; ic = (cell % cpr) * C2 + within % C2; }
+      else { jb = (cell % cpr) * R + within % R; ic = 2 * hb - 1 - ((cell / cpr) * C2 + within / R); }
       const int cb64 = 2 * (o + hb) + ic;
       j.valid = cb64 < 2 * g.nb;
       j.rowA = (o + jb) * 128;
@@ -153,19 +138,13 @@ __device__ __forceinline__ Job decode_job(const JobCtx& g, int tile, int init_de
       j.crow = j.rowA; j.ccol = j.rowB;
     } break;
     case M_LAUUM: {  // Kinv[i, c] = sum_{k >= i} U[i, k] U[c, k]^T  (lower tiles, longest K first)
-      int i, c;
-      if (g.raster) {
-        // L2-aware order: bands of 8 block rows, inside a band cells of 8 x 16 tiles (band b has b + 1 cells, 64 b (b + 1)
-        // tile slots before it); slots beyond the triangle exit.  Grid = lauum_slots(nb).
-        const int ip = (isqrt_floor(4 * (tile >> 6) + 1) - 1) >> 1;
-        const int rem = tile - 64 * ip * (ip + 1);
-        i = ip * 8 + ((rem & 127) >> 4);
-        c = (rem >> 7) * 16 + (rem & 15);
-        j.valid = i < g.nb && c <= 2 * i + 1;
-      } else {
-        i = (isqrt_floor(4 * tile + 1) - 1) >> 1;
-        c = tile - i * (i + 1);
-      }
+      // L2-aware order: bands of 8 block rows, inside a band cells of 8 x 16 tiles (band b has b + 1 cells, 64 b (b + 1)
+      // tile slots before it); slots beyond the triangle exit.  Grid = lauum_slots(nb).
+      const int ip = (isqrt_floor(4 * (tile >> 6) + 1) - 1) >> 1;
+      const int rem = tile - 64 * ip * (ip + 1);
+      const int i = ip * 8 + ((rem & 127) >> 4);
+      const int c = (rem >> 7) * 16 + (rem & 15);
+      j.valid = i < g.nb && c <= 2 * i + 1;
       j.rowA = i * 128; j.kA = i * 128;
       j.rowB = c * 64; j.kB = i * 128;
       j.nk = (g.nb - i) * 8;
@@ -250,13 +229,6 @@ constexpr int SM_XS = STAGES * STAGE_BYTES;                 // 192 feature rows 
 constexpr int SM_COVC = SM_XS + (BM + BN) * DGP_XS * 8;     // CovC
 constexpr int SM_BAR = SM_COVC + ((sizeof(CovC) + 15) / 16) * 16;
 constexpr int SM_TOTAL = SM_BAR + 2 * STAGES * 8 + 1024;    // + alignment slack
-// grad epilogue carve-out inside the (then idle) stage ring
-constexpr int SMG_W = 0;                                    // W tile [128][WS]
-constexpr int SMG_XS = SMG_W + BM * WS * 8;                 // feature rows
-constexpr int SMG_AL = SMG_XS + (BM + BN) * DGP_XS * 8;     // alpha_i[128], alpha_j[64]
-constexpr int SMG_PART = SMG_AL + (BM + BN) * 8;            // [4 warps][8 terms][NSLOT] + noise[4]
-constexpr int SMG_END = SMG_PART + (4 * DGP_MAX_TERMS * NSLOT + 4) * 8;
-static_assert(SMG_END <= STAGES * STAGE_BYTES, "grad epilogue does not fit the stage ring");
 
 // MT = 8-row fragments per consumer warp along M: 8 -> the 128x64 tile; 4 -> 64x64 half tiles (blockIdx = 2 tile + half)
 // for the short launches of the panel chain, whose few tiles leave most SMs idle: twice the CTAs, half the DMMA time.
@@ -273,17 +245,15 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   int tile = MT == 8 ? blockIdx.x : (blockIdx.x >> 1);
-  JobCtx jc{g.mode, g.step, g.nb, g.aux0, g.aux1, g.aux2, g.raster};
-  int site = -1, npts = g.n;   // site >= 0: batched launch
-  double jitter = g.jitter;
+  JobCtx jc{g.mode, g.step, g.nb, g.aux0, g.aux1, g.aux2};
+  int site = -1;   // site >= 0: batched launch
   if (bt.count > 0) {
     int k = 0;
 #pragma unroll 1
     for (int i = 1; i < bt.count; i++) if (tile >= bt.e[i].tile0) k = i;
     const BatchEnt& e = bt.e[k];
-    tile -= e.tile0; site = e.site; npts = e.n;
+    tile -= e.tile0; site = e.site;
     jc.step = e.step; jc.nb = e.nb; jc.aux0 = e.aux0; jc.aux1 = e.aux1; jc.aux2 = e.aux2;
-    jitter = bt.jitv[site];
   }
   // slab offsets of this site (0 for a single-site launch)
   const size_t soff_m = site >= 0 ? (size_t)site * (size_t)bt.ld * (size_t)bt.ld : 0;  // matrices
@@ -294,11 +264,6 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 4); }
     fence_mbar_init();
-    if (g.stagger_ns > 0 && (int)blockIdx.x >= g.stagger_lo && (int)blockIdx.x < 2 * g.stagger_lo) {
-      unsigned long long t0, t1;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-      do { __nanosleep(256); asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1)); } while (t1 - t0 < (unsigned long long)g.stagger_ns);
-    }
   }
   __syncthreads();
   // dependent launch (panel chain): everything above overlapped the predecessor's tail; no global access before this
@@ -357,46 +322,6 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
     } else {
       asm volatile("prefetch.global.L2 [%0];" ::"l"(rowp + 256 * (t >> 6)));
       asm volatile("prefetch.global.L2 [%0];" ::"l"(rowp + 256 * (t >> 6) + 128));
-    }
-  }
-
-  // First-touch tiles come in two kinds (INIT_COV launches).  Generating the covariance tile is a long chain of FP64 ALU work
-  // that shares its datapath with the neighbour CTA's DMMAs; if both CTAs of an SM reach it at the same time the tensor pipe
-  // idles.  So every other wave-sized group of CTAs generates its tile FIRST -- row per thread, straight into the output tile
-  // in global memory (it stays in L2) -- and adds it back in the epilogue like an old tile, while the others generate in the
-  // epilogue: the two CTAs of an SM then tend to be in opposite phases.  Same operands, one rounding: bit-identical.
-  if constexpr (INIT == INIT_COV) {
-    if (job.init == INIT_COV && g.gen_first_mod > 0 && (((int)blockIdx.x / g.gen_first_mod) & 1)) {
-      const int t = threadIdx.x;
-      double* xaT = (double*)(smem + SM_XS);
-      double* xb = xaT + DGP_XS * BM;
-      const size_t soff_v = site >= 0 ? (size_t)site * (size_t)bt.ld : 0;
-      const double* Xw_s = g.Xw + soff_v * DGP_XS;
-      const double* noise_s = g.noise + soff_v;
-      cov_compile(cc, spec, g.theta + (site >= 0 ? site * DGP_MAX_THETA : 0), jitter, t, 128);
-      for (int e = t; e < BM * DGP_XS; e += 128) xaT[(e % DGP_XS) * BM + e / DGP_XS] = Xw_s[(size_t)job.crow * DGP_XS + e];
-      for (int e = t; e < BN * DGP_XS; e += 128) xb[e] = Xw_s[(size_t)job.ccol * DGP_XS + e];
-      consumer_bar();
-      const int gr = job.crow + t;
-      const double dn = (gr < npts) ? (g.latent ? jitter : noise_s[gr] + cc->extra_noise) : 0.0;
-      double* crow = g.C + soff_m + (size_t)gr * g.ldc + job.ccol;
-#pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += COV_V) {
-        double val[COV_V];
-        cov_vals<COV_V>(cc, xaT, BM, t, xb + c0 * DGP_XS, val);
-#pragma unroll
-        for (int v = 0; v < COV_V; v++) {
-          const int gc = job.ccol + c0 + v;
-          if (gr < npts && gc < npts) { if (gr == gc) val[v] += dn; }
-          else val[v] = (gr == gc) ? 1.0 : 0.0;
-        }
-#pragma unroll
-        for (int v = 0; v < COV_V; v += 2) {
-          double2 o; o.x = val[v]; o.y = val[v + 1];
-          *reinterpret_cast<double2*>(crow + c0 + v) = o;
-        }
-      }
-      consumer_bar();   // the tile is read back in the accumulator layout by other threads of this CTA
     }
   }
 
@@ -480,7 +405,7 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
     int bx = blockIdx.x, tx = threadIdx.x;
     asm volatile("" : "+r"(bx), "+r"(tx));
     int tile_e = MT == 8 ? bx : (bx >> 1);
-    JobCtx je{g.mode, g.step, g.nb, g.aux0, g.aux1, g.aux2, g.raster};
+    JobCtx je{g.mode, g.step, g.nb, g.aux0, g.aux1, g.aux2};
     size_t soff_e = 0;
     int site_e = -1, npts_e = g.n;
     if (bt.count > 0) {
@@ -496,11 +421,8 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
     const int crow_e = jo.crow + (MT == 4 ? 64 * (bx & 1) : 0);
     const int lane_e = tx & 31, warp_e = tx >> 5;
     const int g8e = lane_e >> 2, qe = lane_e & 3, wme = warp_e >> 1, wne = warp_e & 1;
-    bool gen = false, gen_done = false;   // gen_done: this CTA generated its tile before the main loop (see there)
-    if constexpr (INIT == INIT_COV) {
-      gen_done = jo.init == INIT_COV && g.gen_first_mod > 0 && ((bx / g.gen_first_mod) & 1);
-      gen = (jo.init == INIT_COV) && !gen_done;
-    }
+    bool gen = false;
+    if constexpr (INIT == INIT_COV) gen = jo.init == INIT_COV;
     if (gen) {
       if constexpr (INIT == INIT_COV) {
         // First touch of the tile: out = K + sign * sum.  The accumulators are parked in the (now idle) operand ring as a
@@ -556,7 +478,7 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
         }
       }
     } else {
-      const bool ldc = ((INIT == INIT_LOAD || INIT == INIT_COV) && jo.init == INIT_LOAD) || gen_done;
+      const bool ldc = (INIT == INIT_LOAD || INIT == INIT_COV) && jo.init == INIT_LOAD;
 #pragma unroll
       for (int mi = 0; mi < MT; mi++) {
         double* crow = g.C + soff_e + (size_t)(crow_e + WROWS * wme + 8 * mi + g8e) * g.ldc + jo.ccol + 32 * wne + 2 * qe;
@@ -606,79 +528,6 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
         const int lr = 64 * wm + 8 * mi + g8;
         g.part[(size_t)cb * g.aux1 + job.crow + lr] = rs[mi] + red[lr];
       }
-    }
-  } else {  // EPI_GRAD: W = alpha_i alpha_j' - Kinv, contracted with regenerated dK/dtheta tiles
-    consumer_bar();  // every warp is done reading the ring
-    double* W = (double*)(smem + SM_STAGES + SMG_W);
-    double* xs = (double*)(smem + SM_STAGES + SMG_XS);
-    double* al = (double*)(smem + SM_STAGES + SMG_AL);
-    double* part = (double*)(smem + SM_STAGES + SMG_PART);
-    const int t = threadIdx.x;
-#pragma unroll
-    for (int mi = 0; mi < 8; mi++) {
-      const int lr = 64 * wm + 8 * mi + g8;
-#pragma unroll
-      for (int ni = 0; ni < 4; ni++) {
-        const int lc = 32 * wn + 8 * ni + 2 * q;
-        W[lr * WS + lc] = acc[mi][ni][0];
-        W[lr * WS + lc + 1] = acc[mi][ni][1];
-        if (g.Kinv != nullptr) {
-          double2 v; v.x = acc[mi][ni][0]; v.y = acc[mi][ni][1];
-          *reinterpret_cast<double2*>(g.Kinv + (size_t)(job.crow + lr) * g.ldc + job.ccol + lc) = v;
-        }
-      }
-    }
-    cov_compile(cc, spec, g.theta, 0.0, t, 128);
-    double* xaT = xs;                 // [DGP_XS][128] row-point features, column-major
-    double* xb = xs + DGP_XS * BM;    // [64][DGP_XS]  column-point features
-    for (int e = t; e < BM * DGP_XS; e += 128) xaT[(e % DGP_XS) * BM + e / DGP_XS] = g.Xw[(size_t)job.crow * DGP_XS + e];
-    for (int e = t; e < BN * DGP_XS; e += 128) xb[e] = g.Xw[(size_t)job.ccol * DGP_XS + e];
-    for (int e = t; e < BM + BN; e += 128) al[e] = g.alpha[(e < BM) ? job.crow + e : job.ccol + (e - BM)];
-    consumer_bar();
-
-    // thread t owns row t of the tile; 4 columns side by side (term_grad_accum_v<4>)
-    const int grow = job.crow + t;
-    const double ai = al[t];
-    double trw = 0.0;
-    for (int term = 0; term < cc->nterms; term++) {
-      double sl[NSLOT];
-#pragma unroll
-      for (int k = 0; k < NSLOT; k++) sl[k] = 0.0;
-      const TermC& tc = cc->t[term];
-#pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += 4) {
-        if (grow >= g.n || job.ccol + c0 > grow) continue;  // padding rows / strictly above the diagonal
-        double w[4];
-#pragma unroll
-        for (int v = 0; v < 4; v++) {
-          const int c = c0 + v, gcol = job.ccol + c;
-          const double wgt = (gcol < grow) ? 2.0 : (gcol == grow ? 1.0 : 0.0);
-          w[v] = wgt * (ai * al[BM + c] - W[t * WS + c]);
-          if (term == 0 && gcol == grow) trw += w[v];
-        }
-        term_grad_accum_v<4>(tc, xaT, BM, t, xb + c0 * DGP_XS, w, sl);
-      }
-#pragma unroll
-      for (int k = 0; k < NSLOT; k++) {
-        double v = sl[k];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == 0) part[(warp * DGP_MAX_TERMS + term) * NSLOT + k] = v;
-      }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) trw += __shfl_xor_sync(0xffffffffu, trw, o);
-    if (lane == 0) part[4 * DGP_MAX_TERMS * NSLOT + warp] = trw;
-    consumer_bar();
-    if (t < cc->ntheta) {
-      double s = 0.0;
-      for (int term = 0; term < cc->nterms; term++)
-        for (int k = 0; k < NSLOT; k++)
-          if (term_slot_theta(cc->t[term], k) == t)
-            for (int w4 = 0; w4 < 4; w4++) s += part[(w4 * DGP_MAX_TERMS + term) * NSLOT + k];
-      if (t == cc->noise_idx)
-        for (int w4 = 0; w4 < 4; w4++) s += part[4 * DGP_MAX_TERMS * NSLOT + w4];
-      g.part[(size_t)blockIdx.x * DGP_MAX_THETA + t] = -0.5 * s;
     }
   }
 }

@@ -134,11 +134,11 @@ k_cov_rect(const __grid_constant__ dgp_spec spec, const double* __restrict__ the
 }
 
 // Matrices of more than this many block columns are written by the standalone generator ahead of the factorisation
-// (both engines, whatever the stream layout: which kernel generates a tile decides how its first update rounds).
+// (both engines: which kernel generates a tile decides how its first update rounds).
 constexpr int DGP_PREGEN_MIN_NB = 8;
 
 // lower-triangle blocks of block columns [ob, ob + gridDim.y) of the work matrix (noise on the diagonal, identity padding),
-// rows from block ob down: grid = (4 (nb - ob), width).  The standalone generator of the pre-generation schedule (DGP_PREGEN).
+// rows from block ob down: grid = (4 (nb - ob), width).  The standalone generator of the pre-generation schedule.
 __global__ void __launch_bounds__(256)
 k_cov_lower(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta, const double* __restrict__ Xw,
             const double* __restrict__ noise, double jitter, double* __restrict__ A, long long ld, int n, int ob) {
@@ -170,164 +170,6 @@ k_cov_lower_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ Sit
   const size_t v = (size_t)st * sd.ld;
   cov_rect_body(spec, theta + st * DGP_MAX_THETA, Xw + v * DGP_XS, Xw + v * DGP_XS, noise + v, jitv[st], A + v * sd.ld, sd.ld,
                 sd.n[st], sd.n[st], 1, 1, nullptr, nullptr, 0, blockIdx.x, col);
-}
-
-// ------------------------------------------------------------------ diagonal block: L, L^-1, L^-T
-// One CTA factors the 128x128 diagonal block A_ss = L L^T and, by running the same right-looking
-// elimination on the identity ("augmented rows"), obtains Y = L^-T: rows of Y are forward-substituted
-// exactly like the rows below the diagonal block.  L lives in the lower triangle of As, Y in its strict
-// upper triangle, diag(Y) = 1 / diag(L) in rd.  Outputs: L -> Lblk (zeros above the diagonal),
-// Y -> Ublk (upper), Y^T = L^-1 -> DIblk (lower).  logdet += sum log L_ii; first bad pivot -> info.
-constexpr int PF_THREADS = 256;
-constexpr int PF_AS = 129;  // row stride of As
-constexpr int PF_PN = 33;   // row stride of the 32-column panel scratch
-constexpr int PF_SMEM = (128 * PF_AS + 256 * PF_PN + 128 + 64) * 8;
-
-template <int REM>
-__device__ __forceinline__ void potf2_trailing(double* As, const double* Pn, int o, int tid) {
-  constexpr int NC = REM / 8;  // columns per thread
-  const int rg = tid >> 3, cg = tid & 7;
-  double acc[4][NC];
-#pragma unroll
-  for (int a = 0; a < 4; a++)
-#pragma unroll
-    for (int b = 0; b < NC; b++) acc[a][b] = 0.0;
-  int vrow[4];
-#pragma unroll
-  for (int a = 0; a < 4; a++) {
-    const int row = rg + 32 * a;
-    vrow[a] = (row < o + 32) ? 128 + row : row;
-  }
-#pragma unroll 4
-  for (int k = 0; k < 32; k++) {
-    double rv[4], cv[NC];
-#pragma unroll
-    for (int a = 0; a < 4; a++) rv[a] = Pn[vrow[a] * PF_PN + k];
-#pragma unroll
-    for (int b = 0; b < NC; b++) cv[b] = Pn[(o + 32 + cg + 8 * b) * PF_PN + k];
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-      for (int b = 0; b < NC; b++) acc[a][b] = fma(rv[a], cv[b], acc[a][b]);
-  }
-#pragma unroll
-  for (int a = 0; a < 4; a++) {
-    const int row = rg + 32 * a;
-#pragma unroll
-    for (int b = 0; b < NC; b++) {
-      const int j = o + 32 + cg + 8 * b;
-      if (row < o + 32 || j <= row) As[row * PF_AS + j] -= acc[a][b];
-    }
-  }
-}
-
-// Tblk (optional, may alias Ablk: the block is fully staged in shared memory before anything is written) receives
-// L^-1 as a full 128x128 block (zeros above the diagonal): the diagonal block of T for the recursive inverse.
-__global__ void __launch_bounds__(PF_THREADS, 1)
-k_potf2(const double* Ablk, double* __restrict__ Lblk, double* __restrict__ Ublk, long long ld,
-        double* __restrict__ DIblk, double* __restrict__ scal, int base, double* Tblk) {
-  extern __shared__ double pf_smem[];
-  double* As = pf_smem;
-  double* Pn = As + 128 * PF_AS;
-  double* rd = Pn + 256 * PF_PN;
-  double* cb = rd + 128;  // [2][32] column exchange buffer of the diagonal sub-block
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-
-#pragma unroll 1
-  for (int e0 = 0; e0 < 128 * 128; e0 += PF_THREADS * 16) {  // 16 independent loads in flight per thread
-    double v[16];
-#pragma unroll
-    for (int u = 0; u < 16; u++) {
-      const int e = e0 + u * PF_THREADS + tid, r = e >> 7, c = e & 127;
-      v[u] = (c <= r) ? Ablk[(size_t)r * ld + c] : 0.0;
-    }
-#pragma unroll
-    for (int u = 0; u < 16; u++) {
-      const int e = e0 + u * PF_THREADS + tid, r = e >> 7, c = e & 127;
-      As[r * PF_AS + c] = v[u];
-    }
-  }
-  __syncthreads();
-
-  for (int kb = 0; kb < 4; kb++) {
-    const int o = 32 * kb;
-    // (1) 32x32 diagonal sub-block, one warp, lane = row, the row in registers.  Column c is exchanged through a
-    // double-buffered shared vector (one STS + broadcast LDS.128 per lane instead of 31 - c register shuffles):
-    //   a[c2] -= a[c] * A[c2][c] / d,  L[r][c] = a[c] / sqrt(d)
-    if (warp == 0) {
-      double a[32];
-#pragma unroll
-      for (int c = 0; c < 32; c++) a[c] = As[(o + lane) * PF_AS + o + c];
-      double myinv = 0.0;
-#pragma unroll
-      for (int c = 0; c < 32; c++) {
-        double* cbuf = cb + (c & 1) * 32;
-        cbuf[lane] = a[c];
-        __syncwarp();
-        const double d = cbuf[c];
-        if (!(d > 0.0) && lane == 0 && scal[SC_INFO] == 0.0) scal[SC_INFO] = (double)(base + o + c + 1);
-        const double inv = rsqrt(d);  // one MUFU + Newton chain instead of sqrt followed by a division
-        const double tfac = a[c] * inv * inv;
-#pragma unroll
-        for (int c2 = c + 1; c2 < 32; c2++) a[c2] = fma(-tfac, cbuf[c2], a[c2]);
-        a[c] = (lane == c) ? d * inv : a[c] * inv;
-        if (lane == c) myinv = inv;
-      }
-#pragma unroll
-      for (int c = 0; c < 32; c++)
-        if (c <= lane) As[(o + lane) * PF_AS + o + c] = a[c];
-      rd[o + lane] = myinv;
-    }
-    __syncthreads();
-    // (2) forward substitution of the 32-column panel: thread t owns row t, which is either a row of A
-    // below the diagonal block (t >= o + 32) or a row of Y = L^-T (t < o + 32)
-    if (tid < 128) {
-      const int t = tid;
-      double x[32];
-      if (t >= o + 32 || t < o) {
-#pragma unroll
-        for (int c = 0; c < 32; c++) x[c] = As[t * PF_AS + o + c];
-      } else {
-#pragma unroll
-        for (int c = 0; c < 32; c++) x[c] = (c == t - o) ? 1.0 : 0.0;
-      }
-#pragma unroll
-      for (int c = 0; c < 32; c++) {
-        x[c] *= rd[o + c];
-#pragma unroll
-        for (int c2 = c + 1; c2 < 32; c2++) x[c2] = fma(-x[c], As[(o + c2) * PF_AS + o + c], x[c2]);
-      }
-      const int v = (t >= o + 32) ? t : 128 + t;
-#pragma unroll
-      for (int c = 0; c < 32; c++) {
-        Pn[v * PF_PN + c] = x[c];
-        if (t >= o + 32 || o + c > t) As[t * PF_AS + o + c] = x[c];
-      }
-    }
-    __syncthreads();
-    // (3) rank-32 update of the remaining columns, rows of A (lower part) and rows of Y alike
-    if (kb == 0) potf2_trailing<96>(As, Pn, o, tid);
-    else if (kb == 1) potf2_trailing<64>(As, Pn, o, tid);
-    else if (kb == 2) potf2_trailing<32>(As, Pn, o, tid);
-    __syncthreads();
-  }
-
-  for (int e = tid; e < 128 * 128; e += PF_THREADS) {
-    const int r = e >> 7, c = e & 127;
-    const double lv = As[r * PF_AS + c];
-    Lblk[(size_t)r * ld + c] = (c <= r) ? lv : 0.0;
-    if (Ublk != nullptr) Ublk[(size_t)r * ld + c] = (c > r) ? lv : (c == r ? rd[r] : 0.0);
-    const double tv = (c < r) ? As[c * PF_AS + r] : (c == r ? rd[r] : 0.0);
-    DIblk[r * 128 + c] = tv;
-    if (Tblk != nullptr) Tblk[(size_t)r * ld + c] = tv;
-  }
-  if (warp == 0) {
-    double s = 0.0;
-    for (int i = lane; i < 128; i += 32) s += log(As[i * PF_AS + i]);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) scal[SC_LOGDET] += s;
-  }
 }
 
 // ------------------------------------------------------------------ forward substitution step

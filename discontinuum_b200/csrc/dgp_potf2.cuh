@@ -200,9 +200,11 @@ __device__ __forceinline__ void p2_st_prog(int* prog, int v) {
 
 #define P2_BARH(nh) asm volatile("bar.sync 1, %0;" ::"r"((nh) * 32) : "memory")
 
-// Same contract as k_potf2 (dgp_panel.cuh): Lblk <- L, Ublk <- L^-T (upper, optional), DIblk <- L^-1 ([128][128]
-// contiguous, optional), Tblk <- L^-1 (optional, leading dimension ld; may alias Ablk: the block is staged in shared
-// memory before anything is written), scal[SC_LOGDET] += sum log L_ii, first bad pivot -> scal[SC_INFO].
+// Factors the 128x128 diagonal block A_ss = L L^T (lower triangle of Ablk, leading dimension ld) and produces its inverses
+// in the same CTA: Lblk <- L (zeros above the diagonal), Ublk <- L^-T (upper, optional), DIblk <- L^-1 ([128][128]
+// contiguous, optional), Tblk <- L^-1 as a full block with zeros above the diagonal (optional, leading dimension ld: the
+// diagonal block of T for the recursive inverse; may alias Ablk: the block is staged in shared memory before anything is
+// written), scal[SC_LOGDET] += sum log L_ii, first bad pivot -> scal[SC_INFO].
 // zero_lu = 0: the 32x32 sub-blocks above the diagonal of Lblk / below the diagonal of Ublk are known to be zero already.
 //
 // Warp roles in phase A of step k: warp 0 pivots; warps 1..3-k follow with the rows of the sub-blocks below and warp 5

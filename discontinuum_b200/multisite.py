@@ -310,7 +310,7 @@ class _GroupRun:
 def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int = 0, group: int = 16,
                     predict: Optional[Dict[int, np.ndarray]] = None, lr: float = 0.05, scheduler: bool = True,
                     patience: int = 60, model="loadest", stats: Optional[dict] = None, concurrency: Optional[int] = None,
-                    partitions: Optional[int] = None, lanes: int = 2) -> Dict[int, dict]:
+                    lanes: int = 2) -> Dict[int, dict]:
     """Fit one GP per site on this rank.  sites: {index: (X, y[, noise])} in model space; model: "loadest", "rating" or a
     kind object (see LoadestKind).  Returns {index: {"theta", "objective", "history", "failed", "n", "mu", "var",
     "var_latent"}} ("var" follows `likelihood(model(x))` like MarginalB200.predict).
@@ -324,10 +324,10 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
     `lanes`: every site sees the same sequence of evaluations.  Evaluations that fail (info != 0 or a non-finite value) climb
     psd_safe_cholesky's jitter ladder per site; a site whose objective stays bad for more than 10 consecutive iterations is
     marked failed, as MarginalB200.fit gives up.
-    `concurrency` / `partitions` select the round-1 per-handle pipelines instead (fit_sites_local_per_handle)."""
-    if concurrency is not None or partitions is not None:
+    `concurrency` selects the round-1 per-handle pipelines instead (fit_sites_local_per_handle)."""
+    if concurrency is not None:
         return fit_sites_local_per_handle(sites, iterations=iterations, device=device, concurrency=concurrency or 4,
-                                          predict=predict, lr=lr, scheduler=scheduler, patience=patience, partitions=partitions)
+                                          predict=predict, lr=lr, scheduler=scheduler, patience=patience)
     kind = _kind(model)
     t_start = time.perf_counter()
     st = {"groups": 0, "evals": 0, "gpu_eval_ms": 0.0, "fit_wall_s": 0.0, "predict_s": 0.0, "host_step_s": 0.0, "retries": 0,
@@ -471,8 +471,7 @@ def _finish_step(s: _SiteState):
 _COMPLETION_ORDER = True  # serve sites as their evaluations finish (False: fixed round, blocking on each in turn)
 
 
-def _open_site(idx, tup, device, lr, scheduler, patience, pool: Optional[List[capi.Engine]] = None,
-               free_parts: Optional[List[int]] = None) -> _SiteState:
+def _open_site(idx, tup, device, lr, scheduler, patience, pool: Optional[List[capi.Engine]] = None) -> _SiteState:
     X, y = np.ascontiguousarray(tup[0], dtype=np.float64), np.ascontiguousarray(tup[1], dtype=np.float64)
     noise = np.ascontiguousarray(tup[2], dtype=np.float64) if len(tup) > 2 else np.full(y.shape[0], LOADEST_FIXED_NOISE)
     module = GPModule(loadest_spec(X.shape[1]))
@@ -482,16 +481,7 @@ def _open_site(idx, tup, device, lr, scheduler, patience, pool: Optional[List[ca
         if k is not None:
             eng = pool.pop(k)
     if eng is None:
-        if free_parts is not None:  # one engine per SM partition: take a free partition, or rebuild a pooled engine's
-            if not free_parts:
-                old = pool.pop(0)
-                free_parts.append(old.partition)
-                old.close()
-            part = free_parts.pop(0)
-            eng = capi.Engine(max_n=X.shape[0], max_m=2048, device=device, partition=part)
-            eng.partition = part
-        else:
-            eng = capi.Engine(max_n=X.shape[0], max_m=2048, device=device)
+        eng = capi.Engine(max_n=X.shape[0], max_m=2048, device=device)
     eng.set_train(module.spec.to_c(), X, y, noise)
     opt = torch.optim.Adam(module.raw_list(), lr=lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-4, fused=True)
     sch = None
@@ -532,23 +522,18 @@ def _close_site(s: _SiteState, predict, pool: Optional[List[capi.Engine]] = None
 
 def fit_sites_local_per_handle(sites: Dict[int, tuple], iterations: int = 100, device: int = 0, concurrency: int = 4,
                                predict: Optional[Dict[int, np.ndarray]] = None, lr: float = 0.05, scheduler: bool = True,
-                               patience: int = 60, partitions: Optional[int] = None) -> Dict[int, dict]:
+                               patience: int = 60) -> Dict[int, dict]:
     """Round-1 driver, kept for comparison and as the reference of the bit-identity tests: `concurrency` loadest sites in
     flight, each a pipeline of its own on its own libdgp handle and streams (dgp_nlml_grad_launch / _ready / _wait), served
-    in completion order; optional SM partitions (`capi.partition_device`, one site per partition)."""
+    in completion order."""
     results: Dict[int, dict] = {}
     queue = sorted(sites, key=lambda i: -sites[i][0].shape[0])  # largest first: later sites fit the pooled workspaces
     active: List[_SiteState] = []
     pool: List[capi.Engine] = []
-    free_parts: Optional[List[int]] = None
-    if partitions and partitions > 1:
-        nparts, _ = capi.partition_device(device, partitions)
-        concurrency = nparts
-        free_parts = list(range(nparts))
 
     def refill():
         while queue and len(active) < max(1, concurrency):
-            s = _open_site(queue[0], sites[queue.pop(0)], device, lr, scheduler, patience, pool, free_parts)
+            s = _open_site(queue[0], sites[queue.pop(0)], device, lr, scheduler, patience, pool)
             if iterations > 0:
                 _launch_step(s)
             active.append(s)

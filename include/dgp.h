@@ -98,17 +98,6 @@ typedef struct dgp_handle_s* dgp_handle;
  * let the handle create its own non-blocking stream. */
 int dgp_create(dgp_handle* out, int device, int max_n, int max_m, void* stream);
 
-/* SM partitions for concurrent, independent sites (the B200 stand-in for the reference's one-Lambda-worker-per-site
- * map, examples/nwqn-loadest-example/nwqn-loadest-example.py:156-157).  Evaluations of different sites sharing all
- * SMs get in each other's way: the short, strictly dependent kernels of one site's panel chain queue behind the
- * long tiles of another site's inverse (no preemption), and every site slows down 3-4x.  dgp_partition_device splits
- * the device's SMs into `parts` disjoint green contexts (CUDA driver API; partition sizes are multiples of 8 SMs);
- * dgp_create_partitioned creates an engine whose streams belong to partition `part`, so that its kernels only
- * ever run there.  Returns the number of partitions available (>= 1; idempotent for the same `parts`), or < 0.
- * sms_out (optional): SMs per partition. */
-int dgp_partition_device(int device, int parts, int* sms_out);
-int dgp_create_partitioned(dgp_handle* out, int device, int max_n, int max_m, int part);
-
 int dgp_destroy(dgp_handle h);
 const char* dgp_last_error(dgp_handle h); /* h may be NULL: error of a failed dgp_create */
 int dgp_abi_version(void);

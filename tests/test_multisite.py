@@ -203,19 +203,6 @@ def test_rating_gauges_through_the_batch_driver(cuda_device):
 
 
 @pytest.mark.gpu
-def test_sites_on_sm_partitions_match_shared_gpu(cuda_device):
-    from discontinuum_b200 import synthetic
-
-    sites = {i: synthetic.loadest_site(n, 1100 + i)[:2] for i, n in enumerate((500, 260, 380, 640))}
-    shared = multisite.fit_sites_local_per_handle(sites, iterations=6, concurrency=2)
-    split = multisite.fit_sites_local_per_handle(sites, iterations=6, partitions=2)
-    for i in sites:
-        assert split[i]["failed"] is None
-        assert np.max(np.abs(np.array(split[i]["history"]) - np.array(shared[i]["history"]))) <= 1e-9
-        assert np.max(np.abs(split[i]["theta"] - shared[i]["theta"])) <= 1e-9
-
-
-@pytest.mark.gpu
 def test_sample_sharded_single_rank_matches_engine_sample(cuda_device):
     """world = 1: the panel-by-panel distributed schedule reproduces dgp_sample (same Philox normals)."""
     import helpers as H

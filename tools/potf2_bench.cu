@@ -1,6 +1,7 @@
-// Micro-benchmark / self-check of the diagonal-block kernels (development aid): k_potf2 vs k_potf2_v2 on one random SPD
-// 128x128 block: max differences of L, L^-1, L^-T, event timing of 200 back-to-back launches and, with -DP2_TIMING,
-// the clock64 stamps of the phases of k_potf2_v2.
+// Micro-benchmark / self-check of the diagonal-block kernel (development aid): k_potf2_v2 on one random SPD 128x128
+// block: event timing of 200 back-to-back launches, the residuals max |L L' - A| and max |T L - I| (T = L^-1) and the
+// agreement of U with T' (and, with P2_FULL set, of the contiguous copy DI with T), and, with -DP2_TIMING, the clock64
+// stamps of its phases.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -DP2_TIMING -o tools/potf2_bench tools/potf2_bench.cu
 #include <cstdio>
 #include <cstdlib>
@@ -17,6 +18,7 @@ using namespace dgp;
 
 int main() {
   const int ld = 256;
+  const bool full = getenv("P2_FULL") != nullptr;
   std::vector<double> A(128 * ld, 0.0), G(128 * 128);
   srand(1);
   for (auto& g : G) g = rand() / (double)RAND_MAX - 0.5;
@@ -28,45 +30,39 @@ int main() {
       A[j * ld + i] = 777.0;  // garbage above the diagonal must be ignored
       if (i == j) A[i * ld + j] = s;
     }
-  double *dA, *dL[2], *dU[2], *dDI[2], *dT[2], *scal;
+  double *dA, *dL, *dU, *dDI, *dT, *scal;
   cudaMalloc(&dA, 128 * ld * 8); cudaMalloc(&scal, 64 * 8);
-  for (int v = 0; v < 2; v++) { cudaMalloc(&dL[v], 128 * ld * 8); cudaMalloc(&dU[v], 128 * ld * 8); cudaMalloc(&dDI[v], 128 * 128 * 8); cudaMalloc(&dT[v], 128 * ld * 8);
-    cudaMemset(dL[v], 0xff, 128 * ld * 8); cudaMemset(dU[v], 0xff, 128 * ld * 8); cudaMemset(dT[v], 0xff, 128 * ld * 8); }
+  cudaMalloc(&dL, 128 * ld * 8); cudaMalloc(&dU, 128 * ld * 8); cudaMalloc(&dDI, 128 * 128 * 8); cudaMalloc(&dT, 128 * ld * 8);
+  cudaMemset(dL, 0xff, 128 * ld * 8); cudaMemset(dU, 0xff, 128 * ld * 8); cudaMemset(dT, 0xff, 128 * ld * 8);
   cudaMemcpy(dA, A.data(), 128 * ld * 8, cudaMemcpyHostToDevice);
   cudaMemset(scal, 0, 64 * 8);
-  cudaFuncSetAttribute(k_potf2, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM);
   cudaFuncSetAttribute(k_potf2_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM);
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
-  for (int v = 0; v < 2; v++) {
-    for (int rep = 0; rep < 2; rep++) {
-      const int iters = rep ? 200 : 3;
-      cudaEventRecord(e0);
-      for (int it = 0; it < iters; it++) {
-        if (v == 0) k_potf2<<<1, PF_THREADS, PF_SMEM>>>(dA, dL[v], dU[v], ld, dDI[v], scal, 0, dT[v]);
-        else k_potf2_v2<<<1, P2_THREADS, P2_SMEM>>>(dA, dL[v], dU[v], ld, getenv("P2_FULL") ? dDI[v] : nullptr, scal, 0, dT[v], getenv("P2_FULL") ? 1 : 0, P2Batch{});
-      }
-      cudaEventRecord(e1); cudaEventSynchronize(e1);
-      float ms; cudaEventElapsedTime(&ms, e0, e1);
-      if (rep) printf("v%d: %.2f us per launch (%s)\n", v + 1, ms * 1e3 / iters, cudaGetErrorString(cudaGetLastError()));
-    }
+  for (int rep = 0; rep < 2; rep++) {
+    const int iters = rep ? 200 : 3;
+    cudaEventRecord(e0);
+    for (int it = 0; it < iters; it++)
+      k_potf2_v2<<<1, P2_THREADS, P2_SMEM>>>(dA, dL, dU, ld, full ? dDI : nullptr, scal, 0, dT, 1, P2Batch{});
+    cudaEventRecord(e1); cudaEventSynchronize(e1);
+    float ms; cudaEventElapsedTime(&ms, e0, e1);
+    if (rep) printf("k_potf2_v2: %.2f us per launch (%s)\n", ms * 1e3 / iters, cudaGetErrorString(cudaGetLastError()));
   }
-  std::vector<double> L[2], U[2], DI[2], T[2];
-  for (int v = 0; v < 2; v++) {
-    L[v].resize(128 * ld); U[v].resize(128 * ld); DI[v].resize(128 * 128); T[v].resize(128 * ld);
-    cudaMemcpy(L[v].data(), dL[v], 128 * ld * 8, cudaMemcpyDeviceToHost);
-    cudaMemcpy(U[v].data(), dU[v], 128 * ld * 8, cudaMemcpyDeviceToHost);
-    cudaMemcpy(DI[v].data(), dDI[v], 128 * 128 * 8, cudaMemcpyDeviceToHost);
-    cudaMemcpy(T[v].data(), dT[v], 128 * ld * 8, cudaMemcpyDeviceToHost);
-  }
-  double dl = 0, du = 0, dd = 0, dt = 0;
+  std::vector<double> L(128 * ld), U(128 * ld), DI(128 * 128), T(128 * ld);
+  cudaMemcpy(L.data(), dL, 128 * ld * 8, cudaMemcpyDeviceToHost);
+  cudaMemcpy(U.data(), dU, 128 * ld * 8, cudaMemcpyDeviceToHost);
+  cudaMemcpy(DI.data(), dDI, 128 * 128 * 8, cudaMemcpyDeviceToHost);
+  cudaMemcpy(T.data(), dT, 128 * ld * 8, cudaMemcpyDeviceToHost);
+  double ra = 0, rt = 0, du = 0, dd = 0;
   for (int i = 0; i < 128; i++)
     for (int j = 0; j < 128; j++) {
-      dl = fmax(dl, fabs(L[0][i * ld + j] - L[1][i * ld + j]));
-      du = fmax(du, fabs(U[0][i * ld + j] - U[1][i * ld + j]));
-      dt = fmax(dt, fabs(T[0][i * ld + j] - T[1][i * ld + j]));
-      dd = fmax(dd, fabs(DI[0][i * 128 + j] - DI[1][i * 128 + j]));
+      double llt = 0, tl = 0;
+      for (int k = 0; k < 128; k++) { llt += L[i * ld + k] * L[j * ld + k]; tl += T[i * ld + k] * L[k * ld + j]; }
+      if (j <= i) ra = fmax(ra, fabs(llt - A[i * ld + j]));
+      rt = fmax(rt, fabs(tl - (i == j ? 1.0 : 0.0)));
+      du = fmax(du, fabs(U[i * ld + j] - T[j * ld + i]));
+      if (full) dd = fmax(dd, fabs(DI[i * 128 + j] - T[i * ld + j]));
     }
-  printf("max |v1 - v2|: L %.3e  U %.3e  DI %.3e  T %.3e\n", dl, du, dd, dt);
+  printf("max |L L' - A| %.3e  |T L - I| %.3e  |U - T'| %.3e  |DI - T| %.3e\n", ra, rt, du, dd);
 #ifdef P2_TIMING
   long long ts[64];
   cudaMemcpyFromSymbol(ts, p2_ts, sizeof(ts));

@@ -17,8 +17,7 @@ for s, n in enumerate(ns):
     sites[s] = (X, y, noise)
     grids[s] = synthetic.daily_grid(X, m)
 t0 = time.perf_counter()
-parts = int(os.environ.get("PARTS", "0")) or None
-res = multisite.fit_sites_local(sites, iterations=iters, device=0, concurrency=conc, predict=grids, partitions=parts)
+res = multisite.fit_sites_local(sites, iterations=iters, device=0, concurrency=conc, predict=grids)
 dt = time.perf_counter() - t0
 flop = sum(float(n) ** 3 * iters for n in ns)
 print(f"sites={S} iters={iters} conc={conc} m={m} n=[{ns.min()}..{ns.max()}] wall={dt:.2f}s sites/s={S/dt:.3f} "
@@ -40,7 +39,7 @@ if os.environ.get("PHASES"):
         a[0] += 1; a[1] += ms[0]; a[2] += ms[1]; a[3] += ms[2]
     multisite._finish_step = f1
     t0 = time.perf_counter()
-    multisite.fit_sites_local(sites, iterations=iters, device=0, concurrency=conc, predict=grids, partitions=parts)
+    multisite.fit_sites_local(sites, iterations=iters, device=0, concurrency=conc, predict=grids)
     print("phases run total", round(time.perf_counter() - t0, 2))
     for n in sorted(acc):
         c, a, b, d = acc[n]
