@@ -15,6 +15,7 @@ import numpy as np
 MAX_TERMS, MAX_FACTORS, MAX_FDIMS, MAX_COLS, MAX_THETA = 8, 3, 4, 8, 48
 ABI_VERSION = 2
 BATCH_MAX_SITES = 32
+BATCH_PREDICT_CHUNK = 1024  # grid rows of every site per launch of dgp_batch_predict (csrc/dgp_batch.cuh)
 
 RBF, MATERN32, MATERN52, PERIODIC = 0, 1, 2, 3
 GATE_NONE, GATE_SIGMOID, GATE_INV_SIGMOID = 0, 1, 2
@@ -93,6 +94,8 @@ _SIGNATURES = [
     ("dgp_batch_nlml_grad_launch", C.c_int, [_P, _P, _P]),
     ("dgp_batch_nlml_grad_ready", C.c_int, [_P]),
     ("dgp_batch_nlml_grad_wait", C.c_int, [_P, _P, _P, _P]),
+    ("dgp_batch_factorize", C.c_int, [_P, _P, _P, _P, _P]),
+    ("dgp_batch_predict", C.c_int, [_P, _P, _P, _P, _P]),
     ("dgp_batch_get_alpha", C.c_int, [_P, C.c_int, _P]),
     ("dgp_batch_launch_count", C.c_longlong, [_P]),
     ("dgp_batch_set_timing", C.c_int, [_P, C.c_int]),
@@ -156,7 +159,8 @@ def _f64(a) -> np.ndarray:
 
 class BatchEngine:
     """One libdgp batch handle (dgp_batch_*): up to `max_sites` independent sites sharing one covariance spec, evaluated
-    by ONE launch sequence per call (NLML + gradient of every site).  Host arrays in, host arrays out."""
+    by ONE launch sequence per call (NLML + gradient of every site; or factorisation, then posterior prediction of every
+    site on its own grid).  Host arrays in, host arrays out."""
 
     def __init__(self, max_sites: int, max_n: int, device: int = 0, stream: int = 0):
         self.lib = load_library()
@@ -235,6 +239,41 @@ class BatchEngine:
         self._check(self.lib.dgp_batch_nlml_grad_wait(self._h, val.ctypes.data, grad.ctypes.data, info.ctypes.data),
                     "dgp_batch_nlml_grad_wait")
         return val, grad, info
+
+    def factorize(self, theta, jitter=None):
+        """(nlml[G], info[G]): factorise every site at theta[G, P] (+ jitter[G]) for predict (Engine.factorize per site)."""
+        th, jit = self._args(theta, jitter)
+        val = np.zeros(self.nsites)
+        info = np.zeros(self.nsites, dtype=np.int32)
+        self._check(self.lib.dgp_batch_factorize(self._h, th.ctypes.data, jit.ctypes.data if jit is not None else None,
+                                                 val.ctypes.data, info.ctypes.data), "dgp_batch_factorize")
+        return val, info
+
+    def predict(self, grids, want_var: bool = True):
+        """Posterior mean and latent variance of every site on its own grid (Engine.predict per site, bit for bit).
+        grids: length-G sequence of Xs[m_s, ndim] host arrays, or None to skip a site.  Returns [(mu, var)] per site: var is
+        None when want_var is false, (None, None) for a skipped site.  Needs factorize of every predicted site first."""
+        if len(grids) != self.nsites:
+            raise ValueError(f"predict: {self.nsites} grids (or None) expected, got {len(grids)}")
+        G = self.nsites
+        xs, out = [], []
+        for Xs in grids:
+            if Xs is None:
+                xs.append(None)
+                out.append((None, None))
+                continue
+            Xs = _f64(Xs)
+            if Xs.ndim != 2 or Xs.shape[1] != self._keep.ndim:
+                raise ValueError("predict: Xs[m, ndim] expected for every site")
+            xs.append(Xs)
+            m = int(Xs.shape[0])
+            out.append((np.empty(m), np.empty(m) if want_var else None))
+        ms = (C.c_int * G)(*[0 if x is None else int(x.shape[0]) for x in xs])
+        px = (_P * G)(*[None if x is None or x.shape[0] == 0 else x.ctypes.data for x in xs])
+        pm = (_P * G)(*[None if o[0] is None or o[0].shape[0] == 0 else o[0].ctypes.data for o in out])
+        pv = (_P * G)(*[None if o[1] is None or o[1].shape[0] == 0 else o[1].ctypes.data for o in out])
+        self._check(self.lib.dgp_batch_predict(self._h, ms, px, pm, pv if want_var else None), "dgp_batch_predict")
+        return out
 
     def alpha(self, site: int) -> np.ndarray:
         a = np.empty(self.ns[site])

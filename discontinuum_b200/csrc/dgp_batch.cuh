@@ -28,6 +28,10 @@ struct dgp_batch_s {
   long long ld = 0;
   int n[DGP_BATCH_MAX] = {0}, nb[DGP_BATCH_MAX] = {0}, off[DGP_BATCH_MAX] = {0}, order[DGP_BATCH_MAX] = {0};
   bool have_train = false, pending = false;
+  // have_T[s]: the last evaluation was a dgp_batch_factorize and site s factorised (info == 0): L^-1 in the lower triangle
+  // of its A slab and alpha are what dgp_batch_predict reads.  Cleared by set_train and by every nlml_grad launch (LAUUM
+  // overwrites T).
+  bool have_T[DGP_BATCH_MAX] = {false};
   dgp_spec spec, user_spec;
   SiteDims sd;
   double *A = nullptr, *L = nullptr, *U = nullptr;
@@ -35,17 +39,25 @@ struct dgp_batch_s {
   double *theta = nullptr, *scal = nullptr, *gpart = nullptr, *zpart = nullptr, *jitv = nullptr;
   double *h_theta = nullptr, *h_scal = nullptr, *h_jit = nullptr;  // pinned
   CUtensorMap tmA, tmL, tmU;
+  // prediction slabs (dgp_batch_predict), allocated by the first prediction on the handle and kept (chunk = DGP_BATCH_CHUNK):
+  // Kx [max_sites][chunk][max_pad], mean / variance partials [max_sites][max_nb | 2 max_nb][chunk], inputs and features
+  // [max_sites][chunk][8], means / mu / var [max_sites][chunk]; pinned staging of the inputs and of mu / var
+  double *Kx = nullptr, *Xs = nullptr, *Xws = nullptr, *means = nullptr, *dot = nullptr, *vpart = nullptr;
+  double *mu = nullptr, *var = nullptr;
+  double *h_xs = nullptr, *h_mu = nullptr, *h_var = nullptr;  // pinned
+  CUtensorMap tmKx;
   long long launches = 0;
   double last_ms[4] = {0, 0, 0, 0};
   std::string err;
 };
 typedef struct dgp_batch_s* dgp_batch_t;
 
-static int make_map3(dgp_batch_t h, CUtensorMap* m, double* base, long long ld, int sites) {
+// slab [sites][rows][ld] (rows = ld: the per-site matrices; the prediction chunk: the cross-covariance slab)
+static int make_map3(dgp_batch_t h, CUtensorMap* m, double* base, long long ld, long long rows, int sites) {
   PFN_encodeTiled enc = get_encode();
   if (!enc) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled entry point not available");
-  cuuint64_t dims[3] = {(cuuint64_t)ld, (cuuint64_t)ld, (cuuint64_t)sites};
-  cuuint64_t strides[2] = {(cuuint64_t)ld * 8, (cuuint64_t)ld * (cuuint64_t)ld * 8};
+  cuuint64_t dims[3] = {(cuuint64_t)ld, (cuuint64_t)rows, (cuuint64_t)sites};
+  cuuint64_t strides[2] = {(cuuint64_t)ld * 8, (cuuint64_t)rows * (cuuint64_t)ld * 8};
   cuuint32_t box[3] = {BK, 64, 1};
   cuuint32_t es[3] = {1, 1, 1};
   CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
@@ -247,9 +259,11 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
 
 // U = L^-T by recursive doubling, all sites per launch, stream W.  b_trtri_advance(Fg): every merge whose block range lies
 // inside the block columns that are final once the global step Fg is reached (site i: its first Fg - off_i columns) and has
-// not been launched yet (trtri_advance of dgp_api.cu); Fg >= NB: everything that is left.
+// not been launched yet (trtri_advance of dgp_api.cu); Fg >= NB: everything that is left.  want_T: also transpose the last
+// level, so that T = L^-1 is complete in the lower triangle of the A slab (dgp_batch_factorize, for the prediction).
 struct BInvProgress {
   short done[16][DGP_BATCH_MAX];
+  bool want_T;
   cudaStream_t W;
 };
 
@@ -270,7 +284,7 @@ int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg) {
       const int pr0 = ip.done[lv][i], cnt = avail - pr0;
       if (cnt <= 0) continue;
       tb.add(i, pr0, nbi, b->n[i], hb, cnt, 0, cnt * hb * 2 * hb);
-      if (2 * hb < nbi) {
+      if (ip.want_T || 2 * hb < nbi) {
         prg.pr0[i] = (short)pr0; prg.cnt[i] = (short)cnt;
         if (cnt * 16 * hb * hb > tmax) tmax = cnt * 16 * hb * hb;
       }
@@ -330,7 +344,9 @@ int b_lauum_grad(dgp_batch_t b, cudaStream_t W) {
   return 0;
 }
 
-int b_enqueue(dgp_batch_t b) {
+// level 1: NLML + gradient (dgp_batch_nlml_grad); level 2: factorise for the prediction (dgp_batch_factorize: the inverse
+// with its last level transposed, no LAUUM, no gradient), as evaluate_enqueue of dgp_api.cu
+int b_enqueue(dgp_batch_t b, int level) {
   int rc;
   const int G = b->G;
   cudaStream_t T = b->stream, W = b->stream_lo ? b->stream_lo : b->stream;
@@ -343,6 +359,7 @@ int b_enqueue(dgp_batch_t b) {
   BInvProgress ip;
   memset(&ip, 0, sizeof(ip));
   ip.W = W;
+  ip.want_T = (level == 2);
   // the merges of the inverse are released as the factorisation passes them at every size (unlike the single-site engine)
   if ((rc = b_potrf(b, W != T ? &ip : nullptr))) return rc;
   if (b->timing) CK(b, cudaEventRecord(b->ev[1], T));
@@ -352,17 +369,50 @@ int b_enqueue(dgp_batch_t b) {
   }
   if ((rc = b_trtri(b, ip))) return rc;
   if (b->timing) CK(b, cudaEventRecord(b->ev[2], W));
-  if ((rc = b_lauum_grad(b, W))) return rc;
+  if (level == 1 && (rc = b_lauum_grad(b, W))) return rc;
   if (b->timing) CK(b, cudaEventRecord(b->ev[3], W));
   if (W != T) {
     CK(b, cudaEventRecord(b->ev_lo[1], W));
     CK(b, cudaStreamWaitEvent(T, b->ev_lo[1], 0));
   }
-  k_finish_b<<<dim3(b->spec.ntheta + 1, G), 256, 0, T>>>(b->spec, b->sd, b->theta, b->gpart, b->z, b->alpha, b->X, b->scal);
+  k_finish_b<<<dim3(b->spec.ntheta + 1, G), 256, 0, T>>>(b->spec, b->sd, b->theta, b->gpart, b->z, b->alpha, b->X, b->scal,
+                                                          level == 1 ? 1 : 0);
   b->launches++;
   CK(b, cudaGetLastError());
   CK(b, cudaMemcpyAsync(b->h_scal, b->scal, sizeof(double) * SC_SIZE * G, cudaMemcpyDeviceToHost, T));
   if (b->timing) CK(b, cudaEventRecord(b->ev[4], T));
+  return 0;
+}
+
+// Rows of every site's prediction grid per batched launch.  1024 keeps the cross-covariance slab at 1024 / (3 max_pad) of the
+// training slabs (64 MB per site at n = 8192) while a launch of the variance GEMM still has 8 x 2 nb tiles per site, a full
+// wave of the 2 x 148 CTA slots for a single site from 19 block columns (n > 2304) on; 2048 rows would only save the 4 launches per chunk.
+constexpr int DGP_BATCH_CHUNK = 1024;
+
+void b_predict_free(dgp_batch_t b) {
+  double* bufs[] = {b->Kx, b->Xs, b->Xws, b->means, b->dot, b->vpart, b->mu, b->var};
+  for (double* p : bufs) if (p) cudaFree(p);
+  double* hbufs[] = {b->h_xs, b->h_mu, b->h_var};
+  for (double* p : hbufs) if (p) cudaFreeHost(p);
+  b->Kx = b->Xs = b->Xws = b->means = b->dot = b->vpart = b->mu = b->var = nullptr;
+  b->h_xs = b->h_mu = b->h_var = nullptr;
+}
+
+// the prediction slabs, once per handle, for max_sites sites of up to max_n points (later calls allocate nothing)
+int b_predict_alloc(dgp_batch_t b) {
+  if (b->Kx) return 0;
+  const size_t S = b->max_sites, C = DGP_BATCH_CHUNK, np = b->max_pad, nbm = np / 128;
+  cudaError_t r = cudaSuccess;
+  auto A = [&](double** p, size_t count) { if (r == cudaSuccess) r = cudaMalloc((void**)p, count * sizeof(double)); };
+  auto H = [&](double** p, size_t count) { if (r == cudaSuccess) r = cudaMallocHost((void**)p, count * sizeof(double)); };
+  A(&b->Kx, S * C * np); A(&b->dot, S * nbm * C); A(&b->vpart, S * 2 * nbm * C);
+  A(&b->Xs, S * C * DGP_MAX_COLS); A(&b->Xws, S * C * DGP_XS); A(&b->means, S * C); A(&b->mu, S * C); A(&b->var, S * C);
+  H(&b->h_xs, S * C * DGP_MAX_COLS); H(&b->h_mu, S * C); H(&b->h_var, S * C);
+  if (r != cudaSuccess) {
+    cudaGetLastError();
+    b_predict_free(b);
+    DGP_FAIL(b, -2, "dgp_batch_predict: allocation of the prediction slabs failed: %s", cudaGetErrorString(r));
+  }
   return 0;
 }
 }  // namespace
@@ -386,6 +436,7 @@ int dgp_batch_destroy(dgp_batch b) {
   for (cudaEvent_t e : b->evs) cudaEventDestroy(e);
   double* bufs[] = {b->A, b->L, b->U, b->X, b->y, b->noise, b->Xw, b->r, b->z, b->alpha, b->theta, b->scal, b->gpart, b->zpart, b->jitv};
   for (double* p : bufs) if (p) cudaFree(p);
+  b_predict_free(b);
   if (b->h_theta) cudaFreeHost(b->h_theta);
   if (b->h_scal) cudaFreeHost(b->h_scal);
   if (b->h_jit) cudaFreeHost(b->h_jit);
@@ -498,29 +549,36 @@ int dgp_batch_set_train(dgp_batch b, const dgp_spec* spec, int nsites, const int
     CK(b, cudaMemcpyAsync(b->noise + (size_t)i * ld, noise[i], (size_t)n[i] * 8, cudaMemcpyHostToDevice, st));
   }
   CK(b, cudaStreamSynchronize(st));
-  if ((rc = make_map3(b, &b->tmA, b->A, b->ld, nsites))) return rc;
-  if ((rc = make_map3(b, &b->tmL, b->L, b->ld, nsites))) return rc;
-  if ((rc = make_map3(b, &b->tmU, b->U, b->ld, nsites))) return rc;
+  for (int i = 0; i < DGP_BATCH_MAX; i++) b->have_T[i] = false;
+  if ((rc = make_map3(b, &b->tmA, b->A, b->ld, b->ld, nsites))) return rc;
+  if ((rc = make_map3(b, &b->tmL, b->L, b->ld, b->ld, nsites))) return rc;
+  if ((rc = make_map3(b, &b->tmU, b->U, b->ld, b->ld, nsites))) return rc;
   b->have_train = true;
   return 0;
 }
 
-int dgp_batch_nlml_grad_launch(dgp_batch b, const double* theta, const double* jitter) {
+// level 1: dgp_batch_nlml_grad_launch; level 2: dgp_batch_factorize
+static int b_launch(dgp_batch b, const double* theta, const double* jitter, int level) {
   if (!b) return -1;
   if (!b->have_train) DGP_FAIL(b, -1, "no training data: call dgp_batch_set_train first");
   if (!theta) DGP_FAIL(b, -1, "theta is NULL");
   if (b->pending) DGP_FAIL(b, -1, "an evaluation is already in flight: call dgp_batch_nlml_grad_wait first");
   CK(b, cudaSetDevice(b->device));
+  for (int i = 0; i < DGP_BATCH_MAX; i++) b->have_T[i] = false;
   const int P = b->spec.ntheta;
   memset(b->h_theta, 0, sizeof(double) * DGP_MAX_THETA * b->G);
   for (int i = 0; i < b->G; i++) {
     memcpy(b->h_theta + (size_t)i * DGP_MAX_THETA, theta + (size_t)i * P, sizeof(double) * P);
     b->h_jit[i] = jitter ? jitter[i] : 0.0;
   }
-  int rc = b_enqueue(b);
+  int rc = b_enqueue(b, level);
   if (rc) return rc;
   b->pending = true;
   return 0;
+}
+
+int dgp_batch_nlml_grad_launch(dgp_batch b, const double* theta, const double* jitter) {
+  return b_launch(b, theta, jitter, 1);
 }
 
 int dgp_batch_nlml_grad_ready(dgp_batch b) {
@@ -569,6 +627,84 @@ int dgp_batch_get_alpha(dgp_batch b, int site, double* alpha_out) {
   CK(b, cudaSetDevice(b->device));
   CK(b, cudaMemcpyAsync(alpha_out, b->alpha + (size_t)site * b->ld, (size_t)b->n[site] * 8, cudaMemcpyDeviceToHost, b->stream));
   CK(b, cudaStreamSynchronize(b->stream));
+  return 0;
+}
+
+int dgp_batch_factorize(dgp_batch b, const double* theta, const double* jitter, double* nlml_out, int* info_out) {
+  int rc = b_launch(b, theta, jitter, 2);
+  if (rc) return rc;
+  if ((rc = dgp_batch_nlml_grad_wait(b, nlml_out, nullptr, info_out)) < 0) return rc;
+  for (int i = 0; i < b->G; i++) b->have_T[i] = (int)b->h_scal[(size_t)i * SC_SIZE + SC_INFO] == 0;
+  return rc;
+}
+
+// dgp_predict for every site of the batch, DGP_BATCH_CHUNK rows of every grid per launch: features of the chunk -> cross
+// covariance + mean partials -> variance GEMM V'[i, c] = sum_k Kx[i, k] T[c, k] with row sums of squares (M_PREDVAR,
+// EPI_SUMSQ) -> mu, var.  Per site, every tile and partial sums the same k range in the same order as the single-site
+// prediction, and rows never mix: the results do not depend on the chunk or on which sites share a launch.
+int dgp_batch_predict(dgp_batch b, const int* m, const double* const* Xs, double* const* mu_out, double* const* var_out) {
+  if (!b) return -1;
+  if (!b->have_train || !m || !Xs || !mu_out) DGP_FAIL(b, -1, "dgp_batch_predict: bad arguments");
+  if (b->pending) DGP_FAIL(b, -1, "dgp_batch_predict: an evaluation is in flight: call dgp_batch_nlml_grad_wait first");
+  const int G = b->G, C = DGP_BATCH_CHUNK, ndim = b->spec.ndim;
+  int mmax = 0;
+  for (int i = 0; i < G; i++) {
+    if (m[i] < 0) DGP_FAIL(b, -1, "dgp_batch_predict: site %d: m = %d", i, m[i]);
+    if (m[i] == 0) continue;
+    if (!Xs[i] || !mu_out[i]) DGP_FAIL(b, -1, "dgp_batch_predict: site %d: NULL grid or output", i);
+    if (!b->have_T[i])
+      DGP_FAIL(b, -1, "dgp_batch_predict: site %d is not factorised: call dgp_batch_factorize first (again after every "
+               "dgp_batch_set_train / dgp_batch_nlml_grad; a site whose factorisation failed cannot predict)", i);
+    if (m[i] > mmax) mmax = m[i];
+  }
+  if (mmax == 0) return 0;
+  CK(b, cudaSetDevice(b->device));
+  int rc;
+  if ((rc = b_predict_alloc(b))) return rc;
+  if ((rc = make_map3(b, &b->tmKx, b->Kx, b->ld, C, G))) return rc;
+  cudaStream_t st = b->stream;
+  for (int m0 = 0; m0 < mmax; m0 += C) {
+    PredChunk pc;
+    memset(&pc, 0, sizeof(pc));
+    TabBuilder tb(b);
+    bool any_var = false;
+    for (int k = 0; k < G; k++) {   // largest sites first in the GEMM's table, as in every other batched launch
+      const int i = b->order[k];
+      const int mc = m[i] - m0 < 0 ? 0 : (m[i] - m0 < C ? m[i] - m0 : C);
+      if (mc == 0) continue;
+      pc.m[i] = mc;
+      pc.var[i] = var_out != nullptr && var_out[i] != nullptr;
+      memcpy(b->h_xs + (size_t)i * C * DGP_MAX_COLS, Xs[i] + (size_t)m0 * ndim, (size_t)mc * ndim * 8);
+      if (pc.var[i]) {
+        const int rb = (mc + 127) / 128;
+        tb.add(i, 0, b->nb[i], b->n[i], rb, C, 0, rb * 2 * b->nb[i]);
+        any_var = true;
+      }
+    }
+    CK(b, cudaMemcpyAsync(b->Xs, b->h_xs, (size_t)G * C * DGP_MAX_COLS * 8, cudaMemcpyHostToDevice, st));
+    k_pred_features_b<<<dim3(C / 256, G), 256, 0, st>>>(b->spec, pc, b->theta, b->Xs, b->Xws, b->means, C);
+    k_cov_rect_pred_b<<<dim3(C / 32, b->NB, G), 256, 0, st>>>(b->spec, b->sd, pc, b->theta, b->Xws, b->Xw, b->noise, b->alpha,
+                                                              b->Kx, b->dot, C);
+    b->launches += 2;
+    CK(b, cudaGetLastError());
+    if (any_var) {
+      GemmArgs g = b_args(b, M_PREDVAR, nullptr, 1.0, tb.total);
+      g.aux1 = C; g.part = b->vpart;
+      if ((rc = launch_gemm<INIT_ZERO, EPI_SUMSQ>(b, b->tmKx, b->tmA, g, st, false, &tb.t))) return rc;
+    }
+    k_pred_finish_b<<<dim3(C / 256, G), 256, 0, st>>>(b->spec, b->sd, pc, b->theta, b->Xws, b->means, b->dot, b->vpart, b->mu,
+                                                      b->var, C);
+    b->launches++;
+    CK(b, cudaGetLastError());
+    CK(b, cudaMemcpyAsync(b->h_mu, b->mu, (size_t)G * C * 8, cudaMemcpyDeviceToHost, st));
+    if (any_var) CK(b, cudaMemcpyAsync(b->h_var, b->var, (size_t)G * C * 8, cudaMemcpyDeviceToHost, st));
+    CK(b, cudaStreamSynchronize(st));
+    for (int i = 0; i < G; i++) {
+      if (pc.m[i] == 0) continue;
+      memcpy(mu_out[i] + m0, b->h_mu + (size_t)i * C, (size_t)pc.m[i] * 8);
+      if (pc.var[i]) memcpy(var_out[i] + m0, b->h_var + (size_t)i * C, (size_t)pc.m[i] * 8);
+    }
+  }
   return 0;
 }
 

@@ -44,7 +44,7 @@ struct GemmArgs {
   const double* noise;          // fixed noise [npad]                    (INIT_COV)
   const double* theta;          // natural parameters on device          (INIT_COV)
   const void* reserved0_;       // unused (see reserved3_)
-  double* part;                 // EPI_SUMSQ: [2 nb][rows]
+  double* part;                 // EPI_SUMSQ: [2 nb][rows] (batched: [site][2 nbmax][rows])
   const void* reserved1_;       // unused (see reserved3_)
   double jitter;
   int latent;                   // INIT_COV: add only `jitter` on the diagonal (latent posterior covariance)
@@ -502,8 +502,17 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
       }
     }
   } else if constexpr (EPI == EPI_SUMSQ) {
-    // row sums of squares of the tile -> part[cblock][row]
-    const int cb = job.ccol / 64;
+    // row sums of squares of the tile -> part[cblock][row]; a batched launch writes site s's partials at part[s][2 nbmax]
+    // [rows] (nbmax = bt.ld / 128), the site found again from the block index like the store epilogue does
+    size_t cb = job.ccol / 64;
+    if (bt.count > 0) {
+      int bx = blockIdx.x;
+      asm volatile("" : "+r"(bx));
+      int k = 0;
+#pragma unroll 1
+      for (int i = 1; i < bt.count; i++) if (bx >= bt.e[i].tile0) k = i;
+      cb += (size_t)bt.e[k].site * (size_t)(bt.ld / 64);
+    }
     double rs[8];
 #pragma unroll
     for (int mi = 0; mi < 8; mi++) {
@@ -526,7 +535,7 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
 #pragma unroll
       for (int mi = 0; mi < 8; mi++) {
         const int lr = 64 * wm + 8 * mi + g8;
-        g.part[(size_t)cb * g.aux1 + job.crow + lr] = rs[mi] + red[lr];
+        g.part[cb * g.aux1 + job.crow + lr] = rs[mi] + red[lr];
       }
     }
   }

@@ -383,24 +383,22 @@ k_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta
 __global__ void __launch_bounds__(256)
 k_finish_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ SiteDims sd, const double* __restrict__ theta,
            const double* __restrict__ part, const double* __restrict__ z, const double* __restrict__ alpha,
-           const double* __restrict__ X, double* __restrict__ scal) {
+           const double* __restrict__ X, double* __restrict__ scal, int want_grad) {
   const int st = blockIdx.y, nb = sd.nb[st];
   const size_t v = (size_t)st * sd.ld;
   finish_body(spec, theta + st * DGP_MAX_THETA, part + (size_t)st * sd.nbmax * (sd.nbmax + 1) * DGP_MAX_THETA, nb * (nb + 1),
-              z + v, alpha + v, X + v * DGP_MAX_COLS, sd.n[st], nb * 128, scal + (size_t)st * SC_SIZE, 1, blockIdx.x);
+              z + v, alpha + v, X + v * DGP_MAX_COLS, sd.n[st], nb * 128, scal + (size_t)st * SC_SIZE, want_grad, blockIdx.x);
 }
 
 // ------------------------------------------------------------------ prediction reductions
 // mu[i] = mean[i] + sum_cb dot[cb][i] ;  var[i] = k(x*_i, x*_i) - sum_cb vpart[cb][i]
-__global__ void __launch_bounds__(256)
-k_pred_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta,
+__device__ __forceinline__ void pred_finish_body(const dgp_spec& spec, const double* __restrict__ theta,
               const double* __restrict__ Xws, const double* __restrict__ mean, const double* __restrict__ dot,
               int ndot, const double* __restrict__ vpart, int nvpart, int ldp, int m, double* __restrict__ mu,
-              double* __restrict__ var) {
+              double* __restrict__ var, int i) {
   __shared__ CovC cc;
   cov_compile(&cc, spec, theta, 0.0, threadIdx.x, 256);
   __syncthreads();
-  const int i = blockIdx.x * 256 + threadIdx.x;
   if (i >= m) return;
   double s = mean[i];
   for (int b = 0; b < ndot; b++) s += dot[(size_t)b * ldp + i];
@@ -413,6 +411,63 @@ k_pred_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ 
     for (int b = 0; b < nvpart; b++) v += vpart[(size_t)b * ldp + i];
     var[i] = cov_entry(&cc, xi, xi) - v;
   }
+}
+__global__ void __launch_bounds__(256)
+k_pred_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta,
+              const double* __restrict__ Xws, const double* __restrict__ mean, const double* __restrict__ dot,
+              int ndot, const double* __restrict__ vpart, int nvpart, int ldp, int m, double* __restrict__ mu,
+              double* __restrict__ var) {
+  pred_finish_body(spec, theta, Xws, mean, dot, ndot, vpart, nvpart, ldp, m, mu, var, blockIdx.x * 256 + threadIdx.x);
+}
+
+// ------------------------------------------------------------------ batched prediction (dgp_batch_predict)
+// One chunk of rows of every site's grid per launch.  Chunk slabs: inputs [site][chunk][DGP_MAX_COLS], features
+// [site][chunk][DGP_XS], means / mu / var [site][chunk], Kx [site][chunk][ld], mean partials [site][nbmax][chunk], variance
+// partials [site][2 nbmax][chunk]; the training side is the batch's slabs (SiteDims).  m[s] = rows of site s in this chunk
+// (0: nothing to do), var[s] = 1: its variance is wanted.  The bodies are those of the single-site prediction.
+struct PredChunk {
+  int m[DGP_BATCH_MAX];
+  int var[DGP_BATCH_MAX];
+};
+
+// grid = (chunk / 256, sites)
+__global__ void k_pred_features_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ PredChunk pc,
+                                  const double* __restrict__ theta, const double* __restrict__ Xs, double* __restrict__ Xws,
+                                  double* __restrict__ means, int chunk) {
+  const int st = blockIdx.y, m = pc.m[st];
+  if (m == 0) return;
+  const size_t v = (size_t)st * chunk;
+  features_body(spec, theta + st * DGP_MAX_THETA, Xs + v * DGP_MAX_COLS, nullptr, Xws + v * DGP_XS, nullptr, means + v, m,
+                (m + 127) / 128 * 128, nullptr, blockIdx.x * blockDim.x + threadIdx.x);
+}
+
+// cross covariance Kx[s] = K(x*, X_s) of the chunk (only where the variance is wanted) fused with the mean partials
+// dot[s][cb][i] = sum_{j in block cb} Kx[s][i, j] alpha_s[j].  grid = (chunk / 32, nbmax, sites)
+__global__ void __launch_bounds__(256)
+k_cov_rect_pred_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ SiteDims sd, const __grid_constant__ PredChunk pc,
+                  const double* __restrict__ theta, const double* __restrict__ Xws, const double* __restrict__ Xw,
+                  const double* __restrict__ noise, const double* __restrict__ alpha, double* __restrict__ Kx,
+                  double* __restrict__ dot, int chunk) {
+  const int st = blockIdx.z, m = pc.m[st];
+  if (m == 0 || (int)blockIdx.x >= (m + 127) / 128 * 4 || (int)blockIdx.y >= sd.nb[st]) return;
+  const size_t v = (size_t)st * sd.ld, c = (size_t)st * chunk;
+  cov_rect_body(spec, theta + st * DGP_MAX_THETA, Xws + c * DGP_XS, Xw + v * DGP_XS, noise + v, 0.0,
+                pc.var[st] ? Kx + c * sd.ld : nullptr, sd.ld, m, sd.n[st], 0, 0, alpha + v, dot + c * sd.nbmax, chunk,
+                blockIdx.x, blockIdx.y);
+}
+
+// grid = (chunk / 256, sites)
+__global__ void __launch_bounds__(256)
+k_pred_finish_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ SiteDims sd, const __grid_constant__ PredChunk pc,
+                const double* __restrict__ theta, const double* __restrict__ Xws, const double* __restrict__ means,
+                const double* __restrict__ dot, const double* __restrict__ vpart, double* __restrict__ mu,
+                double* __restrict__ var, int chunk) {
+  const int st = blockIdx.y, m = pc.m[st], nb = sd.nb[st];
+  if (m == 0) return;
+  const size_t c = (size_t)st * chunk;
+  pred_finish_body(spec, theta + st * DGP_MAX_THETA, Xws + c * DGP_XS, means + c, dot + c * sd.nbmax, nb,
+                   vpart + c * 2 * sd.nbmax, 2 * nb, chunk, m, mu + c, pc.var[st] ? var + c : nullptr,
+                   blockIdx.x * 256 + threadIdx.x);
 }
 
 }  // namespace dgp

@@ -219,19 +219,47 @@ def _groups(order: List[int], group: int) -> List[List[int]]:
     return [order[i:i + group] for i in range(0, len(order), group)]
 
 
-def _predict_site(eng: capi.Engine, s: _Site, theta: np.ndarray, Xs: np.ndarray, res: dict):
-    """Factorise at the fitted theta (psd_safe_cholesky's jitter ladder) and predict the site's grid."""
-    eng.set_train(s.module.spec.to_c(), s.X, s.y, s.noise)
-    for jit in JITTERS:
-        _, info = eng.factorize(theta, jit)
-        if info == 0:
+def _predict_group(batch: capi.BatchEngine, grp: List[_Site], want: List[bool], predict: Dict[int, np.ndarray], kind,
+                   res_of: Dict[int, dict]):
+    """Prediction of a group through its own batch handle (whose training set is the group's): factorise every site at its
+    fitted theta (dgp_batch_factorize), climb psd_safe_cholesky's jitter ladder only for the wanted sites that failed -- the
+    others are re-factorised unchanged and keep their bits -- and predict every wanted site's grid in one dgp_batch_predict.
+    Sites not wanted (not in `predict`, or failed while fitting) are factorised at their last theta, results unused."""
+    G = len(grp)
+    grids: List[Optional[np.ndarray]] = [None] * G
+    thetas = []
+    for k, s in enumerate(grp):
+        if want[k]:
+            grids[k] = np.ascontiguousarray(predict[s.idx], dtype=np.float64)
+            kind.project(s.module, np.concatenate([s.X, grids[k]], axis=0))
+        with torch.no_grad():
+            thetas.append(s.module.natural().numpy().astype(np.float64))
+        if want[k]:
+            res_of[s.idx]["theta"] = thetas[k]
+    thetas = np.ascontiguousarray(np.stack(thetas))
+    jit = np.full(G, JITTERS[0])
+    _, info = batch.factorize(thetas, jit)
+    bad = np.array(want) & (info != 0)
+    for j in JITTERS[1:]:
+        if not bad.any():
             break
-    else:
-        res["failed"] = f"prediction: not positive definite after jitter {JITTERS[-1]:g} (info={info})"
+        jit[bad] = j
+        _, i2 = batch.factorize(thetas, jit)
+        info = np.where(bad, i2, info)
+        bad &= i2 != 0
+    for k in np.nonzero(bad)[0]:
+        res_of[grp[k].idx]["failed"] = f"prediction: not positive definite after jitter {JITTERS[-1]:g} (info={int(info[k])})"
+        grids[k] = None
+    if all(g is None for g in grids):
         return
-    mu, var = eng.predict(Xs)
-    res["mu"], res["var_latent"] = mu, var
-    res["var"] = observed_variance(s.module.spec, theta, var, s.noise, Xs.shape[0])
+    out = batch.predict(grids)
+    for k, s in enumerate(grp):
+        if grids[k] is None:
+            continue
+        mu, var = out[k]
+        res = res_of[s.idx]
+        res["mu"], res["var_latent"] = mu, var
+        res["var"] = observed_variance(s.module.spec, thetas[k], var, s.noise, grids[k].shape[0])
 
 
 class _GroupRun:
@@ -324,6 +352,8 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
     `lanes`: every site sees the same sequence of evaluations.  Evaluations that fail (info != 0 or a non-finite value) climb
     psd_safe_cholesky's jitter ladder per site; a site whose objective stays bad for more than 10 consecutive iterations is
     marked failed, as MarginalB200.fit gives up.
+    The sites of a finished group that have a grid in `predict` are factorised and predicted on the group's own handle
+    (dgp_batch_factorize + dgp_batch_predict: every site's numbers equal a per-site capi.Engine factorize + predict bit for bit).
     `concurrency` selects the round-1 per-handle pipelines instead (fit_sites_local_per_handle)."""
     if concurrency is not None:
         return fit_sites_local_per_handle(sites, iterations=iterations, device=device, concurrency=concurrency or 4,
@@ -353,25 +383,31 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
     st["lanes"] = lanes
     n_max = state[order[0]].X.shape[0]
     handles: List[capi.BatchEngine] = []
-    single: Optional[capi.Engine] = None
 
-    def close_group(grp):
-        nonlocal single
+    def close_group(grp, batch: Optional[capi.BatchEngine] = None):
+        """Results of a finished group; its predictions run on the group's batch handle (idle now: the other lane's group keeps
+        the GPU busy meanwhile), or on a handle of its own when the group was never fitted (iterations <= 0)."""
         t0 = time.perf_counter()
+        res_of = {}
         for s in grp:
             with torch.no_grad():
                 theta = s.module.natural().numpy().astype(np.float64)
-            res = {"theta": theta, "history": s.history, "objective": s.history[-1] if s.history else None,
-                   "failed": s.failed, "n": int(s.X.shape[0])}
-            if predict is not None and s.idx in predict and s.failed is None:
-                if single is None:
-                    single = capi.Engine(max_n=n_max, max_m=2048, device=device)
-                kind.project(s.module, np.concatenate([s.X, predict[s.idx]], axis=0))
-                with torch.no_grad():
-                    theta = s.module.natural().numpy().astype(np.float64)
-                res["theta"] = theta
-                _predict_site(single, s, theta, np.ascontiguousarray(predict[s.idx], dtype=np.float64), res)
-            results[s.idx] = res
+            res_of[s.idx] = {"theta": theta, "history": s.history, "objective": s.history[-1] if s.history else None,
+                             "failed": s.failed, "n": int(s.X.shape[0])}
+        want = [predict is not None and s.idx in predict and s.failed is None for s in grp]
+        if any(want):
+            own = batch is None
+            if own:
+                batch = capi.BatchEngine(max_sites=len(grp), max_n=max(s.X.shape[0] for s in grp), device=device)
+            try:
+                if own:
+                    batch.set_train(grp[0].module.spec.to_c(), [(s.X, s.y, s.noise) for s in grp])
+                _predict_group(batch, grp, want, predict, kind, res_of)
+            finally:
+                if own:
+                    batch.close()
+        for s in grp:
+            results[s.idx] = res_of[s.idx]
         st["predict_s"] += time.perf_counter() - t0
 
     try:
@@ -408,7 +444,7 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
                     if r.left > 0 and not r.launch() and r.left <= 0:
                         r.opt.push()             # (every site of the group has failed: nothing left to evaluate)
                     if r.done:
-                        close_group(r.grp)
+                        close_group(r.grp, r.batch)
                         runs[lane] = next_group(lane)
                         if runs[lane] is not None:
                             runs[lane].launch()
@@ -416,8 +452,6 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
     finally:
         for b in handles:
             b.close()
-        if single is not None:
-            single.close()
     if stats is not None:
         stats.update(st, wall_s=time.perf_counter() - t_start)
     return results

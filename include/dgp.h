@@ -223,14 +223,18 @@ int dgp_gemm_nt(dgp_handle h, const double* A, long long lda, const double* B, l
  * sites, each running MarginalGPyTorch.fit, discontinuum/engines/gpytorch.py:346-444) and the per-gauge loop of
  * docs/source/notebooks/rating-gp-demo.ipynb.  Every kernel launch of the single-site schedule covers all sites (tile
  * index -> (site, tile) through a per-launch prefix table), so the latency-bound panel chain is paid once per block step
- * for the whole batch.  Sites of different n are end-aligned; per site the arithmetic is that of dgp_nlml_grad,
- * bit for bit.  Workspace (3 max_sites x max_n^2 float64 + O(max_sites max_n)) is allocated at create; later calls
- * allocate nothing.  Host pointers throughout. */
+ * for the whole batch.  Sites of different n are end-aligned; per site the arithmetic is that of dgp_nlml_grad (and of
+ * dgp_factorize + dgp_predict), bit for bit.  Workspace (3 max_sites x max_n^2 float64 + O(max_sites max_n)) is allocated
+ * at create.  The first dgp_batch_predict on a handle adds the prediction slabs, once: 8 max_sites x 1024 x (max_pad +
+ * 3 max_pad / 128 + 19) B on the device (max_pad = max_n rounded up to 128; the cross covariance of 1024 grid rows per
+ * site) and 80 max_sites x 1024 B of pinned host memory.  Every other call allocates nothing, and handles that never
+ * predict keep the create-time footprint.  Host pointers throughout. */
 #define DGP_BATCH_MAX_SITES 32
 typedef struct dgp_batch_s* dgp_batch;
 int dgp_batch_create(dgp_batch* out, int device, int max_sites, int max_n, void* stream);
 int dgp_batch_destroy(dgp_batch b);
 const char* dgp_batch_last_error(dgp_batch b); /* b may be NULL: error of a failed dgp_batch_create */
+/* Device bytes allocated by dgp_batch_create (the prediction slabs of the first dgp_batch_predict are not included). */
 size_t dgp_batch_workspace_bytes(int max_sites, int max_n);
 /* Training sets of nsites sites: n[s] points each, X[s][n[s], ndim], y[s][n[s]], noise[s][n[s]] (host arrays of host pointers). */
 int dgp_batch_set_train(dgp_batch b, const dgp_spec* spec, int nsites, const int* n, const double* const* X,
@@ -245,6 +249,16 @@ int dgp_batch_nlml_grad(dgp_batch b, const double* theta, const double* jitter, 
 int dgp_batch_nlml_grad_launch(dgp_batch b, const double* theta, const double* jitter);
 int dgp_batch_nlml_grad_ready(dgp_batch b);
 int dgp_batch_nlml_grad_wait(dgp_batch b, double* nlml_out, double* grad_out, int* info_out);
+/* Factorise every site of the batch at theta[nsites][ntheta] (+ jitter[nsites], NULL: 0) and keep, per site, L^-1 and
+ * alpha resident for dgp_batch_predict (the batch form of dgp_factorize).  nlml_out[nsites], info_out[nsites] may be NULL.
+ * Returns the number of sites with info != 0, or < 0. */
+int dgp_batch_factorize(dgp_batch b, const double* theta, const double* jitter, double* nlml_out, int* info_out);
+/* Posterior mean m(x*) + K*x alpha and LATENT variance k** - |L^-1 Kx*|^2 of every site on its own grid:
+ * m[s] points Xs[s][m[s], ndim] -> mu_out[s][m[s]], var_out[s][m[s]] (host pointers; var_out == NULL or var_out[s] == NULL:
+ * mean only; m[s] == 0: site skipped).  Needs a successful dgp_batch_factorize of every site with m[s] > 0 since the last
+ * dgp_batch_set_train / dgp_batch_nlml_grad; fails (< 0) otherwise.  Grids are walked in chunks of 1024 rows, each chunk
+ * of all sites in one launch sequence; the results equal dgp_predict's bit for bit. */
+int dgp_batch_predict(dgp_batch b, const int* m, const double* const* Xs, double* const* mu_out, double* const* var_out);
 /* Parity accessor: alpha of one site after an evaluation. */
 int dgp_batch_get_alpha(dgp_batch b, int site, double* alpha_out);
 long long dgp_batch_launch_count(dgp_batch b);
