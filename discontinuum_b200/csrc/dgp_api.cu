@@ -317,23 +317,31 @@ static int check_spec(HT h, const dgp_spec* sp) {
   if (sp->ntheta < 1 || sp->ntheta > DGP_MAX_THETA) DGP_FAIL(h, -1, "spec: ntheta out of range");
   auto bad = [&](int idx) { return idx < -1 || idx >= sp->ntheta; };
   if (bad(sp->noise_theta)) DGP_FAIL(h, -1, "spec: noise_theta out of range");
+  if (sp->mean_kind < DGP_MEAN_ZERO || sp->mean_kind > DGP_MEAN_POWERLAW) DGP_FAIL(h, -1, "spec: mean kind %d", sp->mean_kind);
   for (int c = 0; c < sp->ncols; c++) {
     const dgp_col& k = sp->col[c];
+    // the internal DGP_COL_SINP / DGP_COL_COSP kinds are appended by augment_spec, never accepted from a caller
+    if (k.kind < DGP_COL_COPY || k.kind > DGP_COL_GATE) DGP_FAIL(h, -1, "spec: col %d kind %d", c, k.kind);
     if (k.src < 0 || k.src >= sp->ndim) DGP_FAIL(h, -1, "spec: col %d src out of range", c);
     if (k.kind == DGP_COL_GATE && (k.theta < 0 || k.theta >= sp->ntheta)) DGP_FAIL(h, -1, "spec: gate col %d theta", c);
   }
   for (int t = 0; t < sp->nterms; t++) {
     const dgp_term& tm = sp->term[t];
     if (bad(tm.scale) || tm.nfactors < 0 || tm.nfactors > DGP_MAX_FACTORS) DGP_FAIL(h, -1, "spec: term %d", t);
+    if (tm.gate < DGP_GATE_NONE || tm.gate > DGP_GATE_INV_SIGMOID) DGP_FAIL(h, -1, "spec: term %d gate kind %d", t, tm.gate);
     if (tm.gate != DGP_GATE_NONE && (tm.gate_col < 0 || tm.gate_col >= sp->ncols || sp->col[tm.gate_col].kind != DGP_COL_GATE))
       DGP_FAIL(h, -1, "spec: term %d gate column", t);
     for (int f = 0; f < tm.nfactors; f++) {
       const dgp_factor& fa = tm.factor[f];
       if (fa.kind < DGP_RBF || fa.kind > DGP_PERIODIC || fa.ndims < 1 || fa.ndims > DGP_MAX_FDIMS)
         DGP_FAIL(h, -1, "spec: term %d factor %d kind/ndims", t, f);
-      for (int d = 0; d < fa.ndims; d++)
+      for (int d = 0; d < fa.ndims; d++) {
         if (fa.col[d] < 0 || fa.col[d] >= sp->ncols || fa.ls[d] < 0 || fa.ls[d] >= sp->ntheta)
           DGP_FAIL(h, -1, "spec: term %d factor %d dim %d", t, f, d);
+        // a gate column depends on theta[col.theta]; the gradient slots of a factor have no place for that dependence
+        if (sp->col[fa.col[d]].kind == DGP_COL_GATE)
+          DGP_FAIL(h, -1, "spec: term %d factor %d dim %d reads gate column %d", t, f, d, fa.col[d]);
+      }
       if (fa.kind == DGP_PERIODIC && (fa.ndims != 1 || fa.period < 0 || fa.period >= sp->ntheta))
         DGP_FAIL(h, -1, "spec: term %d factor %d periodic", t, f);
     }

@@ -45,10 +45,13 @@ extern "C" {
 enum { DGP_RBF = 0, DGP_MATERN32 = 1, DGP_MATERN52 = 2, DGP_PERIODIC = 3 };
 /* multiplicative gate of a term: g(h)g(h') or (1-g(h))(1-g(h')), g = 1/(1+exp(a(h-b))) */
 enum { DGP_GATE_NONE = 0, DGP_GATE_SIGMOID = 1, DGP_GATE_INV_SIGMOID = 2 };
-/* feature-table column kinds */
+/* feature-table column kinds.  A DGP_COL_GATE column may only be a term's gate_col: no factor dimension may read it,
+ * because its value depends on theta[b] and a factor's gradient has no place for that dependence. */
 enum { DGP_COL_COPY = 0, DGP_COL_LOG = 1 /* log(x + eps) */, DGP_COL_GATE = 2 /* g(x; a, theta[b]) */ };
 /* mean functions */
 enum { DGP_MEAN_ZERO = 0, DGP_MEAN_CONST = 1, DGP_MEAN_POWERLAW = 2 /* a + b log(x - c) */ };
+/* dgp_set_train / dgp_batch_set_train reject (< 0, with a message) a spec with any kind outside the enums above (column,
+ * factor, gate, mean), any theta index or column out of range, or a factor dimension on a DGP_COL_GATE column. */
 
 typedef struct {
   int32_t kind;                 /* DGP_COL_*                                          */
