@@ -84,6 +84,7 @@ _SIGNATURES = [
     ("dgp_get_chol", C.c_int, [_P, _P, C.c_int]),
     ("dgp_set_debug_kinv", C.c_int, [_P, C.c_int]),
     ("dgp_get_kinv", C.c_int, [_P, _P, C.c_int]),
+    ("dgp_get_linv", C.c_int, [_P, _P, C.c_int]),
     ("dgp_gemm_nt", C.c_int, [_P, _P, C.c_longlong, _P, C.c_longlong, _P, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int]),
     ("dgp_batch_create", C.c_int, [C.POINTER(_P), C.c_int, C.c_int, C.c_int, _P]),
     ("dgp_batch_destroy", C.c_int, [_P]),
@@ -413,15 +414,24 @@ class Engine:
                                                       C.addressof(val), grad.ctypes.data), "dgp_mean_functional_grad")
         return val.value, grad
 
-    def sample(self, Xs, Z, jitter: float = 0.0) -> Tuple[np.ndarray, int]:
-        """(draws[S, m], info): info > 0 means the posterior covariance (+ jitter) was not positive definite."""
-        Xs, Z = _f64(Xs), _f64(Z)
+    def sample(self, Xs, Z, jitter: float = 0.0):
+        """(draws[S, m], info): info > 0 means the posterior covariance (+ jitter) was not positive definite.  With Z a CUDA
+        tensor, Xs and the draws are CUDA tensors on its device too (nothing of size S x m crosses PCIe)."""
+        on_dev = hasattr(Z, "data_ptr") and Z.is_cuda
+        if not on_dev and hasattr(Xs, "data_ptr") and Xs.is_cuda:
+            raise ValueError("sample: Xs is a CUDA tensor but Z is not; pass Z on the same device to sample there")
+        if on_dev:
+            import torch
+
+            Xs = torch.as_tensor(Xs, dtype=torch.float64, device=Z.device).contiguous()
+        else:
+            Xs, Z = _f64(Xs), _f64(Z)
         S, m = Z.shape
-        if Xs.shape[0] != m:
+        if Xs.ndim != 2 or Xs.shape[0] != m:
             raise ValueError("sample: Z[S, m] and Xs[m, ndim] expected")
-        out = np.empty((S, m))
-        info = self._check(self.lib.dgp_sample(self._h, Xs.ctypes.data, m, Z.ctypes.data, S, float(jitter), out.ctypes.data, 0),
-                           "dgp_sample")
+        out = torch.empty((S, m), dtype=torch.float64, device=Z.device) if on_dev else np.empty((S, m))
+        info = self._check(self.lib.dgp_sample(self._h, _ptr(Xs)[0], m, _ptr(Z)[0], S, float(jitter), _ptr(out)[0],
+                                               1 if on_dev else 0), "dgp_sample")
         return out, info
 
     def sample_ex(self, Xs, S: int, Z=None, seed: int = 0, jitter: float = 0.0, flux: Optional[dict] = None):
@@ -495,18 +505,35 @@ class Engine:
         self._check(self.lib.dgp_get_alpha(self._h, a.ctypes.data, 0), "dgp_get_alpha")
         return a
 
-    def chol(self) -> np.ndarray:
-        L = np.empty((self.n, self.n))
-        self._check(self.lib.dgp_get_chol(self._h, L.ctypes.data, 0), "dgp_get_chol")
+    def _square_out(self, out):
+        """(buffer, address, on_device) of an [n, n] result: a new numpy array, or the caller's numpy array or contiguous
+        float64 tensor (a CUDA tensor is filled on the device)."""
+        if out is None:
+            out = np.empty((self.n, self.n))
+        if tuple(out.shape) != (self.n, self.n):
+            raise ValueError(f"out must be [{self.n}, {self.n}], got {tuple(out.shape)}")
+        return (out,) + _ptr(out)
+
+    def chol(self, out=None):
+        """L [n, n], lower triangular, of the last evaluation."""
+        L, p, dev = self._square_out(out)
+        self._check(self.lib.dgp_get_chol(self._h, p, dev), "dgp_get_chol")
         return L
 
     def set_debug_kinv(self, on: bool):
         self._check(self.lib.dgp_set_debug_kinv(self._h, 1 if on else 0), "dgp_set_debug_kinv")
 
-    def kinv(self) -> np.ndarray:
-        Ki = np.empty((self.n, self.n))
-        self._check(self.lib.dgp_get_kinv(self._h, Ki.ctypes.data, 0), "dgp_get_kinv")
+    def kinv(self, out=None):
+        """Ky^-1 [n, n] (lower triangle valid) of the last nlml_grad with set_debug_kinv(True)."""
+        Ki, p, dev = self._square_out(out)
+        self._check(self.lib.dgp_get_kinv(self._h, p, dev), "dgp_get_kinv")
         return Ki
+
+    def linv(self, out=None):
+        """T = L^-1 [n, n], lower triangular, of the last successful factorize."""
+        T, p, dev = self._square_out(out)
+        self._check(self.lib.dgp_get_linv(self._h, p, dev), "dgp_get_linv")
+        return T
 
     def gemm_nt(self, A, B, Cm, mode: int = 0):
         """Cm (=, +=, -=) A @ B.T on CUDA float64 tensors (row-major, contiguous)."""

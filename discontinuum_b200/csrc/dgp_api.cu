@@ -1420,6 +1420,26 @@ int dgp_get_kinv(dgp_handle h, double* Kinv_out, int out_on_device) {
   return copy_out(h, Kinv_out, h->bufA, h->n, h->n, h->npad, out_on_device);
 }
 
+// T = L^-1 sits in the lower triangle of bufA after dgp_factorize (the last merge level is transposed there too); the upper
+// triangle holds the inverse's scratch, which the copy replaces with zeros
+int dgp_get_linv(dgp_handle h, double* T_out, int out_on_device) {
+  if (!h) return -1;
+  if (!h->have_T || !T_out) DGP_FAIL(h, -1, "dgp_get_linv: needs a successful dgp_factorize (dgp_nlml* leave Ky^-1 there)");
+  CK(h, cudaSetDevice(h->device));
+  int rc = copy_out(h, T_out, h->bufA, h->n, h->n, h->npad, out_on_device);
+  if (rc) return rc;
+  const int n = h->n;
+  if (out_on_device) {
+    k_zero_strict_upper<<<n, 256, 0, h->stream>>>(T_out, n, n);
+    h->launches++;
+    CK(h, cudaGetLastError());
+    CK(h, cudaStreamSynchronize(h->stream));
+  } else {
+    for (int i = 0; i + 1 < n; i++) memset(T_out + (size_t)i * n + i + 1, 0, (size_t)(n - i - 1) * 8);
+  }
+  return 0;
+}
+
 long long dgp_launch_count(dgp_handle h) { return h ? h->launches : 0; }
 int dgp_set_timing(dgp_handle h, int enable) { if (!h) return -1; h->timing = enable != 0; return 0; }
 int dgp_last_timing(dgp_handle h, double* ms4) {

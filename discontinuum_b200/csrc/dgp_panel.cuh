@@ -485,6 +485,12 @@ k_copy_panel(const double* __restrict__ P, double* __restrict__ A, long long ld,
   }
 }
 
+// zero the strict upper triangle of a dense row-major n x n matrix (leading dimension ld); grid = n rows, block = 256
+__global__ void __launch_bounds__(256) k_zero_strict_upper(double* __restrict__ A, long long ld, int n) {
+  double* row = A + (size_t)blockIdx.x * ld;
+  for (int c = blockIdx.x + 1 + threadIdx.x; c < n; c += 256) row[c] = 0.0;
+}
+
 // Column panel [c0, c0 + w) of the rows >= r0 of A  <->  contiguous buffer P[rows][w]  (dir = 0: pack, 1: unpack).
 // grid = (rows / 8), block = 256; w multiple of 2.
 __global__ void __launch_bounds__(256)

@@ -212,6 +212,9 @@ int dgp_get_chol(dgp_handle h, double* L_out, int out_on_device);
 /* Ky^-1 [n, n] (lower triangle valid), materialised only when debug_kinv was enabled. */
 int dgp_set_debug_kinv(dgp_handle h, int enable);
 int dgp_get_kinv(dgp_handle h, double* Kinv_out, int out_on_device);
+/* T = L^-1 [n, n], lower triangular (zeros above the diagonal): the inverse the variance and sampling products use.  Valid
+ * after a successful dgp_factorize only (dgp_nlml_grad overwrites it with Ky^-1); fails with a message otherwise. */
+int dgp_get_linv(dgp_handle h, double* T_out, int out_on_device);
 
 /* Utility: the FP64 tensor-pipe tile engine as a plain product on device pointers,
  * C[M, N] = A[M, K] B[N, K]' (mode 0), C += A B' (mode 1), C -= A B' (mode -1).

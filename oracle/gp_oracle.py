@@ -3,7 +3,10 @@
 This file is a float64 torch restatement, on the CPU, of what the reference computes on its
 hot path when GPyTorch takes the exact-Cholesky branch (n <= max_cholesky_size).  It is the
 checker for the CUDA engine: only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline /
---impl reference legs may import it.  The product package never does.
+--impl reference legs may import it.  The product package never does.  Every function that takes data tensors creates
+its tensors on their device, so the same code also runs on CUDA tensors: tests/test_factor_schedule.py uses it that way
+as a float64 GPU reference (cuSOLVER / cuBLAS underneath) at sizes the CPU cannot reach in a test.  The initial-value
+and fixed-noise constructors (`*_init_raw`, `loadest_noise`) take no tensors and build theirs on the CPU.
 
 PARITY STATUS.  Two layers, pinned differently:
   * what the REFERENCE owns (which kernels act on which dimensions with which priors, constraints and initial values; the
@@ -87,7 +90,7 @@ def lp_gamma(x, a, b):
 # ----------------------------------------------------------------------------------------
 def _scaled_dist(X1, X2, cols, ls):
     """Euclidean distance of x/ls over `cols`, clamped like gpytorch's covar_dist."""
-    d2 = torch.zeros(X1.shape[0], X2.shape[0], dtype=DT)
+    d2 = torch.zeros(X1.shape[0], X2.shape[0], dtype=DT, device=X1.device)
     for c, l in zip(cols, ls):
         diff = (X1[:, c, None] - X2[None, :, c]) / l
         d2 = d2 + diff * diff
@@ -393,7 +396,7 @@ def sample(cov, mean, nat, X, y, noise, Xs, Z, extra_noise=None, jitter=0.0):
     mu, _, _ = predict(cov, mean, nat, X, y, noise, Xs, extra_noise)
     S = posterior_cov(cov, nat, X, noise, Xs, extra_noise)
     S = 0.5 * (S + S.T)
-    Lp = torch.linalg.cholesky(S + jitter * torch.eye(S.shape[0], dtype=DT))
+    Lp = torch.linalg.cholesky(S + jitter * torch.eye(S.shape[0], dtype=DT, device=S.device))
     return mu[None, :] + Z @ Lp.T, Lp
 
 
@@ -418,7 +421,7 @@ def pymc_loadest_cov(X1, X2, v):
 def pymc_loadest_neg_logp(v, X, y, sigma=0.1, jitter=1e-6):
     """-(log N(y | 0, K + (sigma^2 + jitter) I) + sum log prior), the quantity pm.find_MAP minimises (no Jacobian)."""
     n = X.shape[0]
-    Ky = pymc_loadest_cov(X, X, v) + (sigma ** 2 + jitter) * torch.eye(n, dtype=DT)
+    Ky = pymc_loadest_cov(X, X, v) + (sigma ** 2 + jitter) * torch.eye(n, dtype=DT, device=X.device)
     val = nlml_from_K(Ky, y)[0]
     lp = lp_halfnormal(v["eta_per"], 1.0).sum() + lp_gamma(v["ls_pdecay"], 10.0, 1.0).sum() + lp_normal(v["period"], 1.0, 0.05).sum()
     lp = lp + lp_gamma(v["ls_psmooth"], 4.0, 3.0).sum() + (-math.log(1.5) - v["eta_trend"] / 1.5).sum()

@@ -46,7 +46,7 @@ def spec_features(spec, X, theta):
 def spec_cov(spec, X1, X2, theta):
     """K(X1, X2) = sum over terms of scale x gate(x1) gate(x2) x product of factors on feature columns (no noise)."""
     W1, W2 = spec_features(spec, X1, theta), spec_features(spec, X2, theta)
-    K = torch.zeros(X1.shape[0], X2.shape[0], dtype=DT)
+    K = torch.zeros(X1.shape[0], X2.shape[0], dtype=DT, device=X1.device)
     for t in spec.terms:
         v = theta[t.scale] * torch.ones_like(K) if t.scale >= 0 else torch.ones_like(K)
         if t.gate != GATE_NONE:
@@ -71,7 +71,7 @@ def spec_cov(spec, X1, X2, theta):
 def spec_mean(spec, X, theta):
     """m(x): zero, theta[c], or the power law a + b log(x[mean_col] - c)."""
     if spec.mean_kind == MEAN_ZERO:
-        return torch.zeros(X.shape[0], dtype=DT)
+        return torch.zeros(X.shape[0], dtype=DT, device=X.device)
     if spec.mean_kind == MEAN_CONST:
         return theta[spec.mean_theta[0]].expand(X.shape[0])
     if spec.mean_kind == MEAN_POWERLAW:
