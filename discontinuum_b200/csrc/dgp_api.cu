@@ -1229,12 +1229,16 @@ int dgp_dist_end(dgp_dist d) {
   return 0;
 }
 
-// rows [row0, row1) (multiples of 128) of V' = Kx T' and of the posterior mean
+// rows [row0, row1) (multiples of 128) of V' = Kx T' and of the posterior mean.  Both ends are clamped to mpad first: a
+// shard of rows_per_rank rows lies wholly past mpad when world is large for mb (world 3, mb 1: rank 2 gets [256, 384)),
+// and such a range is an empty shard, not an error.
 int dgp_dist_vt_rows(dgp_dist d, int row0, int row1) {
   if (!d) return -1;
   dgp_handle h = d->h;
-  if (row0 < 0 || row0 % 128 || row1 % 128 || row1 < row0) DGP_FAIL(h, -1, "dgp_dist_vt_rows: bad row range");
+  if (row0 < 0 || row0 % 128 || row1 % 128) DGP_FAIL(h, -1, "dgp_dist_vt_rows: bad row range");
+  if (row0 > d->mpad) row0 = d->mpad;
   if (row1 > d->mpad) row1 = d->mpad;
+  if (row1 < row0) DGP_FAIL(h, -1, "dgp_dist_vt_rows: bad row range");
   CK(h, cudaSetDevice(h->device));
   int rc;
   const int npad = h->npad;

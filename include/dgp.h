@@ -186,7 +186,10 @@ int dgp_reserve(dgp_handle h, int max_m_sample, int max_S, int max_groups);
  *                                       (passed per call: the caller may double-buffer it)
  *   Od   [Spad, mpad]                   partial draws, all-reduced (sum) by the caller
  *   mu   [mpad]                         posterior mean, each rank fills its rows (zeros elsewhere): all-reduce (sum)
- * dgp_dist_dims -> {mpad, npad, Spad, panel_cols, npanels, rows_per_rank}.  Call order per rank:
+ * dgp_dist_dims -> {mpad, npad, Spad, panel_cols, npanels, rows_per_rank}.  Rank r's V' shard is rows
+ * [r rows_per_rank, (r + 1) rows_per_rank); dgp_dist_vt_rows clamps both ends to mpad, so a shard may be empty: when world
+ * is large for mb = mpad / 128 (world 3 with mb 1, world 8 with mb 41) the last ranks' shards lie at or past mpad, and
+ * vt_rows on them succeeds and does nothing.  A rank that owns no panel is valid too.  Call order per rank:
  *   begin -> vt_rows(my shard) -> [all_gather VT, all_reduce mu] -> sigma ->
  *   for p: (owner: panel_factor) -> [broadcast pack] -> (others: panel_unpack) -> trail(p, p+1, npanels-1)
  *          (look-ahead: trail(p, p+1, p+1) first, factor panel p+1 on a side stream while trail(p, p+2, ...) runs)
