@@ -97,6 +97,7 @@ _SIGNATURES = [
     ("dgp_batch_nlml_grad_wait", C.c_int, [_P, _P, _P, _P]),
     ("dgp_batch_factorize", C.c_int, [_P, _P, _P, _P, _P]),
     ("dgp_batch_predict", C.c_int, [_P, _P, _P, _P, _P]),
+    ("dgp_batch_mean_functional_grad", C.c_int, [_P, _P, _P, _P, _P, _P]),
     ("dgp_batch_get_alpha", C.c_int, [_P, C.c_int, _P]),
     ("dgp_batch_launch_count", C.c_longlong, [_P]),
     ("dgp_batch_set_timing", C.c_int, [_P, C.c_int]),
@@ -275,6 +276,33 @@ class BatchEngine:
         pv = (_P * G)(*[None if o[1] is None or o[1].shape[0] == 0 else o[1].ctypes.data for o in out])
         self._check(self.lib.dgp_batch_predict(self._h, ms, px, pm, pv if want_var else None), "dgp_batch_predict")
         return out
+
+    def mean_functional_grad(self, points, c):
+        """(val[G], grad[G, P]): F_s = sum_p c[s][p] mu_s(points[s][p]) and dF_s/dtheta_s of every site at the theta of its
+        last successful nlml_grad / factorize (Engine.mean_functional_grad per site, bit for bit).  points[s] / c[s] None:
+        site skipped (val 0, grad zeros).  At most BATCH_PREDICT_CHUNK points per site."""
+        if len(points) != self.nsites or len(c) != self.nsites:
+            raise ValueError(f"mean_functional_grad: {self.nsites} point sets and weight vectors (or None) expected")
+        G = self.nsites
+        xs, cs = [], []
+        for Xs, cv in zip(points, c):
+            if Xs is None or cv is None:
+                xs.append(None)
+                cs.append(None)
+                continue
+            Xs, cv = _f64(Xs), _f64(cv).reshape(-1)
+            if Xs.ndim != 2 or Xs.shape[1] != self._keep.ndim or cv.shape[0] != Xs.shape[0]:
+                raise ValueError("mean_functional_grad: points[m, ndim] and c[m] expected for every site")
+            xs.append(Xs)
+            cs.append(cv)
+        ms = (C.c_int * G)(*[0 if x is None else int(x.shape[0]) for x in xs])
+        px = (_P * G)(*[None if x is None or x.shape[0] == 0 else x.ctypes.data for x in xs])
+        pc = (_P * G)(*[None if v is None or v.shape[0] == 0 else v.ctypes.data for v in cs])
+        val = np.zeros(G)
+        grad = np.zeros((G, self.ntheta))
+        self._check(self.lib.dgp_batch_mean_functional_grad(self._h, ms, px, pc, val.ctypes.data, grad.ctypes.data),
+                    "dgp_batch_mean_functional_grad")
+        return val, grad
 
     def alpha(self, site: int) -> np.ndarray:
         a = np.empty(self.ns[site])

@@ -32,6 +32,10 @@ struct dgp_batch_s {
   // of its A slab and alpha are what dgp_batch_predict reads.  Cleared by set_train and by every nlml_grad launch (LAUUM
   // overwrites T).
   bool have_T[DGP_BATCH_MAX] = {false};
+  // have_eval[s]: the last evaluation (nlml_grad or factorize) finished and site s had info == 0: alpha and U = L^-T are
+  // resident, which is what the mean-only prediction and dgp_batch_mean_functional_grad read.  Cleared by set_train and
+  // by every launch.
+  bool have_eval[DGP_BATCH_MAX] = {false};
   dgp_spec spec, user_spec;
   SiteDims sd;
   double *A = nullptr, *L = nullptr, *U = nullptr;
@@ -46,6 +50,12 @@ struct dgp_batch_s {
   double *mu = nullptr, *var = nullptr;
   double *h_xs = nullptr, *h_mu = nullptr, *h_var = nullptr;  // pinned
   CUtensorMap tmKx;
+  // adjoint slabs (dgp_batch_mean_functional_grad), allocated by its first call and kept: c [max_sites][chunk], v / gamma
+  // and the intermediate U'v [max_sites][max_pad], its row-block partials [max_sites][max_nb][max_pad], the contraction
+  // partials [max_sites][mfg_pstride], results [max_sites][1 + DGP_MAX_THETA]; pinned staging of c and of the results
+  double *cvec = nullptr, *vvec = nullptr, *tmpz = nullptr, *gam = nullptr, *gzpart = nullptr, *wpart = nullptr, *mfg = nullptr;
+  double *h_c = nullptr, *h_mfg = nullptr;  // pinned
+  long long mfg_pstride = 0;
   long long launches = 0;
   double last_ms[4] = {0, 0, 0, 0};
   std::string err;
@@ -398,6 +408,15 @@ void b_predict_free(dgp_batch_t b) {
   b->h_xs = b->h_mu = b->h_var = nullptr;
 }
 
+void b_mfg_free(dgp_batch_t b) {
+  double* bufs[] = {b->cvec, b->vvec, b->tmpz, b->gam, b->gzpart, b->wpart, b->mfg};
+  for (double* p : bufs) if (p) cudaFree(p);
+  if (b->h_c) cudaFreeHost(b->h_c);
+  if (b->h_mfg) cudaFreeHost(b->h_mfg);
+  b->cvec = b->vvec = b->tmpz = b->gam = b->gzpart = b->wpart = b->mfg = nullptr;
+  b->h_c = b->h_mfg = nullptr;
+}
+
 // the prediction slabs, once per handle, for max_sites sites of up to max_n points (later calls allocate nothing)
 int b_predict_alloc(dgp_batch_t b) {
   if (b->Kx) return 0;
@@ -412,6 +431,25 @@ int b_predict_alloc(dgp_batch_t b) {
     cudaGetLastError();
     b_predict_free(b);
     DGP_FAIL(b, -2, "dgp_batch_predict: allocation of the prediction slabs failed: %s", cudaGetErrorString(r));
+  }
+  return 0;
+}
+
+// the adjoint slabs, once per handle (the partials of a site: (chunk / 128 + nb) (2 nb) tiles at the largest m and n)
+int b_mfg_alloc(dgp_batch_t b) {
+  if (b->cvec) return 0;
+  const size_t S = b->max_sites, C = DGP_BATCH_CHUNK, np = b->max_pad, nbm = np / 128;
+  b->mfg_pstride = (long long)((C / 128 + nbm) * (np / 64) * DGP_MAX_THETA);
+  cudaError_t r = cudaSuccess;
+  auto A = [&](double** p, size_t count) { if (r == cudaSuccess) r = cudaMalloc((void**)p, count * sizeof(double)); };
+  auto H = [&](double** p, size_t count) { if (r == cudaSuccess) r = cudaMallocHost((void**)p, count * sizeof(double)); };
+  A(&b->cvec, S * C); A(&b->vvec, S * np); A(&b->tmpz, S * np); A(&b->gam, S * np); A(&b->gzpart, S * nbm * np);
+  A(&b->wpart, S * (size_t)b->mfg_pstride); A(&b->mfg, S * (1 + DGP_MAX_THETA));
+  H(&b->h_c, S * C); H(&b->h_mfg, S * (1 + DGP_MAX_THETA));
+  if (r != cudaSuccess) {
+    cudaGetLastError();
+    b_mfg_free(b);
+    DGP_FAIL(b, -2, "dgp_batch_mean_functional_grad: allocation of the adjoint slabs failed: %s", cudaGetErrorString(r));
   }
   return 0;
 }
@@ -437,6 +475,7 @@ int dgp_batch_destroy(dgp_batch b) {
   double* bufs[] = {b->A, b->L, b->U, b->X, b->y, b->noise, b->Xw, b->r, b->z, b->alpha, b->theta, b->scal, b->gpart, b->zpart, b->jitv};
   for (double* p : bufs) if (p) cudaFree(p);
   b_predict_free(b);
+  b_mfg_free(b);
   if (b->h_theta) cudaFreeHost(b->h_theta);
   if (b->h_scal) cudaFreeHost(b->h_scal);
   if (b->h_jit) cudaFreeHost(b->h_jit);
@@ -549,7 +588,7 @@ int dgp_batch_set_train(dgp_batch b, const dgp_spec* spec, int nsites, const int
     CK(b, cudaMemcpyAsync(b->noise + (size_t)i * ld, noise[i], (size_t)n[i] * 8, cudaMemcpyHostToDevice, st));
   }
   CK(b, cudaStreamSynchronize(st));
-  for (int i = 0; i < DGP_BATCH_MAX; i++) b->have_T[i] = false;
+  for (int i = 0; i < DGP_BATCH_MAX; i++) b->have_T[i] = b->have_eval[i] = false;
   if ((rc = make_map3(b, &b->tmA, b->A, b->ld, b->ld, nsites))) return rc;
   if ((rc = make_map3(b, &b->tmL, b->L, b->ld, b->ld, nsites))) return rc;
   if ((rc = make_map3(b, &b->tmU, b->U, b->ld, b->ld, nsites))) return rc;
@@ -564,7 +603,7 @@ static int b_launch(dgp_batch b, const double* theta, const double* jitter, int 
   if (!theta) DGP_FAIL(b, -1, "theta is NULL");
   if (b->pending) DGP_FAIL(b, -1, "an evaluation is already in flight: call dgp_batch_nlml_grad_wait first");
   CK(b, cudaSetDevice(b->device));
-  for (int i = 0; i < DGP_BATCH_MAX; i++) b->have_T[i] = false;
+  for (int i = 0; i < DGP_BATCH_MAX; i++) b->have_T[i] = b->have_eval[i] = false;
   const int P = b->spec.ntheta;
   memset(b->h_theta, 0, sizeof(double) * DGP_MAX_THETA * b->G);
   for (int i = 0; i < b->G; i++) {
@@ -609,6 +648,7 @@ int dgp_batch_nlml_grad_wait(dgp_batch b, double* nlml_out, double* grad_out, in
     if (grad_out) memcpy(grad_out + (size_t)i * P, sc + SC_GRAD, sizeof(double) * P);
     const int info = (int)sc[SC_INFO];
     if (info_out) info_out[i] = info;
+    b->have_eval[i] = info == 0;
     if (info != 0) bad++;
   }
   return bad;
@@ -652,9 +692,13 @@ int dgp_batch_predict(dgp_batch b, const int* m, const double* const* Xs, double
     if (m[i] < 0) DGP_FAIL(b, -1, "dgp_batch_predict: site %d: m = %d", i, m[i]);
     if (m[i] == 0) continue;
     if (!Xs[i] || !mu_out[i]) DGP_FAIL(b, -1, "dgp_batch_predict: site %d: NULL grid or output", i);
-    if (!b->have_T[i])
+    const bool want_var = var_out != nullptr && var_out[i] != nullptr;
+    if (want_var && !b->have_T[i])
       DGP_FAIL(b, -1, "dgp_batch_predict: site %d is not factorised: call dgp_batch_factorize first (again after every "
                "dgp_batch_set_train / dgp_batch_nlml_grad; a site whose factorisation failed cannot predict)", i);
+    if (!want_var && !b->have_eval[i])
+      DGP_FAIL(b, -1, "dgp_batch_predict: site %d has no successful evaluation: the mean needs dgp_batch_nlml_grad or "
+               "dgp_batch_factorize first (again after every dgp_batch_set_train; a site whose evaluation failed cannot predict)", i);
     if (m[i] > mmax) mmax = m[i];
   }
   if (mmax == 0) return 0;
@@ -704,6 +748,80 @@ int dgp_batch_predict(dgp_batch b, const int* m, const double* const* Xs, double
       memcpy(mu_out[i] + m0, b->h_mu + (size_t)i * C, (size_t)pc.m[i] * 8);
       if (pc.var[i]) memcpy(var_out[i] + m0, b->h_var + (size_t)i * C, (size_t)pc.m[i] * 8);
     }
+  }
+  return 0;
+}
+
+// dgp_mean_functional_grad for every site of the batch, each step one launch over all sites: features, cross covariance
+// and mu of the points (the prediction kernels on the chunk slabs; Kx is kept) -> v = Kx' c -> gamma = U (U' v) on the U
+// slab (U = L^-T is intact after both evaluations: LAUUM writes Ky^-1 into A) -> both weighted contractions of dK/dtheta
+// -> the per-site reductions.  alpha, z and zpart, which later predictions and evaluations read, are not touched.
+int dgp_batch_mean_functional_grad(dgp_batch b, const int* m, const double* const* Xs, const double* const* c,
+                                   double* val_out, double* grad_out) {
+  if (!b) return -1;
+  if (!b->have_train || !m || !Xs || !c || !val_out || !grad_out)
+    DGP_FAIL(b, -1, "dgp_batch_mean_functional_grad: bad arguments (NULL pointer or no training data)");
+  if (b->pending) DGP_FAIL(b, -1, "dgp_batch_mean_functional_grad: an evaluation is in flight: call dgp_batch_nlml_grad_wait first");
+  const int G = b->G, C = DGP_BATCH_CHUNK, ndim = b->spec.ndim, P = b->spec.ntheta;
+  MfgTab mt;
+  memset(&mt, 0, sizeof(mt));
+  for (int i = 0; i < G; i++) {
+    if (m[i] < 0 || m[i] > C) DGP_FAIL(b, -1, "dgp_batch_mean_functional_grad: site %d: m = %d (0 <= m <= %d)", i, m[i], C);
+    if (m[i] == 0) continue;
+    if (!Xs[i] || !c[i]) DGP_FAIL(b, -1, "dgp_batch_mean_functional_grad: site %d: NULL points or weights", i);
+    if (!b->have_eval[i])
+      DGP_FAIL(b, -1, "dgp_batch_mean_functional_grad: site %d has no successful evaluation: call dgp_batch_nlml_grad or "
+               "dgp_batch_factorize first (again after every dgp_batch_set_train; a site whose evaluation failed has no adjoint)", i);
+    mt.m[i] = m[i];
+  }
+  for (int i = 0; i < G; i++) mt.tile0[i + 1] = mt.tile0[i] + (mt.m[i] == 0 ? 0 : ((mt.m[i] + 127) / 128 + b->nb[i]) * 2 * b->nb[i]);
+  memset(val_out, 0, sizeof(double) * G);
+  memset(grad_out, 0, sizeof(double) * G * P);
+  if (mt.tile0[G] == 0) return 0;
+  CK(b, cudaSetDevice(b->device));
+  int rc;
+  if ((rc = b_predict_alloc(b))) return rc;
+  if ((rc = b_mfg_alloc(b))) return rc;
+  cudaStream_t st = b->stream;
+  PredChunk pk, pm;   // pk: write the cross covariance (kept for v = Kx' c); pm: the mean alone
+  memset(&pk, 0, sizeof(pk));
+  memset(&pm, 0, sizeof(pm));
+  for (int i = 0; i < G; i++) {
+    pk.m[i] = pm.m[i] = mt.m[i];
+    pk.var[i] = mt.m[i] > 0;
+    if (mt.m[i] == 0) continue;
+    const int mpad = (mt.m[i] + 127) / 128 * 128;
+    memcpy(b->h_xs + (size_t)i * C * DGP_MAX_COLS, Xs[i], (size_t)mt.m[i] * ndim * 8);
+    memcpy(b->h_c + (size_t)i * C, c[i], (size_t)mt.m[i] * 8);
+    memset(b->h_c + (size_t)i * C + mt.m[i], 0, (size_t)(mpad - mt.m[i]) * 8);
+  }
+  CK(b, cudaMemcpyAsync(b->Xs, b->h_xs, (size_t)G * C * DGP_MAX_COLS * 8, cudaMemcpyHostToDevice, st));
+  CK(b, cudaMemcpyAsync(b->cvec, b->h_c, (size_t)G * C * 8, cudaMemcpyHostToDevice, st));
+  const unsigned gl = (unsigned)((b->ld + 255) / 256);
+  k_pred_features_b<<<dim3(C / 256, G), 256, 0, st>>>(b->spec, pk, b->theta, b->Xs, b->Xws, b->means, C);
+  k_cov_rect_pred_b<<<dim3(C / 32, b->NB, G), 256, 0, st>>>(b->spec, b->sd, pk, b->theta, b->Xws, b->Xw, b->noise, b->alpha,
+                                                            b->Kx, b->dot, C);
+  k_pred_finish_b<<<dim3(C / 256, G), 256, 0, st>>>(b->spec, b->sd, pm, b->theta, b->Xws, b->means, b->dot, b->vpart, b->mu,
+                                                    b->var, C);
+  // gamma = Ky^-1 (Kx*' c) = U (U' v)
+  k_colsum_weighted_b<<<dim3(gl, G), 256, 0, st>>>(b->sd, mt, b->Kx, b->cvec, b->vvec, C);
+  k_upperT_gemv_part_b<<<dim3(b->NB, b->NB, G), 256, 0, st>>>(b->sd, b->U, b->vvec, b->gzpart);
+  k_upperT_gemv_sum_b<<<dim3(gl, G), 256, 0, st>>>(b->sd, b->gzpart, b->tmpz);
+  k_upper_gemv_b<<<dim3((unsigned)(b->ld / 8), G), 256, 0, st>>>(b->sd, b->U, b->tmpz, b->gam);
+  // the two weighted contractions of dK/dtheta, then the per-site reductions
+  k_wgrad_b<<<mt.tile0[G], 128, 0, st>>>(b->spec, b->sd, mt, b->theta, b->Xws, b->Xw, b->cvec, b->gam, b->alpha, b->wpart, C,
+                                         b->mfg_pstride);
+  k_mfg_finish_b<<<dim3(P + 1, G), 256, 0, st>>>(b->spec, b->sd, mt, b->theta, b->wpart, b->cvec, b->mu, b->Xs, b->gam,
+                                                 b->alpha, b->X, b->mfg, C, b->mfg_pstride);
+  b->launches += 9;
+  CK(b, cudaGetLastError());
+  CK(b, cudaMemcpyAsync(b->h_mfg, b->mfg, (size_t)G * (1 + DGP_MAX_THETA) * 8, cudaMemcpyDeviceToHost, st));
+  CK(b, cudaStreamSynchronize(st));
+  for (int i = 0; i < G; i++) {
+    if (mt.m[i] == 0) continue;
+    const double* o = b->h_mfg + (size_t)i * (1 + DGP_MAX_THETA);
+    val_out[i] = o[0];
+    memcpy(grad_out + (size_t)i * P, o + 1, sizeof(double) * P);
   }
   return 0;
 }

@@ -572,17 +572,18 @@ k_flux_reduce(const double* __restrict__ D, long long ld, const double* __restri
 //   gamma = Ky^-1 Kx* c  (adjoint of the solve).  Both sums are rank-1-weighted contractions of dK/dtheta:
 // k_wgrad: part[cta][t] = sgn * sum_{i in rows, j in cols of this 128x64 tile} wa_i wb_j dk(xa_i, xb_j)/dtheta_t.
 // grid = (col blocks of 64, row blocks of 128), block = 128 (thread = row); wa / wb are zero on padding.
-__global__ void __launch_bounds__(128)
-k_wgrad(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta, const double* __restrict__ XwA,
-        const double* __restrict__ XwB, const double* __restrict__ wa, const double* __restrict__ wb, double sgn,
-        double* __restrict__ part) {
+// (bx, by) = (column block, row block) of the CTA, ncb = column blocks: part index by * ncb + bx.
+__device__ __forceinline__ void wgrad_body(const dgp_spec& spec, const double* __restrict__ theta, const double* __restrict__ XwA,
+                                           const double* __restrict__ XwB, const double* __restrict__ wa,
+                                           const double* __restrict__ wb, double sgn, double* __restrict__ part, int bx, int by,
+                                           int ncb) {
   __shared__ CovC cc;
   __shared__ double xaT[DGP_XS * 128];
   __shared__ double xb[64 * DGP_XS];
   __shared__ double wbs[64];
   __shared__ double red[4 * DGP_MAX_TERMS * NSLOT];
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  const size_t r0 = (size_t)blockIdx.y * 128, c0b = (size_t)blockIdx.x * 64;
+  const size_t r0 = (size_t)by * 128, c0b = (size_t)bx * 64;
   cov_compile(&cc, spec, theta, 0.0, t, 128);
   for (int e = t; e < 128 * DGP_XS; e += 128) xaT[(e % DGP_XS) * 128 + e / DGP_XS] = XwA[r0 * DGP_XS + e];
   for (int e = t; e < 64 * DGP_XS; e += 128) xb[e] = XwB[c0b * DGP_XS + e];
@@ -617,8 +618,14 @@ k_wgrad(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta,
         for (int k = 0; k < NSLOT; k++)
           if (term_slot_theta(cc.t[term], k) == t)
             for (int w4 = 0; w4 < 4; w4++) s += red[(w4 * DGP_MAX_TERMS + term) * NSLOT + k];
-    part[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * DGP_MAX_THETA + t] = sgn * s;
+    part[((size_t)by * ncb + bx) * DGP_MAX_THETA + t] = sgn * s;
   }
+}
+__global__ void __launch_bounds__(128)
+k_wgrad(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta, const double* __restrict__ XwA,
+        const double* __restrict__ XwB, const double* __restrict__ wa, const double* __restrict__ wb, double sgn,
+        double* __restrict__ part) {
+  wgrad_body(spec, theta, XwA, XwB, wa, wb, sgn, part, blockIdx.x, blockIdx.y, gridDim.x);
 }
 
 // ------------------------------------------------------------------ NLML gradient contraction as its own pass
@@ -735,24 +742,27 @@ k_grad_contract_b(const __grid_constant__ dgp_spec spec, const __grid_constant__
 }
 
 // v[j] = sum_p c[p] Kx[p, j]   (p < mpad), grid = npad / 256
-__global__ void __launch_bounds__(256)
-k_colsum_weighted(const double* __restrict__ Kx, long long ld, const double* __restrict__ c, int mpad, double* __restrict__ v) {
-  const int j = blockIdx.x * 256 + threadIdx.x;
-  if (j >= ld) return;
+__device__ __forceinline__ void colsum_weighted_body(const double* __restrict__ Kx, long long ld, const double* __restrict__ c,
+                                                     int mpad, double* __restrict__ v, int npad, int j) {
+  if (j >= npad) return;
   double s = 0.0;
   for (int p = 0; p < mpad; p++) s = fma(c[p], Kx[(size_t)p * ld + j], s);
   v[j] = s;
 }
+__global__ void __launch_bounds__(256)
+k_colsum_weighted(const double* __restrict__ Kx, long long ld, const double* __restrict__ c, int mpad, double* __restrict__ v) {
+  colsum_weighted_body(Kx, ld, c, mpad, v, (int)ld, blockIdx.x * 256 + threadIdx.x);
+}
 
 // block b < ntheta: grad[b] = sum_parts part[.][b] + mean-parameter terms + learned-noise term; block ntheta: F = c'mu.
 // out[0] = F, out[1 + b] = dF/dtheta_b.
-__global__ void __launch_bounds__(256)
-k_mfg_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta, const double* __restrict__ part,
-             int nparts, const double* __restrict__ c, const double* __restrict__ mu, const double* __restrict__ Xs, int m,
-             const double* __restrict__ gamma, const double* __restrict__ alpha, const double* __restrict__ X, int n,
-             double* __restrict__ out) {
+__device__ __forceinline__ void mfg_finish_body(const dgp_spec& spec, const double* __restrict__ theta,
+                                                const double* __restrict__ part, int nparts, const double* __restrict__ c,
+                                                const double* __restrict__ mu, const double* __restrict__ Xs, int m,
+                                                const double* __restrict__ gamma, const double* __restrict__ alpha,
+                                                const double* __restrict__ X, int n, double* __restrict__ out, int b) {
   __shared__ double red[256];
-  const int tid = threadIdx.x, b = blockIdx.x;
+  const int tid = threadIdx.x;
   double s = 0.0;
   if (b == spec.ntheta) {
     for (int p = tid; p < m; p += 256) s = fma(c[p], mu[p], s);
@@ -786,5 +796,70 @@ k_mfg_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ t
     __syncthreads();
   }
   if (tid == 0) out[(b == spec.ntheta) ? 0 : 1 + b] = red[0];
+}
+__global__ void __launch_bounds__(256)
+k_mfg_finish(const __grid_constant__ dgp_spec spec, const double* __restrict__ theta, const double* __restrict__ part,
+             int nparts, const double* __restrict__ c, const double* __restrict__ mu, const double* __restrict__ Xs, int m,
+             const double* __restrict__ gamma, const double* __restrict__ alpha, const double* __restrict__ X, int n,
+             double* __restrict__ out) {
+  mfg_finish_body(spec, theta, part, nparts, c, mu, Xs, m, gamma, alpha, X, n, out, blockIdx.x);
+}
+
+// ------------------------------------------------------------------ batched adjoint of the posterior mean
+// (dgp_batch_mean_functional_grad).  Per site s with m[s] > 0: the chunk slabs of the prediction hold its points (Xs, Xws,
+// mu: [site][chunk]..., Kx: [site][chunk][ld]), c / v / gamma are [site][chunk] / [site][ld] / [site][ld], and its partials
+// [site][pstride] are laid out as those of dgp_mean_functional_grad for ITS OWN sizes: mpad = 128 ceil(m / 128) and
+// npad = 128 nb, (mpad / 128 + nb) (npad / 64) tiles, the first mpad / 128 row blocks c x alpha, the rest -gamma x alpha.
+// The bodies and the order of every sum are the single-site ones, so the results are bit-identical to it.
+struct MfgTab {
+  int m[DGP_BATCH_MAX];
+  int tile0[DGP_BATCH_MAX + 1];   // prefix of the per-site tile counts (mpad / 128 + nb) (npad / 64)
+};
+
+// v[s][j] = sum_{p < mpad_s} c[s][p] Kx[s][p, j], j < npad_s;  grid = (ceil(ld / 256), sites)
+__global__ void __launch_bounds__(256)
+k_colsum_weighted_b(const __grid_constant__ SiteDims sd, const __grid_constant__ MfgTab mt, const double* __restrict__ Kx,
+                    const double* __restrict__ c, double* __restrict__ v, int chunk) {
+  const int st = blockIdx.y;
+  const size_t cc = (size_t)st * chunk;
+  colsum_weighted_body(Kx + cc * sd.ld, sd.ld, c + cc, (mt.m[st] + 127) / 128 * 128, v + (size_t)st * sd.ld, sd.nb[st] * 128,
+                       blockIdx.x * 256 + threadIdx.x);
+}
+
+// both weighted contractions of every site in one launch: grid = mt.tile0[sites] (prefix lookup, no empty CTAs)
+__global__ void __launch_bounds__(128)
+k_wgrad_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ SiteDims sd, const __grid_constant__ MfgTab mt,
+          const double* __restrict__ theta, const double* __restrict__ Xws, const double* __restrict__ Xw,
+          const double* __restrict__ c, const double* __restrict__ gamma, const double* __restrict__ alpha,
+          double* __restrict__ part, int chunk, long long pstride) {
+  int st = 0;
+#pragma unroll 1
+  for (int i = 1; i < sd.count; i++) if ((int)blockIdx.x >= mt.tile0[i]) st = i;
+  const int t = (int)blockIdx.x - mt.tile0[st], ncb = sd.nb[st] * 2, mb = (mt.m[st] + 127) / 128;
+  const size_t v = (size_t)st * sd.ld, cc = (size_t)st * chunk;
+  const double* th = theta + st * DGP_MAX_THETA;
+  double* pt = part + (size_t)st * pstride;
+  if (t < mb * ncb) {
+    wgrad_body(spec, th, Xws + cc * DGP_XS, Xw + v * DGP_XS, c + cc, alpha + v, 1.0, pt, t % ncb, t / ncb, ncb);
+  } else {
+    const int u = t - mb * ncb;
+    wgrad_body(spec, th, Xw + v * DGP_XS, Xw + v * DGP_XS, gamma + v, alpha + v, -1.0, pt + (size_t)mb * ncb * DGP_MAX_THETA,
+               u % ncb, u / ncb, ncb);
+  }
+}
+
+// grid = (ntheta + 1, sites); out: [site][1 + DGP_MAX_THETA]
+__global__ void __launch_bounds__(256)
+k_mfg_finish_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ SiteDims sd, const __grid_constant__ MfgTab mt,
+               const double* __restrict__ theta, const double* __restrict__ part, const double* __restrict__ c,
+               const double* __restrict__ mu, const double* __restrict__ Xs, const double* __restrict__ gamma,
+               const double* __restrict__ alpha, const double* __restrict__ X, double* __restrict__ out, int chunk,
+               long long pstride) {
+  const int st = blockIdx.y, m = mt.m[st], nb = sd.nb[st];
+  if (m == 0) return;
+  const size_t v = (size_t)st * sd.ld, cc = (size_t)st * chunk;
+  mfg_finish_body(spec, theta + st * DGP_MAX_THETA, part + (size_t)st * pstride, ((m + 127) / 128 + nb) * 2 * nb, c + cc, mu + cc,
+                  Xs + cc * DGP_MAX_COLS, m, gamma + v, alpha + v, X + v * DGP_MAX_COLS, sd.n[st],
+                  out + (size_t)st * (1 + DGP_MAX_THETA), blockIdx.x);
 }
 }  // namespace dgp

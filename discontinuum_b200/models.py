@@ -198,9 +198,11 @@ class RatingGPMarginalB200(RatingDataMixin, MarginalB200):
 
     def fit(self, covariates, target, target_unc=None, iterations=100, optimizer=None, learning_rate=None,
             early_stopping=False, patience=60, scheduler=True, resume=False, monotonic_penalty_weight: float = 0.0,
-            grid_size: int = 64, monotonic_penalty_interval: int = 1, **kw):
+            grid_size: int = 64, monotonic_penalty_interval: int = 1, penalty_generator: Optional[torch.Generator] = None,
+            **kw):
         """src/rating_gp/models/gpytorch.py:81-202: optional penalty on negative dQ/dStage of the posterior mean over a
-        random (time uniform, stage log-uniform) grid, every `monotonic_penalty_interval` iterations."""
+        random (time uniform, stage log-uniform) grid, every `monotonic_penalty_interval` iterations.  The grids are drawn
+        from torch's global generator, or from `penalty_generator`."""
         if monotonic_penalty_weight <= 0:
             return super().fit(covariates=covariates, target=target, target_unc=target_unc, iterations=iterations,
                                optimizer=optimizer, learning_rate=learning_rate, early_stopping=early_stopping,
@@ -213,7 +215,7 @@ class RatingGPMarginalB200(RatingDataMixin, MarginalB200):
             step["i"] += 1
             if monotonic_penalty_interval > 1 and (step["i"] % monotonic_penalty_interval) != 0:
                 return torch.zeros((), dtype=torch.float64)
-            grid = monotonic_penalty_grid(self.dm.X, grid_size)
+            grid = monotonic_penalty_grid(self.dm.X, grid_size, generator=penalty_generator)
             pen = _MonotonicPenalty.apply(self.model.natural(), self, grid, 1e-3)
             if monotonic_penalty_interval > 1:
                 pen = pen * float(monotonic_penalty_interval)
@@ -225,15 +227,16 @@ class RatingGPMarginalB200(RatingDataMixin, MarginalB200):
                            penalty_weight=float(monotonic_penalty_weight), **kw)
 
 
-def monotonic_penalty_grid(X: np.ndarray, grid_size: int = 64, time_dim: int = 0, stage_dim: int = 1) -> np.ndarray:
-    """The reference's random grid (rating_gp/models/gpytorch.py:139-158): float32 draws from torch's global generator,
-    time uniform over the training range (drawn first), stage log-uniform."""
+def monotonic_penalty_grid(X: np.ndarray, grid_size: int = 64, time_dim: int = 0, stage_dim: int = 1,
+                           generator: Optional[torch.Generator] = None) -> np.ndarray:
+    """The reference's random grid (rating_gp/models/gpytorch.py:139-158): float32 draws from torch's global generator
+    (or from `generator`), time uniform over the training range (drawn first), stage log-uniform."""
     x_min, x_max = X.min(axis=0), X.max(axis=0)
-    u_time = torch.rand((grid_size,), dtype=torch.float32)
+    u_time = torch.rand((grid_size,), dtype=torch.float32, generator=generator)
     time_grid = u_time * (x_max[time_dim] - x_min[time_dim]) + x_min[time_dim]
     eps = 1e-6
     log_xmin, log_xmax = float(np.log(x_min[stage_dim] + eps)), float(np.log(x_max[stage_dim] + eps))
-    u_stage = torch.rand((grid_size,), dtype=torch.float32)
+    u_stage = torch.rand((grid_size,), dtype=torch.float32, generator=generator)
     stage_grid = torch.exp(u_stage * (log_xmax - log_xmin) + log_xmin)
     cols = [None, None]
     cols[time_dim], cols[stage_dim] = time_grid, stage_grid

@@ -18,7 +18,7 @@ import torch
 
 from . import capi
 from .engine import JITTERS, MIN_VARIANCE
-from .models import LOADEST_FIXED_NOISE, loadest_spec
+from .models import LOADEST_FIXED_NOISE, loadest_spec, monotonic_penalty_grid
 from .spec import GPModule
 
 
@@ -213,6 +213,13 @@ class _Site:
     history: List[float] = field(default_factory=list)
     failed: Optional[str] = None
     bad_streak: int = 0
+    # early stopping (MarginalB200.fit's rule) and the monotonicity penalty
+    best: float = float("inf")
+    patience_counter: int = 0
+    stopped_at: Optional[int] = None
+    good_iters: int = 0
+    penalty_gen: Optional[torch.Generator] = None
+    penalty: Optional[float] = None
 
 
 def _groups(order: List[int], group: int) -> List[List[int]]:
@@ -262,13 +269,31 @@ def _predict_group(batch: capi.BatchEngine, grp: List[_Site], want: List[bool], 
         res["var"] = observed_variance(s.module.spec, thetas[k], var, s.noise, grids[k].shape[0])
 
 
+@dataclass
+class PenaltyConfig:
+    """The rating-gp monotonicity penalty of a driver fit (RatingGP.fit's monotonic_penalty_weight / grid_size /
+    monotonic_penalty_interval); site `idx` draws its grids from torch.Generator().manual_seed(seed + idx)."""
+    weight: float
+    grid_size: int = 64
+    interval: int = 1
+    seed: int = 0
+    fd_eps: float = 1e-3
+
+
+_MIN_IMPROVEMENT = 1e-6   # MarginalB200.fit's early-stopping threshold
+
+
 class _GroupRun:
     """One group of sites on one batch handle: `launch()` enqueues the next optimiser iteration's NLML + gradient evaluation of
     the whole group, `finish()` collects it and takes the host step.  Two of these in flight on one GPU fill each other's
     latency-bound stretches (measured: +1 % for two groups of n ~ 7k sites, +8 % for two groups of n ~ 2-3k sites)."""
 
-    def __init__(self, grp, batch, kind, iterations, lr, scheduler, patience, st, timed):
+    def __init__(self, grp, batch, kind, iterations, lr, scheduler, patience, st, timed, early_stopping=False, penalty=None):
         self.grp, self.batch, self.kind, self.left, self.st = grp, batch, kind, int(iterations), st
+        self.iterations, self.patience, self.early_stopping, self.pen = int(iterations), int(patience), bool(early_stopping), penalty
+        if penalty is not None:
+            for s in grp:
+                s.penalty_gen = torch.Generator().manual_seed(int(penalty.seed) + int(s.idx))
         self.G = len(grp)
         batch.set_train(grp[0].module.spec.to_c(), [(s.X, s.y, s.noise) for s in grp])
         batch.set_timing(timed)
@@ -284,11 +309,14 @@ class _GroupRun:
     def launch(self):
         if self.left <= 0:
             return False
-        self.alive = np.array([s.failed is None for s in self.grp])
+        self.alive = np.array([s.failed is None and s.stopped_at is None for s in self.grp])
         if not self.alive.any():
             self.left = 0
             return False
+        stopped = np.array([s.stopped_at is not None for s in self.grp])
+        kept = self.opt.raw[stopped].copy()      # a stopped site keeps its last parameters as they are
         self.kind.project_raw(self.opt.raw, self.opt.modules, [s.X for s in self.grp])
+        self.opt.raw[stopped] = kept
         self.nat, self.dnat, self.lp, self.dlp = self.opt.chain()
         self.theta = np.ascontiguousarray(self.nat)
         self.batch.nlml_grad_launch(self.theta)
@@ -301,6 +329,8 @@ class _GroupRun:
         self.inflight = False
         self.left -= 1
         st["evals"] += 1
+        st["site_evals"] += G
+        st["wasted_site_evals"] += int(G - alive.sum())   # stopped / failed sites still evaluated with their group
         if self.timed:
             st["gpu_eval_ms"] += sum(self.batch.last_timing())
         bad = alive & ((info != 0) | ~np.isfinite(val))
@@ -317,8 +347,17 @@ class _GroupRun:
                     break
         t0 = time.perf_counter()
         obj = (val - self.lp) / self.ns
-        graw = (grad - self.dlp) * self.dnat / self.ns[:, None]
         ok = alive & ~bad & np.isfinite(obj)
+        if self.pen is None:
+            graw = (grad - self.dlp) * self.dnat / self.ns[:, None]
+        else:
+            t1 = time.perf_counter()
+            wpen, dpen = self._penalty(ok)
+            st["penalty_s"] += time.perf_counter() - t1
+            t0 += time.perf_counter() - t1
+            obj = obj + wpen
+            graw = ((grad - self.dlp) / self.ns[:, None] + dpen) * self.dnat
+            ok &= np.isfinite(obj)
         for k, s in enumerate(grp):
             if not alive[k]:
                 continue
@@ -330,15 +369,65 @@ class _GroupRun:
                 if s.bad_streak > 10:
                     s.failed = f"more than 10 consecutive bad objectives (info={int(info[k])})"
         self.opt.step(np.where(ok[:, None], graw, 0.0), obj, ok)
+        if self.early_stopping:   # MarginalB200.fit: bad iterations neither count nor reset the counter
+            for k in np.nonzero(ok)[0]:
+                s = grp[k]
+                if s.history[-1] < s.best - _MIN_IMPROVEMENT:
+                    s.best, s.patience_counter = s.history[-1], 0
+                else:
+                    s.patience_counter += 1
+                if s.patience_counter >= self.patience:
+                    s.stopped_at = self.iterations - self.left
         st["host_step_s"] += time.perf_counter() - t0
         if self.left <= 0:
             self.opt.push()
+
+    def _penalty(self, ok):
+        """(w pen [G], w d pen / d natural theta [G, P]) of the sites whose evaluation is good (zeros elsewhere and between
+        penalty iterations): RatingGP.fit's _MonotonicPenalty for the whole group, with one mean-only dgp_batch_predict of
+        every site's [grid; grid + eps e_stage] at the evaluated theta and one dgp_batch_mean_functional_grad of c'mu with
+        the active set fixed.  Every `interval`-th good iteration of a site, scaled by the interval."""
+        pen, G, gs, eps = self.pen, self.G, int(self.pen.grid_size), float(self.pen.fd_eps)
+        wpen, dpen = np.zeros(G), np.zeros((G, self.theta.shape[1]))
+        pts: List[Optional[np.ndarray]] = [None] * G
+        for k, s in enumerate(self.grp):
+            if not ok[k]:
+                continue
+            s.good_iters += 1
+            if pen.interval > 1 and s.good_iters % pen.interval != 0:
+                continue
+            grid = monotonic_penalty_grid(s.X, gs, generator=s.penalty_gen)
+            plus = grid.copy()
+            plus[:, 1] += eps
+            pts[k] = np.ascontiguousarray(np.concatenate([grid, plus], axis=0))
+        if all(p is None for p in pts):
+            return wpen, dpen
+        out = self.batch.predict(pts, want_var=False)
+        cs: List[Optional[np.ndarray]] = [None] * G
+        for k, s in enumerate(self.grp):
+            if pts[k] is None:
+                continue
+            mu = out[k][0]
+            d = (mu[gs:] - mu[:gs]) / eps
+            active = d < 0.0
+            c = np.zeros(2 * gs)
+            c[:gs][active] = 1.0 / (gs * eps)
+            c[gs:][active] = -1.0 / (gs * eps)
+            cs[k] = c
+            s.penalty = float(np.maximum(-d, 0.0).mean())
+            wpen[k] = pen.weight * (s.penalty * pen.interval)
+        _, g = self.batch.mean_functional_grad(pts, cs)
+        for k in range(G):
+            if pts[k] is not None:
+                dpen[k] = pen.weight * (g[k] * pen.interval)
+        return wpen, dpen
 
 
 def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int = 0, group: int = 16,
                     predict: Optional[Dict[int, np.ndarray]] = None, lr: float = 0.05, scheduler: bool = True,
                     patience: int = 60, model="loadest", stats: Optional[dict] = None, concurrency: Optional[int] = None,
-                    lanes: int = 2) -> Dict[int, dict]:
+                    lanes: int = 2, early_stopping: bool = False, monotonic_penalty_weight: float = 0.0, grid_size: int = 64,
+                    monotonic_penalty_interval: int = 1, penalty_seed: int = 0) -> Dict[int, dict]:
     """Fit one GP per site on this rank.  sites: {index: (X, y[, noise])} in model space; model: "loadest", "rating" or a
     kind object (see LoadestKind).  Returns {index: {"theta", "objective", "history", "failed", "n", "mu", "var",
     "var_latent"}} ("var" follows `likelihood(model(x))` like MarginalB200.predict).
@@ -354,14 +443,35 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
     marked failed, as MarginalB200.fit gives up.
     The sites of a finished group that have a grid in `predict` are factorised and predicted on the group's own handle
     (dgp_batch_factorize + dgp_batch_predict: every site's numbers equal a per-site capi.Engine factorize + predict bit for bit).
-    `concurrency` selects the round-1 per-handle pipelines instead (fit_sites_local_per_handle)."""
+    `early_stopping` applies MarginalB200.fit's rule per site (best objective, improvement 1e-6, stop when `patience`
+    good iterations in a row did not improve it; bad iterations neither count nor reset): a stopped site is frozen at its
+    last parameters ("stopped_at": the iteration it stopped after, else None) and a group ends when every site has stopped
+    or failed.  Stopped and failed sites are still evaluated with their group until it ends.
+    `monotonic_penalty_weight` > 0 (rating kind only) adds RatingGP.fit's penalty on negative dQ/dstage of the posterior
+    mean over a random grid of `grid_size` points (<= 512: grid and shifted grid share one 1024-row chunk), drawn by site
+    `idx` from torch.Generator().manual_seed(penalty_seed + idx), every `monotonic_penalty_interval`-th good iteration
+    and scaled by the interval; its gradient comes from dgp_batch_mean_functional_grad.  "penalty" holds the last
+    (unweighted) value.  Neither depends on `lanes`, on the group a site lands in, or on the rank.
+    `concurrency` selects the round-1 per-handle pipelines instead (fit_sites_local_per_handle), which has neither."""
+    pen = None
+    if monotonic_penalty_weight > 0.0:
+        if getattr(_kind(model), "name", None) != "rating":
+            raise ValueError("monotonic_penalty_weight applies to rating gauges only (model='rating')")
+        if not 1 <= int(grid_size) <= capi.BATCH_PREDICT_CHUNK // 2:
+            raise ValueError(f"grid_size must be in [1, {capi.BATCH_PREDICT_CHUNK // 2}]: the grid and its shifted copy share "
+                             f"one {capi.BATCH_PREDICT_CHUNK}-row chunk")
+        if int(monotonic_penalty_interval) < 1:
+            raise ValueError("monotonic_penalty_interval must be >= 1")
+        pen = PenaltyConfig(float(monotonic_penalty_weight), int(grid_size), int(monotonic_penalty_interval), int(penalty_seed))
     if concurrency is not None:
+        if early_stopping or pen is not None:
+            raise ValueError("early_stopping and the monotonicity penalty need the batch driver (concurrency=None)")
         return fit_sites_local_per_handle(sites, iterations=iterations, device=device, concurrency=concurrency or 4,
                                           predict=predict, lr=lr, scheduler=scheduler, patience=patience)
     kind = _kind(model)
     t_start = time.perf_counter()
     st = {"groups": 0, "evals": 0, "gpu_eval_ms": 0.0, "fit_wall_s": 0.0, "predict_s": 0.0, "host_step_s": 0.0, "retries": 0,
-          "lanes": 1}
+          "lanes": 1, "penalty_s": 0.0, "site_evals": 0, "wasted_site_evals": 0}
     results: Dict[int, dict] = {}
     if not sites:
         if stats is not None:
@@ -393,7 +503,9 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
             with torch.no_grad():
                 theta = s.module.natural().numpy().astype(np.float64)
             res_of[s.idx] = {"theta": theta, "history": s.history, "objective": s.history[-1] if s.history else None,
-                             "failed": s.failed, "n": int(s.X.shape[0])}
+                             "failed": s.failed, "n": int(s.X.shape[0]), "stopped_at": s.stopped_at}
+            if pen is not None:
+                res_of[s.idx]["penalty"] = s.penalty
         want = [predict is not None and s.idx in predict and s.failed is None for s in grp]
         if any(want):
             own = batch is None
@@ -426,7 +538,7 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
                 members = pending.pop(0) if lane == 0 else pending.pop()   # lane 0 from the large end, the others from the small end
                 st["groups"] += 1
                 return _GroupRun([state[i] for i in members], handles[lane], kind, iterations, lr, scheduler, patience, st,
-                                 stats is not None)
+                                 stats is not None, early_stopping, pen)
 
             # rolling: every lane always has an evaluation in flight (wait -> host step -> launch the next one), so the GPU
             # works on one group while the host steps the other
@@ -596,9 +708,11 @@ def fit_sites_local_per_handle(sites: Dict[int, tuple], iterations: int = 100, d
 
 def fit_sites(sites: Dict[int, tuple], iterations: int = 100, predict: Optional[Dict[int, np.ndarray]] = None,
               group: int = 16, dist=None, device: int = 0, model="loadest", stats: Optional[dict] = None,
-              concurrency: Optional[int] = None, lanes: int = 2) -> Optional[Dict[int, dict]]:
+              concurrency: Optional[int] = None, lanes: int = 2, early_stopping: bool = False, patience: int = 60,
+              monotonic_penalty_weight: float = 0.0, grid_size: int = 64, monotonic_penalty_interval: int = 1,
+              penalty_seed: int = 0) -> Optional[Dict[int, dict]]:
     """Shard `sites` (every rank holds the same dict, or at least the same keys and sizes) over the ranks of
-    `dist`, fit this rank's share, gather everything on rank 0."""
+    `dist`, fit this rank's share, gather everything on rank 0.  The fit options are fit_sites_local's."""
     world = dist.get_world_size() if dist is not None and dist.is_initialized() else 1
     rank = dist.get_rank() if world > 1 else 0
     keys = sorted(sites)
@@ -606,7 +720,9 @@ def fit_sites(sites: Dict[int, tuple], iterations: int = 100, predict: Optional[
     mine = [keys[i] for i in assign_sites(costs, world)[rank]]
     local = fit_sites_local({k: sites[k] for k in mine}, iterations=iterations, device=device, group=group,
                             predict={k: predict[k] for k in mine} if predict else None, model=model, stats=stats,
-                            concurrency=concurrency, lanes=lanes)
+                            concurrency=concurrency, lanes=lanes, early_stopping=early_stopping, patience=patience,
+                            monotonic_penalty_weight=monotonic_penalty_weight, grid_size=grid_size,
+                            monotonic_penalty_interval=monotonic_penalty_interval, penalty_seed=penalty_seed)
     return gather_results(local, dist)
 
 

@@ -264,10 +264,22 @@ int dgp_batch_nlml_grad_wait(dgp_batch b, double* nlml_out, double* grad_out, in
 int dgp_batch_factorize(dgp_batch b, const double* theta, const double* jitter, double* nlml_out, int* info_out);
 /* Posterior mean m(x*) + K*x alpha and LATENT variance k** - |L^-1 Kx*|^2 of every site on its own grid:
  * m[s] points Xs[s][m[s], ndim] -> mu_out[s][m[s]], var_out[s][m[s]] (host pointers; var_out == NULL or var_out[s] == NULL:
- * mean only; m[s] == 0: site skipped).  Needs a successful dgp_batch_factorize of every site with m[s] > 0 since the last
- * dgp_batch_set_train / dgp_batch_nlml_grad; fails (< 0) otherwise.  Grids are walked in chunks of 1024 rows, each chunk
+ * mean only; m[s] == 0: site skipped).  The variance of a site needs its successful dgp_batch_factorize since the last
+ * dgp_batch_set_train / dgp_batch_nlml_grad; the mean alone needs a successful dgp_batch_factorize or dgp_batch_nlml_grad
+ * of the site (as dgp_predict); fails (< 0) otherwise.  Grids are walked in chunks of 1024 rows, each chunk
  * of all sites in one launch sequence; the results equal dgp_predict's bit for bit. */
 int dgp_batch_predict(dgp_batch b, const int* m, const double* const* Xs, double* const* mu_out, double* const* var_out);
+/* Batch form of dgp_mean_functional_grad: for every site s with m[s] > 0, F_s = sum_p c[s][p] mu_s(Xs[s][p]) and
+ * dF_s/dtheta_s (natural parameters, including mean and learned-noise parameters) at the theta of the site's last
+ * successful dgp_batch_nlml_grad or dgp_batch_factorize.  m[s] <= 1024; m[s] == 0: site skipped (val 0, grad zeros).
+ * val_out[nsites], grad_out[nsites][ntheta] (host).  Results equal dgp_mean_functional_grad of a per-site handle bit for bit.
+ * Fails (< 0) on NULL pointers, m[s] > 1024, a site with m[s] > 0 whose last evaluation did not succeed (or none since
+ * dgp_batch_set_train), and while an evaluation is in flight.  Each step is one launch over all sites.  The first call on a
+ * handle adds the adjoint slabs, once: 8 max_sites x (1024 + max_pad (3 + max_pad / 128) + (8 + max_pad / 128)
+ * (max_pad / 64) 48 + 49) B on the device, next to the prediction slabs (which it also uses and allocates if
+ * dgp_batch_predict has not), and 8 max_sites x 1073 B of pinned host memory.  Later calls allocate nothing. */
+int dgp_batch_mean_functional_grad(dgp_batch b, const int* m, const double* const* Xs, const double* const* c,
+                                   double* val_out, double* grad_out);
 /* Parity accessor: alpha of one site after an evaluation. */
 int dgp_batch_get_alpha(dgp_batch b, int site, double* alpha_out);
 long long dgp_batch_launch_count(dgp_batch b);
