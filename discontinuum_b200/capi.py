@@ -85,6 +85,7 @@ _SIGNATURES = [
     ("dgp_set_debug_kinv", C.c_int, [_P, C.c_int]),
     ("dgp_get_kinv", C.c_int, [_P, _P, C.c_int]),
     ("dgp_get_linv", C.c_int, [_P, _P, C.c_int]),
+    ("dgp_get_uinv", C.c_int, [_P, _P, C.c_int]),
     ("dgp_gemm_nt", C.c_int, [_P, _P, C.c_longlong, _P, C.c_longlong, _P, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int]),
     ("dgp_batch_create", C.c_int, [C.POINTER(_P), C.c_int, C.c_int, C.c_int, _P]),
     ("dgp_batch_destroy", C.c_int, [_P]),
@@ -562,6 +563,12 @@ class Engine:
         T, p, dev = self._square_out(out)
         self._check(self.lib.dgp_get_linv(self._h, p, dev), "dgp_get_linv")
         return T
+
+    def uinv(self, out=None):
+        """U = L^-T [n, n], upper triangular, of the last nlml_grad or factorize (the LAUUM's operand)."""
+        U, p, dev = self._square_out(out)
+        self._check(self.lib.dgp_get_uinv(self._h, p, dev), "dgp_get_uinv")
+        return U
 
     def gemm_nt(self, A, B, Cm, mode: int = 0):
         """Cm (=, +=, -=) A @ B.T on CUDA float64 tensors (row-major, contiguous)."""

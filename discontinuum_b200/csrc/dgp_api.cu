@@ -31,6 +31,7 @@
 #include "../../include/dgp.h"
 #include "dgp_cov.cuh"
 #include "dgp_gemm.cuh"
+#include "dgp_lauum8.cuh"
 #include "dgp_panel.cuh"
 #include "dgp_potf2.cuh"
 
@@ -65,6 +66,24 @@ constexpr int STRIP_BLOCKS = 8;
 static_assert(STRIP_BLOCKS % PANEL_BLOCKS == 0, "a strip holds whole panels");
 // the merges of the inverse are launched as the factorisation passes them up to this many block columns (single-site engine)
 constexpr int EAGER_INV_MAX_NB = 96;
+// sites of at least this many padded points form Ky^-1 for the gradient on the INT8 tensor cores (dgp_lauum8.cuh), in both
+// engines alike; below it the FP64 DMMA LAUUM is faster (tools/lauum_emul_probe.py)
+constexpr int L8_MIN_NPAD = 8192;
+inline bool lauum_emulated(int npad) { return npad >= L8_MIN_NPAD && npad <= L8_MAX_NPAD; }
+
+// residue buffers of the emulated LAUUM, allocated by the first evaluation that needs them and kept until destroy:
+// R [16][npad][npad] int8 (operand residues in the upper block triangle, product residues in the strictly lower one),
+// D [16][npad][128] int8 (product residues of the diagonal blocks), the row scale exponents [npad]
+struct L8Work {
+  int8_t *R = nullptr, *D = nullptr;
+  int* sexp = nullptr;
+  void release() {
+    if (R) cudaFree(R);
+    if (D) cudaFree(D);
+    if (sexp) cudaFree(sexp);
+    R = D = nullptr; sexp = nullptr;
+  }
+};
 
 }  // namespace
 
@@ -102,6 +121,7 @@ struct dgp_handle_s {
   double *mu = nullptr, *var = nullptr;
   // pinned host staging
   double *h_theta = nullptr, *h_scal = nullptr;
+  L8Work l8;
   CUtensorMap tmA, tmL, tmU, tmDI, tmKx;
   cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   double last_ms[4] = {0, 0, 0, 0};
@@ -180,6 +200,47 @@ static cudaError_t launch_ex(void (*kern)(KArgs...), int grid, int block, size_t
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+}
+
+// Ky^-1 = U U' (lower block triangle of K, leading dimension ld) of one site of npad points on the INT8 tensor cores;
+// the residue buffers are allocated on first use for sites of up to cap padded points
+template <typename HT>
+static int lauum_i8(HT h, L8Work& w, long long cap, const double* U, double* K, long long ld, int npad, cudaStream_t st) {
+  const int nb = npad / 128;
+  if (!w.R) {
+    const size_t c = (size_t)cap;
+    cudaError_t e = cudaMalloc((void**)&w.R, L8_NMOD * c * c);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&w.D, L8_NMOD * c * 128);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&w.sexp, c * sizeof(int));
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      w.release();
+      DGP_FAIL(h, -2, "INT8 LAUUM workspace (%zu B for %lld padded points) not allocated: %s",
+               (size_t)L8_NMOD * c * (c + 128) + c * sizeof(int), cap, cudaGetErrorString(e));
+    }
+    static bool attr_set[64] = {false};
+    const int dev = (h->device >= 0 && h->device < 64) ? h->device : 0;
+    if (!attr_set[dev]) {
+      CK(h, cudaFuncSetAttribute(k_l8_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, L8_SMEM));
+      attr_set[dev] = true;
+    }
+  }
+  PFN_encodeTiled enc = get_encode();
+  if (!enc) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled entry point not available");
+  CUtensorMap tm;
+  cuuint64_t dims[3] = {(cuuint64_t)npad, (cuuint64_t)npad, (cuuint64_t)L8_NMOD};
+  cuuint64_t strides[2] = {(cuuint64_t)npad, (cuuint64_t)npad * (cuuint64_t)npad};
+  cuuint32_t box[3] = {128, 128, 1};
+  cuuint32_t es[3] = {1, 1, 1};
+  CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, w.R, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled (int8 residues) failed (%d) npad=%d", (int)r, npad);
+  k_l8_convert<<<npad, 256, 0, st>>>(U, ld, npad, l8_bits(npad), w.R, npad, w.sexp);
+  k_l8_gemm<<<L8_NMOD * l8_slots(nb), 128, L8_SMEM, st>>>(tm, nb, w.R, w.D, npad);
+  k_l8_recon<<<nb * (nb + 1) / 2, 256, 0, st>>>(w.R, w.D, npad, w.sexp, K, ld);
+  h->launches += 3;
+  CK(h, cudaGetLastError());
+  return 0;
 }
 
 static const BatchTab g_no_batch = {};   // count == 0: single-site launch
@@ -298,6 +359,7 @@ int dgp_destroy(dgp_handle h) {
                     h->scal, h->gpart, h->zpart, h->cvec, h->vvec, h->gam, h->tmpz, h->mfg_out, h->wpart, h->Kx, h->Xs, h->Xws, h->means, h->dot, h->vpart, h->mu, h->var};
   for (double* p : bufs) if (p) cudaFree(p);
   if (h->arena) cudaFree(h->arena);
+  h->l8.release();
   if (h->h_theta) cudaFreeHost(h->h_theta);
   if (h->h_scal) cudaFreeHost(h->h_scal);
   if (h->h_mfg) cudaFreeHost(h->h_mfg);
@@ -722,9 +784,14 @@ static int run_trtri(dgp_handle h, InvProgress& ip) {
 // contracts W = alpha alpha' - Ky^-1 with the regenerated dK/dtheta tiles (measured 3-4 ms faster at n = 16384 than the
 // contraction fused into the LAUUM epilogue, whose dependent FP64 chains wait behind the co-resident CTA's DMMA issue).
 static int run_lauum_grad(dgp_handle h) {
-  GemmArgs g = base_args(h, M_LAUUM, 0);
-  g.C = h->bufA; g.ntiles = lauum_slots(h->nb);
-  int rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmU, h->tmU, g);
+  int rc;
+  if (lauum_emulated(h->npad)) {
+    rc = lauum_i8(h, h->l8, h->max_pad, h->bufU, h->bufA, h->npad, h->npad, h->stream);
+  } else {
+    GemmArgs g = base_args(h, M_LAUUM, 0);
+    g.C = h->bufA; g.ntiles = lauum_slots(h->nb);
+    rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmU, h->tmU, g);
+  }
   if (rc) return rc;
   k_grad_contract<<<h->nb * (h->nb + 1), 128, 0, h->stream>>>(h->spec, h->theta, h->Xw, h->alpha, h->bufA, h->npad, h->n, h->gpart);
   h->launches++;
@@ -1422,6 +1489,14 @@ int dgp_get_kinv(dgp_handle h, double* Kinv_out, int out_on_device) {
     DGP_FAIL(h, -1, "dgp_get_kinv: needs dgp_set_debug_kinv(1) + dgp_nlml_grad");
   CK(h, cudaSetDevice(h->device));
   return copy_out(h, Kinv_out, h->bufA, h->n, h->n, h->npad, out_on_device);
+}
+
+int dgp_get_uinv(dgp_handle h, double* U_out, int out_on_device) {
+  if (!h) return -1;
+  if (!h->factorized || h->pending_grad < 1 || !U_out)
+    DGP_FAIL(h, -1, "dgp_get_uinv: needs a successful dgp_nlml_grad or dgp_factorize");
+  CK(h, cudaSetDevice(h->device));
+  return copy_out(h, U_out, h->bufU, h->n, h->n, h->npad, out_on_device);
 }
 
 // T = L^-1 sits in the lower triangle of bufA after dgp_factorize (the last merge level is transposed there too); the upper

@@ -43,6 +43,7 @@ struct dgp_batch_s {
   double *theta = nullptr, *scal = nullptr, *gpart = nullptr, *zpart = nullptr, *jitv = nullptr;
   double *h_theta = nullptr, *h_scal = nullptr, *h_jit = nullptr;  // pinned
   CUtensorMap tmA, tmL, tmU;
+  L8Work l8;   // residue buffers of the INT8 LAUUM (sites of L8_MIN_NPAD padded points or more, one site at a time)
   // prediction slabs (dgp_batch_predict), allocated by the first prediction on the handle and kept (chunk = DGP_BATCH_CHUNK):
   // Kx [max_sites][chunk][max_pad], mean / variance partials [max_sites][max_nb | 2 max_nb][chunk], inputs and features
   // [max_sites][chunk][8], means / mu / var [max_sites][chunk]; pinned staging of the inputs and of mu / var
@@ -339,14 +340,22 @@ int b_trtri(dgp_batch_t b, BInvProgress& ip) {
 }
 
 // LAUUM -> Ky^-1 (lower tiles, over the dead T) and the gradient contraction W (.) dK/dtheta; all sites per launch.
+// Sites the size rule of the single-site engine sends to the INT8 tensor cores go there one by one, the others share
+// one DMMA launch.
 int b_lauum_grad(dgp_batch_t b, cudaStream_t W) {
   TabBuilder tb(b);
+  int rc;
   for (int k = 0; k < b->G; k++) {
     const int i = b->order[k];
-    tb.add(i, 0, b->nb[i], b->n[i], 0, 0, 0, lauum_slots(b->nb[i]));
+    if (lauum_emulated(b->nb[i] * 128)) {
+      const size_t so = (size_t)i * (size_t)b->ld * (size_t)b->ld;
+      if ((rc = lauum_i8(b, b->l8, b->max_pad, b->U + so, b->A + so, b->ld, b->nb[i] * 128, W))) return rc;
+    } else {
+      tb.add(i, 0, b->nb[i], b->n[i], 0, 0, 0, lauum_slots(b->nb[i]));
+    }
   }
   GemmArgs g = b_args(b, M_LAUUM, b->A, 1.0, tb.total);
-  int rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmU, b->tmU, g, W, false, &tb.t);
+  rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmU, b->tmU, g, W, false, &tb.t);
   if (rc) return rc;
   k_grad_contract_b<<<b->sd.tile0[b->G], 128, 0, W>>>(b->spec, b->sd, b->theta, b->Xw, b->alpha, b->A, b->gpart);
   b->launches++;
@@ -476,6 +485,7 @@ int dgp_batch_destroy(dgp_batch b) {
   for (double* p : bufs) if (p) cudaFree(p);
   b_predict_free(b);
   b_mfg_free(b);
+  b->l8.release();
   if (b->h_theta) cudaFreeHost(b->h_theta);
   if (b->h_scal) cudaFreeHost(b->h_scal);
   if (b->h_jit) cudaFreeHost(b->h_jit);

@@ -98,12 +98,17 @@ typedef struct dgp_handle_s* dgp_handle;
 /* Create an engine on CUDA device `device` for up to max_n training points and prediction chunks
  * of up to max_m points (0 -> default).  Allocates every workspace (3 padded n x n float64 panels +
  * prediction chunk); later calls allocate nothing.  stream: a cudaStream_t to run on, or NULL to
- * let the handle create its own non-blocking stream. */
+ * let the handle create its own non-blocking stream.  Exception: the first gradient evaluation of a training set of
+ * at least 8192 padded points (n rounded up to 128) forms Ky^-1 on the INT8 tensor cores and allocates its residue
+ * buffers then, kept until destroy: 16 max_pad^2 + 2048 max_pad + 4 max_pad B (max_pad = max_n rounded up to 128).  If
+ * that allocation fails the evaluation returns an error. */
 int dgp_create(dgp_handle* out, int device, int max_n, int max_m, void* stream);
 
 int dgp_destroy(dgp_handle h);
 const char* dgp_last_error(dgp_handle h); /* h may be NULL: error of a failed dgp_create */
 int dgp_abi_version(void);
+/* Device bytes allocated by dgp_create; the INT8 LAUUM's residue buffers (16 max_pad^2 + 2052 max_pad B, allocated by the
+ * first gradient evaluation of a training set of >= 8192 padded points) are not included. */
 size_t dgp_workspace_bytes(int max_n, int max_m);
 
 /* Training set of one site.  X[n, ndim], y[n], noise[n] (fixed per-point noise variances).
@@ -218,6 +223,9 @@ int dgp_get_kinv(dgp_handle h, double* Kinv_out, int out_on_device);
 /* T = L^-1 [n, n], lower triangular (zeros above the diagonal): the inverse the variance and sampling products use.  Valid
  * after a successful dgp_factorize only (dgp_nlml_grad overwrites it with Ky^-1); fails with a message otherwise. */
 int dgp_get_linv(dgp_handle h, double* T_out, int out_on_device);
+/* U = L^-T [n, n], upper triangular: the operand of the LAUUM that forms Ky^-1.  Valid after dgp_nlml_grad or
+ * dgp_factorize; fails with a message otherwise. */
+int dgp_get_uinv(dgp_handle h, double* U_out, int out_on_device);
 
 /* Utility: the FP64 tensor-pipe tile engine as a plain product on device pointers,
  * C[M, N] = A[M, K] B[N, K]' (mode 0), C += A B' (mode 1), C -= A B' (mode -1).
@@ -237,13 +245,16 @@ int dgp_gemm_nt(dgp_handle h, const double* A, long long lda, const double* B, l
  * at create.  The first dgp_batch_predict on a handle adds the prediction slabs, once: 8 max_sites x 1024 x (max_pad +
  * 3 max_pad / 128 + 19) B on the device (max_pad = max_n rounded up to 128; the cross covariance of 1024 grid rows per
  * site) and 80 max_sites x 1024 B of pinned host memory.  Every other call allocates nothing, and handles that never
- * predict keep the create-time footprint.  Host pointers throughout. */
+ * predict keep the create-time footprint.  The first dgp_batch_nlml_grad with a site of at least 8192 padded points
+ * adds the residue buffers of the INT8 LAUUM once, for one site at a time: 16 max_pad^2 + 2052 max_pad B.  Host pointers
+ * throughout. */
 #define DGP_BATCH_MAX_SITES 32
 typedef struct dgp_batch_s* dgp_batch;
 int dgp_batch_create(dgp_batch* out, int device, int max_sites, int max_n, void* stream);
 int dgp_batch_destroy(dgp_batch b);
 const char* dgp_batch_last_error(dgp_batch b); /* b may be NULL: error of a failed dgp_batch_create */
-/* Device bytes allocated by dgp_batch_create (the prediction slabs of the first dgp_batch_predict are not included). */
+/* Device bytes allocated by dgp_batch_create (the prediction slabs of the first dgp_batch_predict and the INT8 LAUUM's
+ * residue buffers of the first gradient evaluation with a site of >= 8192 padded points are not included). */
 size_t dgp_batch_workspace_bytes(int max_sites, int max_n);
 /* Training sets of nsites sites: n[s] points each, X[s][n[s], ndim], y[s][n[s]], noise[s][n[s]] (host arrays of host pointers). */
 int dgp_batch_set_train(dgp_batch b, const dgp_spec* spec, int nsites, const int* n, const double* const* X,

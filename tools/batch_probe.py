@@ -43,6 +43,10 @@ if "all" in which or "config4" in which:
         run([int(v) for v in ns_all[g:g + 16]], f"config-4 group {g // 16} ({ns_all[g]}..{ns_all[g + 15]})")
     run([int(v) for v in ns_all[:32]], "config-4 32 largest")
     run([int(v) for v in ns_all[::8]], "config-4 every 8th (mixed)")
+if "rule" in which:   # groups just below (FP64 DMMA LAUUM) and at (INT8 LAUUM, one site at a time) the 8192-point size rule
+    for g in (1, 4, 8):
+        run([8064] * g, f"{g} x 8064")
+        run([8192] * g, f"{g} x 8192")
 if "single" in which:
     for n in (2048, 4096, 7680, 8192, 16384):
         run([n], f"1 x {n}")

@@ -8,7 +8,7 @@ HEAD = """# cuobjdump -sass discontinuum_b200/libdgp.so, instruction counts per 
 # build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -shared -Xcompiler -fPIC -o libdgp.so dgp_api.cu (CUDA 12.9)
 # DMMA = FP64 tensor-core MMA (mma.sync.m8n8k4.f64; tcgen05 has no f64 kind), UTMALDG = TMA tensor load (cp.async.bulk.tensor),
 # SYNCS = mbarrier ops, USETMAXREG = warpgroup register reallocation (setmaxnreg), STL / LDL = local-memory spills (none inside
-# the DMMA main loops).  No UTC*MMA (tcgen05) expected: the path is FP64."""
+# the DMMA main loops).  UTCIMMA (tcgen05.mma kind::i8) appears in k_l8_gemm only: the INT8 modular LAUUM of dgp_lauum8.cuh."""
 
 
 def main(tag):
