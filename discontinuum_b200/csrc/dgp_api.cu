@@ -21,6 +21,7 @@
 // latency-bound inside a GEMM epilogue; the extra 2 x 8 n^2 bytes are 3 % of the evaluation's DRAM traffic, DESIGN 4.6).
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -70,10 +71,21 @@ constexpr int EAGER_INV_MAX_NB = 96;
 // engines alike; below it the FP64 DMMA LAUUM is faster (tools/lauum_emul_probe.py)
 constexpr int L8_MIN_NPAD = 8192;
 inline bool lauum_emulated(int npad) { return npad >= L8_MIN_NPAD && npad <= L8_MAX_NPAD; }
+// a merge of the inverse (block ranges of hb and w2 <= hb blocks) forms its two products on the INT8 tensor cores
+// (inv_merge_i8) when hb >= INV8_MIN_HB and w2 >= INV8_MIN_W2, in both engines alike; smaller merges stay on the FP64 DMMA
+// tile engine.  Measured per merge (tools/inv_emul_probe.py, DESIGN.md 4.1b): 16 | 16 loses, 32 | 32, 64 | 16 and above
+// win; hb = 32 stays on DMMA so that the batched sites up to 64 blocks keep their shared launches.  Monotone in w2: at one
+// level only the ragged last pair can fall below it.
+constexpr int INV8_MIN_HB = 64;
+constexpr int INV8_MIN_W2 = 16;
+inline bool inv_emulated(int hb, int w2) { return hb >= INV8_MIN_HB && w2 >= INV8_MIN_W2 && 128 * hb <= L8_MAX_NPAD; }
+// blocks of the second range of merge pair pr at level hb of an nb-block inverse
+inline int pair_w2(int nb, int hb, int pr) { return std::min(hb, nb - (2 * pr + 1) * hb); }
 
-// residue buffers of the emulated LAUUM, allocated by the first evaluation that needs them and kept until destroy:
-// R [16][npad][npad] int8 (operand residues in the upper block triangle, product residues in the strictly lower one),
-// D [16][npad][128] int8 (product residues of the diagonal blocks), the row scale exponents [npad]
+// residue buffers of the emulated LAUUM and inverse merges, allocated by the first evaluation that needs them and kept until
+// destroy: R [16][npad][npad] int8 (LAUUM: operand residues in the upper block triangle, product residues in the strictly
+// lower one; a merge: the planes of its two operands and of its product, 16 (hb^2 + 2 hb w2) 128^2 <= 16 npad^2 bytes),
+// D [16][npad][128] int8 (LAUUM: product residues of the diagonal blocks), the row scale exponents [npad]
 struct L8Work {
   int8_t *R = nullptr, *D = nullptr;
   int* sexp = nullptr;
@@ -202,45 +214,100 @@ static cudaError_t launch_ex(void (*kern)(KArgs...), int grid, int block, size_t
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
-// Ky^-1 = U U' (lower block triangle of K, leading dimension ld) of one site of npad points on the INT8 tensor cores;
-// the residue buffers are allocated on first use for sites of up to cap padded points
+// the residue buffers, allocated on first use for sites of up to cap padded points
+template <typename HT>
+static int l8_ensure(HT h, L8Work& w, long long cap) {
+  if (w.R) return 0;
+  const size_t c = (size_t)cap;
+  cudaError_t e = cudaMalloc((void**)&w.R, L8_NMOD * c * c);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&w.D, L8_NMOD * c * 128);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&w.sexp, c * sizeof(int));
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    w.release();
+    DGP_FAIL(h, -2, "INT8 emulation workspace (%zu B for %lld padded points) not allocated: %s",
+             (size_t)L8_NMOD * c * (c + 128) + c * sizeof(int), cap, cudaGetErrorString(e));
+  }
+  static bool attr_set[64] = {false};
+  const int dev = (h->device >= 0 && h->device < 64) ? h->device : 0;
+  if (!attr_set[dev]) {
+    CK(h, cudaFuncSetAttribute(k_l8_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, L8_SMEM));
+    CK(h, cudaFuncSetAttribute(k_l8_gemm_ab, cudaFuncAttributeMaxDynamicSharedMemorySize, L8_SMEM));
+    attr_set[dev] = true;
+  }
+  return 0;
+}
+
+// 3-D map of 16 int8 residue planes [16][rows][kw] (128 x 128 boxes, the operand layout of l8_tile)
+template <typename HT>
+static int l8_map(HT h, CUtensorMap* tm, int8_t* base, long long rows, long long kw) {
+  PFN_encodeTiled enc = get_encode();
+  if (!enc) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled entry point not available");
+  cuuint64_t dims[3] = {(cuuint64_t)kw, (cuuint64_t)rows, (cuuint64_t)L8_NMOD};
+  cuuint64_t strides[2] = {(cuuint64_t)kw, (cuuint64_t)kw * (cuuint64_t)rows};
+  cuuint32_t box[3] = {128, 128, 1};
+  cuuint32_t es[3] = {1, 1, 1};
+  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled (int8 residues) failed (%d) rows=%lld kw=%lld", (int)r, rows, kw);
+  return 0;
+}
+
+// Ky^-1 = U U' (lower block triangle of K, leading dimension ld) of one site of npad points on the INT8 tensor cores
 template <typename HT>
 static int lauum_i8(HT h, L8Work& w, long long cap, const double* U, double* K, long long ld, int npad, cudaStream_t st) {
   const int nb = npad / 128;
-  if (!w.R) {
-    const size_t c = (size_t)cap;
-    cudaError_t e = cudaMalloc((void**)&w.R, L8_NMOD * c * c);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&w.D, L8_NMOD * c * 128);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&w.sexp, c * sizeof(int));
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      w.release();
-      DGP_FAIL(h, -2, "INT8 LAUUM workspace (%zu B for %lld padded points) not allocated: %s",
-               (size_t)L8_NMOD * c * (c + 128) + c * sizeof(int), cap, cudaGetErrorString(e));
-    }
-    static bool attr_set[64] = {false};
-    const int dev = (h->device >= 0 && h->device < 64) ? h->device : 0;
-    if (!attr_set[dev]) {
-      CK(h, cudaFuncSetAttribute(k_l8_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, L8_SMEM));
-      attr_set[dev] = true;
-    }
-  }
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled entry point not available");
+  int rc;
+  if ((rc = l8_ensure(h, w, cap))) return rc;
   CUtensorMap tm;
-  cuuint64_t dims[3] = {(cuuint64_t)npad, (cuuint64_t)npad, (cuuint64_t)L8_NMOD};
-  cuuint64_t strides[2] = {(cuuint64_t)npad, (cuuint64_t)npad * (cuuint64_t)npad};
-  cuuint32_t box[3] = {128, 128, 1};
-  cuuint32_t es[3] = {1, 1, 1};
-  CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, w.R, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) DGP_FAIL(h, -3, "cuTensorMapEncodeTiled (int8 residues) failed (%d) npad=%d", (int)r, npad);
-  k_l8_convert<<<npad, 256, 0, st>>>(U, ld, npad, l8_bits(npad), w.R, npad, w.sexp);
+  if ((rc = l8_map(h, &tm, w.R, npad, npad))) return rc;
+  k_l8_convert<<<npad, 256, 0, st>>>(U, ld, npad, l8_bits(npad), true, false, w.R, npad, (long long)npad * npad, w.sexp);
   k_l8_gemm<<<L8_NMOD * l8_slots(nb), 128, L8_SMEM, st>>>(tm, nb, w.R, w.D, npad);
   k_l8_recon<<<nb * (nb + 1) / 2, 256, 0, st>>>(w.R, w.D, npad, w.sexp, K, ld);
   h->launches += 3;
   CK(h, cudaGetLastError());
   return 0;
+}
+
+// C = sign A B' (ra x rb tiles, leading dimension ldc) on the INT8 tensor cores, A = rows [0, 128 ra) and B = rows
+// [0, 128 rb) of their k ranges [0, 128 kb) (leading dimension ld): A upper block triangular and the k blocks [i, kb) of
+// tile row i when kupper, else B lower triangular at 64-row granularity and the k blocks [0, c + 1) of tile column c.
+// The operand width b depends on the k extent 128 kb alone.
+template <typename HT>
+static int gemm_ab_i8(HT h, L8Work& w, const double* A, const double* B, long long ld, int ra, int rb, int kb, bool kupper,
+                      double sign, double* C, long long ldc, cudaStream_t st) {
+  const long long kw = 128LL * kb, rowsA = 128LL * ra, rowsB = 128LL * rb;
+  int8_t* PA = w.R;
+  int8_t* PB = PA + L8_NMOD * rowsA * kw;
+  int8_t* PC = PB + L8_NMOD * rowsB * kw;
+  int* sa = w.sexp;
+  int* sb = w.sexp + rowsA;
+  const int b = l8_bits(kw);
+  int rc;
+  CUtensorMap tmA, tmB;
+  if ((rc = l8_map(h, &tmA, PA, rowsA, kw)) || (rc = l8_map(h, &tmB, PB, rowsB, kw))) return rc;
+  k_l8_convert<<<(unsigned)rowsA, 256, 0, st>>>(A, ld, (int)kw, b, kupper, false, PA, kw, rowsA * kw, sa);
+  k_l8_convert<<<(unsigned)rowsB, 256, 0, st>>>(B, ld, (int)kw, b, false, !kupper, PB, kw, rowsB * kw, sb);
+  k_l8_gemm_ab<<<L8_NMOD * 64 * ((ra + 7) / 8) * ((rb + 7) / 8), 128, L8_SMEM, st>>>(tmA, tmB, ra, rb, kb, kupper, PC);
+  k_l8_recon_ab<<<ra * rb, 256, 0, st>>>(PC, ra, rb, sa, sb, sign, C, ldc);
+  h->launches += 4;
+  CK(h, cudaGetLastError());
+  return 0;
+}
+
+// one merge of the inverse (block ranges [o, o + hb) | [o + hb, o + hb + w2)) on the INT8 tensor cores, the products of
+// M_INV_M and M_INV_U (dgp_gemm.cuh) over the same operand entries:
+//   M'  = U11 L21'  -> upper triangle of A (work matrix), k over the blocks [row block, hb) of range 1
+//   U12 = -M' T22'  -> U, k over range 2 up to the 64-row half of T22's row (T22 in the lower triangle of A)
+template <typename HT>
+static int inv_merge_i8(HT h, L8Work& w, long long cap, double* A, const double* L, double* U, long long ld, int o, int hb,
+                        int w2, cudaStream_t st) {
+  int rc;
+  if ((rc = l8_ensure(h, w, cap))) return rc;
+  const size_t r1 = (size_t)o * 128, r2 = (size_t)(o + hb) * 128;
+  double* Mp = A + r1 * ld + r2;
+  if ((rc = gemm_ab_i8(h, w, U + r1 * ld + r1, L + r2 * ld + r1, ld, hb, w2, hb, true, 1.0, Mp, ld, st))) return rc;
+  return gemm_ab_i8(h, w, Mp, A + r2 * ld + r2, ld, hb, w2, w2, false, -1.0, U + r1 * ld + r2, ld, st);
 }
 
 static const BatchTab g_no_batch = {};   // count == 0: single-site launch
@@ -740,15 +807,21 @@ static int trtri_advance(dgp_handle h, InvProgress& ip, int F) {
     const int avail = F >= nb ? npairs : F / (2 * hb);
     const int pr0 = ip.done[lv], cnt = avail - pr0;
     if (cnt <= 0) continue;
-    {
-      GemmArgs g = base_args(h, M_INV_M, pr0);
-      g.aux0 = hb; g.aux1 = cnt; g.C = h->bufA; g.ntiles = cnt * hb * 2 * hb;
-      if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmU, h->tmL, g, ip.W))) return rc;
-    }
-    {
-      GemmArgs g = base_args(h, M_INV_U, pr0);
-      g.aux0 = hb; g.aux1 = cnt; g.C = h->bufU; g.ntiles = cnt * hb * 2 * hb; g.sign = -1.0;
-      if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmA, h->tmA, g, ip.W))) return rc;
+    int pe = pr0;   // pairs [pr0, pe) on the INT8 tensor cores, [pe, avail) on the DMMA tile engine
+    for (; pe < avail && inv_emulated(hb, pair_w2(nb, hb, pe)); pe++)
+      if ((rc = inv_merge_i8(h, h->l8, h->max_pad, h->bufA, h->bufL, h->bufU, h->npad, pe * 2 * hb, hb, pair_w2(nb, hb, pe),
+                             ip.W))) return rc;
+    if (pe < avail) {
+      {
+        GemmArgs g = base_args(h, M_INV_M, pe);
+        g.aux0 = hb; g.aux1 = avail - pe; g.C = h->bufA; g.ntiles = (avail - pe) * hb * 2 * hb;
+        if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmU, h->tmL, g, ip.W))) return rc;
+      }
+      {
+        GemmArgs g = base_args(h, M_INV_U, pe);
+        g.aux0 = hb; g.aux1 = avail - pe; g.C = h->bufU; g.ntiles = (avail - pe) * hb * 2 * hb; g.sign = -1.0;
+        if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(h, h->tmA, h->tmA, g, ip.W))) return rc;
+      }
     }
     if (ip.want_T || 2 * hb < nb) {
       k_transpose_pairs<<<cnt * 16 * hb * hb, 256, 0, ip.W>>>(h->bufU, h->bufA, h->npad, hb, h->npad, pr0);

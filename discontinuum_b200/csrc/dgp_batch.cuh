@@ -294,21 +294,24 @@ int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg) {
       const int avail = F >= nbi ? npairs : (F > 0 ? F / (2 * hb) : 0);
       const int pr0 = ip.done[lv][i], cnt = avail - pr0;
       if (cnt <= 0) continue;
-      tb.add(i, pr0, nbi, b->n[i], hb, cnt, 0, cnt * hb * 2 * hb);
+      // merges the size rule sends to the INT8 tensor cores leave the shared table and run one site at a time
+      int pe = pr0;
+      const size_t so = (size_t)i * (size_t)b->ld * (size_t)b->ld;
+      for (; pe < avail && inv_emulated(hb, pair_w2(nbi, hb, pe)); pe++)
+        if ((rc = inv_merge_i8(b, b->l8, b->max_pad, b->A + so, b->L + so, b->U + so, b->ld, pe * 2 * hb, hb,
+                               pair_w2(nbi, hb, pe), ip.W))) return rc;
+      tb.add(i, pe, nbi, b->n[i], hb, avail - pe, 0, (avail - pe) * hb * 2 * hb);
       if (ip.want_T || 2 * hb < nbi) {
         prg.pr0[i] = (short)pr0; prg.cnt[i] = (short)cnt;
         if (cnt * 16 * hb * hb > tmax) tmax = cnt * 16 * hb * hb;
       }
       ip.done[lv][i] = (short)avail;
     }
-    if (tb.total <= 0) continue;
-    {
-      GemmArgs g = b_args(b, M_INV_M, b->A, 1.0, tb.total);
-      if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmU, b->tmL, g, ip.W, false, &tb.t))) return rc;
-    }
-    {
-      GemmArgs g = b_args(b, M_INV_U, b->U, -1.0, tb.total);
-      if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmA, b->tmA, g, ip.W, false, &tb.t))) return rc;
+    if (tb.total > 0) {   // (none when every merge of the level went to the INT8 tensor cores; the transposes still run)
+      GemmArgs gm = b_args(b, M_INV_M, b->A, 1.0, tb.total);
+      if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmU, b->tmL, gm, ip.W, false, &tb.t))) return rc;
+      GemmArgs gu = b_args(b, M_INV_U, b->U, -1.0, tb.total);
+      if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmA, b->tmA, gu, ip.W, false, &tb.t))) return rc;
     }
     if (tmax > 0) {
       k_transpose_pairs_b<<<dim3(tmax, G), 256, 0, ip.W>>>(b->sd, prg, b->U, b->A, hb);

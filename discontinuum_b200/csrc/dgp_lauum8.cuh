@@ -17,6 +17,7 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <string.h>
 #include "dgp_gemm.cuh"
 
 namespace dgp {
@@ -75,10 +76,24 @@ __host__ __device__ __forceinline__ int l8_residue(unsigned long long a, bool ne
   return r > m / 2 ? r - m : r;
 }
 
+// x 2^k, as ldexp: one multiplication by 2^k while that is a normal double (the exact product, rounded once if it is
+// subnormal), instead of ldexp's general range handling on every call
+__host__ __device__ __forceinline__ double l8_ldexp(double x, int k) {
+  if (k < -1022 || k > 1023) return ldexp(x, k);
+  const unsigned long long p = (unsigned long long)(k + 1023) << 52;
+#ifdef __CUDA_ARCH__
+  return x * __longlong_as_double((long long)p);
+#else
+  double f;
+  memcpy(&f, &p, sizeof(f));
+  return x * f;
+#endif
+}
+
 // the 126-bit magnitude x, rounded once to double (round to nearest even), times 2^sc
 __host__ __device__ __forceinline__ double l8_round(u128 x, int sc) {
   const unsigned long long hi = (unsigned long long)(x >> 64), lo = (unsigned long long)x;
-  if (hi == 0) return ldexp((double)lo, sc);
+  if (hi == 0) return l8_ldexp((double)lo, sc);
 #ifdef __CUDA_ARCH__
   const int lz = __clzll((long long)hi);
 #else
@@ -87,21 +102,34 @@ __host__ __device__ __forceinline__ double l8_round(u128 x, int sc) {
   const int sh = 64 - lz;                                   // 1 .. 61
   unsigned long long top = (hi << lz) | (lo >> sh);         // bit 63 set
   top |= (lo << lz) != 0 ? 1ull : 0ull;                     // sticky bit, below the rounding bit
-  return ldexp((double)top, sh + sc);
+  return l8_ldexp((double)top, sh + sc);
 }
 
-// exact C' from its 16 symmetric residues, rounded to double and scaled by 2^sc
+// exact C' from its 16 symmetric residues, rounded to double and scaled by 2^sc.  S = sum_j t_j (M / m_j) with
+// t_j = y_j (M / m_j)^-1 mod m_j < 256 is accumulated in four 32-bit limbs of M / m_j (one mad.wide.u32 each): every limb
+// sum stays below 16 2^8 2^32 < 2^44, so the carries are propagated once after the loop.  S < 16 M; q = floor(S / M) is
+// taken from the top 33 bits of S against the top limb of M, rounded up (q is exact or one too small), and fixed with one
+// comparison.  Same x = S mod M as a 128-bit sum reduced after every step: the result is bit-identical.
 __host__ __device__ __forceinline__ double l8_crt(const int (&y)[L8_NMOD], int sc) {
   const u128 M = ((u128)L8_M_HI << 64) | L8_M_LO;
-  u128 x = 0;
+  unsigned long long a0 = 0, a1 = 0, a2 = 0, a3 = 0;
 #pragma unroll
   for (int j = 0; j < L8_NMOD; j++) {
     const L8Mod md = l8_mod(j);
-    const int yy = y[j] < 0 ? y[j] + md.m : y[j];
-    const unsigned long long t = (unsigned long long)((yy * md.inv) % md.m);
-    x += (((u128)(t * md.hi)) << 64) + (u128)t * md.lo;
-    if (x >= M) x -= M;
+    const unsigned yy = (unsigned)(y[j] < 0 ? y[j] + md.m : y[j]);
+    const unsigned t = (yy * (unsigned)md.inv) % (unsigned)md.m;
+    a0 += (unsigned long long)t * (unsigned)md.lo;
+    a1 += (unsigned long long)t * (unsigned)(md.lo >> 32);
+    a2 += (unsigned long long)t * (unsigned)md.hi;
+    a3 += (unsigned long long)t * (unsigned)(md.hi >> 32);
   }
+  a1 += a0 >> 32;
+  a2 += a1 >> 32;
+  a3 += a2 >> 32;   // S = a3 2^96 + (a2 mod 2^32) 2^64 + (a1 mod 2^32) 2^32 + (a0 mod 2^32), a3 < 2^33
+  const unsigned long long q = a3 / ((L8_M_HI >> 32) + 1);
+  u128 x = ((u128)a3 << 96) | ((u128)(a2 & 0xffffffffull) << 64) | ((a1 & 0xffffffffull) << 32) | (a0 & 0xffffffffull);
+  x -= (u128)q * M;   // mod 2^128: the true difference is below 2 M < 2^128
+  if (x >= M) x -= M;
   const bool neg = x > (M >> 1);
   return neg ? -l8_round(M - x, sc) : l8_round(x, sc);
 }
@@ -113,15 +141,21 @@ __host__ __device__ inline int l8_slots(int nb) {
   return 32 * B * (B + 1);
 }
 
-// ---------------------------------------------------------------- 1. conversion: one CTA per row of U
-__global__ void __launch_bounds__(256) k_l8_convert(const double* __restrict__ U, long long ldu, int npad, int b,
-                                                    int8_t* __restrict__ R, long long ldr, int* __restrict__ sexp) {
+// ---------------------------------------------------------------- 1. conversion: one CTA per operand row
+// Row i of the operand src[i][0, kw) (leading dimension lds), entries outside [k_lo(i), k_hi(i)) taken as zeros:
+// k_lo(i) = 128 (i / 128) when lo_blk (upper block triangle: nothing left of the row's diagonal block is stored, the GEMM
+// reads no k block left of it), else 0; k_hi(i) = 64 (i / 64 + 1) when hi64 (lower triangle at the 64-row granularity the
+// DMMA tile engine reads), else kw.  Residues of plane j at R + j plane + i ldr + k.
+__global__ void __launch_bounds__(256) k_l8_convert(const double* __restrict__ src, long long lds, int kw, int b, bool lo_blk,
+                                                    bool hi64, int8_t* __restrict__ R, long long ldr, long long plane,
+                                                    int* __restrict__ sexp) {
   const int i = blockIdx.x;
-  const int k0 = (i / 128) * 128;   // U[i, k] = 0 left of the row's diagonal block
-  const double* row = U + (size_t)i * ldu;
+  const int k0 = lo_blk ? (i / 128) * 128 : 0;
+  const int k1 = hi64 ? (i / 64 + 1) * 64 : kw;
+  const double* row = src + (size_t)i * lds;
   __shared__ double red[8];
   double mx = 0.0;
-  for (int k = k0 + threadIdx.x; k < npad; k += 256) mx = fmax(mx, fabs(row[k]));
+  for (int k = k0 + threadIdx.x; k < k1; k += 256) mx = fmax(mx, fabs(row[k]));
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = mx;
@@ -133,14 +167,14 @@ __global__ void __launch_bounds__(256) k_l8_convert(const double* __restrict__ U
   if (mx > 0.0) frexp(mx, &e);      // mx < 2^e
   const int s = mx > 0.0 ? b - 1 - e : 0;
   if (threadIdx.x == 0) sexp[i] = s;
-  const size_t plane = (size_t)ldr * ldr;
   int8_t* out = R + (size_t)i * ldr;
-  for (int k = k0 + 8 * threadIdx.x; k < npad; k += 8 * 256) {
+  for (int k = k0 + 8 * threadIdx.x; k < kw; k += 8 * 256) {
+    const bool in = k < k1;   // k1 is a multiple of 64: the 8 entries lie wholly inside or outside the row's range
     unsigned long long a[8];
     bool neg[8];
 #pragma unroll
     for (int v = 0; v < 8; v++) {
-      const double x = rint(ldexp(row[k + v], s));   // exact scaling; |x| <= 2^(b-1) < 2^62
+      const double x = in ? rint(ldexp(row[k + v], s)) : 0.0;   // exact scaling; |x| <= 2^(b-1) < 2^62
       neg[v] = x < 0.0;
       a[v] = (unsigned long long)fabs(x);
     }
@@ -173,23 +207,16 @@ __device__ __forceinline__ void l8_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-// grid = 16 * l8_slots(nb), modulus-major; modulus j is plane j of R (the third TMA coordinate) and of D
-__global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUtensorMap tmR, int nb, int8_t* __restrict__ R,
-                                                    int8_t* __restrict__ D, long long ld) {
+// one 128 x 128 output tile of plane j: C_j = sum over the k blocks kb0 .. kb0 + nk - 1 of A_j[rowA0 + 128) B_j[rowB0 + 128)'
+// mod m_j (A_j, B_j: plane j of the two tensor maps), stored as int8 residues at dst (row stride lds)
+__device__ __forceinline__ void l8_tile(const CUtensorMap* tmA, const CUtensorMap* tmB, int j, int rowA0, int rowB0, int kb0,
+                                        int nk, int8_t* __restrict__ dst, long long lds) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   uint64_t* full = (uint64_t*)(smem + L8_STAGES * L8_STAGE_BYTES);
   uint64_t* empty = full + L8_STAGES;
   uint64_t* done = empty + L8_STAGES;
   uint32_t* tslot = (uint32_t*)(done + 1);
-
-  const int slots = l8_slots(nb);
-  const int j = blockIdx.x / slots, tile = blockIdx.x - j * slots;
-  const int p = (isqrt_floor(4 * (tile >> 5) + 1) - 1) >> 1;
-  const int rem = tile - 32 * p * (p + 1);
-  const int i = 8 * p + ((rem & 63) >> 3), c = 8 * (rem >> 6) + (rem & 7);
-  if (i >= nb || c > i) return;
-  const int plane = j;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
@@ -205,7 +232,6 @@ __global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUte
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem = *tslot;
-  const int nk = nb - i;   // 128-wide k blocks i .. nb-1
 
   if (threadIdx.x == 0) {   // TMA producer
     for (int it = 0; it < nk; it++) {
@@ -213,8 +239,8 @@ __global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUte
       if (it >= L8_STAGES) mbar_wait(&empty[s], ((it / L8_STAGES) - 1) & 1);
       uint8_t* st = smem + s * L8_STAGE_BYTES;
       mbar_expect_tx(&full[s], L8_STAGE_BYTES);
-      tma_load_3d(st, &tmR, &full[s], (i + it) * 128, i * 128, plane);
-      tma_load_3d(st + L8_TILE_BYTES, &tmR, &full[s], (i + it) * 128, c * 128, plane);
+      tma_load_3d(st, tmA, &full[s], (kb0 + it) * 128, rowA0, j);
+      tma_load_3d(st + L8_TILE_BYTES, tmB, &full[s], (kb0 + it) * 128, rowB0, j);
     }
   } else if (threadIdx.x == 32) {   // MMA issuer
     for (int it = 0; it < nk; it++) {
@@ -236,9 +262,7 @@ __global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUte
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const int m = l8_mod(j).m;
   const double rinv = 1.0 / (double)m;
-  const int r = i * 128 + 32 * warp + lane;
-  int8_t* dst = (i == c) ? D + (size_t)plane * ld * 128 + (size_t)r * 128
-                         : R + (size_t)plane * ld * ld + (size_t)r * ld + (size_t)c * 128;
+  dst += (size_t)(32 * warp + lane) * lds;
 #pragma unroll 1
   for (int q = 0; q < 4; q++) {
     uint32_t v[32];
@@ -272,7 +296,67 @@ __global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUte
   }
 }
 
-// ---------------------------------------------------------------- 3. reconstruction: one CTA per lower 128 x 128 tile
+// LAUUM: grid = 16 * l8_slots(nb), modulus-major; modulus j is plane j of R (the third TMA coordinate) and of D
+__global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUtensorMap tmR, int nb, int8_t* __restrict__ R,
+                                                    int8_t* __restrict__ D, long long ld) {
+  const int slots = l8_slots(nb);
+  const int j = blockIdx.x / slots, tile = blockIdx.x - j * slots;
+  const int p = (isqrt_floor(4 * (tile >> 5) + 1) - 1) >> 1;
+  const int rem = tile - 32 * p * (p + 1);
+  const int i = 8 * p + ((rem & 63) >> 3), c = 8 * (rem >> 6) + (rem & 7);
+  if (i >= nb || c > i) return;
+  int8_t* dst = (i == c) ? D + (size_t)j * ld * 128 + (size_t)i * 128 * 128
+                         : R + (size_t)j * ld * ld + (size_t)i * 128 * ld + (size_t)c * 128;
+  l8_tile(&tmR, &tmR, j, i * 128, c * 128, i, nb - i, dst, i == c ? 128 : ld);   // k blocks i .. nb-1
+}
+
+// C = A B' over ra x rb tiles (C residues [16][128 ra][128 rb]), k blocks [i, kb) of tile (i, c) when kupper (A upper block
+// triangular, kb its block width), [0, c + 1) otherwise (B lower block triangular).  Grid = 16 * 64 ceil(ra / 8) ceil(rb / 8):
+// cells of 8 x 8 tiles, the longest K first (kupper: row-major from the top; else column-major from the right).
+__global__ void __launch_bounds__(128, 2) k_l8_gemm_ab(const __grid_constant__ CUtensorMap tmA,
+                                                       const __grid_constant__ CUtensorMap tmB, int ra, int rb, int kb,
+                                                       bool kupper, int8_t* __restrict__ C) {
+  const int cr = (ra + 7) / 8, cc = (rb + 7) / 8, slots = 64 * cr * cc;
+  const int j = blockIdx.x / slots, tile = blockIdx.x - j * slots;
+  const int cell = tile >> 6, w = tile & 63;
+  const int i = 8 * (kupper ? cell / cc : cell % cr) + (w >> 3);
+  const int c = kupper ? 8 * (cell % cc) + (w & 7) : 8 * (cc - 1 - cell / cr) + 7 - (w & 7);
+  if (i >= ra || c < 0 || c >= rb) return;
+  const long long ldc = 128LL * rb;
+  int8_t* dst = C + (size_t)j * 128 * ra * ldc + (size_t)i * 128 * ldc + (size_t)c * 128;
+  if (kupper) l8_tile(&tmA, &tmB, j, i * 128, c * 128, i, kb - i, dst, ldc);
+  else l8_tile(&tmA, &tmB, j, i * 128, c * 128, 0, c + 1, dst, ldc);
+}
+
+// ---------------------------------------------------------------- 3. reconstruction: one CTA per 128 x 128 tile
+// out[r][c] = sign 2^-(sr[r] + sc[c]) C'[r][c] for the tile whose residues of plane j start at src + j plane (row stride ls)
+__device__ __forceinline__ void l8_recon_tile(const int8_t* __restrict__ src, size_t plane, size_t ls,
+                                              const int* __restrict__ sr, const int* __restrict__ sc, double sign,
+                                              double* __restrict__ out, long long ldo) {
+  const int cq = 4 * (threadIdx.x & 31);
+  const int sc0 = sc[cq], sc1 = sc[cq + 1], sc2 = sc[cq + 2], sc3 = sc[cq + 3];
+#pragma unroll 1
+  for (int rr = threadIdx.x >> 5; rr < 128; rr += 8) {
+    const int8_t* p = src + (size_t)rr * ls + cq;
+    int y[4][L8_NMOD];
+#pragma unroll
+    for (int j = 0; j < L8_NMOD; j++) {
+      const uint32_t w = *reinterpret_cast<const uint32_t*>(p + j * plane);
+#pragma unroll
+      for (int v = 0; v < 4; v++) y[v][j] = (int)(int8_t)(w >> (8 * v));
+    }
+    const int s = sr[rr];
+    double2 o0, o1;
+    o0.x = sign * l8_crt(y[0], -(s + sc0));
+    o0.y = sign * l8_crt(y[1], -(s + sc1));
+    o1.x = sign * l8_crt(y[2], -(s + sc2));
+    o1.y = sign * l8_crt(y[3], -(s + sc3));
+    double* kp = out + (size_t)rr * ldo + cq;
+    *reinterpret_cast<double2*>(kp) = o0;
+    *reinterpret_cast<double2*>(kp + 2) = o1;
+  }
+}
+
 // Kinv[r, c] for the lower block triangle (diagonal blocks in full), the region M_LAUUM writes
 __global__ void __launch_bounds__(256) k_l8_recon(const int8_t* __restrict__ R, const int8_t* __restrict__ D, long long ld,
                                                   const int* __restrict__ sexp, double* __restrict__ K,
@@ -282,33 +366,20 @@ __global__ void __launch_bounds__(256) k_l8_recon(const int8_t* __restrict__ R, 
   while (i * (i + 1) / 2 > t) --i;
   while ((i + 1) * (i + 2) / 2 <= t) ++i;
   const int c = t - i * (i + 1) / 2;
-  const int8_t* src;
-  size_t plane, ls;
-  if (i == c) { src = D; plane = (size_t)ld * 128; ls = 128; }
-  else { src = R + (size_t)c * 128; plane = (size_t)ld * ld; ls = ld; }
-  const int cq = 4 * (threadIdx.x & 31);
-  const int sc0 = sexp[c * 128 + cq], sc1 = sexp[c * 128 + cq + 1], sc2 = sexp[c * 128 + cq + 2], sc3 = sexp[c * 128 + cq + 3];
-#pragma unroll 1
-  for (int rr = threadIdx.x >> 5; rr < 128; rr += 8) {
-    const int r = i * 128 + rr;
-    const int8_t* p = src + (size_t)r * ls + cq;
-    int y[4][L8_NMOD];
-#pragma unroll
-    for (int j = 0; j < L8_NMOD; j++) {
-      const uint32_t w = *reinterpret_cast<const uint32_t*>(p + j * plane);
-#pragma unroll
-      for (int v = 0; v < 4; v++) y[v][j] = (int)(int8_t)(w >> (8 * v));
-    }
-    const int sr = sexp[r];
-    double2 o0, o1;
-    o0.x = l8_crt(y[0], -(sr + sc0));
-    o0.y = l8_crt(y[1], -(sr + sc1));
-    o1.x = l8_crt(y[2], -(sr + sc2));
-    o1.y = l8_crt(y[3], -(sr + sc3));
-    double* kp = K + (size_t)r * ldk + c * 128 + cq;
-    *reinterpret_cast<double2*>(kp) = o0;
-    *reinterpret_cast<double2*>(kp + 2) = o1;
-  }
+  if (i == c) l8_recon_tile(D + (size_t)i * 128 * 128, (size_t)ld * 128, 128, sexp + i * 128, sexp + c * 128, 1.0,
+                            K + (size_t)i * 128 * ldk + c * 128, ldk);
+  else l8_recon_tile(R + (size_t)i * 128 * ld + c * 128, (size_t)ld * ld, ld, sexp + i * 128, sexp + c * 128, 1.0,
+                     K + (size_t)i * 128 * ldk + c * 128, ldk);
+}
+
+// out[128 ra][128 rb] (leading dimension ldo) = sign C from the residues of k_l8_gemm_ab; one CTA per tile
+__global__ void __launch_bounds__(256) k_l8_recon_ab(const int8_t* __restrict__ C, int ra, int rb, const int* __restrict__ sa,
+                                                     const int* __restrict__ sb, double sign, double* __restrict__ out,
+                                                     long long ldo) {
+  const int i = blockIdx.x / rb, c = blockIdx.x - i * rb;
+  const size_t ldc = (size_t)128 * rb;
+  l8_recon_tile(C + (size_t)i * 128 * ldc + c * 128, (size_t)128 * ra * ldc, ldc, sa + i * 128, sb + c * 128, sign,
+                out + (size_t)i * 128 * ldo + c * 128, ldo);
 }
 
 }  // namespace dgp

@@ -77,7 +77,7 @@ int main(int argc, char** argv) {
     memset(&spec, 0, sizeof(spec));
     const int b = l8_bits(npad);
     auto dmma = [&]() { k_gemm<INIT_ZERO, EPI_STORE><<<g.ntiles, GEMM_THREADS, SM_TOTAL>>>(tmU, tmU, spec, g, bt); };
-    auto conv = [&]() { k_l8_convert<<<npad, 256>>>(U, npad, npad, b, R, npad, sexp); };
+    auto conv = [&]() { k_l8_convert<<<npad, 256>>>(U, npad, npad, b, true, false, R, npad, (long long)nn, sexp); };
     auto gemm = [&]() { k_l8_gemm<<<L8_NMOD * l8_slots(nb), 128, L8_SMEM>>>(tmR, nb, R, D, npad); };
     auto recon = [&]() { k_l8_recon<<<nb * (nb + 1) / 2, 256>>>(R, D, npad, sexp, Ke, npad); };
     dmma(); conv(); gemm(); recon();
