@@ -8,6 +8,8 @@
 //        (programmatic dependent launches; 64-row half tiles while a launch is smaller than the GPU)
 //     T / T2: rank-512 update right of the panel in fixed column strips, strip j on stream j mod 2; the next panel's
 //        columns are the head of their strip: first column | its other columns | the rest of the strip       (n^3/3, DMMA)
+//     from SYRK_MIN_NB block columns split at hs: left of hs the updates stop at column hs, and the lower-right quadrant
+//        takes them all at once as A22 -= L21 L21' on the INT8 tensor cores (syrk_i8)               (44 % of the n^3/3)
 //   W: U = L^-T by recursive doubling (two long-K products and a transpose per level; up to 96 block columns and in batches
 //      the merges are launched as the factorisation passes them)                                            (n^3/3, DMMA)
 //      z = U'r, alpha = U z, LAUUM -> Ky^-1 (lower tiles), gradient contraction W (.) dK/dtheta              (n^3/3, DMMA)
@@ -79,6 +81,18 @@ inline bool lauum_emulated(int npad) { return npad >= L8_MIN_NPAD && npad <= L8_
 constexpr int INV8_MIN_HB = 64;
 constexpr int INV8_MIN_W2 = 16;
 inline bool inv_emulated(int hb, int w2) { return hb >= INV8_MIN_HB && w2 >= INV8_MIN_W2 && 128 * hb <= L8_MAX_NPAD; }
+// a training matrix of SYRK_MIN_NB block columns or more is factorised split at hs = syrk_split(nb) block columns
+// (potrf_core): the panels left of hs update only the block columns left of it, and the lower-right quadrant receives all
+// their updates as one product A22 -= L21 L21' on the INT8 tensor cores (syrk_i8), K = 128 hs.  In both engines alike, a
+// function of nb only.  hs = 3 nb / 8 rounded to a whole strip (DESIGN.md 4.5, tools/syrk_emul_probe.py).
+constexpr int SYRK_MIN_NB = 96;
+constexpr int SYRK_NUM = 3, SYRK_DEN = 8;
+static_assert(SYRK_MIN_NB > DGP_PREGEN_MIN_NB, "the quadrant is always a pre-generated matrix");
+static_assert(EAGER_INV_MAX_NB < 2 * INV8_MIN_HB, "no INT8 merge of the eager inverse shares the residue buffers with syrk_i8");
+inline int syrk_split(int nb) {
+  if (nb < SYRK_MIN_NB || 128 * nb > L8_MAX_NPAD) return 0;
+  return (SYRK_NUM * nb + SYRK_DEN * STRIP_BLOCKS / 2) / (SYRK_DEN * STRIP_BLOCKS) * STRIP_BLOCKS;
+}
 // blocks of the second range of merge pair pr at level hb of an nb-block inverse
 inline int pair_w2(int nb, int hb, int pr) { return std::min(hb, nb - (2 * pr + 1) * hb); }
 
@@ -288,9 +302,33 @@ static int gemm_ab_i8(HT h, L8Work& w, const double* A, const double* B, long lo
   if ((rc = l8_map(h, &tmA, PA, rowsA, kw)) || (rc = l8_map(h, &tmB, PB, rowsB, kw))) return rc;
   k_l8_convert<<<(unsigned)rowsA, 256, 0, st>>>(A, ld, (int)kw, b, kupper, false, PA, kw, rowsA * kw, sa);
   k_l8_convert<<<(unsigned)rowsB, 256, 0, st>>>(B, ld, (int)kw, b, false, !kupper, PB, kw, rowsB * kw, sb);
-  k_l8_gemm_ab<<<L8_NMOD * 64 * ((ra + 7) / 8) * ((rb + 7) / 8), 128, L8_SMEM, st>>>(tmA, tmB, ra, rb, kb, kupper, PC);
-  k_l8_recon_ab<<<ra * rb, 256, 0, st>>>(PC, ra, rb, sa, sb, sign, C, ldc);
+  k_l8_gemm_ab<<<L8_NMOD * 64 * ((ra + 7) / 8) * ((rb + 7) / 8), 128, L8_SMEM, st>>>(tmA, tmB, ra, rb, kb,
+                                                                                      kupper ? L8_KUPPER_A : L8_KLOWER_B, PC);
+  k_l8_recon_ab<<<ra * rb, 256, 0, st>>>(PC, ra, rb, sa, sb, sign, C, ldc, false);
   h->launches += 4;
+  CK(h, cudaGetLastError());
+  return 0;
+}
+
+// the lower-right quadrant update of a split factorisation (potrf_core) on the INT8 tensor cores: A22 -= L21 L21', L21 = rows
+// [128 hs, 128 nb) x columns [0, 128 hs) of L, over the lower tiles of A22 with its diagonal blocks in full (the region the
+// DMMA trailing updates write).  Operand planes [16][128 r][128 hs], product planes [16][128 r][128 r] (r = nb - hs): together
+// 16 128^2 r nb bytes, inside the LAUUM's 16 npad^2.  Every entry is the exact product rounded once, then one subtraction.
+template <typename HT>
+static int syrk_i8(HT h, L8Work& w, long long cap, const double* L, double* A, long long ld, int nb, int hs, cudaStream_t st) {
+  int rc;
+  if ((rc = l8_ensure(h, w, cap))) return rc;
+  const int r = nb - hs;
+  const long long kw = 128LL * hs, rows = 128LL * r;
+  int8_t* PA = w.R;
+  int8_t* PC = PA + L8_NMOD * rows * kw;
+  CUtensorMap tm;
+  if ((rc = l8_map(h, &tm, PA, rows, kw))) return rc;
+  const size_t o = (size_t)hs * 128;
+  k_l8_convert<<<(unsigned)rows, 256, 0, st>>>(L + o * ld, ld, (int)kw, l8_bits(kw), false, false, PA, kw, rows * kw, w.sexp);
+  k_l8_gemm_ab<<<L8_NMOD * l8_slots(r), 128, L8_SMEM, st>>>(tm, tm, r, r, hs, L8_KFULL_SYRK, PC);
+  k_l8_recon_ab<<<r * (r + 1) / 2, 256, 0, st>>>(PC, r, r, w.sexp, w.sexp, -1.0, A + o * ld + o, ld, true);
+  h->launches += 3;
   CK(h, cudaGetLastError());
   return 0;
 }
@@ -683,7 +721,11 @@ struct PanelHook { int (*fn)(dgp_handle, void*, cudaEvent_t, int) = nullptr; voi
 // the standalone generator covers every matrix it is used for with at least two column strips
 static_assert(DGP_PREGEN_MIN_NB >= STRIP_BLOCKS, "pre-generated matrices span more than one strip");
 
-static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jitter, bool fwd, PanelHook hook = PanelHook()) {
+// hs > 0 (training matrices, syrk_split): the panels ending at or before block column hs update the block columns [pe, hs)
+// only, all rows below included, so L21 comes out exactly as without the split; after the panel ending at hs, syrk_i8
+// applies all their updates to the lower-right quadrant at once and the panels from hs on run as without the split.
+static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jitter, bool fwd, PanelHook hook = PanelHook(),
+                      int hs = 0) {
   const int nb = b.nb;
   const long long ld = b.ld;
   int rc;
@@ -729,13 +771,21 @@ static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jit
     CK(h, cudaEventRecord(ev_panel(p), P));
     CK(h, cudaStreamWaitEvent(T, ev_panel(p), 0));
     if (hook.fn && pe < nb && (rc = hook.fn(h, hook.ctx, ev_panel(p), pe))) return rc;
-    if (pe < nb) {
+    if (pe == hs) {   // the quadrant update; the generator's strips right of hs have not been waited for yet
+      CK(h, cudaStreamWaitEvent(T, ev_gen(nstrips - 1), 0));
+      trace_mark(h, T, "syrk<", p);
+      if ((rc = syrk_i8(h, h->l8, h->max_pad, b.L, b.A, ld, nb, hs, T))) return rc;
+      trace_mark(h, T, "syrk>", p);
+      CK(h, cudaEventRecord(ev_col0(p + 1), T));
+      CK(h, cudaEventRecord(ev_cols(p + 1), T));
+    } else if (pe < nb) {
       // Column strips on two streams.  The trailing matrix is cut into fixed strips of `sw` block columns; strip j is
       // always updated on stream j mod 2, so the strips of one stream form their own dependency chain (panel after
       // panel) and the two streams never wait for each other: while one launch drains its last partial wave, the other
       // stream's CTAs take the free slots (a single stream loses about half a wave per launch, 3 launches per panel).
       // The next panel's columns are the head of their strip: first column | its other columns | the rest of the strip.
       // Launches with fewer tiles than the GPU has CTA slots run on 64-row half tiles (a K = 512 tile is 34 us on its own).
+      const int ce = pe < hs ? hs : nb;   // end of the block columns this panel updates
       const int ne = (pe + pw < nb) ? pe + pw : nb, w = ne - pe, m = nb - pe;
       const int slots = 2 * h->sms;
       const bool first = generate && p == 0 && !pregen;
@@ -758,13 +808,13 @@ static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jit
                                       (m - 1) * 2 * (w - 1) <= slots))) return rc;
       trace_mark(h, S0, "cols>", p);
       CK(h, cudaEventRecord(ev_cols(p + 1), S0));
-      const int e0 = ((j0 + 1) * sw < nb) ? (j0 + 1) * sw : nb;
+      const int e0 = ((j0 + 1) * sw < ce) ? (j0 + 1) * sw : ce;
       if (ne < e0) {
         const int tiles = (nb - ne) * 2 * (e0 - ne);
         if ((rc = launch_trail(h, b, pb, pe - pb, ne, e0 - ne, tiles, first, jitter, S0, tiles <= slots))) return rc;
       }
-      for (int j = j0 + 1; j * sw < nb; j++) {
-        const int o = j * sw, wj = (o + sw < nb) ? sw : nb - o, tiles = (nb - o) * 2 * wj;
+      for (int j = j0 + 1; j * sw < ce; j++) {
+        const int o = j * sw, wj = (o + sw < ce) ? sw : ce - o, tiles = (nb - o) * 2 * wj;
         if ((rc = launch_trail(h, b, pb, pe - pb, o, wj, tiles, first, jitter, strip_stream(j), tiles <= slots))) return rc;
       }
       trace_mark(h, T, "rest>", p);
@@ -780,7 +830,7 @@ static int potrf_core(dgp_handle h, const CholBufs& b, bool generate, double jit
 
 static int run_potrf(dgp_handle h, double jitter, bool fwd, PanelHook hook = PanelHook()) {
   CholBufs b{h->bufA, h->bufL, h->bufU, h->DI, h->scal, &h->tmA, &h->tmL, &h->tmDI, h->nb, h->npad};
-  return potrf_core(h, b, true, jitter, fwd, hook);
+  return potrf_core(h, b, true, jitter, fwd, hook, syrk_split(h->nb));
 }
 
 // U = L^-T (upper) by recursive doubling: the diagonal 128-blocks come from k_potf2_v2 (U_ss in bufU, T_ss = L_ss^-1 in

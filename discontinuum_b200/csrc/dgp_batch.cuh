@@ -124,7 +124,13 @@ int b_ensure_events(dgp_batch_t b, size_t count) {
 }
 
 // Two-level right-looking Cholesky with look-ahead (potrf_core of dgp_api.cu) over all sites, end-aligned.
-struct BInvProgress;
+// want_T: also transpose the last level of the inverse, so that T = L^-1 is complete in the lower triangle of the A slab
+// (dgp_batch_factorize, for the prediction)
+struct BInvProgress {
+  short done[16][DGP_BATCH_MAX];
+  bool want_T;
+  cudaStream_t W;
+};
 int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg);
 int b_eager(dgp_batch_t b, BInvProgress* ip, cudaEvent_t ev_panel, int pe);
 
@@ -136,7 +142,7 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
   const int npanels = (NB + pw - 1) / pw;
   int rc;
   bool any2 = false;
-  if ((rc = b_ensure_events(b, 3 * (size_t)npanels + 3))) return rc;
+  if ((rc = b_ensure_events(b, 3 * (size_t)npanels + 4))) return rc;
   auto ev_panel = [&](int p) { return b->evs[3 * p]; };
   auto ev_cols = [&](int p) { return b->evs[3 * p + 1]; };
   auto ev_col0 = [&](int p) { return b->evs[3 * p + 2]; };
@@ -155,6 +161,13 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
     any_pre |= pre[i];
   }
   cudaEvent_t ev_gen = b->evs[3 * (size_t)npanels + 1];
+  // split factorisation (syrk_split, potrf_core of dgp_api.cu) of every site the rule sends there, at its local block column
+  // hs[i]; the quadrant updates run one site at a time and share the residue buffers with the eager inverse's INT8 merges on
+  // stream W, so the two are ordered by events both ways
+  int hs[DGP_BATCH_MAX];
+  for (int i = 0; i < G; i++) hs[i] = syrk_split(b->nb[i]);
+  cudaEvent_t ev_w = b->evs[3 * (size_t)npanels + 2], ev_syrk = b->evs[3 * (size_t)npanels + 3];
+  bool w_pending = false, syrk_pending = false;
   if (any_pre) {
     CK(b, cudaStreamWaitEvent(b->stream_lo, ev_cols(0), 0));
     k_cov_lower_b<<<dim3(4 * NB, NB - 1, G), 256, 0, b->stream_lo>>>(b->spec, b->sd, b->theta, b->Xw, b->noise, b->jitv, b->A,
@@ -208,7 +221,12 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
     CK(b, cudaEventRecord(ev_panel(p), P));
     CK(b, cudaStreamWaitEvent(T, ev_panel(p), 0));
     if (any_pre && !wT) { wT = true; CK(b, cudaStreamWaitEvent(T, ev_gen, 0)); }
-    if (eager != nullptr && pe < NB && (rc = b_eager(b, eager, ev_panel(p), pe))) return rc;
+    if (eager != nullptr && pe < NB) {
+      if (syrk_pending) { syrk_pending = false; CK(b, cudaStreamWaitEvent(eager->W, ev_syrk, 0)); }
+      if ((rc = b_eager(b, eager, ev_panel(p), pe))) return rc;
+      CK(b, cudaEventRecord(ev_w, eager->W));
+      w_pending = true;
+    }
     // ---- rank-(128 pw) update right of the panel.  Column strips on two streams (potrf_core of dgp_api.cu): fixed strips
     // of `sw` block columns in the end-aligned (global) column numbering, strip j always on stream j mod 2; the next panel's
     // columns are the head of their strip: first column | its other columns | the rest of the strip.
@@ -228,13 +246,22 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
       if (lpb < 0 || lpb >= nbi) continue;
       const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
       if (lpe >= nbi) continue;
+      if (lpe == hs[i]) {   // the site's quadrant update, ahead of ev_col0(p + 1) on S0
+        if (w_pending) { w_pending = false; CK(b, cudaStreamWaitEvent(S0, ev_w, 0)); }
+        const size_t so = (size_t)i * (size_t)ld * (size_t)ld;
+        if ((rc = syrk_i8(b, b->l8, b->max_pad, b->L + so, b->A + so, ld, nbi, hs[i], S0))) return rc;
+        CK(b, cudaEventRecord(ev_syrk, S0));
+        syrk_pending = true;
+        continue;
+      }
+      const int ce = lpe < hs[i] ? hs[i] : nbi;   // end of the block columns this panel updates
       const int kb = lpe - lpb, ne = (lpe + pw < nbi) ? lpe + pw : nbi, w = ne - lpe, m = nbi - lpe;
       const bool first = (lpb == 0) && !pre[i];
       const int a2 = first ? 0 : 1;
       ta.add(i, lpb, nbi, b->n[i], lpe | (1 << 16), kb, a2, m * 2);
       ta.any_first |= first;
       if (w > 1) { tb2.add(i, lpb, nbi, b->n[i], (lpe + 1) | ((w - 1) << 16), kb, a2, (m - 1) * 2 * (w - 1)); tb2.any_first |= first; }
-      const int e0 = ((j0 + 1) * sw - b->off[i] < nbi) ? (j0 + 1) * sw - b->off[i] : nbi;   // local end of the near strip
+      const int e0 = ((j0 + 1) * sw - b->off[i] < ce) ? (j0 + 1) * sw - b->off[i] : ce;   // local end of the near strip
       if (ne < e0) { tr.add(i, lpb, nbi, b->n[i], ne | ((e0 - ne) << 16), kb, a2, (nbi - ne) * 2 * (e0 - ne)); tr.any_first |= first; }
       const int jl = (b->off[i] + nbi - 1) / sw;   // last global strip this site reaches
       if (jl > jmax) jmax = jl;
@@ -250,9 +277,9 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
         const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
         if (lpb < 0 || lpb >= nbi) continue;
         const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
-        const int o = j * sw - b->off[i];
-        if (lpe >= nbi || o >= nbi) continue;
-        const int wj = (o + sw < nbi) ? sw : nbi - o;
+        const int o = j * sw - b->off[i], ce = lpe < hs[i] ? hs[i] : nbi;
+        if (lpe >= nbi || lpe == hs[i] || o >= ce) continue;
+        const int wj = (o + sw < ce) ? sw : ce - o;
         const bool first = (lpb == 0) && !pre[i];
         ts.add(i, lpb, nbi, b->n[i], o | (wj << 16), lpe - lpb, first ? 0 : 1, (nbi - o) * 2 * wj);
         ts.any_first |= first;
@@ -270,13 +297,7 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
 
 // U = L^-T by recursive doubling, all sites per launch, stream W.  b_trtri_advance(Fg): every merge whose block range lies
 // inside the block columns that are final once the global step Fg is reached (site i: its first Fg - off_i columns) and has
-// not been launched yet (trtri_advance of dgp_api.cu); Fg >= NB: everything that is left.  want_T: also transpose the last
-// level, so that T = L^-1 is complete in the lower triangle of the A slab (dgp_batch_factorize, for the prediction).
-struct BInvProgress {
-  short done[16][DGP_BATCH_MAX];
-  bool want_T;
-  cudaStream_t W;
-};
+// not been launched yet (trtri_advance of dgp_api.cu); Fg >= NB: everything that is left.
 
 int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg) {
   const int G = b->G, NB = b->NB;

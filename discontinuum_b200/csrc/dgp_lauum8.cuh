@@ -10,6 +10,9 @@
 //   3. k_l8_recon: the Chinese remainder theorem in 128-bit integer arithmetic gives C' = A' A'' exactly (|C'| < M / 2,
 //      M = prod m_j ~ 2^124.95, which is what fixes b), rounded once to double and scaled by 2^-(s_r + s_c).
 //
+// The same kernels form C = sign A B' for the merges of the inverse (k_l8_gemm_ab, k_l8_recon_ab) and the quadrant update
+// A22 -= L21 L21' of the split factorisation (L8_KFULL_SYRK, accumulating reconstruction); see dgp_api.cu.
+//
 // The result is a deterministic function of U and npad alone (no tiling or launch order enters it), so a batched
 // launch reproduces a single-site one bit for bit.  b = l8_bits(npad) is the largest b with 2 npad 2^(2b-2) < M: 55 at
 // npad = 16384 and 32768, one rounding of each operand at 2^-54 relative to its row's largest entry.
@@ -310,29 +313,47 @@ __global__ void __launch_bounds__(128, 2) k_l8_gemm(const __grid_constant__ CUte
   l8_tile(&tmR, &tmR, j, i * 128, c * 128, i, nb - i, dst, i == c ? 128 : ld);   // k blocks i .. nb-1
 }
 
-// C = A B' over ra x rb tiles (C residues [16][128 ra][128 rb]), k blocks [i, kb) of tile (i, c) when kupper (A upper block
-// triangular, kb its block width), [0, c + 1) otherwise (B lower block triangular).  Grid = 16 * 64 ceil(ra / 8) ceil(rb / 8):
-// cells of 8 x 8 tiles, the longest K first (kupper: row-major from the top; else column-major from the right).
+// k ranges of k_l8_gemm_ab
+enum { L8_KLOWER_B = 0, L8_KUPPER_A = 1, L8_KFULL_SYRK = 2 };
+
+// C = A B' over ra x rb tiles (C residues [16][128 ra][128 rb]), the k blocks of tile (i, c) by kmode:
+//   L8_KUPPER_A: [i, kb) (A upper block triangular, kb its block width); L8_KLOWER_B: [0, c + 1) (B lower block triangular);
+//   L8_KFULL_SYRK: [0, kb), the lower tiles c <= i of a square product (rb = ra, A and B the same planes) only.
+// Grid = 16 * 64 ceil(ra / 8) ceil(rb / 8): cells of 8 x 8 tiles, the longest K first (L8_KUPPER_A: row-major from the top;
+// L8_KLOWER_B: column-major from the right); L8_KFULL_SYRK: 16 * l8_slots(ra), the band order of k_l8_gemm.
 __global__ void __launch_bounds__(128, 2) k_l8_gemm_ab(const __grid_constant__ CUtensorMap tmA,
                                                        const __grid_constant__ CUtensorMap tmB, int ra, int rb, int kb,
-                                                       bool kupper, int8_t* __restrict__ C) {
+                                                       int kmode, int8_t* __restrict__ C) {
+  const long long ldc = 128LL * rb;
+  if (kmode == L8_KFULL_SYRK) {
+    const int slots = l8_slots(ra);
+    const int j = blockIdx.x / slots, tile = blockIdx.x - j * slots;
+    const int p = (isqrt_floor(4 * (tile >> 5) + 1) - 1) >> 1;
+    const int rem = tile - 32 * p * (p + 1);
+    const int i = 8 * p + ((rem & 63) >> 3), c = 8 * (rem >> 6) + (rem & 7);
+    if (i >= ra || c > i) return;
+    int8_t* dst = C + (size_t)j * 128 * ra * ldc + (size_t)i * 128 * ldc + (size_t)c * 128;
+    l8_tile(&tmA, &tmB, j, i * 128, c * 128, 0, kb, dst, ldc);
+    return;
+  }
+  const bool kupper = kmode == L8_KUPPER_A;
   const int cr = (ra + 7) / 8, cc = (rb + 7) / 8, slots = 64 * cr * cc;
   const int j = blockIdx.x / slots, tile = blockIdx.x - j * slots;
   const int cell = tile >> 6, w = tile & 63;
   const int i = 8 * (kupper ? cell / cc : cell % cr) + (w >> 3);
   const int c = kupper ? 8 * (cell % cc) + (w & 7) : 8 * (cc - 1 - cell / cr) + 7 - (w & 7);
   if (i >= ra || c < 0 || c >= rb) return;
-  const long long ldc = 128LL * rb;
   int8_t* dst = C + (size_t)j * 128 * ra * ldc + (size_t)i * 128 * ldc + (size_t)c * 128;
   if (kupper) l8_tile(&tmA, &tmB, j, i * 128, c * 128, i, kb - i, dst, ldc);
   else l8_tile(&tmA, &tmB, j, i * 128, c * 128, 0, c + 1, dst, ldc);
 }
 
 // ---------------------------------------------------------------- 3. reconstruction: one CTA per 128 x 128 tile
-// out[r][c] = sign 2^-(sr[r] + sc[c]) C'[r][c] for the tile whose residues of plane j start at src + j plane (row stride ls)
+// out[r][c] = sign 2^-(sr[r] + sc[c]) C'[r][c] for the tile whose residues of plane j start at src + j plane (row stride ls);
+// acc: out[r][c] += that instead (the product rounded once, then one FP64 addition)
 __device__ __forceinline__ void l8_recon_tile(const int8_t* __restrict__ src, size_t plane, size_t ls,
                                               const int* __restrict__ sr, const int* __restrict__ sc, double sign,
-                                              double* __restrict__ out, long long ldo) {
+                                              double* __restrict__ out, long long ldo, bool acc = false) {
   const int cq = 4 * (threadIdx.x & 31);
   const int sc0 = sc[cq], sc1 = sc[cq + 1], sc2 = sc[cq + 2], sc3 = sc[cq + 3];
 #pragma unroll 1
@@ -352,6 +373,11 @@ __device__ __forceinline__ void l8_recon_tile(const int8_t* __restrict__ src, si
     o1.x = sign * l8_crt(y[2], -(s + sc2));
     o1.y = sign * l8_crt(y[3], -(s + sc3));
     double* kp = out + (size_t)rr * ldo + cq;
+    if (acc) {
+      const double2 a0 = *reinterpret_cast<const double2*>(kp), a1 = *reinterpret_cast<const double2*>(kp + 2);
+      o0.x = __dadd_rn(a0.x, o0.x); o0.y = __dadd_rn(a0.y, o0.y);
+      o1.x = __dadd_rn(a1.x, o1.x); o1.y = __dadd_rn(a1.y, o1.y);
+    }
     *reinterpret_cast<double2*>(kp) = o0;
     *reinterpret_cast<double2*>(kp + 2) = o1;
   }
@@ -372,14 +398,24 @@ __global__ void __launch_bounds__(256) k_l8_recon(const int8_t* __restrict__ R, 
                      K + (size_t)i * 128 * ldk + c * 128, ldk);
 }
 
-// out[128 ra][128 rb] (leading dimension ldo) = sign C from the residues of k_l8_gemm_ab; one CTA per tile
+// out[128 ra][128 rb] (leading dimension ldo) = sign C from the residues of k_l8_gemm_ab; one CTA per tile.
+// syrk (the L8_KFULL_SYRK product, rb = ra): out += sign C on the lower tiles only (diagonal tiles in full), grid ra (ra + 1) / 2
 __global__ void __launch_bounds__(256) k_l8_recon_ab(const int8_t* __restrict__ C, int ra, int rb, const int* __restrict__ sa,
                                                      const int* __restrict__ sb, double sign, double* __restrict__ out,
-                                                     long long ldo) {
-  const int i = blockIdx.x / rb, c = blockIdx.x - i * rb;
+                                                     long long ldo, bool syrk) {
+  int i, c;
+  if (syrk) {
+    const int t = blockIdx.x;
+    i = (int)((sqrt(8.0 * t + 1.0) - 1.0) * 0.5);
+    while (i * (i + 1) / 2 > t) --i;
+    while ((i + 1) * (i + 2) / 2 <= t) ++i;
+    c = t - i * (i + 1) / 2;
+  } else {
+    i = blockIdx.x / rb; c = blockIdx.x - i * rb;
+  }
   const size_t ldc = (size_t)128 * rb;
   l8_recon_tile(C + (size_t)i * 128 * ldc + c * 128, (size_t)128 * ra * ldc, ldc, sa + i * 128, sb + c * 128, sign,
-                out + (size_t)i * 128 * ldo + c * 128, ldo);
+                out + (size_t)i * 128 * ldo + c * 128, ldo, syrk);
 }
 
 }  // namespace dgp

@@ -124,9 +124,10 @@ int main(int argc, char** argv) {
         k_l8_convert<<<(unsigned)r2, 256>>>(T22, npad, (int)kw, b, false, true, PB, kw, r2 * kw, sexp + r1);
       }
       cudaEventRecord(ev[1]);
-      k_l8_gemm_ab<<<L8_NMOD * 64 * ((hb + 7) / 8) * ((w2 + 7) / 8), 128, L8_SMEM>>>(ta, tb, hb, w2, kb, first, PC);
+      k_l8_gemm_ab<<<L8_NMOD * 64 * ((hb + 7) / 8) * ((w2 + 7) / 8), 128, L8_SMEM>>>(ta, tb, hb, w2, kb,
+                                                                                 first ? L8_KUPPER_A : L8_KLOWER_B, PC);
       cudaEventRecord(ev[2]);
-      k_l8_recon_ab<<<hb * w2, 256>>>(PC, hb, w2, sexp, sexp + r1, first ? 1.0 : -1.0, first ? Me : Ue, r2);
+      k_l8_recon_ab<<<hb * w2, 256>>>(PC, hb, w2, sexp, sexp + r1, first ? 1.0 : -1.0, first ? Me : Ue, r2, false);
       cudaEventRecord(ev[3]);
     };
     cudaEvent_t ev[6];
