@@ -16,6 +16,11 @@ MAX_TERMS, MAX_FACTORS, MAX_FDIMS, MAX_COLS, MAX_THETA = 8, 3, 4, 8, 48
 ABI_VERSION = 2
 BATCH_MAX_SITES = 32
 BATCH_PREDICT_CHUNK = 1024  # grid rows of every site per launch of dgp_batch_predict (csrc/dgp_batch.cuh)
+# Default cap on the sampling arena of one dgp_batch_sample_ex call (BatchEngine.sample).  A config-4 site (m = 10 958
+# daily points, n <= 8 000, S = 1000) needs 1.9 GB, a group of 16 about 30 GB, so one call covers such a group; two lanes
+# of 16 such sites then hold 2 x (25 GB of training slabs + 1 GB of prediction slabs + 32 GB of arena) = 116 GB of the
+# B200's 180 GB.
+BATCH_SAMPLE_MAX_BYTES = 32 << 30
 
 RBF, MATERN32, MATERN52, PERIODIC = 0, 1, 2, 3
 GATE_NONE, GATE_SIGMOID, GATE_INV_SIGMOID = 0, 1, 2
@@ -99,6 +104,8 @@ _SIGNATURES = [
     ("dgp_batch_factorize", C.c_int, [_P, _P, _P, _P, _P]),
     ("dgp_batch_predict", C.c_int, [_P, _P, _P, _P, _P]),
     ("dgp_batch_mean_functional_grad", C.c_int, [_P, _P, _P, _P, _P, _P]),
+    ("dgp_batch_sample_ex", C.c_int, [_P, _P, _P, C.c_int, _P, _P, _P, _P, _P, _P]),
+    ("dgp_batch_sample_bytes", C.c_size_t, [_P, _P, C.c_int, _P]),
     ("dgp_batch_get_alpha", C.c_int, [_P, C.c_int, _P]),
     ("dgp_batch_launch_count", C.c_longlong, [_P]),
     ("dgp_batch_set_timing", C.c_int, [_P, C.c_int]),
@@ -158,6 +165,17 @@ def _ptr(a) -> Tuple[int, int]:
 
 def _f64(a) -> np.ndarray:
     return np.ascontiguousarray(np.asarray(a, dtype=np.float64))
+
+
+def _flux_reduce(flux: dict, m: int):
+    """(DgpFluxReduce, arrays it points into) of a flux dict of Engine.sample_ex over a grid of m points."""
+    w = _f64(flux["weight"]).reshape(-1)
+    gs = np.ascontiguousarray(np.asarray(flux["group_start"], dtype=np.int32))
+    if w.shape[0] != m:
+        raise ValueError("sample: weight[m] expected")
+    red = DgpFluxReduce(float(flux["y_mean"]), float(flux["y_scale"]), int(flux.get("log_transform", 1)),
+                        int(gs.shape[0] - 1), w.ctypes.data, gs.ctypes.data)
+    return red, (w, gs)
 
 
 class BatchEngine:
@@ -277,6 +295,95 @@ class BatchEngine:
         pv = (_P * G)(*[None if o[1] is None or o[1].shape[0] == 0 else o[1].ctypes.data for o in out])
         self._check(self.lib.dgp_batch_predict(self._h, ms, px, pm, pv if want_var else None), "dgp_batch_predict")
         return out
+
+    def _sample_call(self, sites, m, xs, S, Z, seeds, jitter, reds, outs):
+        G = self.nsites
+        ms = (C.c_int * G)(*[m[i] if i in sites else 0 for i in range(G)])
+        red_arr = (C.POINTER(DgpFluxReduce) * G)(*[C.pointer(reds[i]) if i in sites and reds[i] is not None else None
+                                                   for i in range(G)])
+        px = (_P * G)(*[xs[i].ctypes.data if i in sites else None for i in range(G)])
+        po = (_P * G)(*[outs[i].ctypes.data if i in sites else None for i in range(G)])
+        pz = (_P * G)(*[Z[i].ctypes.data if i in sites else None for i in range(G)]) if Z is not None else None
+        seed_arr = (C.c_ulonglong * G)(*seeds)
+        jit = (C.c_double * G)(*jitter)
+        info = np.zeros(G, dtype=np.int32)
+        self._check(self.lib.dgp_batch_sample_ex(self._h, ms, px, int(S), pz, seed_arr, jit, red_arr, po, info.ctypes.data),
+                    "dgp_batch_sample_ex")
+        return info
+
+    def sample_bytes(self, m, S: int, flux=None) -> int:
+        """Device bytes of the sampling arena of one dgp_batch_sample_ex call over the sites with m[s] > 0."""
+        G = self.nsites
+        ms = (C.c_int * G)(*[int(v) for v in m])
+        keep = [_flux_reduce(flux[i], int(m[i])) if flux is not None and flux[i] is not None and m[i] > 0 else None
+                for i in range(G)]   # the structures and the arrays they point into, alive through the call
+        red_arr = (C.POINTER(DgpFluxReduce) * G)(*[C.pointer(r[0]) if r is not None else None for r in keep])
+        return int(self.lib.dgp_batch_sample_bytes(self._h, ms, int(S), red_arr))
+
+    def sample(self, grids, S: int, seeds=None, Z=None, jitter=None, flux=None, max_bytes: int = BATCH_SAMPLE_MAX_BYTES):
+        """Joint posterior draws of every site on its own grid (Engine.sample_ex per site, bit for bit).
+        grids: length-G sequence of Xs[m_s, ndim] host arrays, or None to skip a site.  seeds[G]: Philox key of each site's
+        normals (default 0); Z: length-G sequence of host normals [S, m_s] (or None for skipped sites) instead;
+        jitter[G]: added to the diagonal of each site's posterior covariance (default 0); flux: length-G sequence of the
+        dicts Engine.sample_ex takes (or None: raw draws for that site).  Returns [(out, info)] per site: out [S, m_s], or
+        [S, groups] with a reduction; (None, 0) for a skipped site.  Needs factorize of every sampled site first.
+        The sampled sites go to the device in consecutive calls whose arena (sample_bytes) stays at or below max_bytes (a
+        site that alone needs more gets a call of its own); the results do not depend on the split.  The default
+        (BATCH_SAMPLE_MAX_BYTES, 32 GiB) holds a group of 16 config-4 sites (1.9 GB each) in one call, so that two lanes of
+        16 such sites fit on a 180 GB B200 next to their training and prediction slabs."""
+        G = self.nsites
+        if len(grids) != G:
+            raise ValueError(f"sample: {G} grids (or None) expected, got {len(grids)}")
+        S = int(S)
+        seeds = [0] * G if seeds is None else [int(v) for v in seeds]
+        jitter = [0.0] * G if jitter is None else [float(v) for v in _f64(jitter).reshape(-1)]
+        if len(seeds) != G or len(jitter) != G:
+            raise ValueError("sample: seeds and jitter need one entry per site")
+        if Z is not None and len(Z) != G:
+            raise ValueError("sample: Z needs one entry (or None) per site")
+        if flux is not None and len(flux) != G:
+            raise ValueError("sample: flux needs one entry (or None) per site")
+        xs, m, reds, keep, outs, Zs = [None] * G, [0] * G, [None] * G, [], [None] * G, [None] * G
+        for i, Xs in enumerate(grids):
+            if Xs is None:
+                continue
+            Xs = _f64(Xs)
+            if Xs.ndim != 2 or Xs.shape[1] != self._keep.ndim:
+                raise ValueError("sample: Xs[m, ndim] expected for every site")
+            if Xs.shape[0] == 0:
+                continue
+            xs[i], m[i] = Xs, int(Xs.shape[0])
+            if Z is not None:
+                if Z[i] is None:
+                    raise ValueError(f"sample: site {i} has a grid but no normals")
+                Zs[i] = _f64(Z[i])
+                if Zs[i].shape != (S, m[i]):
+                    raise ValueError(f"sample: Z[{i}] must be [S, m] = [{S}, {m[i]}]")
+            if flux is not None and flux[i] is not None:
+                reds[i], arrs = _flux_reduce(flux[i], m[i])
+                keep.append(arrs)
+                outs[i] = np.empty((S, reds[i].ngroups))
+            else:
+                outs[i] = np.empty((S, m[i]))
+        infos = np.zeros(G, dtype=np.int32)
+        sampled = [i for i in range(G) if m[i] > 0]
+        calls, cur = [], []
+        for i in sampled:
+            trial = cur + [i]
+            need = self.sample_bytes([m[j] if j in trial else 0 for j in range(G)], S,
+                                     [flux[j] if flux is not None and j in trial else None for j in range(G)])
+            if cur and need > max_bytes:
+                calls.append(cur)
+                cur = [i]
+            else:
+                cur = trial
+        if cur:
+            calls.append(cur)
+        for sites in calls:
+            info = self._sample_call(set(sites), m, xs, S, Zs if Z is not None else None, seeds, jitter, reds, outs)
+            for i in sites:
+                infos[i] = info[i]
+        return [(outs[i], int(infos[i])) for i in range(G)]
 
     def mean_functional_grad(self, points, c):
         """(val[G], grad[G, P]): F_s = sum_p c[s][p] mu_s(points[s][p]) and dF_s/dtheta_s of every site at the theta of its

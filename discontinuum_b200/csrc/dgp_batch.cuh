@@ -15,6 +15,69 @@
 // Included at the end of dgp_api.cu (uses its launch helpers).
 #pragma once
 
+namespace dgp {
+// ------------------------------------------------------------------ batched joint posterior samples (dgp_batch_sample_ex)
+// The sites one call samples, by slot k (the index of the sampling arena's slabs, in batch order): site[k] = the batch
+// site, m[k] = grid points, seed[k] = Philox key of its normals, ng[k] > 0: groups of its flux reduction.
+struct SampleTab {
+  int site[DGP_BATCH_MAX], m[DGP_BATCH_MAX], ng[DGP_BATCH_MAX], logt[DGP_BATCH_MAX];
+  unsigned long long seed[DGP_BATCH_MAX];
+  double mean[DGP_BATCH_MAX], scale[DGP_BATCH_MAX];
+};
+
+// k_copy_panel of the in-place factorisation for the entries of pk (blockIdx.y): staging slab [site][ld][128], matrix
+// slab [site][ld][ld].  grid = (largest row-block count below the diagonal block, entries)
+__global__ void __launch_bounds__(256)
+k_copy_panel_b(const double* __restrict__ P, double* __restrict__ A, long long ld, const __grid_constant__ P2Batch pk,
+               const __grid_constant__ SiteDims sd) {
+  const int st = pk.site[blockIdx.y], s = pk.step[blockIdx.y];
+  if ((int)blockIdx.x >= sd.nb[st] - s - 1) return;
+  copy_panel_body(P + (size_t)st * (size_t)ld * 128, A + (size_t)st * (size_t)ld * (size_t)ld, ld, s, blockIdx.x);
+}
+
+// rows of one prediction chunk (starting at grid row m0) of the features and the posterior mean of batch site site[k]
+// (chunk slabs [site][chunk][...]) -> slot k of the whole-grid slabs [slot][mld][...].  grid = (chunk / 256, slots)
+__global__ void __launch_bounds__(256)
+k_sample_gather(const __grid_constant__ SampleTab tab, const __grid_constant__ PredChunk pc, const double* __restrict__ Xws,
+                const double* __restrict__ mu, int chunk, int m0, double* __restrict__ Xws_all, double* __restrict__ mu_all,
+                long long mld) {
+  const int k = blockIdx.y, st = tab.site[k], r = blockIdx.x * 256 + threadIdx.x, mc = pc.m[st];
+  if (r >= (mc + 127) / 128 * 128) return;
+  const double* src = Xws + ((size_t)st * chunk + r) * DGP_XS;
+  double* dst = Xws_all + ((size_t)k * mld + m0 + r) * DGP_XS;
+#pragma unroll
+  for (int e = 0; e < DGP_XS; e++) dst[e] = src[e];
+  if (r < mc) mu_all[(size_t)k * mld + m0 + r] = mu[(size_t)st * chunk + r];
+}
+
+// k_fill_normals of every slot: Z[k][s, i] = normal number s m[k] + i of the stream seed[k].  grid = (ceil(max m / 256), S, slots)
+__global__ void __launch_bounds__(256)
+k_fill_normals_b(double* __restrict__ Z, long long ld, long long slab, const __grid_constant__ SampleTab tab) {
+  const int k = blockIdx.z, m = tab.m[k], i = blockIdx.x * 256 + threadIdx.x;
+  if (i < m)
+    Z[(size_t)k * slab + (size_t)blockIdx.y * ld + i] = philox_normal(tab.seed[k], (unsigned long long)blockIdx.y * (unsigned long long)m + i);
+}
+
+// k_add_rowvec of every slot: out[k][s, i] += mu[k][i].  grid = (ceil(max m / 256), S, slots)
+__global__ void __launch_bounds__(256)
+k_add_rowvec_b(double* __restrict__ out, long long ld, long long slab, const double* __restrict__ mu, const __grid_constant__ SampleTab tab) {
+  const int k = blockIdx.z, i = blockIdx.x * 256 + threadIdx.x;
+  if (i < tab.m[k]) out[(size_t)k * slab + (size_t)blockIdx.y * ld + i] += mu[(size_t)k * ld + i];
+}
+
+// k_flux_reduce of every slot with a reduction: draws [slot][S][ld] (slab apart), weights [slot][ld], group starts
+// [slot][gld], sums [slot][S][ng] (oslab apart).  grid = (largest group count, ceil(S / 8), slots)
+__global__ void __launch_bounds__(256)
+k_flux_reduce_b(const double* __restrict__ D, long long ld, long long slab, const double* __restrict__ w,
+                const int* __restrict__ start, int gld, int S, const __grid_constant__ SampleTab tab, double* __restrict__ out,
+                long long oslab) {
+  const int k = blockIdx.z, g = blockIdx.x;
+  if (g >= tab.ng[k]) return;
+  flux_reduce_body(D + (size_t)k * slab, ld, w + (size_t)k * ld, start + (size_t)k * gld, tab.ng[k], S, tab.mean[k],
+                   tab.scale[k], tab.logt[k], out + (size_t)k * oslab, g, blockIdx.y * 8 + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+}  // namespace dgp
+
 struct dgp_batch_s {
   int device = 0, sms = 148;
   cudaStream_t stream = nullptr, stream_hi = nullptr, stream_lo = nullptr, stream_t2 = nullptr;
@@ -57,6 +120,9 @@ struct dgp_batch_s {
   double *cvec = nullptr, *vvec = nullptr, *tmpz = nullptr, *gam = nullptr, *gzpart = nullptr, *wpart = nullptr, *mfg = nullptr;
   double *h_c = nullptr, *h_mfg = nullptr;  // pinned
   long long mfg_pstride = 0;
+  // sampling arena (dgp_batch_sample_ex): grow-only, sized by dgp_batch_sample_bytes of the largest call so far
+  double* sarena = nullptr;
+  size_t sarena_count = 0;
   long long launches = 0;
   double last_ms[4] = {0, 0, 0, 0};
   std::string err;
@@ -82,9 +148,9 @@ struct TabBuilder {
   BatchTab t;
   int total = 0;
   bool any_first = false;
-  explicit TabBuilder(dgp_batch_t b) {
+  explicit TabBuilder(dgp_batch_t b, long long ld = 0) {
     memset(&t, 0, sizeof(t));
-    t.ld = b->ld;
+    t.ld = ld ? ld : b->ld;
     t.jitv = b->jitv;
   }
   void add(int site, int step, int nb, int n, int a0, int a1, int a2, int ntiles) {
@@ -104,14 +170,34 @@ GemmArgs b_args(dgp_batch_t b, int mode, double* C, double sign, int ntiles) {
   return g;
 }
 
+// The matrices b_potrf factorises, all sites of one launch sequence: the training covariances of the batch (generate:
+// written by the covariance generator, L and U apart from the work slab A, the INT8 quadrant split and the eager inverse as
+// in the training factorisation) or the posterior covariances of dgp_batch_sample_ex (in place, L == A, as potrf_core's
+// generate = false, hs = 0 path: the diagonal-block kernel leaves T_ss in DI, the panel solve stages its block column in P
+// and k_copy_panel_b puts it back).  Per-site sizes, the leading dimension and the site count are those of *sd.
+struct BChol {
+  double *A, *L, *U, *scal;          // slabs [site][ld][ld] (U: NULL in place), [site][SC_SIZE]
+  const CUtensorMap *tA, *tL;
+  double *DI, *P;                    // in place: [site][ld][128] each
+  const CUtensorMap* tDI;
+  const SiteDims* sd;
+  const int *off, *order;            // end-aligned start step of each site, sites largest first
+  bool generate;
+};
+
+BChol b_train_chol(dgp_batch_t b) {
+  return BChol{b->A, b->L, b->U, b->scal, &b->tmA, &b->tmL, nullptr, nullptr, nullptr, &b->sd, b->off, b->order, true};
+}
+
 // one rank-(128 kb) update launch over the sites of `tb` (M_TRAIL_COL entries); half_limit: largest tile count that still
 // runs on 64-row half tiles
-int b_launch_trail(dgp_batch_t b, const TabBuilder& tb, cudaStream_t st, int half_limit, bool pdl) {
+int b_launch_trail(dgp_batch_t b, const BChol& c, const TabBuilder& tb, cudaStream_t st, int half_limit, bool pdl) {
   if (tb.total <= 0) return 0;
-  GemmArgs g = b_args(b, M_TRAIL_COL, b->A, -1.0, tb.total);
-  if (tb.any_first) return launch_gemm<INIT_COV, EPI_STORE>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
-  if (tb.total <= half_limit) return launch_gemm<INIT_LOAD, EPI_STORE, 4>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
-  return launch_gemm<INIT_LOAD, EPI_STORE>(b, b->tmL, b->tmL, g, st, pdl, &tb.t);
+  GemmArgs g = b_args(b, M_TRAIL_COL, c.A, -1.0, tb.total);
+  g.nb = c.sd->nbmax; g.ldc = c.sd->ld;
+  if (tb.any_first) return launch_gemm<INIT_COV, EPI_STORE>(b, *c.tL, *c.tL, g, st, pdl, &tb.t);
+  if (tb.total <= half_limit) return launch_gemm<INIT_LOAD, EPI_STORE, 4>(b, *c.tL, *c.tL, g, st, pdl, &tb.t);
+  return launch_gemm<INIT_LOAD, EPI_STORE>(b, *c.tL, *c.tL, g, st, pdl, &tb.t);
 }
 
 int b_ensure_events(dgp_batch_t b, size_t count) {
@@ -134,10 +220,15 @@ struct BInvProgress {
 int b_trtri_advance(dgp_batch_t b, BInvProgress& ip, int Fg);
 int b_eager(dgp_batch_t b, BInvProgress* ip, cudaEvent_t ev_panel, int pe);
 
-int b_potrf(dgp_batch_t b, BInvProgress* eager) {
-  const int G = b->G, NB = b->NB;
+int b_potrf(dgp_batch_t b, const BChol& c, BInvProgress* eager) {
+  const SiteDims& sd = *c.sd;
+  const int G = sd.count, NB = sd.nbmax;
+  const int* nb = sd.nb;
+  const int* off = c.off;
+  const int* order = c.order;
   constexpr int pw = PANEL_BLOCKS, sw = STRIP_BLOCKS;
-  const long long ld = b->ld;
+  const long long ld = sd.ld;
+  const bool inplace = c.L == c.A;
   cudaStream_t T = b->stream, P = b->stream_hi, T2 = b->stream_t2;
   const int npanels = (NB + pw - 1) / pw;
   int rc;
@@ -146,9 +237,11 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
   auto ev_panel = [&](int p) { return b->evs[3 * p]; };
   auto ev_cols = [&](int p) { return b->evs[3 * p + 1]; };
   auto ev_col0 = [&](int p) { return b->evs[3 * p + 2]; };
-  k_cov_col0_b<<<dim3(4 * NB, 1, G), 256, 0, T>>>(b->spec, b->sd, b->theta, b->Xw, b->noise, b->jitv, b->A);
-  b->launches++;
-  CK(b, cudaGetLastError());
+  if (c.generate) {
+    k_cov_col0_b<<<dim3(4 * NB, 1, G), 256, 0, T>>>(b->spec, sd, b->theta, b->Xw, b->noise, b->jitv, c.A);
+    b->launches++;
+    CK(b, cudaGetLastError());
+  }
   CK(b, cudaEventRecord(ev_cols(0), T));
   CK(b, cudaStreamWaitEvent(P, ev_cols(0), 0));
   // standalone generator (as in potrf_core): the sites with more than DGP_PREGEN_MIN_NB block columns get their
@@ -157,20 +250,20 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
   bool pre[DGP_BATCH_MAX];
   bool any_pre = false, wP = false, wT = false, w2 = false;
   for (int i = 0; i < G; i++) {
-    pre[i] = b->nb[i] > DGP_PREGEN_MIN_NB;
+    pre[i] = c.generate && nb[i] > DGP_PREGEN_MIN_NB;
     any_pre |= pre[i];
   }
   cudaEvent_t ev_gen = b->evs[3 * (size_t)npanels + 1];
   // split factorisation (syrk_split, potrf_core of dgp_api.cu) of every site the rule sends there, at its local block column
   // hs[i]; the quadrant updates run one site at a time and share the residue buffers with the eager inverse's INT8 merges on
-  // stream W, so the two are ordered by events both ways
+  // stream W, so the two are ordered by events both ways.  No split in place (hs = 0, as in potrf_core).
   int hs[DGP_BATCH_MAX];
-  for (int i = 0; i < G; i++) hs[i] = syrk_split(b->nb[i]);
+  for (int i = 0; i < G; i++) hs[i] = c.generate ? syrk_split(nb[i]) : 0;
   cudaEvent_t ev_w = b->evs[3 * (size_t)npanels + 2], ev_syrk = b->evs[3 * (size_t)npanels + 3];
   bool w_pending = false, syrk_pending = false;
   if (any_pre) {
     CK(b, cudaStreamWaitEvent(b->stream_lo, ev_cols(0), 0));
-    k_cov_lower_b<<<dim3(4 * NB, NB - 1, G), 256, 0, b->stream_lo>>>(b->spec, b->sd, b->theta, b->Xw, b->noise, b->jitv, b->A,
+    k_cov_lower_b<<<dim3(4 * NB, NB - 1, G), 256, 0, b->stream_lo>>>(b->spec, sd, b->theta, b->Xw, b->noise, b->jitv, c.A,
                                                                             DGP_PREGEN_MIN_NB);
     b->launches++;
     CK(b, cudaGetLastError());
@@ -185,37 +278,54 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
       P2Batch pk;
       memset(&pk, 0, sizeof(pk));
       pk.slab = ld * ld;
-      TabBuilder trsm(b), inp(b);
+      if (inplace) pk.dslab = ld * 128;
+      TabBuilder trsm(b, ld), inp(b, ld);
+      int mmax = 0;
       for (int k = 0; k < G; k++) {
-        const int i = b->order[k], s = t - b->off[i], nbi = b->nb[i];
+        const int i = order[k], s = t - off[i], nbi = nb[i];
         if (s < 0 || s >= nbi) continue;
         pk.site[pk.count] = (short)i; pk.step[pk.count] = (short)s; pk.count++;
         const int m = nbi - s - 1;
-        trsm.add(i, s, nbi, b->n[i], 0, 1, 0, 2 * m);
-        const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
+        if (m > mmax) mmax = m;
+        // in place: into the staging slab P (aux0 = 1), T_ss from the block-inverse slab DI (aux1 = 0)
+        trsm.add(i, s, nbi, sd.n[i], inplace ? 1 : 0, inplace ? 0 : 1, 0, 2 * m);
+        const int lpe = (pe - off[i] < nbi) ? pe - off[i] : nbi;
         if (s + 1 < lpe) {   // right-looking, like the single-site engine: the two must agree for bit-identical results
           const int w = lpe - s - 1;
-          const bool first = (s == 0) && !pre[i];
-          inp.add(i, s, nbi, b->n[i], (s + 1) | (w << 16), 1, first ? 0 : 1, m * 2 * w);
+          const bool first = (s == 0) && c.generate && !pre[i];
+          inp.add(i, s, nbi, sd.n[i], (s + 1) | (w << 16), 1, first ? 0 : 1, m * 2 * w);
           inp.any_first |= first && m > 0;
         }
       }
       if (pk.count == 0) continue;
-      // dependent launch behind the in-panel update of the previous block column (same stream, nothing in between)
-      CK(b, launch_ex(k_potf2_v2, pk.count, P2_THREADS, (size_t)P2_SMEM, P, t > pb, (const double*)b->A, b->L, b->U, ld,
-                      (double*)nullptr, b->scal, 0, b->A, 0, pk));
+      // dependent launch behind the in-panel update of the previous block column (same stream, nothing in between; in
+      // place the copy of the staged panel is in between, as in factor_panel)
+      CK(b, launch_ex(k_potf2_v2, pk.count, P2_THREADS, (size_t)P2_SMEM, P, t > pb && !inplace, (const double*)c.A, c.L, c.U, ld,
+                      c.DI, c.scal, 0, inplace ? (double*)nullptr : c.A, inplace ? 1 : 0, pk));
       b->launches++;
       if (trsm.total > 0) {  // panel solve: L[i, s] = A[i, s] T_ss', T_ss read from the diagonal block of the work matrix
-        GemmArgs g = b_args(b, M_TRSM, b->L, 1.0, trsm.total);
-        if (2 * trsm.total <= slots) { if ((rc = launch_gemm<INIT_ZERO, EPI_STORE, 4>(b, b->tmA, b->tmA, g, P, true, &trsm.t))) return rc; }
-        else if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmA, b->tmA, g, P, true, &trsm.t))) return rc;
+        GemmArgs g = b_args(b, M_TRSM, c.L, 1.0, trsm.total);
+        g.nb = NB; g.ldc = ld;
+        const CUtensorMap* tB = c.tA;
+        if (inplace) {
+          g.C = c.P; g.ldc = 128; tB = c.tDI;
+          trsm.t.cstride = ld * 128;
+          for (int k = 0; k < G; k++) trsm.t.cslot[k] = (short)k;
+        }
+        if (2 * trsm.total <= slots) { if ((rc = launch_gemm<INIT_ZERO, EPI_STORE, 4>(b, *c.tA, *tB, g, P, true, &trsm.t))) return rc; }
+        else if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, *c.tA, *tB, g, P, true, &trsm.t))) return rc;
+        if (inplace) {
+          k_copy_panel_b<<<dim3(mmax, pk.count), 256, 0, P>>>(c.P, c.A, ld, pk, sd);
+          b->launches++;
+          CK(b, cudaGetLastError());
+        }
       }
       if (inp.total > 0) {   // rank-128 update of the panel's own remaining columns
         const bool waited = (t == pb && p > 0);
         if (waited) CK(b, cudaStreamWaitEvent(P, ev_cols(p), 0));
         const bool gen_wait = any_pre && !wP;
         if (gen_wait) { wP = true; CK(b, cudaStreamWaitEvent(P, ev_gen, 0)); }
-        if ((rc = b_launch_trail(b, inp, P, b->sms, !waited && !gen_wait))) return rc;
+        if ((rc = b_launch_trail(b, c, inp, P, b->sms, !waited && !gen_wait && !inplace))) return rc;
       }
     }
     CK(b, cudaEventRecord(ev_panel(p), P));
@@ -239,52 +349,52 @@ int b_potrf(dgp_batch_t b, BInvProgress* eager) {
       return T2;
     };
     cudaStream_t S0 = strip_stream(j0);
-    TabBuilder ta(b), tb2(b), tr(b);
+    TabBuilder ta(b, ld), tb2(b, ld), tr(b, ld);
     int jmax = j0;
     for (int k = 0; k < G; k++) {
-      const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
+      const int i = order[k], nbi = nb[i], lpb = pb - off[i];
       if (lpb < 0 || lpb >= nbi) continue;
-      const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
+      const int lpe = (pe - off[i] < nbi) ? pe - off[i] : nbi;
       if (lpe >= nbi) continue;
       if (lpe == hs[i]) {   // the site's quadrant update, ahead of ev_col0(p + 1) on S0
         if (w_pending) { w_pending = false; CK(b, cudaStreamWaitEvent(S0, ev_w, 0)); }
         const size_t so = (size_t)i * (size_t)ld * (size_t)ld;
-        if ((rc = syrk_i8(b, b->l8, b->max_pad, b->L + so, b->A + so, ld, nbi, hs[i], S0))) return rc;
+        if ((rc = syrk_i8(b, b->l8, b->max_pad, c.L + so, c.A + so, ld, nbi, hs[i], S0))) return rc;
         CK(b, cudaEventRecord(ev_syrk, S0));
         syrk_pending = true;
         continue;
       }
       const int ce = lpe < hs[i] ? hs[i] : nbi;   // end of the block columns this panel updates
       const int kb = lpe - lpb, ne = (lpe + pw < nbi) ? lpe + pw : nbi, w = ne - lpe, m = nbi - lpe;
-      const bool first = (lpb == 0) && !pre[i];
+      const bool first = (lpb == 0) && c.generate && !pre[i];
       const int a2 = first ? 0 : 1;
-      ta.add(i, lpb, nbi, b->n[i], lpe | (1 << 16), kb, a2, m * 2);
+      ta.add(i, lpb, nbi, sd.n[i], lpe | (1 << 16), kb, a2, m * 2);
       ta.any_first |= first;
-      if (w > 1) { tb2.add(i, lpb, nbi, b->n[i], (lpe + 1) | ((w - 1) << 16), kb, a2, (m - 1) * 2 * (w - 1)); tb2.any_first |= first; }
-      const int e0 = ((j0 + 1) * sw - b->off[i] < ce) ? (j0 + 1) * sw - b->off[i] : ce;   // local end of the near strip
-      if (ne < e0) { tr.add(i, lpb, nbi, b->n[i], ne | ((e0 - ne) << 16), kb, a2, (nbi - ne) * 2 * (e0 - ne)); tr.any_first |= first; }
-      const int jl = (b->off[i] + nbi - 1) / sw;   // last global strip this site reaches
+      if (w > 1) { tb2.add(i, lpb, nbi, sd.n[i], (lpe + 1) | ((w - 1) << 16), kb, a2, (m - 1) * 2 * (w - 1)); tb2.any_first |= first; }
+      const int e0 = ((j0 + 1) * sw - off[i] < ce) ? (j0 + 1) * sw - off[i] : ce;   // local end of the near strip
+      if (ne < e0) { tr.add(i, lpb, nbi, sd.n[i], ne | ((e0 - ne) << 16), kb, a2, (nbi - ne) * 2 * (e0 - ne)); tr.any_first |= first; }
+      const int jl = (off[i] + nbi - 1) / sw;   // last global strip this site reaches
       if (jl > jmax) jmax = jl;
     }
-    if ((rc = b_launch_trail(b, ta, S0, slots, false))) return rc;
+    if ((rc = b_launch_trail(b, c, ta, S0, slots, false))) return rc;
     if (p + 1 < npanels) CK(b, cudaEventRecord(ev_col0(p + 1), S0));
-    if ((rc = b_launch_trail(b, tb2, S0, slots, false))) return rc;
+    if ((rc = b_launch_trail(b, c, tb2, S0, slots, false))) return rc;
     if (p + 1 < npanels) CK(b, cudaEventRecord(ev_cols(p + 1), S0));
-    if ((rc = b_launch_trail(b, tr, S0, slots, false))) return rc;
+    if ((rc = b_launch_trail(b, c, tr, S0, slots, false))) return rc;
     for (int j = j0 + 1; j <= jmax; j++) {
-      TabBuilder ts(b);
+      TabBuilder ts(b, ld);
       for (int k = 0; k < G; k++) {
-        const int i = b->order[k], nbi = b->nb[i], lpb = pb - b->off[i];
+        const int i = order[k], nbi = nb[i], lpb = pb - off[i];
         if (lpb < 0 || lpb >= nbi) continue;
-        const int lpe = (pe - b->off[i] < nbi) ? pe - b->off[i] : nbi;
-        const int o = j * sw - b->off[i], ce = lpe < hs[i] ? hs[i] : nbi;
+        const int lpe = (pe - off[i] < nbi) ? pe - off[i] : nbi;
+        const int o = j * sw - off[i], ce = lpe < hs[i] ? hs[i] : nbi;
         if (lpe >= nbi || lpe == hs[i] || o >= ce) continue;
         const int wj = (o + sw < ce) ? sw : ce - o;
-        const bool first = (lpb == 0) && !pre[i];
-        ts.add(i, lpb, nbi, b->n[i], o | (wj << 16), lpe - lpb, first ? 0 : 1, (nbi - o) * 2 * wj);
+        const bool first = (lpb == 0) && c.generate && !pre[i];
+        ts.add(i, lpb, nbi, sd.n[i], o | (wj << 16), lpe - lpb, first ? 0 : 1, (nbi - o) * 2 * wj);
         ts.any_first |= first;
       }
-      if (ts.total > 0 && (rc = b_launch_trail(b, ts, strip_stream(j), slots, false))) return rc;
+      if (ts.total > 0 && (rc = b_launch_trail(b, c, ts, strip_stream(j), slots, false))) return rc;
     }
     if (used2) any2 = true;
   }
@@ -404,7 +514,7 @@ int b_enqueue(dgp_batch_t b, int level) {
   ip.W = W;
   ip.want_T = (level == 2);
   // the merges of the inverse are released as the factorisation passes them at every size (unlike the single-site engine)
-  if ((rc = b_potrf(b, W != T ? &ip : nullptr))) return rc;
+  if ((rc = b_potrf(b, b_train_chol(b), W != T ? &ip : nullptr))) return rc;
   if (b->timing) CK(b, cudaEventRecord(b->ev[1], T));
   if (W != T) {
     CK(b, cudaEventRecord(b->ev_lo[0], T));
@@ -486,6 +596,63 @@ int b_mfg_alloc(dgp_batch_t b) {
   }
   return 0;
 }
+
+// The arena of one dgp_batch_sample_ex call over G sites (slots), mld = largest padded grid, ld = the batch's padded n,
+// Spad = S rounded up to 128, ngmax = largest group count of a reduction (0: none); slabs [slot][...], carved in this order.
+struct SampleArena {
+  double *VT, *Sig, *Pb, *DI, *Z, *O, *Xw, *mu, *scal, *theta, *jit, *w, *gout;
+  int* gstart;
+};
+size_t b_sample_carve(SampleArena* a, double* base, size_t G, size_t mld, size_t ld, size_t Spad, size_t S, size_t ngmax) {
+  ArenaCarver c(base);
+  a->VT = c.take(G * mld * ld);            // V' = Kx T'          [slot][mld][ld]
+  a->Sig = c.take(G * mld * mld);          // Sigma*, then Lpost  [slot][mld][mld]
+  a->Pb = c.take(G * mld * 128);           // panel-solve staging [slot][mld][128]
+  a->DI = c.take(G * mld * 128);           // block inverses      [slot][mld][128]
+  a->Z = c.take(G * Spad * mld);           // normals             [slot][Spad][mld]
+  a->O = c.take(G * Spad * mld);           // draws               [slot][Spad][mld]
+  a->Xw = c.take(G * mld * DGP_XS);        // grid features
+  a->mu = c.take(G * mld);                 // posterior mean
+  a->scal = c.take(G * SC_SIZE);
+  a->theta = c.take(G * DGP_MAX_THETA);
+  a->jit = c.take(G);
+  a->w = a->gout = nullptr;
+  a->gstart = nullptr;
+  if (ngmax) {
+    a->w = c.take(G * mld);
+    a->gout = c.take(G * S * ngmax);
+    a->gstart = (int*)c.take((G * (ngmax + 1) + 1) / 2);
+  }
+  return c.used;
+}
+
+// what a call samples: the slots (sites with m > 0, in batch order), their largest padded grid and group count;
+// < 0 with the handle's error set for a malformed call
+int b_sample_plan(dgp_batch_t b, const int* m, int S, const dgp_flux_reduce* const* red, int* slot_site, int* G_out,
+                  size_t* mld, size_t* ngmax) {
+  if (!b->have_train || !m) DGP_FAIL(b, -1, "dgp_batch_sample_ex: bad arguments (NULL m or no training data)");
+  if (S < 1) DGP_FAIL(b, -1, "dgp_batch_sample_ex: S = %d (S >= 1)", S);
+  int G = 0;
+  *mld = 0; *ngmax = 0;
+  for (int i = 0; i < b->G; i++) {
+    if (m[i] < 0) DGP_FAIL(b, -1, "dgp_batch_sample_ex: site %d: m = %d", i, m[i]);
+    if (m[i] == 0) continue;
+    const dgp_flux_reduce* r = red ? red[i] : nullptr;
+    if (r) {
+      if (r->ngroups < 1 || !r->weight || !r->group_start) DGP_FAIL(b, -1, "dgp_batch_sample_ex: site %d: bad reduction spec", i);
+      if (r->group_start[0] < 0 || r->group_start[r->ngroups] > m[i])
+        DGP_FAIL(b, -1, "dgp_batch_sample_ex: site %d: group range outside the grid", i);
+      for (int g = 0; g < r->ngroups; g++)
+        if (r->group_start[g] > r->group_start[g + 1]) DGP_FAIL(b, -1, "dgp_batch_sample_ex: site %d: group_start must be non-decreasing", i);
+      if ((size_t)r->ngroups > *ngmax) *ngmax = r->ngroups;
+    }
+    const size_t mp = round_up(m[i], 128);
+    if (mp > *mld) *mld = mp;
+    slot_site[G++] = i;
+  }
+  *G_out = G;
+  return 0;
+}
 }  // namespace
 
 extern "C" {
@@ -509,6 +676,7 @@ int dgp_batch_destroy(dgp_batch b) {
   for (double* p : bufs) if (p) cudaFree(p);
   b_predict_free(b);
   b_mfg_free(b);
+  if (b->sarena) cudaFree(b->sarena);
   b->l8.release();
   if (b->h_theta) cudaFreeHost(b->h_theta);
   if (b->h_scal) cudaFreeHost(b->h_scal);
@@ -858,6 +1026,200 @@ int dgp_batch_mean_functional_grad(dgp_batch b, const int* m, const double* cons
     memcpy(grad_out + (size_t)i * P, o + 1, sizeof(double) * P);
   }
   return 0;
+}
+
+size_t dgp_batch_sample_bytes(dgp_batch b, const int* m, int S, const dgp_flux_reduce* const* red) {
+  if (!b) return 0;
+  int slot_site[DGP_BATCH_MAX], G = 0;
+  size_t mld = 0, ngmax = 0;
+  if (b_sample_plan(b, m, S, red, slot_site, &G, &mld, &ngmax) < 0 || G == 0) return 0;
+  SampleArena a;
+  return b_sample_carve(&a, nullptr, G, mld, b->ld, round_up(S, 128), S, ngmax) * sizeof(double);
+}
+
+// dgp_sample_ex for every site of the batch, each step one launch sequence over all sampled sites (slots):
+//   normals (Philox per slot, or the caller's Z) -> per prediction chunk: features, cross covariance and mean partials, the
+//   posterior mean, both gathered into whole-grid slot slabs, and V' = Kx T' (M_GENERIC, triangular k range) into the V'
+//   slab -> Sigma* = K** + jitter I - V'V' (M_GENERIC lower tiles, covariance generated as the accumulator's start) ->
+//   Lpost in place (b_potrf, end-aligned) -> draws Z Lpost' -> + mu -> grouped sums.
+// Per slot, every tile sums the same k range in the same order as dgp_sample_ex: bit-identical draws, sums and info.
+int dgp_batch_sample_ex(dgp_batch b, const int* m, const double* const* Xs, int S, const double* const* Z,
+                        const unsigned long long* seed, const double* jitter, const dgp_flux_reduce* const* red,
+                        double* const* out, int* info_out) {
+  if (!b) return -1;
+  if (!Xs || !out || !info_out) DGP_FAIL(b, -1, "dgp_batch_sample_ex: bad arguments (NULL Xs, out or info_out)");
+  if (!Z && !seed) DGP_FAIL(b, -1, "dgp_batch_sample_ex: Z and seed are both NULL (device normals need a seed per site)");
+  if (b->pending) DGP_FAIL(b, -1, "dgp_batch_sample_ex: an evaluation is in flight: call dgp_batch_nlml_grad_wait first");
+  int slot_site[DGP_BATCH_MAX], G = 0, rc;
+  size_t mldz = 0, ngmax = 0;
+  if ((rc = b_sample_plan(b, m, S, red, slot_site, &G, &mldz, &ngmax)) < 0) return rc;
+  for (int k = 0; k < G; k++) {
+    const int i = slot_site[k];
+    if (!Xs[i] || !out[i] || (Z && !Z[i])) DGP_FAIL(b, -1, "dgp_batch_sample_ex: site %d: NULL grid, normals or output", i);
+    if (!b->have_T[i])
+      DGP_FAIL(b, -1, "dgp_batch_sample_ex: site %d is not factorised: call dgp_batch_factorize first (again after every "
+               "dgp_batch_set_train / dgp_batch_nlml_grad; a site whose factorisation failed cannot sample)", i);
+  }
+  for (int i = 0; i < b->G; i++) info_out[i] = 0;
+  if (G == 0) return 0;
+  CK(b, cudaSetDevice(b->device));
+  const long long ld = b->ld, mld = (long long)mldz, Spad = round_up(S, 128), C = DGP_BATCH_CHUNK;
+  const int ndim = b->spec.ndim;
+  cudaStream_t st = b->stream;
+  {  // the grow-only arena
+    SampleArena a0;
+    const size_t count = b_sample_carve(&a0, nullptr, G, mld, ld, Spad, S, ngmax);
+    if (b->sarena_count < count) {
+      CK(b, cudaStreamSynchronize(st));
+      if (b->sarena) cudaFree(b->sarena);
+      b->sarena = nullptr; b->sarena_count = 0;
+      const cudaError_t e = cudaMalloc((void**)&b->sarena, count * sizeof(double));
+      if (e != cudaSuccess) {
+        cudaGetLastError();
+        DGP_FAIL(b, -2, "dgp_batch_sample_ex: sampling arena of %.1f GB not allocated: %s", (double)count * 8e-9, cudaGetErrorString(e));
+      }
+      b->sarena_count = count;
+    }
+  }
+  SampleArena a;
+  b_sample_carve(&a, b->sarena, G, mld, ld, Spad, S, ngmax);
+  if ((rc = b_predict_alloc(b))) return rc;
+  SampleTab tab;
+  memset(&tab, 0, sizeof(tab));
+  int mmax = 0, kslot[DGP_BATCH_MAX];
+  for (int i = 0; i < DGP_BATCH_MAX; i++) kslot[i] = -1;
+  std::vector<double> jit(G);
+  for (int k = 0; k < G; k++) {
+    const int i = slot_site[k];
+    const dgp_flux_reduce* r = red ? red[i] : nullptr;
+    kslot[i] = k;
+    tab.site[k] = i; tab.m[k] = m[i]; tab.seed[k] = seed ? seed[i] : 0ull;
+    if (r) { tab.ng[k] = r->ngroups; tab.mean[k] = r->y_mean; tab.scale[k] = r->y_scale; tab.logt[k] = r->log_transform; }
+    jit[k] = jitter ? jitter[i] : 0.0;
+    if (m[i] > mmax) mmax = m[i];
+  }
+  // ---- inputs: theta of the slots, jitter, normals, reduction weights and group starts
+  CK(b, cudaMemsetAsync(a.scal, 0, (size_t)G * SC_SIZE * 8, st));
+  CK(b, cudaMemsetAsync(a.Z, 0, (size_t)G * Spad * mld * 8, st));
+  CK(b, cudaMemcpyAsync(a.jit, jit.data(), (size_t)G * 8, cudaMemcpyHostToDevice, st));
+  for (int k = 0; k < G; k++) {
+    const int i = slot_site[k];
+    CK(b, cudaMemcpyAsync(a.theta + (size_t)k * DGP_MAX_THETA, b->theta + (size_t)i * DGP_MAX_THETA, DGP_MAX_THETA * 8,
+                          cudaMemcpyDeviceToDevice, st));
+    if (Z) CK(b, cudaMemcpy2DAsync(a.Z + (size_t)k * Spad * mld, (size_t)mld * 8, Z[i], (size_t)m[i] * 8, (size_t)m[i] * 8, S,
+                                   cudaMemcpyHostToDevice, st));
+    if (tab.ng[k]) {
+      CK(b, cudaMemcpyAsync(a.w + (size_t)k * mld, red[i]->weight, (size_t)m[i] * 8, cudaMemcpyHostToDevice, st));
+      CK(b, cudaMemcpyAsync(a.gstart + (size_t)k * (ngmax + 1), red[i]->group_start, (size_t)(tab.ng[k] + 1) * sizeof(int),
+                            cudaMemcpyHostToDevice, st));
+    }
+  }
+  if (!Z) {
+    k_fill_normals_b<<<dim3((mmax + 255) / 256, S, G), 256, 0, st>>>(a.Z, mld, Spad * mld, tab);
+    b->launches++;
+    CK(b, cudaGetLastError());
+  }
+  // ---- cross covariance, posterior mean and V', one prediction chunk of every grid per step
+  CUtensorMap tVT, tSig, tDI, tZ;
+  if ((rc = make_map3(b, &b->tmKx, b->Kx, ld, C, b->G))) return rc;
+  if ((rc = make_map3(b, &tVT, a.VT, ld, mld, G))) return rc;
+  if ((rc = make_map3(b, &tSig, a.Sig, mld, mld, G))) return rc;
+  if ((rc = make_map3(b, &tDI, a.DI, 128, mld, G))) return rc;
+  if ((rc = make_map3(b, &tZ, a.Z, mld, Spad, G))) return rc;
+  for (int m0 = 0; m0 < mmax; m0 += (int)C) {
+    PredChunk pc, pm;   // pc: write the cross covariance; pm: the mean alone
+    memset(&pc, 0, sizeof(pc));
+    TabBuilder tb(b);
+    tb.t.cstride = mld * ld;
+    for (int k = 0; k < b->G; k++) {   // largest sites first in the GEMM's table, as in every other batched launch
+      const int i = b->order[k];
+      if (kslot[i] < 0) continue;
+      const int mc = m[i] - m0 < 0 ? 0 : (m[i] - m0 < C ? m[i] - m0 : (int)C);
+      if (mc == 0) continue;
+      pc.m[i] = mc; pc.var[i] = 1;
+      tb.t.cslot[i] = (short)kslot[i];
+      CK(b, cudaMemcpyAsync(b->Xs + (size_t)i * C * DGP_MAX_COLS, Xs[i] + (size_t)m0 * ndim, (size_t)mc * ndim * 8,
+                            cudaMemcpyHostToDevice, st));
+      const int rb = (mc + 127) / 128;   // V'[k][m0 + rows of the chunk, 0 .. 128 nb) = Kx T'
+      tb.add(i, 0, rb, mc, 2 * b->nb[i], 8 * b->nb[i], 1, rb * 2 * b->nb[i]);
+    }
+    pm = pc;
+    for (int i = 0; i < DGP_BATCH_MAX; i++) pm.var[i] = 0;
+    k_pred_features_b<<<dim3(C / 256, b->G), 256, 0, st>>>(b->spec, pc, b->theta, b->Xs, b->Xws, b->means, (int)C);
+    k_cov_rect_pred_b<<<dim3(C / 32, b->NB, b->G), 256, 0, st>>>(b->spec, b->sd, pc, b->theta, b->Xws, b->Xw, b->noise,
+                                                                 b->alpha, b->Kx, b->dot, (int)C);
+    k_pred_finish_b<<<dim3(C / 256, b->G), 256, 0, st>>>(b->spec, b->sd, pm, b->theta, b->Xws, b->means, b->dot, b->vpart,
+                                                         b->mu, b->var, (int)C);
+    k_sample_gather<<<dim3(C / 256, G), 256, 0, st>>>(tab, pc, b->Xws, b->mu, (int)C, m0, a.Xw, a.mu, mld);
+    b->launches += 4;
+    CK(b, cudaGetLastError());
+    GemmArgs g = b_args(b, M_GENERIC, a.VT + (size_t)m0 * ld, 1.0, tb.total);
+    if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, b->tmKx, b->tmA, g, st, false, &tb.t))) return rc;
+  }
+  // ---- the slots' own per-site sizes, largest first, end-aligned (as set_train lays out the training matrices)
+  SiteDims psd;
+  memset(&psd, 0, sizeof(psd));
+  int off[DGP_BATCH_MAX], order[DGP_BATCH_MAX];
+  psd.count = G; psd.nbmax = (int)(mld / 128); psd.ld = mld;
+  for (int k = 0; k < G; k++) {
+    psd.n[k] = m[slot_site[k]]; psd.nb[k] = round_up(psd.n[k], 128) / 128;
+    off[k] = ((psd.nbmax - psd.nb[k]) / PANEL_BLOCKS) * PANEL_BLOCKS;
+    order[k] = k;
+  }
+  for (int i = 1; i < G; i++)
+    for (int k = i; k > 0 && psd.nb[order[k]] > psd.nb[order[k - 1]]; k--) std::swap(order[k], order[k - 1]);
+  {  // Sigma* = K** + jitter I - V'V'  (lower tiles)
+    TabBuilder ts(b, mld);
+    ts.t.jitv = a.jit;
+    for (int k = 0; k < G; k++) {
+      const int s = order[k], mb = psd.nb[s];
+      ts.add(s, 0, mb, psd.n[s], 2 * mb, 8 * b->nb[slot_site[s]], 2, mb * (mb + 1));
+    }
+    GemmArgs g = b_args(b, M_GENERIC, a.Sig, -1.0, ts.total);
+    g.ldc = mld; g.Xw = a.Xw; g.theta = a.theta; g.latent = 1;
+    g.noise = a.mu;   // not read: the latent covariance adds only the jitter on its diagonal
+    if ((rc = launch_gemm<INIT_COV, EPI_STORE>(b, tVT, tVT, g, st, false, &ts.t))) return rc;
+  }
+  {  // Lpost, in place
+    const BChol c{a.Sig, a.Sig, nullptr, a.scal, &tSig, &tSig, a.DI, a.Pb, &tDI, &psd, off, order, false};
+    if ((rc = b_potrf(b, c, nullptr))) return rc;
+  }
+  {  // draws = Z Lpost'
+    TabBuilder td(b, mld);
+    td.t.cstride = Spad * mld;
+    for (int k = 0; k < G; k++) {
+      const int s = order[k], mb = psd.nb[s];
+      td.t.cslot[s] = (short)s;
+      td.add(s, 0, (int)(Spad / 128), S, 2 * mb, 8 * mb, 1, (int)(Spad / 128) * 2 * mb);
+    }
+    GemmArgs g = b_args(b, M_GENERIC, a.O, 1.0, td.total);
+    g.ldc = mld;
+    if ((rc = launch_gemm<INIT_ZERO, EPI_STORE>(b, tZ, tSig, g, st, false, &td.t))) return rc;
+  }
+  k_add_rowvec_b<<<dim3((mmax + 255) / 256, S, G), 256, 0, st>>>(a.O, mld, Spad * mld, a.mu, tab);
+  b->launches++;
+  CK(b, cudaGetLastError());
+  if (ngmax) {   // annual (grouped) flux of every draw, reduced where the draws are
+    k_flux_reduce_b<<<dim3((unsigned)ngmax, (S + 7) / 8, G), 256, 0, st>>>(a.O, mld, Spad * mld, a.w, a.gstart, (int)ngmax + 1,
+                                                                          S, tab, a.gout, (long long)S * (long long)ngmax);
+    b->launches++;
+    CK(b, cudaGetLastError());
+  }
+  for (int k = 0; k < G; k++) {
+    const int i = slot_site[k];
+    if (tab.ng[k]) CK(b, cudaMemcpyAsync(out[i], a.gout + (size_t)k * S * ngmax, (size_t)S * tab.ng[k] * 8, cudaMemcpyDeviceToHost, st));
+    else CK(b, cudaMemcpy2DAsync(out[i], (size_t)m[i] * 8, a.O + (size_t)k * Spad * mld, (size_t)mld * 8, (size_t)m[i] * 8, S,
+                                 cudaMemcpyDeviceToHost, st));
+  }
+  std::vector<double> sc((size_t)G * SC_SIZE);
+  CK(b, cudaMemcpyAsync(sc.data(), a.scal, sc.size() * 8, cudaMemcpyDeviceToHost, st));
+  CK(b, cudaStreamSynchronize(st));
+  int bad = 0;
+  for (int k = 0; k < G; k++) {
+    info_out[slot_site[k]] = (int)sc[(size_t)k * SC_SIZE + SC_INFO];
+    if (info_out[slot_site[k]] != 0) bad++;
+  }
+  return bad;
 }
 
 long long dgp_batch_launch_count(dgp_batch b) { return b ? b->launches : 0; }

@@ -57,13 +57,20 @@ struct GemmArgs {
 // dependent GemmArgs fields.  Every per-site array lives in a slab indexed by the site: matrices [site][ld][ld] behind 3-D
 // tensor maps (the site is the third TMA coordinate), per-point vectors [site][ld], theta [site][DGP_MAX_THETA].
 // count == 0: a plain single-site launch (GemmArgs as given, 2-D tensor maps).
+// cstride == 0: the output matrix of site s is C + s ld^2 (the [site][ld][ld] slabs); else it is C + cslot[s] cstride, for
+// outputs of another shape ([site][rows][ldc]) or kept per sampled site rather than per batch site (dgp_batch_sample_ex).
 struct BatchEnt { int tile0, site, step, nb, n, aux0, aux1, aux2; };
 struct BatchTab {
   int count, pad_;
   long long ld;                 // leading dimension of every slab matrix = rows of a per-point vector slab
   const double* jitv;           // [sites] diagonal jitter of each site
+  long long cstride;            // elements between the output matrices of consecutive slots (0: ld^2, slot = site)
   BatchEnt e[DGP_BATCH_MAX];
+  short cslot[DGP_BATCH_MAX];   // output slot of each site (cstride != 0)
 };
+__device__ __forceinline__ size_t out_slab(const BatchTab& bt, int site) {
+  return bt.cstride ? (size_t)bt.cslot[site] * (size_t)bt.cstride : (size_t)site * (size_t)bt.ld * (size_t)bt.ld;
+}
 
 // tile slots of an M_LAUUM launch over nb block rows (8-row bands of 8 x 16 cells, see decode_job)
 __host__ __device__ inline int lauum_slots(int nb) {
@@ -256,7 +263,7 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
     jc.step = e.step; jc.nb = e.nb; jc.aux0 = e.aux0; jc.aux1 = e.aux1; jc.aux2 = e.aux2;
   }
   // slab offsets of this site (0 for a single-site launch)
-  const size_t soff_m = site >= 0 ? (size_t)site * (size_t)bt.ld * (size_t)bt.ld : 0;  // matrices
+  const size_t soff_m = site >= 0 ? out_slab(bt, site) : 0;  // output matrix
   Job job = decode_job(jc, tile, INIT);
   if (!job.valid) return;
   if (MT == 4) { job.rowA += 64 * (blockIdx.x & 1); job.crow += 64 * (blockIdx.x & 1); }
@@ -415,7 +422,7 @@ k_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensor
       const BatchEnt& e = bt.e[k];
       tile_e -= e.tile0; site_e = e.site; npts_e = e.n;
       je.step = e.step; je.nb = e.nb; je.aux0 = e.aux0; je.aux1 = e.aux1; je.aux2 = e.aux2;
-      soff_e = (size_t)e.site * (size_t)bt.ld * (size_t)bt.ld;
+      soff_e = out_slab(bt, e.site);
     }
     const Job jo = decode_job(je, tile_e, INIT);
     const int crow_e = jo.crow + (MT == 4 ? 64 * (bx & 1) : 0);

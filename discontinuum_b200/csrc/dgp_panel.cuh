@@ -475,14 +475,17 @@ k_pred_finish_b(const __grid_constant__ dgp_spec spec, const __grid_constant__ S
 namespace dgp {
 // In-place factorisation: block column s of L, staged by the panel solve in P[rows][128], goes back into the matrix.
 // grid = (row blocks below the diagonal block), block = 256.
-__global__ void __launch_bounds__(256)
-k_copy_panel(const double* __restrict__ P, double* __restrict__ A, long long ld, int s) {
-  const size_t row0 = (size_t)(s + 1 + blockIdx.x) * 128;
+__device__ __forceinline__ void copy_panel_body(const double* __restrict__ P, double* __restrict__ A, long long ld, int s, int bx) {
+  const size_t row0 = (size_t)(s + 1 + bx) * 128;
   for (int e = threadIdx.x; e < 128 * 64; e += 256) {
     const int r = e >> 6, c2 = (e & 63) * 2;
     const double2 v = *reinterpret_cast<const double2*>(P + (row0 + r) * 128 + c2);
     *reinterpret_cast<double2*>(A + (row0 + r) * ld + (size_t)s * 128 + c2) = v;
   }
+}
+__global__ void __launch_bounds__(256)
+k_copy_panel(const double* __restrict__ P, double* __restrict__ A, long long ld, int s) {
+  copy_panel_body(P, A, ld, s, blockIdx.x);
 }
 
 // zero the strict upper triangle of a dense row-major n x n matrix (leading dimension ld); grid = n rows, block = 256
@@ -547,11 +550,10 @@ k_fill_normals(double* __restrict__ Z, long long ld, int m, unsigned long long s
 // out[s, g] = sum_{i in [start[g], start[g+1])} w[i] * T(draw[s, i]),  T(z) = exp(z * scale + mean) (log pipelines,
 // clipped below at 1e-6 like the reference's inverse transform), z * scale + mean clipped at 0 (standard pipeline), or affine:
 // concentration_to_flux + resample("YE").sum() of src/loadest_gp/utils.py:14-56,89 without moving the draws.
-// grid = (groups, ceil(S / 8)), block = 256: one warp per (draw, group).
-__global__ void __launch_bounds__(256)
-k_flux_reduce(const double* __restrict__ D, long long ld, const double* __restrict__ w, const int* __restrict__ start,
-              int ngroups, int S, double mean, double scale, int log_transform, double* __restrict__ out) {
-  const int g = blockIdx.x, s = blockIdx.y * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+// k_flux_reduce: grid = (groups, ceil(S / 8)), block = 256: one warp per (draw, group).
+__device__ __forceinline__ void flux_reduce_body(const double* __restrict__ D, long long ld, const double* __restrict__ w,
+                                                 const int* __restrict__ start, int ngroups, int S, double mean, double scale,
+                                                 int log_transform, double* __restrict__ out, int g, int s, int lane) {
   if (s >= S) return;
   const double* row = D + (size_t)s * ld;
   double acc = 0.0;
@@ -564,6 +566,12 @@ k_flux_reduce(const double* __restrict__ D, long long ld, const double* __restri
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if (lane == 0) out[(size_t)s * ngroups + g] = acc;
+}
+__global__ void __launch_bounds__(256)
+k_flux_reduce(const double* __restrict__ D, long long ld, const double* __restrict__ w, const int* __restrict__ start,
+              int ngroups, int S, double mean, double scale, int log_transform, double* __restrict__ out) {
+  flux_reduce_body(D, ld, w, start, ngroups, S, mean, scale, log_transform, out, blockIdx.x, blockIdx.y * 8 + (threadIdx.x >> 5),
+                   threadIdx.x & 31);
 }
 
 // ------------------------------------------------------------------ gradient of a linear functional of the posterior mean

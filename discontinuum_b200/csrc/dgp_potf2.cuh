@@ -212,10 +212,12 @@ __device__ __forceinline__ void p2_st_prog(int* prog, int v) {
 // and takes the scalings; the helpers (warps 6, 7; at k = 3 warps 1, 2, 3, 6, 7) finish the previous row of the inverse.
 //
 // Batched launch (pb.count > 0, one CTA per site): Ablk / Lblk / Ublk / Tblk are then the bases of the [site][ld][ld]
-// slabs and scal the base of [site][SC_SIZE]; CTA b factors the diagonal block pb.step[b] of site pb.site[b].
+// slabs and scal the base of [site][SC_SIZE]; CTA b factors the diagonal block pb.step[b] of site pb.site[b].  DIblk, when
+// given, is the base of a [site][rows][128] slab of block inverses (dslab elements per site; the in-place factorisation).
 struct P2Batch {
   int count, pad_;
   long long slab;               // elements between the matrices of consecutive sites
+  long long dslab;              // elements between the block-inverse tables of consecutive sites
   short site[DGP_BATCH_MAX], step[DGP_BATCH_MAX];
 };
 
@@ -229,6 +231,7 @@ k_potf2_v2(const double* Ablk, double* Lblk, double* Ublk, long long ld, double*
     Ablk += off; Lblk += off;
     if (Ublk != nullptr) Ublk += off;
     if (Tblk != nullptr) Tblk += off;
+    if (DIblk != nullptr) DIblk += (size_t)st * (size_t)pb.dslab + (size_t)s * 128 * 128;
     scal += (size_t)st * SC_SIZE;
     base = s * 128;
   }

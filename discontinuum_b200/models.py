@@ -9,6 +9,7 @@ CovSpec trees for the CUDA tile generator.
 """
 from __future__ import annotations
 
+from dataclasses import dataclass
 from typing import Optional
 
 import numpy as np
@@ -106,6 +107,54 @@ from .engine import JITTERS, DataMixin, MarginalB200, ModelConfig  # noqa: E402
 from .spec import GPModule  # noqa: E402
 
 
+def annual_flux_groups(time, flow, target_pipeline):
+    """(weight[m], group_start[G + 1], years[G], log_transform) of the annual-flux reduction over a strictly increasing
+    time grid: weight = flow * dt * 1e-3 (concentration_to_flux, src/loadest_gp/utils.py:14-56), groups = calendar years
+    (resample(time="YE").sum(), utils.py:89), log_transform the dgp_flux_reduce kind of the target pipeline."""
+    time = np.asarray(time).astype("datetime64[ns]")
+    if np.any(np.diff(time) <= np.timedelta64(0, "ns")):
+        raise ValueError("sample_annual_flux needs a strictly increasing time grid")
+    dts = np.unique(np.diff(time).astype("timedelta64[ns]").astype(np.int64))
+    if dts.shape[0] != 1:
+        import warnings
+
+        warnings.warn("Time delta is not constant", UserWarning, stacklevel=3)
+    dt_s = float(dts[0]) * 1e-9
+    weight = np.asarray(flow, dtype=np.float64) * dt_s * 1e-3
+    years = time.astype("datetime64[Y]").astype(np.int64) + 1970
+    uniq, first = np.unique(years, return_index=True)
+    group_start = np.concatenate([first, [time.shape[0]]]).astype(np.int32)
+    log_t = 1 if isinstance(target_pipeline, LogStandardPipeline) else 2  # exp clipped at 1e-6 | affine clipped at 0 (data.py pipelines)
+    return weight, group_start, uniq, log_t
+
+
+@dataclass
+class FluxSpec:
+    """The annual-flux reduction of one site's posterior draws on `grid` (model-space inputs [m, ndim]): the dgp_flux_reduce
+    of LoadestGPMarginalB200.sample_annual_flux.  years[G] labels the groups."""
+    grid: np.ndarray
+    weight: np.ndarray
+    group_start: np.ndarray
+    years: np.ndarray
+    y_mean: float
+    y_scale: float
+    log_transform: int
+
+    @classmethod
+    def from_series(cls, grid, time, flow, target_pipeline) -> "FluxSpec":
+        """From the grid, its time stamps and flow (original units) and the fitted target pipeline of the site."""
+        weight, group_start, years, log_t = annual_flux_groups(time, flow, target_pipeline)
+        grid = np.ascontiguousarray(grid, dtype=np.float64)
+        if grid.shape[0] != weight.shape[0]:
+            raise ValueError("FluxSpec: grid, time and flow must have the same length")
+        return cls(grid, weight, group_start, years, float(target_pipeline.mean_), float(target_pipeline.scale_), log_t)
+
+    def reduce(self) -> dict:
+        """The `flux` dict of Engine.sample_ex / BatchEngine.sample."""
+        return dict(y_mean=self.y_mean, y_scale=self.y_scale, log_transform=self.log_transform, weight=self.weight,
+                    group_start=self.group_start)
+
+
 class LoadestDataMixin(DataMixin):
     """src/loadest_gp/models/base.py:7-19."""
 
@@ -144,21 +193,8 @@ class LoadestGPMarginalB200(LoadestDataMixin, MarginalB200):
         if not self.is_fitted:
             raise RuntimeError("The model hasn't been fitted yet, call .fit().")
         cov = _cov_dict(covariates)
-        time = np.asarray(cov[time_key]).astype("datetime64[ns]")
-        if np.any(np.diff(time) <= np.timedelta64(0, "ns")):
-            raise ValueError("sample_annual_flux needs a strictly increasing time grid")
-        dts = np.unique(np.diff(time).astype("timedelta64[ns]").astype(np.int64))
-        if dts.shape[0] != 1:
-            import warnings
-
-            warnings.warn("Time delta is not constant", UserWarning, stacklevel=2)
-        dt_s = float(dts[0]) * 1e-9
-        weight = np.asarray(cov[flow_key], dtype=np.float64) * dt_s * 1e-3
-        years = time.astype("datetime64[Y]").astype(np.int64) + 1970
-        uniq, first = np.unique(years, return_index=True)
-        group_start = np.concatenate([first, [time.shape[0]]]).astype(np.int32)
+        weight, group_start, uniq, log_t = annual_flux_groups(cov[time_key], cov[flow_key], self.dm.target_pipeline)
         tp = self.dm.target_pipeline
-        log_t = 1 if isinstance(tp, LogStandardPipeline) else 2  # exp clipped at 1e-6 | affine clipped at 0 (data.py pipelines)
         Xnew = np.ascontiguousarray(self.dm.Xnew(covariates), dtype=np.float64)
         self._ensure_factorized(Xnew)
         for jit in JITTERS:

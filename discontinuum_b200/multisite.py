@@ -18,7 +18,7 @@ import torch
 
 from . import capi
 from .engine import JITTERS, MIN_VARIANCE
-from .models import LOADEST_FIXED_NOISE, loadest_spec, monotonic_penalty_grid
+from .models import LOADEST_FIXED_NOISE, FluxSpec, loadest_spec, monotonic_penalty_grid
 from .spec import GPModule
 
 
@@ -34,9 +34,12 @@ def assign_sites(costs: Sequence[float], world: int) -> List[List[int]]:
     return out
 
 
-def site_cost(n: int, iterations: int, m_predict: int = 0) -> float:
-    """flop model of one site: iterations * n^3 (NLML+grad) + factorise + n^2 per predicted point (SURVEY 8d)."""
-    return float(iterations) * float(n) ** 3 + float(n) ** 3 + float(m_predict) * float(n) ** 2
+def site_cost(n: int, iterations: int, m_predict: int = 0, m_sample: int = 0, draws: int = 1000) -> float:
+    """flop model of one site: iterations * n^3 (NLML+grad) + factorise + n^2 per predicted point (SURVEY 8d) + the joint
+    sampling of `draws` draws on m_sample points, m^2 n + m^3 / 3 + 2 m^2 S (BASELINE.md section 3)."""
+    m = float(m_sample)
+    return (float(iterations) * float(n) ** 3 + float(n) ** 3 + float(m_predict) * float(n) ** 2
+            + m * m * float(n) + m ** 3 / 3.0 + 2.0 * m * m * float(draws))
 
 
 def gather_results(local: Dict[int, dict], dist=None) -> Optional[Dict[int, dict]]:
@@ -227,26 +230,34 @@ def _groups(order: List[int], group: int) -> List[List[int]]:
 
 
 def _predict_group(batch: capi.BatchEngine, grp: List[_Site], want: List[bool], predict: Dict[int, np.ndarray], kind,
-                   res_of: Dict[int, dict]):
+                   res_of: Dict[int, dict], sample_want: Optional[List[bool]] = None,
+                   annual_flux: Optional[Dict[int, FluxSpec]] = None) -> np.ndarray:
     """Prediction of a group through its own batch handle (whose training set is the group's): factorise every site at its
     fitted theta (dgp_batch_factorize), climb psd_safe_cholesky's jitter ladder only for the wanted sites that failed -- the
     others are re-factorised unchanged and keep their bits -- and predict every wanted site's grid in one dgp_batch_predict.
-    Sites not wanted (not in `predict`, or failed while fitting) are factorised at their last theta, results unused."""
+    Sites not wanted (not in `predict`, or failed while fitting) are factorised at their last theta, results unused.
+    sample_want[k]: the site is to be sampled on annual_flux[idx].grid as well (it is factorised and climbs the ladder even
+    when it is not predicted; its parameters are projected over that grid when it is not predicted).  Returns, per site,
+    whether it is wanted for either and factorised."""
     G = len(grp)
+    sample_want = sample_want or [False] * G
+    factor_want = np.array(want) | np.array(sample_want)
     grids: List[Optional[np.ndarray]] = [None] * G
     thetas = []
     for k, s in enumerate(grp):
         if want[k]:
             grids[k] = np.ascontiguousarray(predict[s.idx], dtype=np.float64)
             kind.project(s.module, np.concatenate([s.X, grids[k]], axis=0))
+        elif sample_want[k]:
+            kind.project(s.module, np.concatenate([s.X, annual_flux[s.idx].grid], axis=0))
         with torch.no_grad():
             thetas.append(s.module.natural().numpy().astype(np.float64))
-        if want[k]:
+        if factor_want[k]:
             res_of[s.idx]["theta"] = thetas[k]
     thetas = np.ascontiguousarray(np.stack(thetas))
     jit = np.full(G, JITTERS[0])
     _, info = batch.factorize(thetas, jit)
-    bad = np.array(want) & (info != 0)
+    bad = factor_want & (info != 0)
     for j in JITTERS[1:]:
         if not bad.any():
             break
@@ -255,10 +266,15 @@ def _predict_group(batch: capi.BatchEngine, grp: List[_Site], want: List[bool], 
         info = np.where(bad, i2, info)
         bad &= i2 != 0
     for k in np.nonzero(bad)[0]:
-        res_of[grp[k].idx]["failed"] = f"prediction: not positive definite after jitter {JITTERS[-1]:g} (info={int(info[k])})"
+        msg = f"not positive definite after jitter {JITTERS[-1]:g} (info={int(info[k])})"
+        if want[k]:
+            res_of[grp[k].idx]["failed"] = "prediction: " + msg
+        if sample_want[k]:
+            res_of[grp[k].idx]["flux_failed"] = "factorisation: " + msg
         grids[k] = None
+    ok = factor_want & ~bad
     if all(g is None for g in grids):
-        return
+        return ok
     out = batch.predict(grids)
     for k, s in enumerate(grp):
         if grids[k] is None:
@@ -267,6 +283,35 @@ def _predict_group(batch: capi.BatchEngine, grp: List[_Site], want: List[bool], 
         res = res_of[s.idx]
         res["mu"], res["var_latent"] = mu, var
         res["var"] = observed_variance(s.module.spec, thetas[k], var, s.noise, grids[k].shape[0])
+    return ok
+
+
+def _sample_group(batch: capi.BatchEngine, grp: List[_Site], ok: np.ndarray, annual_flux: Dict[int, FluxSpec], draws: int,
+                  sample_seed: int, res_of: Dict[int, dict]):
+    """Annual flux of the group's factorised sites that have a FluxSpec, on the same handle and factorisation
+    (dgp_batch_sample_ex: every site's numbers equal a per-site capi.Engine sample_ex bit for bit): site `idx` draws from
+    the Philox stream sample_seed + idx, and only the sites whose posterior covariance was not positive definite (or whose
+    sums came back non-finite) are sampled again, at the next jitter of sample_annual_flux's ladder."""
+    G = len(grp)
+    specs = [annual_flux.get(s.idx) for s in grp]
+    todo = [bool(ok[k]) and specs[k] is not None for k in range(G)]
+    seeds = [int(sample_seed) + s.idx for s in grp]
+    for j in JITTERS:
+        if not any(todo):
+            break
+        out = batch.sample([specs[k].grid if todo[k] else None for k in range(G)], int(draws), seeds=seeds,
+                           jitter=np.full(G, j), flux=[specs[k].reduce() if todo[k] else None for k in range(G)])
+        for k in range(G):
+            if not todo[k]:
+                continue
+            flux, info = out[k]
+            if info == 0 and np.all(np.isfinite(flux)):
+                res_of[grp[k].idx]["annual_flux"] = flux
+                res_of[grp[k].idx]["flux_years"] = specs[k].years
+                todo[k] = False
+    for k in range(G):
+        if todo[k]:
+            res_of[grp[k].idx]["flux_failed"] = f"posterior covariance not positive definite after jitter {JITTERS[-1]:g}"
 
 
 @dataclass
@@ -427,7 +472,8 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
                     predict: Optional[Dict[int, np.ndarray]] = None, lr: float = 0.05, scheduler: bool = True,
                     patience: int = 60, model="loadest", stats: Optional[dict] = None, concurrency: Optional[int] = None,
                     lanes: int = 2, early_stopping: bool = False, monotonic_penalty_weight: float = 0.0, grid_size: int = 64,
-                    monotonic_penalty_interval: int = 1, penalty_seed: int = 0) -> Dict[int, dict]:
+                    monotonic_penalty_interval: int = 1, penalty_seed: int = 0,
+                    annual_flux: Optional[Dict[int, FluxSpec]] = None, draws: int = 1000, sample_seed: int = 0) -> Dict[int, dict]:
     """Fit one GP per site on this rank.  sites: {index: (X, y[, noise])} in model space; model: "loadest", "rating" or a
     kind object (see LoadestKind).  Returns {index: {"theta", "objective", "history", "failed", "n", "mu", "var",
     "var_latent"}} ("var" follows `likelihood(model(x))` like MarginalB200.predict).
@@ -452,7 +498,15 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
     `idx` from torch.Generator().manual_seed(penalty_seed + idx), every `monotonic_penalty_interval`-th good iteration
     and scaled by the interval; its gradient comes from dgp_batch_mean_functional_grad.  "penalty" holds the last
     (unweighted) value.  Neither depends on `lanes`, on the group a site lands in, or on the rank.
-    `concurrency` selects the round-1 per-handle pipelines instead (fit_sites_local_per_handle), which has neither."""
+    `annual_flux` {index: FluxSpec}: the sites listed there get LoadestGPMarginalB200.sample_annual_flux's product right
+    after their group's predictions, on the same handle and factorisation: `draws` joint posterior draws on FluxSpec.grid
+    (which may differ from the prediction grid; a site may be sampled without being predicted) reduced to annual sums on
+    the device (dgp_batch_sample_ex).  Site `idx` draws from the Philox stream sample_seed + idx, so the numbers do not
+    depend on the rank, the group, its size or `lanes`.  The posterior climbs sample_annual_flux's jitter ladder per site.
+    "annual_flux" [draws, years] and "flux_years" hold the result; a site whose posterior covariance stays not positive
+    definite, whose factorisation failed, or whose fit failed gets "flux_failed" instead (its other results stay).  The
+    time spent sampling counts in stats["predict_s"].
+    `concurrency` selects the round-1 per-handle pipelines instead (fit_sites_local_per_handle), which has none of these."""
     pen = None
     if monotonic_penalty_weight > 0.0:
         if getattr(_kind(model), "name", None) != "rating":
@@ -464,8 +518,8 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
             raise ValueError("monotonic_penalty_interval must be >= 1")
         pen = PenaltyConfig(float(monotonic_penalty_weight), int(grid_size), int(monotonic_penalty_interval), int(penalty_seed))
     if concurrency is not None:
-        if early_stopping or pen is not None:
-            raise ValueError("early_stopping and the monotonicity penalty need the batch driver (concurrency=None)")
+        if early_stopping or pen is not None or annual_flux is not None:
+            raise ValueError("early_stopping, the monotonicity penalty and annual_flux need the batch driver (concurrency=None)")
         return fit_sites_local_per_handle(sites, iterations=iterations, device=device, concurrency=concurrency or 4,
                                           predict=predict, lr=lr, scheduler=scheduler, patience=patience)
     kind = _kind(model)
@@ -507,14 +561,20 @@ def fit_sites_local(sites: Dict[int, tuple], iterations: int = 100, device: int 
             if pen is not None:
                 res_of[s.idx]["penalty"] = s.penalty
         want = [predict is not None and s.idx in predict and s.failed is None for s in grp]
-        if any(want):
+        sample_want = [annual_flux is not None and s.idx in annual_flux and s.failed is None for s in grp]
+        for s in grp:
+            if annual_flux is not None and s.idx in annual_flux and s.failed is not None:
+                res_of[s.idx]["flux_failed"] = "not sampled: the fit failed"
+        if any(want) or any(sample_want):
             own = batch is None
             if own:
                 batch = capi.BatchEngine(max_sites=len(grp), max_n=max(s.X.shape[0] for s in grp), device=device)
             try:
                 if own:
                     batch.set_train(grp[0].module.spec.to_c(), [(s.X, s.y, s.noise) for s in grp])
-                _predict_group(batch, grp, want, predict, kind, res_of)
+                ok = _predict_group(batch, grp, want, predict, kind, res_of, sample_want, annual_flux)
+                if any(sample_want):
+                    _sample_group(batch, grp, ok, annual_flux, draws, sample_seed, res_of)
             finally:
                 if own:
                     batch.close()
@@ -710,19 +770,23 @@ def fit_sites(sites: Dict[int, tuple], iterations: int = 100, predict: Optional[
               group: int = 16, dist=None, device: int = 0, model="loadest", stats: Optional[dict] = None,
               concurrency: Optional[int] = None, lanes: int = 2, early_stopping: bool = False, patience: int = 60,
               monotonic_penalty_weight: float = 0.0, grid_size: int = 64, monotonic_penalty_interval: int = 1,
-              penalty_seed: int = 0) -> Optional[Dict[int, dict]]:
+              penalty_seed: int = 0, annual_flux: Optional[Dict[int, FluxSpec]] = None, draws: int = 1000,
+              sample_seed: int = 0) -> Optional[Dict[int, dict]]:
     """Shard `sites` (every rank holds the same dict, or at least the same keys and sizes) over the ranks of
     `dist`, fit this rank's share, gather everything on rank 0.  The fit options are fit_sites_local's."""
     world = dist.get_world_size() if dist is not None and dist.is_initialized() else 1
     rank = dist.get_rank() if world > 1 else 0
     keys = sorted(sites)
-    costs = [site_cost(sites[k][0].shape[0], iterations, predict[k].shape[0] if predict and k in predict else 0) for k in keys]
+    costs = [site_cost(sites[k][0].shape[0], iterations, predict[k].shape[0] if predict and k in predict else 0,
+                       annual_flux[k].grid.shape[0] if annual_flux and k in annual_flux else 0, draws) for k in keys]
     mine = [keys[i] for i in assign_sites(costs, world)[rank]]
     local = fit_sites_local({k: sites[k] for k in mine}, iterations=iterations, device=device, group=group,
                             predict={k: predict[k] for k in mine} if predict else None, model=model, stats=stats,
                             concurrency=concurrency, lanes=lanes, early_stopping=early_stopping, patience=patience,
                             monotonic_penalty_weight=monotonic_penalty_weight, grid_size=grid_size,
-                            monotonic_penalty_interval=monotonic_penalty_interval, penalty_seed=penalty_seed)
+                            monotonic_penalty_interval=monotonic_penalty_interval, penalty_seed=penalty_seed,
+                            annual_flux={k: annual_flux[k] for k in mine if k in annual_flux} if annual_flux else None,
+                            draws=draws, sample_seed=sample_seed)
     return gather_results(local, dist)
 
 

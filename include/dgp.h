@@ -15,6 +15,10 @@
  *                         (discontinuum/engines/gpytorch.py:618-622)
  *   dgp_predict        <- MarginalGPyTorch.__gpytorch_predict, discontinuum/engines/gpytorch.py:599-626
  *   dgp_sample         <- f_preds.sample(...), discontinuum/engines/gpytorch.py:578-580
+ *   dgp_batch_sample_ex <- per site of nwqn-loadest-example.py:156-157: the joint draws and their annual flux,
+ *                         loadest_gp/utils.py:14-56,89 (concentration_to_flux + resample("YE").sum()), for a whole group of
+ *                         sites in one launch sequence on the batch handle's factorisation; its workspace is a grow-only
+ *                         sampling arena on the handle (dgp_batch_sample_bytes)
  *
  * Conventions: plain pointers and sizes only.  All matrices are float64, row-major.  Every call
  * returns an int status: 0 = ok; > 0 = LAPACK-style info (1-based index of the first non-positive
@@ -291,6 +295,32 @@ int dgp_batch_predict(dgp_batch b, const int* m, const double* const* Xs, double
  * dgp_batch_predict has not), and 8 max_sites x 1073 B of pinned host memory.  Later calls allocate nothing. */
 int dgp_batch_mean_functional_grad(dgp_batch b, const int* m, const double* const* Xs, const double* const* c,
                                    double* val_out, double* grad_out);
+/* Batch form of dgp_sample_ex.  For every site s with m[s] > 0: S joint latent draws of the posterior on Xs[s][m[s], ndim]
+ * (out[s][S, m[s]]) or, with red != NULL and red[s] != NULL, their grouped sums (out[s][S, red[s]->ngroups]).  Z == NULL:
+ * the normals of site s are the Philox4x32-10 stream keyed by seed[s] (dgp_sample_ex's numbering); else Z[s][S, m[s]] host
+ * normals (seed may then be NULL).  jitter[s] (NULL: 0) is added to the diagonal of site s's posterior covariance.
+ * info_out[nsites]: LAPACK-style, 0 = ok (and 0 for skipped sites); a site whose posterior covariance is not positive
+ * definite gets info > 0 and does not affect the others.  Per site the draws, sums and info equal those of dgp_sample_ex
+ * on a handle factorised at the same training set, theta and jitter, bit for bit.  Each step is one launch over all
+ * sampled sites: normals, per 1024-row chunk the cross covariance and V' = Kx T', Sigma* = K** + jitter I - V'V', the
+ * in-place posterior Cholesky (end-aligned like the training factorisation), the draws, the mean, the grouped sums.
+ * Needs a successful dgp_batch_factorize of every sampled site since the last dgp_batch_set_train / dgp_batch_nlml_grad;
+ * reads T = L^-1, alpha and the training features and writes nothing later factorisations, predictions or evaluations
+ * read.  Fails (< 0) on NULL pointers, m[s] < 0, S < 1, a malformed red[s] (the checks of dgp_sample_ex), a sampled site
+ * without that factorisation, and while an evaluation is in flight.  Returns the number of sampled sites with info != 0.
+ * Workspace: a grow-only sampling arena on the handle (freed at destroy, allocated only when a call needs more than the
+ * largest before) of, per sampled site, in doubles, with mld = the largest m[s] of the call rounded up to 128, ld = the
+ * largest training n of the batch rounded up to 128, Spad = S rounded up to 128:
+ *   mld^2 + mld ld + 2 Spad mld + 2 128 mld + 9 mld + 105 (+ mld + S ng + (ng + 1) / 2 when any site reduces, ng = the
+ *   largest ngroups), every slab rounded up to 256 B
+ * (1.9 GB per site at m = 10 958, n <= 8 000, S = 1000).  The prediction slabs of dgp_batch_predict are used (and
+ * allocated if no prediction has). */
+int dgp_batch_sample_ex(dgp_batch b, const int* m, const double* const* Xs, int S, const double* const* Z,
+                        const unsigned long long* seed, const double* jitter, const dgp_flux_reduce* const* red,
+                        double* const* out, int* info_out);
+/* Device bytes of the sampling arena a dgp_batch_sample_ex call with these m[] / S / red[] needs (0 for a malformed call or
+ * one that samples no site). */
+size_t dgp_batch_sample_bytes(dgp_batch b, const int* m, int S, const dgp_flux_reduce* const* red);
 /* Parity accessor: alpha of one site after an evaluation. */
 int dgp_batch_get_alpha(dgp_batch b, int site, double* alpha_out);
 long long dgp_batch_launch_count(dgp_batch b);
