@@ -84,7 +84,9 @@ _SIGNATURES = [
     ("dgp_dist_trail", C.c_int, [_P, C.c_int, C.c_int, C.c_int]),
     ("dgp_dist_draws_partial", C.c_int, [_P]),
     ("dgp_dist_finish", C.c_int, [_P, _P]),
+    ("dgp_dist_finish_ex", C.c_int, [_P, C.POINTER(DgpFluxReduce), _P]),
     ("dgp_dist_end", C.c_int, [_P]),
+    ("dgp_dist_arena_bytes", C.c_size_t, [_P, C.c_int, C.c_int, C.c_int, C.c_int]),
     ("dgp_get_alpha", C.c_int, [_P, _P, C.c_int]),
     ("dgp_get_chol", C.c_int, [_P, _P, C.c_int]),
     ("dgp_set_debug_kinv", C.c_int, [_P, C.c_int]),
@@ -621,6 +623,16 @@ class Engine:
 
     def dist_call(self, name: str, tok, *args) -> int:
         return self._check(getattr(self.lib, "dgp_dist_" + name)(tok, *args), "dgp_dist_" + name)
+
+    def dist_arena_bytes(self, m: int, S: int, world: int, rank: int) -> int:
+        """Device bytes dist_begin(m, S, rank, world) carves from the engine's workspace (the panel slabs of `rank`, the
+        receive slots, Z and the staging buffers); the caller's VT / Od / mu / pack buffers are not included."""
+        if not (m >= 1 and S >= 1 and world >= 1 and 0 <= rank < world):
+            raise ValueError("dist_arena_bytes: needs m, S, world >= 1 and 0 <= rank < world")
+        nbytes = int(self.lib.dgp_dist_arena_bytes(self._h, int(m), int(S), int(world), int(rank)))
+        if nbytes == 0:
+            raise DgpError("dgp_dist_arena_bytes: no training data")
+        return nbytes
 
     # -- parity / debug
     def covmat(self, theta) -> np.ndarray:

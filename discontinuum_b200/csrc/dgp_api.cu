@@ -27,7 +27,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <string>
+#include <tuple>
 #include <utility>
 #include <vector>
 
@@ -650,8 +652,10 @@ static int launch_trail(dgp_handle h, const CholBufs& b, int k0, int kb, int o, 
 //   for s: potf2(s) -> TRSM(s) on every row below [-> forward substitution(s)] -> rank-128 update of columns (s, pe)
 // mid_wait: event the in-panel update of the first block column has to wait for (the trailing update of the panel's
 // other columns, which stream T applies while the first column is already being factored)
+// piv0: index of b's row 0 in the whole matrix, so that a failing pivot is reported as a global 1-based index when b is a
+// trailing submatrix (the panel slabs of dgp_dist_*)
 static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool generate, double jitter, bool fwd, cudaStream_t P,
-                        cudaEvent_t mid_wait = nullptr) {
+                        cudaEvent_t mid_wait = nullptr, int piv0 = 0) {
   const int nb = b.nb;
   const long long ld = b.ld;
   int rc;
@@ -674,7 +678,7 @@ static int factor_panel(dgp_handle h, const CholBufs& b, int pb, int pe, bool ge
     const bool lu_clean = !inplace && h->lu_zeroed && b.L == h->bufL && (b.U == nullptr || b.U == h->bufU);
     if (!(skip & 1))  // dependent launch behind the in-panel update of the previous block column (same stream, nothing in between)
       CK(h, launch_ex(k_potf2_v2, 1, P2_THREADS, (size_t)P2_SMEM, P, pdl && s > pb && !inplace && !fwd, (const double*)(b.A + off), b.L + off,
-                      b.U ? b.U + off : (double*)nullptr, ld, t_in_a ? (double*)nullptr : b.DI + (size_t)s * 128 * 128, b.scal, s * 128,
+                      b.U ? b.U + off : (double*)nullptr, ld, t_in_a ? (double*)nullptr : b.DI + (size_t)s * 128 * 128, b.scal, piv0 + s * 128,
                       inplace ? (double*)nullptr : b.A + off, lu_clean ? 0 : 1, g_no_p2batch));
     h->launches++;
     CK(h, cudaGetLastError());
@@ -1185,17 +1189,18 @@ struct ArenaCarver {
   explicit ArenaCarver(double* b) : base(b) {}
   double* take(size_t count) { double* p = base ? base + used : nullptr; used += (count + 31) / 32 * 32; return p; }
 };
-// doubles dgp_sample_ex(m, S, ngroups) / dgp_dist_begin(m, S) carve for a training set padded to npad (nb blocks)
-static size_t sample_arena_count(size_t mpad, size_t Spad, size_t npad, size_t nb, size_t S, size_t ngroups, bool dist) {
+// doubles dgp_sample_ex(m, S, ngroups) carves for a training set padded to npad (nb blocks)
+static size_t sample_arena_count(size_t mpad, size_t Spad, size_t npad, size_t nb, size_t S, size_t ngroups) {
   ArenaCarver c(nullptr);
   c.take(mpad * DGP_MAX_COLS); c.take(mpad * DGP_XS); c.take(mpad); c.take(nb * mpad);
-  if (!dist) { c.take(mpad); c.take(mpad * npad); }
+  c.take(mpad); c.take(mpad * npad);
   c.take(mpad * mpad); c.take(mpad * 128); c.take(mpad * 128); c.take(Spad * mpad);
-  if (!dist) c.take(Spad * mpad);
+  c.take(Spad * mpad);
   c.take(mpad); c.take(SC_SIZE);
   if (ngroups) { c.take(mpad); c.take(S * ngroups); c.take((ngroups + 2) / 2 + 1); }
   return c.used;
 }
+static size_t dist_arena_count(int m, int S, int world, int rank, size_t nb);  // dgp_dist_begin's (below)
 static int ensure_arena(dgp_handle h, size_t count) {
   if (h->arena_count >= count) return 0;
   CK(h, cudaStreamSynchronize(h->stream));
@@ -1221,8 +1226,8 @@ int dgp_reserve(dgp_handle h, int max_m_sample, int max_S, int max_groups) {
     return 0;
   }
   const size_t mpad = round_up(max_m_sample, 128), Spad = round_up(max_S > 0 ? max_S : 1, 128), npad = h->max_pad, nb = npad / 128;
-  const size_t a = sample_arena_count(mpad, Spad, npad, nb, (size_t)(max_S > 0 ? max_S : 1), (size_t)max_groups, false);
-  const size_t b = sample_arena_count(mpad, Spad, npad, nb, 0, 0, true);
+  const size_t a = sample_arena_count(mpad, Spad, npad, nb, (size_t)(max_S > 0 ? max_S : 1), (size_t)max_groups);
+  const size_t b = dist_arena_count(max_m_sample, max_S > 0 ? max_S : 1, 1, 0, nb);  // world 1: the slabs of every panel
   return ensure_arena(h, a > b ? a : b);
 }
 
@@ -1232,15 +1237,22 @@ int dgp_sample(dgp_handle h, const double* Xs, int m, const double* Z, int S, do
   return dgp_sample_ex(h, Xs, m, Z, 0ull, S, jitter, nullptr, out, on_device);
 }
 
+// the checks dgp_sample_ex and dgp_dist_finish_ex apply to a reduction over an m-point grid
+static int check_flux_reduce(dgp_handle h, const dgp_flux_reduce* red, int m, const char* who) {
+  if (red->ngroups < 1 || !red->weight || !red->group_start) DGP_FAIL(h, -1, "%s: bad reduction spec", who);
+  if (red->group_start[0] < 0 || red->group_start[red->ngroups] > m) DGP_FAIL(h, -1, "%s: group range outside the grid", who);
+  for (int g = 0; g < red->ngroups; g++)
+    if (red->group_start[g] > red->group_start[g + 1]) DGP_FAIL(h, -1, "%s: group_start must be non-decreasing", who);
+  return 0;
+}
+
 int dgp_sample_ex(dgp_handle h, const double* Xs, int m, const double* Z, unsigned long long seed, int S, double jitter,
                   const dgp_flux_reduce* red, double* out, int on_device) {
   if (!h) return -1;
   if (!Xs || !out || m < 1 || S < 1) DGP_FAIL(h, -1, "dgp_sample: bad arguments");
-  if (red && (red->ngroups < 1 || !red->weight || !red->group_start)) DGP_FAIL(h, -1, "dgp_sample_ex: bad reduction spec");
   if (red) {
-    if (red->group_start[0] < 0 || red->group_start[red->ngroups] > m) DGP_FAIL(h, -1, "dgp_sample_ex: group range outside the grid");
-    for (int g = 0; g < red->ngroups; g++)
-      if (red->group_start[g] > red->group_start[g + 1]) DGP_FAIL(h, -1, "dgp_sample_ex: group_start must be non-decreasing");
+    int rc = check_flux_reduce(h, red, m, "dgp_sample_ex");
+    if (rc) return rc;
   }
   if (!h->factorized || !h->have_T) DGP_FAIL(h, -1, "dgp_sample: call dgp_factorize first");
   CK(h, cudaSetDevice(h->device));
@@ -1252,7 +1264,7 @@ int dgp_sample_ex(dgp_handle h, const double* Xs, int m, const double* Z, unsign
   // factorisation, Z and the draws.  The cross covariance goes through the handle's prediction chunk, so the footprint is
   // 8 (m n + m^2) B + O(m): 106 GB at m = 100k, n = 32k.
   {
-    int rca = ensure_arena(h, sample_arena_count(mpad, Spad, npad, h->nb, S, red ? red->ngroups : 0, false));
+    int rca = ensure_arena(h, sample_arena_count(mpad, Spad, npad, h->nb, S, red ? red->ngroups : 0));
     if (rca) return rca;
   }
   ArenaCarver ar(h->arena);
@@ -1338,12 +1350,18 @@ int dgp_sample_ex(dgp_handle h, const double* Xs, int m, const double* Z, unsign
 // ------------------------------------------------------------------ distributed joint posterior sampling
 // SURVEY 8e: exact joint draws need the Cholesky factor of the m x m posterior covariance.  Across G ranks the block
 // columns are dealt out panel-cyclically (panel p -> rank p mod G); every rank holds the training factorisation and
-// keeps Sigma* in the same padded m x m layout, but only generates, updates and factors ITS panels' columns:
+// stores, generates, updates and factors only ITS panels' columns:
 //   V'   rows sharded over ranks              -> caller all-gathers V'        (m n^2 / G flop per rank)
 //   Sigma* columns of my panels               (m^2 n / G flop per rank)
 //   for p: owner factors panel p, packs its sub-diagonal rows -> caller broadcasts -> others unpack
 //          every rank applies the rank-(128 pw) update to its own panels right of p        (m^3 / 3G flop per rank)
 //   draws: partial Z[:, my columns] L[:, my columns]' -> caller all-reduces, adds the mean
+// Storage: one slab per owned panel j of block columns [jb, je): the trailing submatrix Sigma*[jb 128 :, jb 128 : je 128],
+// (mb - jb) 128 rows, leading dimension (je - jb) 128, the slabs one after another in the handle's arena -- the lower
+// trapezoids of the rank's panels, about 4 mpad^2 / G bytes.  A slab has the same offset on rows and columns, so the
+// tile modes of the single-GPU factorisation run on it unchanged in slab coordinates (block indices minus jb); every
+// operand that lives in a larger buffer (V', Z, another panel) gets a tensor map based at the matching offset into it.  A
+// received panel p goes to receive slot p mod 2, indexed by global row, so that the maps of a slot serve all its panels.
 // The caller (multisite.sample_sharded: torch.distributed over NCCL) owns the exchanged buffers and the collectives;
 // this side is the per-rank kernels, all on the handle's stream.
 struct dgp_dist_s {
@@ -1351,12 +1369,62 @@ struct dgp_dist_s {
   int m = 0, mpad = 0, mb = 0, S = 0, Spad = 0, pw = 0, npanels = 0, rank = 0, world = 1;
   double jitter = 0.0;
   double *VT = nullptr, *Od = nullptr, *mu = nullptr;  // caller-owned device buffers
-  double *Xsd = nullptr, *Xws = nullptr, *means = nullptr, *dot = nullptr, *Sig = nullptr, *Pb = nullptr, *DI2 = nullptr;
-  double *Zd = nullptr, *zero = nullptr, *scal2 = nullptr;
-  CUtensorMap tVT, tSig, tDI2, tZ;
-  CholBufs bufs() { return CholBufs{Sig, Sig, nullptr, DI2, scal2, &tSig, &tSig, &tDI2, mb, mpad, Pb}; }
+  int vt_rows = 0;                                      // rows of VT (world rows_per_rank)
+  double *Xsd = nullptr, *Xws = nullptr, *means = nullptr, *dot = nullptr, *zero = nullptr, *scal2 = nullptr;
+  double *Pb = nullptr, *DI2 = nullptr, *Zd = nullptr;  // from Pb on, nothing is read after the partial draws
+  double* slot[2] = {nullptr, nullptr};                 // received panels: row = global row, leading dimension pw 128
+  std::vector<double*> slab;                            // slab of owned panel p: slab[p / world]
+  CUtensorMap tDI2;
+  std::map<std::tuple<const double*, int, int, long long>, CUtensorMap> maps;  // (base, rows, cols, ld) -> map
   bool mine(int p) const { return p % world == rank; }
+  int pbeg(int p) const { return p * pw; }
+  int pend(int p) const { return (p * pw + pw < mb) ? p * pw + pw : mb; }
+  // tensor map of the rows x cols matrix at `base`: encoded on first use, then reused (a world-1 run at m = 100 000 makes
+  // about 19 000 trailing launches)
+  int map(const double* base, int rows, int cols, long long ld, const CUtensorMap** out) {
+    const auto key = std::make_tuple(base, rows, cols, ld);
+    auto it = maps.find(key);
+    if (it == maps.end()) {
+      CUtensorMap tm;
+      int rc = make_map(h, &tm, const_cast<double*>(base), rows, cols, ld);
+      if (rc) return rc;
+      it = maps.emplace(key, tm).first;
+    }
+    *out = &it->second;
+    return 0;
+  }
 };
+
+static void dist_geometry(dgp_dist_s* d, int m, int S, int world, int rank) {
+  d->m = m; d->mpad = round_up(m, 128); d->mb = d->mpad / 128; d->S = S; d->Spad = round_up(S, 128);
+  d->pw = PANEL_BLOCKS; d->npanels = (d->mb + d->pw - 1) / d->pw; d->rank = rank; d->world = world;
+}
+
+// carve d's buffers out of `base` (nullptr: count only) -> doubles used.  The slabs come last: everything before them is
+// the same on every rank.
+static size_t dist_carve(dgp_dist_s* d, double* base, size_t nb) {
+  ArenaCarver ar(base);
+  const size_t mpad = d->mpad, pcols = (size_t)d->pw * 128;
+  d->Xsd = ar.take(mpad * DGP_MAX_COLS); d->Xws = ar.take(mpad * DGP_XS); d->means = ar.take(mpad); d->dot = ar.take(nb * mpad);
+  d->zero = ar.take(mpad); d->scal2 = ar.take(SC_SIZE);
+  d->Pb = ar.take(mpad * 128); d->DI2 = ar.take(pcols * 128); d->Zd = ar.take((size_t)d->Spad * mpad);
+  for (int k = 0; k < 2; k++) d->slot[k] = ar.take(mpad * pcols);
+  d->slab.clear();
+  for (int p = d->rank; p < d->npanels; p += d->world)
+    d->slab.push_back(ar.take((size_t)(d->mb - d->pbeg(p)) * 128 * (size_t)(d->pend(p) - d->pbeg(p)) * 128));
+  return ar.used;
+}
+
+static size_t dist_arena_count(int m, int S, int world, int rank, size_t nb) {
+  dgp_dist_s d;
+  dist_geometry(&d, m, S, world, rank);
+  return dist_carve(&d, nullptr, nb);
+}
+
+size_t dgp_dist_arena_bytes(dgp_handle h, int m, int S, int world, int rank) {
+  if (!h || m < 1 || S < 1 || world < 1 || rank < 0 || rank >= world || !h->have_train) return 0;
+  return dist_arena_count(m, S, world, rank, h->nb) * sizeof(double);
+}
 
 int dgp_dist_dims(dgp_handle h, int m, int S, int world, long long* dims) {
   if (!h || !dims || m < 1 || S < 1 || world < 1) return -1;
@@ -1376,18 +1444,15 @@ int dgp_dist_begin(dgp_handle h, const double* Xs, int m, int S, const double* Z
   if (!h->factorized || !h->have_T) DGP_FAIL(h, -1, "dgp_dist_begin: call dgp_factorize first");
   CK(h, cudaSetDevice(h->device));
   dgp_dist d = new dgp_dist_s();
-  d->h = h; d->m = m; d->mpad = round_up(m, 128); d->mb = d->mpad / 128; d->S = S; d->Spad = round_up(S, 128);
-  d->pw = PANEL_BLOCKS; d->npanels = (d->mb + d->pw - 1) / d->pw; d->rank = rank; d->world = world; d->jitter = jitter;
+  d->h = h; d->jitter = jitter;
+  dist_geometry(d, m, S, world, rank);
   d->VT = VT; d->Od = Od; d->mu = mu;
   const size_t mpad = d->mpad;
   {
-    int rca = ensure_arena(h, sample_arena_count(mpad, d->Spad, h->npad, h->nb, 0, 0, true));
+    int rca = ensure_arena(h, dist_carve(d, nullptr, h->nb));
     if (rca) { delete d; return rca; }
   }
-  ArenaCarver ar(h->arena);
-  d->Xsd = ar.take(mpad * DGP_MAX_COLS); d->Xws = ar.take(mpad * DGP_XS); d->means = ar.take(mpad); d->dot = ar.take((size_t)h->nb * mpad);
-  d->Sig = ar.take(mpad * mpad); d->Pb = ar.take(mpad * 128); d->DI2 = ar.take(mpad * 128); d->Zd = ar.take((size_t)d->Spad * mpad);
-  d->zero = ar.take(mpad); d->scal2 = ar.take(SC_SIZE);
+  dist_carve(d, h->arena, h->nb);
   cudaStream_t st = h->stream;
   int rc;
   CK(h, cudaMemsetAsync(d->zero, 0, mpad * 8, st));
@@ -1404,10 +1469,8 @@ int dgp_dist_begin(dgp_handle h, const double* Xs, int m, int S, const double* Z
   CK(h, cudaGetLastError());
   long long dims[6];
   dgp_dist_dims(h, m, S, world, dims);
-  if ((rc = make_map(h, &d->tVT, VT, (int)(dims[5] * world), h->npad, h->npad))) { dgp_dist_end(d); return rc; }
-  if ((rc = make_map(h, &d->tSig, d->Sig, d->mpad, d->mpad, d->mpad))) { dgp_dist_end(d); return rc; }
-  if ((rc = make_map(h, &d->tDI2, d->DI2, d->mpad, 128, 128))) { dgp_dist_end(d); return rc; }
-  if ((rc = make_map(h, &d->tZ, d->Zd, d->Spad, d->mpad, d->mpad))) { dgp_dist_end(d); return rc; }
+  d->vt_rows = (int)(dims[5] * world);
+  if ((rc = make_map(h, &d->tDI2, d->DI2, d->pw * 128, 128, 128))) { dgp_dist_end(d); return rc; }
   *out = d;
   return 0;
 }
@@ -1456,20 +1519,24 @@ int dgp_dist_vt_rows(dgp_dist d, int row0, int row1) {
   return 0;
 }
 
-// Sigma* = K** + jitter I - V'V on the block columns of this rank's panels (needs the complete V')
+// Sigma* = K** + jitter I - V'V on the slabs of this rank's panels (needs the complete V').  In slab coordinates: V' from
+// row jb 128 on, the features from point jb 128 on and n = m - jb 128, so the diagonal, the jitter and the identity
+// padding land where they are in the full matrix.
 int dgp_dist_sigma(dgp_dist d) {
   if (!d) return -1;
   dgp_handle h = d->h;
   CK(h, cudaSetDevice(h->device));
   int rc;
-  for (int p = d->rank; p < d->npanels; p += d->world) {
-    const int pb = p * d->pw, pe = (pb + d->pw < d->mb) ? pb + d->pw : d->mb, w = pe - pb;
+  for (size_t k = 0; k < d->slab.size(); k++) {
+    const int p = d->rank + (int)k * d->world, jb = d->pbeg(p), w = d->pend(p) - jb, r0 = jb * 128;
+    const CUtensorMap* tv;
+    if ((rc = d->map(d->VT + (size_t)r0 * h->npad, d->vt_rows - r0, h->npad, h->npad, &tv))) return rc;
     GemmArgs g = base_args(h, M_TRAIL_COL, 0);
-    g.nb = d->mb; g.n = d->m; g.ldc = d->mpad;
-    g.aux0 = pb | (w << 16); g.aux1 = h->npad / 128; g.aux2 = 0;
-    g.C = d->Sig; g.ntiles = (d->mb - pb) * 2 * w; g.sign = -1.0;
-    g.Xw = d->Xws; g.noise = d->zero; g.jitter = d->jitter; g.latent = 1;
-    if ((rc = launch_gemm<INIT_COV, EPI_STORE>(h, d->tVT, d->tVT, g))) return rc;
+    g.nb = d->mb - jb; g.n = d->m - r0; g.ldc = (long long)w * 128;
+    g.aux0 = 0 | (w << 16); g.aux1 = h->npad / 128; g.aux2 = 0;
+    g.C = d->slab[k]; g.ntiles = (d->mb - jb) * 2 * w; g.sign = -1.0;
+    g.Xw = d->Xws + (size_t)r0 * DGP_XS; g.noise = d->zero; g.jitter = d->jitter; g.latent = 1;
+    if ((rc = launch_gemm<INIT_COV, EPI_STORE>(h, *tv, *tv, g))) return rc;
   }
   return 0;
 }
@@ -1483,84 +1550,127 @@ int dgp_dist_panel_factor(dgp_dist d, int p, double* pack, void* stream) {
   if (!pack || p < 0 || p >= d->npanels || !d->mine(p)) DGP_FAIL(h, -1, "dgp_dist_panel_factor: panel %d is not owned by rank %d", p, d->rank);
   CK(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-  const int pb = p * d->pw, pe = (pb + d->pw < d->mb) ? pb + d->pw : d->mb;
-  CholBufs b = d->bufs();
-  int rc = factor_panel(h, b, pb, pe, false, 0.0, false, st);
+  const int pb = d->pbeg(p), w = d->pend(p) - pb, nbl = d->mb - pb;
+  const long long ld = (long long)w * 128;
+  double* sl = d->slab[p / d->world];
+  const CUtensorMap* ts;
+  int rc = d->map(sl, nbl * 128, w * 128, ld, &ts);
   if (rc) return rc;
-  const long long rows = (long long)(d->mb - pe) * 128;
+  CholBufs b{sl, sl, nullptr, d->DI2, d->scal2, ts, ts, &d->tDI2, nbl, ld, d->Pb};
+  if ((rc = factor_panel(h, b, 0, w, false, 0.0, false, st, nullptr, pb * 128))) return rc;
+  const long long rows = (long long)(nbl - w) * 128;
   if (rows > 0) {
-    k_pack_panel<<<(unsigned)(rows / 8), 256, 0, st>>>(d->Sig, d->mpad, (long long)pe * 128, (long long)pb * 128, (pe - pb) * 128, pack, 0);
+    k_pack_panel<<<(unsigned)(rows / 8), 256, 0, st>>>(sl, ld, ld, 0, w * 128, pack, 0);
     h->launches++;
     CK(h, cudaGetLastError());
   }
   return 0;
 }
 
-// other ranks: put the received panel (rows below its diagonal blocks) in place
+// other ranks: copy the received panel (rows below its diagonal blocks) into receive slot p mod 2.  The handle's stream
+// orders the slot's reuse (by panel p + 2) behind the trailing updates with panel p.
 int dgp_dist_panel_unpack(dgp_dist d, int p, double* pack) {
   if (!d) return -1;
   dgp_handle h = d->h;
   if (!pack || p < 0 || p >= d->npanels) DGP_FAIL(h, -1, "dgp_dist_panel_unpack: bad panel");
   CK(h, cudaSetDevice(h->device));
-  const int pb = p * d->pw, pe = (pb + d->pw < d->mb) ? pb + d->pw : d->mb;
+  const int pb = d->pbeg(p), pe = d->pend(p);
   const long long rows = (long long)(d->mb - pe) * 128;
   if (rows > 0) {
-    k_pack_panel<<<(unsigned)(rows / 8), 256, 0, h->stream>>>(d->Sig, d->mpad, (long long)pe * 128, (long long)pb * 128, (pe - pb) * 128,
-                                                              pack, 1);
+    k_pack_panel<<<(unsigned)(rows / 8), 256, 0, h->stream>>>(d->slot[p & 1], (long long)d->pw * 128, (long long)pe * 128, 0,
+                                                              (pe - pb) * 128, pack, 1);
     h->launches++;
     CK(h, cudaGetLastError());
   }
   return 0;
 }
 
-// rank-(128 pw) update, with panel p, of this rank's panels j in [j_first, j_last]
+// rank-(128 pw) update, with panel p, of this rank's panels j in [j_first, j_last].  Panel p's rows from jb 128 on (its
+// own slab on the owner, the receive slot elsewhere) are the operand, behind a map based at that row; the update is the
+// single-GPU factorisation's, on slab j at o = 0 with step 0.
 int dgp_dist_trail(dgp_dist d, int p, int j_first, int j_last) {
   if (!d) return -1;
   dgp_handle h = d->h;
+  if (p < 0 || p >= d->npanels) DGP_FAIL(h, -1, "dgp_dist_trail: bad panel");
   CK(h, cudaSetDevice(h->device));
-  const int pb = p * d->pw, pe = (pb + d->pw < d->mb) ? pb + d->pw : d->mb;
-  CholBufs b = d->bufs();
+  const int pb = d->pbeg(p), wp = d->pend(p) - pb;
   int rc;
   if (j_first < p + 1) j_first = p + 1;
   if (j_last > d->npanels - 1) j_last = d->npanels - 1;
   for (int j = j_first; j <= j_last; j++) {
     if (!d->mine(j)) continue;
-    const int jb = j * d->pw, je = (jb + d->pw < d->mb) ? jb + d->pw : d->mb, w = je - jb;
-    if ((rc = launch_trail(h, b, pb, pe - pb, jb, w, (d->mb - jb) * 2 * w, false, 0.0, h->stream))) return rc;
+    const int jb = d->pbeg(j), wj = d->pend(j) - jb, nbl = d->mb - jb;
+    const double* src;
+    long long ld;
+    if (d->mine(p)) { ld = (long long)wp * 128; src = d->slab[p / d->world] + (size_t)(jb - pb) * 128 * ld; }
+    else { ld = (long long)d->pw * 128; src = d->slot[p & 1] + (size_t)jb * 128 * ld; }
+    const CUtensorMap* tp;
+    if ((rc = d->map(src, nbl * 128, wp * 128, ld, &tp))) return rc;
+    CholBufs b{d->slab[j / d->world], nullptr, nullptr, nullptr, nullptr, nullptr, tp, nullptr, nbl, (long long)wj * 128};
+    if ((rc = launch_trail(h, b, 0, wp, 0, wj, nbl * 2 * wj, false, 0.0, h->stream))) return rc;
   }
   return 0;
 }
 
-// Od += Z[:, my columns] L[:, my columns]'   (partial sums of the draws; the caller all-reduces Od)
+// Od += Z[:, my columns] L[:, my columns]'   (partial sums of the draws; the caller all-reduces Od).  Panel p in slab
+// coordinates: Z from column pb 128 on, the draws' columns from pb 128 on.
 int dgp_dist_draws_partial(dgp_dist d) {
   if (!d) return -1;
   dgp_handle h = d->h;
   CK(h, cudaSetDevice(h->device));
   int rc;
-  for (int p = d->rank; p < d->npanels; p += d->world) {
-    const int pb = p * d->pw, pe = (pb + d->pw < d->mb) ? pb + d->pw : d->mb;
-    GemmArgs g = base_args(h, M_ZL, pb);
-    g.nb = d->mb; g.n = d->S; g.aux1 = pe - pb;
-    g.ntiles = (d->Spad / 128) * 2 * (d->mb - pb); g.C = d->Od; g.ldc = d->mpad;
-    if ((rc = launch_gemm<INIT_LOAD, EPI_STORE>(h, d->tZ, d->tSig, g))) return rc;
+  for (size_t k = 0; k < d->slab.size(); k++) {
+    const int p = d->rank + (int)k * d->world, pb = d->pbeg(p), w = d->pend(p) - pb, nbl = d->mb - pb;
+    const CUtensorMap *tz, *ts;
+    if ((rc = d->map(d->Zd + (size_t)pb * 128, d->Spad, d->mpad - pb * 128, d->mpad, &tz))) return rc;
+    if ((rc = d->map(d->slab[k], nbl * 128, w * 128, (long long)w * 128, &ts))) return rc;
+    GemmArgs g = base_args(h, M_ZL, 0);
+    g.nb = nbl; g.n = d->S; g.aux1 = w;
+    g.ntiles = (d->Spad / 128) * 2 * nbl; g.C = d->Od + (size_t)pb * 128; g.ldc = d->mpad;
+    if ((rc = launch_gemm<INIT_LOAD, EPI_STORE>(h, *tz, *ts, g))) return rc;
   }
   return 0;
 }
 
-// after the all-reduce of Od and of mu: out[S, m] = Od + mu (host); returns the LAPACK-style info of THIS rank's panels
-int dgp_dist_finish(dgp_dist d, double* out) {
+// after the all-reduce of Od and of mu: Od + mu, then out[S, m] = the draws, or (red) out[S, ngroups] = their grouped
+// flux sums (k_flux_reduce, as dgp_sample_ex); returns the LAPACK-style info of THIS rank's panels
+int dgp_dist_finish_ex(dgp_dist d, const dgp_flux_reduce* red, double* out) {
   if (!d) return -1;
   dgp_handle h = d->h;
   if (!out) DGP_FAIL(h, -1, "dgp_dist_finish: out is NULL");
+  if (red) {
+    int rc = check_flux_reduce(h, red, d->m, "dgp_dist_finish_ex");
+    if (rc) return rc;
+  }
   CK(h, cudaSetDevice(h->device));
   k_add_rowvec<<<dim3((d->m + 255) / 256, d->S), 256, 0, h->stream>>>(d->Od, d->mpad, d->mu, d->m);
   h->launches++;
   CK(h, cudaGetLastError());
-  CK(h, cudaMemcpy2DAsync(out, (size_t)d->m * 8, d->Od, (size_t)d->mpad * 8, (size_t)d->m * 8, d->S, cudaMemcpyDeviceToHost, h->stream));
+  if (red == nullptr) {
+    CK(h, cudaMemcpy2DAsync(out, (size_t)d->m * 8, d->Od, (size_t)d->mpad * 8, (size_t)d->m * 8, d->S, cudaMemcpyDeviceToHost, h->stream));
+  } else {
+    // the reduction's buffers take the place of the panel staging, Z, the receive slots and the slabs, which nothing
+    // reads any more
+    ArenaCarver ar(d->Pb);
+    double* wd = ar.take(d->mpad);
+    double* gstart = ar.take((size_t)(red->ngroups + 2) / 2 + 1);
+    double* gout = ar.take((size_t)d->S * red->ngroups);
+    if ((size_t)(d->Pb - h->arena) + ar.used > h->arena_count)
+      DGP_FAIL(h, -1, "dgp_dist_finish_ex: %d groups of %d draws do not fit the workspace", red->ngroups, d->S);
+    CK(h, cudaMemcpyAsync(wd, red->weight, (size_t)d->m * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(h, cudaMemcpyAsync(gstart, red->group_start, (size_t)(red->ngroups + 1) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    k_flux_reduce<<<dim3(red->ngroups, (d->S + 7) / 8), 256, 0, h->stream>>>(d->Od, d->mpad, wd, (const int*)gstart, red->ngroups,
+                                                                            d->S, red->y_mean, red->y_scale, red->log_transform, gout);
+    h->launches++;
+    CK(h, cudaGetLastError());
+    CK(h, cudaMemcpyAsync(out, gout, (size_t)d->S * red->ngroups * 8, cudaMemcpyDeviceToHost, h->stream));
+  }
   CK(h, cudaMemcpyAsync(h->h_scal, d->scal2, SC_SIZE * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   return (int)h->h_scal[SC_INFO];
 }
+
+int dgp_dist_finish(dgp_dist d, double* out) { return dgp_dist_finish_ex(d, nullptr, out); }
 
 // ------------------------------------------------------------------ generic NT product on the tile engine
 int dgp_gemm_nt(dgp_handle h, const double* A, long long lda, const double* B, long long ldb, double* Cm, long long ldc,

@@ -9,6 +9,7 @@ The only collective is the final gather.
 """
 from __future__ import annotations
 
+import ctypes
 import time
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional, Sequence
@@ -832,10 +833,14 @@ def panel_owner(p: int, world: int) -> int:
 
 
 def sample_sharded(engine, Xs: np.ndarray, S: int, dist=None, seed: int = 0, jitter: float = 0.0, Z: Optional[np.ndarray] = None,
-                   stats: Optional[dict] = None):
+                   stats: Optional[dict] = None, flux=None):
     """Exact joint posterior draws [S, m] with the m x m posterior-covariance Cholesky distributed over the ranks of
     `dist` (torch.distributed, NCCL).  Every rank holds the same training factorisation (`engine.factorize` at the same
-    theta) and calls this with the same arguments; every rank returns (draws, info).
+    theta) and calls this with the same arguments; every rank returns (draws, info).  Each rank stores only its own
+    panels of the posterior covariance (stats["arena_bytes"]: the engine workspace this takes on this rank).
+
+    flux: a FluxSpec, or the dict of FluxSpec.reduce() (Engine.sample_ex's `flux`): every rank then reduces the draws to
+    their grouped flux sums on the device and returns (sums [S, ngroups], info) instead.
 
     Exchange steps (the only collectives): all_gather of V' (m x n), all_reduce of the mean, one broadcast of the
     sub-diagonal rows of each factored panel from its owner, all_reduce of the partial draws.  Look-ahead: the owner of
@@ -847,6 +852,9 @@ def sample_sharded(engine, Xs: np.ndarray, S: int, dist=None, seed: int = 0, jit
     m = Xs.shape[0]
     world = dist.get_world_size() if dist is not None and dist.is_initialized() else 1
     rank = dist.get_rank() if world > 1 else 0
+    red = None   # (DgpFluxReduce, the arrays it points into)
+    if flux is not None:
+        red = capi._flux_reduce(flux.reduce() if isinstance(flux, FluxSpec) else flux, m)
     dims = engine.dist_dims(m, S, world)
     dev = torch.device("cuda", engine.device)
     f64 = dict(dtype=torch.float64, device=dev)
@@ -868,11 +876,12 @@ def sample_sharded(engine, Xs: np.ndarray, S: int, dist=None, seed: int = 0, jit
     def rows_below(p):
         return (mb - min((p + 1) * pw_blocks, mb)) * 128
 
-    if stats is not None:   # bytes each collective moves (payload of the buffer it is called on), for the bench line
+    if stats is not None:   # bytes each collective moves (payload of the buffer it is called on) and this rank's workspace
         stats.update(world=world, npanels=npanels, all_gather_VT_bytes=int(VT.numel()) * 8 if world > 1 else 0,
                      all_reduce_mu_bytes=int(mu.numel()) * 8 if world > 1 else 0,
                      broadcast_panel_bytes=sum(rows_below(p) for p in range(npanels)) * dims["panel_cols"] * 8 if world > 1 else 0,
-                     all_reduce_draws_bytes=int(Od.numel()) * 8 if world > 1 else 0)
+                     all_reduce_draws_bytes=int(Od.numel()) * 8 if world > 1 else 0,
+                     arena_bytes=engine.dist_arena_bytes(m, S, world, rank))
     tok = engine.dist_begin(Xs, S, Z, seed, jitter, rank, world, VT, Od, mu)
     try:
         engine.dist_call("vt_rows", tok, rank * rpr, min((rank + 1) * rpr, dims["mpad"]))
@@ -920,8 +929,12 @@ def sample_sharded(engine, Xs: np.ndarray, S: int, dist=None, seed: int = 0, jit
             fence()
             dist.all_reduce(Od)
             fence()
-        out = np.empty((S, m))
-        info = engine.dist_call("finish", tok, out.ctypes.data)
+        if red is None:
+            out = np.empty((S, m))
+            info = engine.dist_call("finish", tok, out.ctypes.data)
+        else:
+            out = np.empty((S, red[0].ngroups))
+            info = engine.dist_call("finish_ex", tok, ctypes.byref(red[0]), out.ctypes.data)
         if world > 1:
             t = torch.tensor([info if info > 0 else 2 ** 31 - 1], dtype=torch.int64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MIN)  # first failing pivot over all ranks

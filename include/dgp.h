@@ -183,12 +183,17 @@ int dgp_sample_ex(dgp_handle h, const double* Xs, int m, const double* Z, unsign
                   double jitter, const dgp_flux_reduce* red, double* out, int on_device);
 
 /* Workspace of dgp_sample / dgp_sample_ex / dgp_dist_*: sized ahead of time for grids of up to max_m_sample points, max_S
- * draws and max_groups flux groups, so that those calls allocate nothing (8 (m n + m^2) B + O(m)).  Without it the first
- * call that needs more grows the workspace once and keeps it.  max_m_sample = 0 releases it. */
+ * draws and max_groups flux groups, so that those calls allocate nothing (dgp_sample_ex: 8 (m n + m^2) B + O(m); the
+ * dgp_dist_* term is that of world 1, the largest: dgp_dist_arena_bytes(h, m, S, 1, 0), about 4 m^2 B + O(m)).  Without it
+ * the first call that needs more grows the workspace once and keeps it.  max_m_sample = 0 releases it. */
 int dgp_reserve(dgp_handle h, int max_m_sample, int max_S, int max_groups);
 
 /* Distributed joint posterior sampling: the per-rank half of a panel-cyclic Cholesky of the m x m posterior covariance
- * (the exchange step of SURVEY 8e).  Panel p (panel_cols / 128 block columns) belongs to rank p mod world.  The caller
+ * (the exchange step of SURVEY 8e).  Panel p (panel_cols / 128 block columns) belongs to rank p mod world, and only its
+ * owner stores it: the rows from the panel's diagonal down (the lower trapezoid of its columns), so the posterior
+ * covariance takes about 4 mpad^2 / world bytes per rank.  The handle's workspace holds those slabs, two receive slots
+ * [mpad, panel_cols] for broadcast panels, Z and the staging buffers: dgp_dist_arena_bytes(h, m, S, world, rank) bytes
+ * (0 on bad arguments or without training data), allocated by dgp_dist_begin unless dgp_reserve made room.  The caller
  * owns the collectives and the exchanged DEVICE buffers (row-major float64):
  *   VT   [rows_per_rank * world, npad]  V' = Kx T'; every rank fills its row shard, the caller all-gathers
  *   pack [mpad, panel_cols]             rows below a factored panel's diagonal blocks, broadcast from its owner
@@ -202,7 +207,7 @@ int dgp_reserve(dgp_handle h, int max_m_sample, int max_S, int max_groups);
  *   begin -> vt_rows(my shard) -> [all_gather VT, all_reduce mu] -> sigma ->
  *   for p: (owner: panel_factor) -> [broadcast pack] -> (others: panel_unpack) -> trail(p, p+1, npanels-1)
  *          (look-ahead: trail(p, p+1, p+1) first, factor panel p+1 on a side stream while trail(p, p+2, ...) runs)
- *   -> draws_partial -> [all_reduce Od] -> finish(out host [S, m]) -> end.
+ *   -> draws_partial -> [all_reduce Od] -> finish(out host [S, m]) or finish_ex -> end.
  * Everything is enqueued on the handle's stream (pass the stream the collectives are ordered against to dgp_create).
  * Z: host base normals [S, m] or NULL for the Philox stream `seed` (identical on every rank). */
 typedef struct dgp_dist_s* dgp_dist;
@@ -216,7 +221,11 @@ int dgp_dist_panel_unpack(dgp_dist d, int p, double* pack);
 int dgp_dist_trail(dgp_dist d, int p, int j_first, int j_last);
 int dgp_dist_draws_partial(dgp_dist d);
 int dgp_dist_finish(dgp_dist d, double* out);  /* > 0: first non-positive pivot met on THIS rank's panels */
+/* dgp_dist_finish with the grouped flux reduction of dgp_sample_ex (red != NULL: out host [S, ngroups], computed on the
+ * device from this rank's all-reduced draws; the checks on red are dgp_sample_ex's).  red == NULL: dgp_dist_finish. */
+int dgp_dist_finish_ex(dgp_dist d, const dgp_flux_reduce* red, double* out);
 int dgp_dist_end(dgp_dist d);
+size_t dgp_dist_arena_bytes(dgp_handle h, int m, int S, int world, int rank);
 
 /* Parity accessors (valid after dgp_nlml* / dgp_factorize): alpha[n]; L[n, n] lower triangular. */
 int dgp_get_alpha(dgp_handle h, double* alpha_out, int out_on_device);
